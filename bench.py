@@ -50,7 +50,20 @@ def parse():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--cols", type=int, default=COLS)
     ap.add_argument("--no-extras", action="store_true", help="skip the ntt / prove_shaped / cpu_baseline sections")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the commitments of the last timed step as DIR/<name>.npy (rank 0's columns), so that two "
+                         "builds can be compared output for output; the inputs depend only on the arguments")
     return ap.parse_args()
+
+
+def dump_outputs(path, points):
+    """points: {name: (n, 8) G1Affine, 64-bit Montgomery limbs} -> DIR/<name>.npy, (n, 2, 8) float64: x and y as eight
+    little-endian 32-bit limbs each, which float64 holds exactly"""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, p in points.items():
+        limbs = np.ascontiguousarray(p, dtype="<u8").view("<u4").reshape(len(p), 2, 8)
+        np.save(os.path.join(path, name + ".npy"), limbs.astype(np.float64))
 
 
 # ----------------------------------------------------------------------------------- clocks
@@ -136,9 +149,11 @@ def run_reference(args, rank, world, out):
         O.best_multiexp(cols[0], bases, threads)
     t = time.perf_counter()
     for _ in range(args.steps):
-        for c in cols:
-            O.best_multiexp(c, bases, threads)
+        last = [O.best_multiexp(c, bases, threads) for c in cols]
     dt = time.perf_counter() - t
+    if args.dump_outputs:
+        import numpy as np
+        dump_outputs(args.dump_outputs, {"commitments": np.stack([O.g1_to_affine(p) for p in last])})
     v = args.steps * sample_cols * N / dt / 1e6
     sample = f"{sample_cols} columns of 2^16 uniform Fr per step (of the {args.cols}-column batch), best_multiexp over {threads} threads"
     print(file=out, *[json.dumps({
@@ -271,6 +286,8 @@ def _main(args, real_stdout):
     dt_e2e = max_over_ranks(e0.elapsed_time(e1) * 1e-3)
     e2e_value = world * args.steps * cols * N / dt_e2e / 1e6
     assert (out_host[0] == got0).all(), "device-resident and host-facing paths disagree"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"commitments": d_out.cpu().numpy().view(np.uint64), "commitments_e2e": out_host})
 
     acc_ms = kernel_ms["msm_accumulate"] / args.steps           # one launch per step (all columns)
     macs = cols * N * MSM_MACS_PER_POINT[K]
