@@ -140,6 +140,8 @@ def lib():
         L.h2v_quotient_gates_ptrs_dev.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]
         L.h2v_quotient_permutation_ptrs_dev.argtypes = ([C.c_void_p] * 5 + [C.c_size_t, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p,
                                                         C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32])
+        L.h2v_quotient_permutation_range_ptrs_dev.argtypes = ([C.c_void_p] * 5 + [C.c_size_t] * 4 + [C.c_int]
+                                                              + [C.c_void_p] * 3 + [C.c_size_t] + [C.c_void_p] * 3 + [C.c_uint32])
         L.h2v_pk_load.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_void_p, C.POINTER(C.c_void_p)]
         L.h2v_pk_free.argtypes = [C.c_void_p]
         L.h2v_pk_free.restype = None
@@ -662,6 +664,16 @@ class EvaluationDomain:
         _check(lib().h2v_quotient_permutation_dev(self._h, d_h, _ptr(_fr1(y)), _ptr(_fr1(beta)), _ptr(_fr1(gamma)),
                                                   n_cols, chunk_len, d_cols, cols_stride, d_sigma, sigma_stride, d_z, z_stride,
                                                   d_l0, d_l_last, d_l_active, blinding_factors))
+
+    def quotient_permutation_range(self, d_h, y, beta, gamma, n_cols, chunk_len, set_begin, set_end, with_head, d_col_ptrs,
+                                   d_sigma_ptrs, d_z, z_stride, d_l0, d_l_last, d_l_active, blinding_factors):
+        """The permutation terms of the sets [set_begin, set_end) only (a prover that streams the extended columns through
+        HBM in slices).  d_col_ptrs / d_sigma_ptrs are device tables of column pointers whose entry 0 is column
+        set_begin * chunk_len; d_z holds all the sets' z columns.  `with_head` folds the terms that precede the per-set
+        products: set it on the first call only, and consecutive ranges fold to the result of one quotient_permutation."""
+        _check(lib().h2v_quotient_permutation_range_ptrs_dev(self._h, d_h, _ptr(_fr1(y)), _ptr(_fr1(beta)), _ptr(_fr1(gamma)), n_cols,
+                                                             chunk_len, set_begin, set_end, int(bool(with_head)), d_col_ptrs,
+                                                             d_sigma_ptrs, d_z, z_stride, d_l0, d_l_last, d_l_active, blinding_factors))
 
     def quotient_lookup(self, d_h, y, beta, gamma, d_input, d_table, d_perm_input, d_perm_table, d_z, d_l0, d_l_last, d_l_active):
         _check(lib().h2v_quotient_lookup_dev(self._h, d_h, _ptr(_fr1(y)), _ptr(_fr1(beta)), _ptr(_fr1(gamma)),
