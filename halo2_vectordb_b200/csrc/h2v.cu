@@ -5,7 +5,6 @@
 //   h2v_srs     <-> halo2-axiom poly/kzg/commitment.rs ParamsKZG            (scaffold mod.rs:260)
 //   h2v_domain  <-> halo2-axiom poly/domain.rs EvaluationDomain             (scaffold mod.rs:273,296)
 #include <cuda_runtime.h>
-#include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -18,6 +17,7 @@
 #include <vector>
 
 #include "h2v.h"
+#include "internal.hpp"
 #include "msm.cuh"
 #include "ntt.cuh"
 #include "poly.cuh"
@@ -53,16 +53,6 @@ thread_local float g_last_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 thread_local uint32_t t_entry_counts[64];
 thread_local int t_entry_launches = 0;
 thread_local uint64_t g_last_entries = 0;
-
-int fail(int code, const char *fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    g_err = buf;
-    return code;
-}
 }  // namespace
 // shared with the other translation units of the library (internal.hpp)
 namespace h2v {
@@ -74,47 +64,11 @@ void count_launches(uint64_t n) { g_launches.fetch_add(n, std::memory_order_rela
 int current_device() { return g_devs[0]; }
 }  // namespace h2v
 namespace {
-#define CU(x)                                                                                      \
-    do {                                                                                           \
-        cudaError_t e_ = (x);                                                                      \
-        if (e_ != cudaSuccess) return fail(H2V_ECUDA, "%s failed: %s", #x, cudaGetErrorString(e_)); \
-    } while (0)
-#define LAUNCHED()                                                                                  \
-    do {                                                                                            \
-        g_launches.fetch_add(1, std::memory_order_relaxed);                                         \
-        cudaError_t e_ = cudaGetLastError();                                                        \
-        if (e_ != cudaSuccess) return fail(H2V_ECUDA, "kernel launch failed (%s:%d): %s", __FILE__, __LINE__, cudaGetErrorString(e_)); \
-    } while (0)
-
 int use_device() {
     cudaError_t e = cudaSetDevice(cur_dev());
-    if (e != cudaSuccess) return fail(H2V_ECUDA, "cudaSetDevice(%d): %s (libh2v has no CPU fallback)", cur_dev(), cudaGetErrorString(e));
+    if (e != cudaSuccess) return failf(H2V_ECUDA, "cudaSetDevice(%d): %s (libh2v has no CPU fallback)", cur_dev(), cudaGetErrorString(e));
     return H2V_OK;
 }
-
-struct DevBuf {
-    void *p = nullptr;
-    size_t cap = 0;
-    int ensure(size_t bytes) {
-        if (bytes <= cap) return H2V_OK;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-        cudaError_t e = cudaMalloc(&p, bytes);
-        if (e != cudaSuccess) {
-            cudaGetLastError();
-            return fail(H2V_ENOMEM, "cudaMalloc(%zu bytes): %s", bytes, cudaGetErrorString(e));
-        }
-        cap = bytes;
-        return H2V_OK;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
-    template <class T> T *as() const { return reinterpret_cast<T *>(p); }
-};
 
 // Column staging between caller-owned host columns and a device staging area: columns that are adjacent in host memory
 // (one Vec / tensor holding a whole batch) and land contiguously on the device move as ONE copy -- fewer, larger DMA
@@ -169,6 +123,33 @@ struct Timer {   // CUDA-event stopwatch on one stream, accumulating per kernel 
     }
 };
 
+// A synchronous `_dev` call: enqueue(tm) on `st` (created on first use) under `mu`, then wait for the stream.  The
+// device time of the call is recorded for h2v_last_kernel_ms as kernel class `cls`, or, with cls < 0, in the spans
+// enqueue records on `tm` itself.  An error of enqueue wins over a CUDA error of the stream.
+template <class Fn> int sync_call(std::mutex &mu, cudaStream_t &st, int cls, const char *what, Fn enqueue) {
+    std::lock_guard<std::mutex> lk(mu);
+    if (!st) H2V_CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+    Timer tm(st);
+    if (cls >= 0) tm.begin(cls);
+    int rc = enqueue(tm);
+    if (cls >= 0) tm.end();
+    cudaError_t e = cudaStreamSynchronize(st);
+    tm.collect(true);
+    if (rc) return rc;
+    if (e != cudaSuccess) return failf(H2V_ECUDA, "%s: %s", what, cudaGetErrorString(e));
+    return H2V_OK;
+}
+
+// The lane of a small host-facing call on replica `r`, locked: the lowest free one (a single-threaded caller keeps reusing
+// lane 0 and its buffers), else the next one in round-robin order.
+template <class Rep> typename Rep::Lane *lock_lane(Rep *r) {
+    for (auto &ln : r->lanes)
+        if (ln.mu.try_lock()) return &ln;
+    typename Rep::Lane *ln = &r->lanes[r->next_lane.fetch_add(1) % Rep::H2V_LANES];
+    ln->mu.lock();
+    return ln;
+}
+
 // ================================================================== NTT host side
 const size_t NTT_SMEM_BYTES = (2 * 2048 + H2V_NTT_PLANE_PAD) * 16;
 std::once_flag g_ntt_attr_once[H2V_MAX_DEV];      // function attributes are per device
@@ -191,7 +172,7 @@ int run_ntt(cudaStream_t st, const fe *src, size_t src_stride, fe *dst, size_t d
             const fe *pre, uint32_t pre_mod, uint32_t n_in, const fe *post, uint32_t post_mod, uint32_t n_out,
             size_t n_cols, uint32_t post_shift = 0) {
     if (n_cols == 0) return H2V_OK;
-    if ((const void *)src == (const void *)dst) return fail(H2V_EINVAL, "run_ntt: in-place transform needs distinct buffers");
+    if ((const void *)src == (const void *)dst) return failf(H2V_EINVAL, "run_ntt: in-place transform needs distinct buffers");
     std::call_once(g_ntt_attr_once[cur_dev()], [] {
         cudaFuncSetAttribute(ntt_pass_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NTT_SMEM_BYTES);
         cudaFuncSetAttribute(ntt_pass_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NTT_SMEM_BYTES);
@@ -218,7 +199,7 @@ int run_ntt(cudaStream_t st, const fe *src, size_t src_stride, fe *dst, size_t d
         if (L <= 2) {
             p.first = p.last = 1;
             ntt_tiny_kernel<<<cols, 32, 0, st>>>(p);
-            LAUNCHED();
+            H2V_LAUNCHED();
             continue;
         }
         NttPlan pl = ntt_plan(L);
@@ -245,7 +226,7 @@ int run_ntt(cudaStream_t st, const fe *src, size_t src_stride, fe *dst, size_t d
             }();
             if (L <= shoup_max_l) ntt_pass_kernel<true><<<dim3(tiles, cols), threads, smem, st>>>(p);
             else ntt_pass_kernel<false><<<dim3(tiles, cols), threads, smem, st>>>(p);
-            LAUNCHED();
+            H2V_LAUNCHED();
             t0 += S;
         }
     }
@@ -265,7 +246,7 @@ int build_twiddles(cudaStream_t st, DevBuf &buf, const fe &omega, int L) {
     }
     tp.half_n = (uint32_t)half;
     twiddle_kernel<<<(unsigned)((half + 255) / 256), 256, 0, st>>>(buf.as<fe>(), tp);
-    LAUNCHED();
+    H2V_LAUNCHED();
     return H2V_OK;
 }
 
@@ -312,8 +293,29 @@ struct DomRep {
     Lane lanes[H2V_LANES];
     std::atomic<unsigned> next_lane{0};
 };
+// public handle: one replica per device
+struct h2v_domain {
+    std::vector<DomRep *> rep;
+};
 
 namespace {
+DomRep *dom_on(h2v_domain *h, int dev) {
+    for (DomRep *r : h->rep)
+        if (r->dev == dev) return r;
+    return nullptr;
+}
+// the replica a call on `h` runs on, made the calling thread's device: the one on the device that holds `ptr`, the primary
+// one for host columns (ptr = NULL).  NULL (error recorded) when there is none.
+DomRep *dom_rep(h2v_domain *h, const void *ptr) {
+    if (!h) {
+        failf(H2V_EINVAL, "NULL domain");
+        return nullptr;
+    }
+    DomRep *r = ptr ? dom_on(h, device_of(ptr)) : h->rep[0];
+    if (!r) failf(H2V_EINVAL, "the columns live on device %d, which is not in the h2v_init list", device_of(ptr));
+    else t_dev = r->dev;
+    return r;
+}
 
 // twiddle tables are built once per domain and direction, synchronously, so that any stream may use them
 int domain_twiddles(DomRep *d, int which, const fe **out) {
@@ -322,7 +324,7 @@ int domain_twiddles(DomRep *d, int which, const fe **out) {
         const fe &w = which == 0 ? d->omega : which == 1 ? d->omega_inv : which == 2 ? d->ext_omega : d->ext_omega_inv;
         int rc = build_twiddles(d->stream, d->tw[which], w, which < 2 ? (int)d->k : (int)d->ek);
         if (rc) return rc;
-        CU(cudaStreamSynchronize(d->stream));
+        H2V_CU(cudaStreamSynchronize(d->stream));
         d->tw_ready[which] = true;
     }
     *out = d->tw[which].as<fe>();
@@ -352,7 +354,7 @@ int domain_op_dev(DomRep *d, cudaStream_t st, int op, const fe *in, size_t in_st
         if ((rc = domain_twiddles(d, 3, &tw))) return rc;
         return run_ntt(st, in, in_stride, out, out_stride, d->ek, tw, dc + 8, d->nt, en, dc + 4, 3, n * (d->j - 1), n_cols);
     default:
-        return fail(H2V_EINVAL, "unknown domain op %d", op);
+        return failf(H2V_EINVAL, "unknown domain op %d", op);
     }
 }
 size_t op_in_len(const DomRep *d, int op) {
@@ -543,12 +545,12 @@ int run_msm(cudaStream_t st, MsmWorkspace &ws, const fe *d_scalars, size_t col_s
             const affine *points, MsmCfg cfg, size_t pstride, affine *d_out_aff, jacobian *d_out_jac, Timer *tm, double density = 1.0) {
     if (n_cols == 0) return H2V_OK;
     if (len == 0) {   // empty sum = identity: affine (0, 0); Jacobian (0, 1, 0) as halo2curves `G1::identity()`
-        if (d_out_aff) CU(cudaMemsetAsync(d_out_aff, 0, n_cols * sizeof(affine), st));
+        if (d_out_aff) H2V_CU(cudaMemsetAsync(d_out_aff, 0, n_cols * sizeof(affine), st));
         if (d_out_jac) {
             std::vector<jacobian> id(n_cols);
             for (auto &j : id) { j.x = fe_zero(); j.y = fe_one<Fq>(); j.z = fe_zero(); }
-            CU(cudaMemcpyAsync(d_out_jac, id.data(), n_cols * sizeof(jacobian), cudaMemcpyHostToDevice, st));
-            CU(cudaStreamSynchronize(st));
+            H2V_CU(cudaMemcpyAsync(d_out_jac, id.data(), n_cols * sizeof(jacobian), cudaMemcpyHostToDevice, st));
+            H2V_CU(cudaStreamSynchronize(st));
         }
         return H2V_OK;
     }
@@ -570,7 +572,7 @@ int run_msm(cudaStream_t st, MsmWorkspace &ws, const fe *d_scalars, size_t col_s
     {
         MsmLayout probe = msm_layout(nullptr, sh, (uint32_t)max_cols);
         uint64_t ent = (uint64_t)max_cols * sh.W * sh.n;
-        if (ent >= (1ull << 32) - 64) return fail(H2V_EINVAL, "MSM too large: %llu bucket entries", (unsigned long long)ent);
+        if (ent >= (1ull << 32) - 64) return failf(H2V_EINVAL, "MSM too large: %llu bucket entries", (unsigned long long)ent);
         int rc = ws.buf.ensure(probe.bytes);
         if (rc) return rc;
     }
@@ -583,23 +585,23 @@ int run_msm(cudaStream_t st, MsmWorkspace &ws, const fe *d_scalars, size_t col_s
         sh.chunk = chunk_for(cols);
         MsmLayout L = msm_layout(ws.buf.p, sh, cols);
         const fe *sc = d_scalars + c0 * col_stride;
-        CU(cudaMemsetAsync(L.counts, 0, ((size_t)L.n_buckets + 8) * sizeof(uint32_t), st));
+        H2V_CU(cudaMemsetAsync(L.counts, 0, ((size_t)L.n_buckets + 8) * sizeof(uint32_t), st));
         unsigned gx = (unsigned)((len + 255) / 256);
         if (tm) tm->begin(0);
-        if (!launch_count(sh.c, dim3(gx, cols), st, sc, col_stride, L.counts, sh)) return fail(H2V_EINVAL, "MSM window size %u unsupported", sh.c);
-        LAUNCHED();
+        if (!launch_count(sh.c, dim3(gx, cols), st, sc, col_stride, L.counts, sh)) return failf(H2V_EINVAL, "MSM window size %u unsupported", sh.c);
+        H2V_LAUNCHED();
         if (tm) { tm->end(); tm->begin(1); }
         {
             const uint32_t ntiles = (L.n_buckets + H2V_SCAN_TILE - 1) / H2V_SCAN_TILE;
             msm_scan_tiles_kernel<<<ntiles, 256, 0, st>>>(L.counts, L.tile_sums, L.n_buckets);
-            LAUNCHED();
+            H2V_LAUNCHED();
             msm_scan_top_kernel<<<1, 256, 0, st>>>(L.tile_sums, ntiles, L.offsets + L.n_buckets);
-            LAUNCHED();
+            H2V_LAUNCHED();
             msm_scan_apply_kernel<<<ntiles, 256, 0, st>>>(L.counts, L.tile_sums, L.offsets, L.cursor, L.n_buckets);
-            LAUNCHED();
+            H2V_LAUNCHED();
         }
         if (tm && t_entry_launches < 64)
-            CU(cudaMemcpyAsync(&t_entry_counts[t_entry_launches++], L.offsets + L.n_buckets, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+            H2V_CU(cudaMemcpyAsync(&t_entry_counts[t_entry_launches++], L.offsets + L.n_buckets, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
         if (tm) { tm->end(); tm->begin(2); }
         {
             // A single very large MSM (>= 1 GiB of sorted entries) sweeps the bucket space in 4 slices: the
@@ -615,22 +617,22 @@ int run_msm(cudaStream_t st, MsmWorkspace &ws, const fe *d_scalars, size_t col_s
             const uint32_t per = (sh.nb + slices - 1) / slices;
             for (uint32_t sl = 0; sl < slices; ++sl) {
                 launch_scatter(sh.c, dim3(gx, cols), st, sc, col_stride, L.cursor, L.entries, sh, sl * per, std::min(sh.nb, (sl + 1) * per));
-                LAUNCHED();
+                H2V_LAUNCHED();
             }
         }
         if (tm) { tm->end(); tm->begin(3); }
         const uint32_t acc_threads = L.nthreads;
         msm_accumulate_kernel<<<(acc_threads + 127) / 128, 128, 0, st>>>(L.entries, L.offsets, L.n_buckets, points, L.buckets, L.edges, sh.chunk,
                                                                         L.strad_list, L.strad_count);
-        LAUNCHED();
+        H2V_LAUNCHED();
         if (tm) { tm->end(); tm->begin(4); }
         {
             const unsigned fg = (unsigned)std::min<uint64_t>(((uint64_t)acc_threads + 127) / 128, 148ull * 16);
             msm_finish_kernel<<<fg, 128, 0, st>>>(L.offsets, L.strad_list, L.strad_count, L.edges, L.buckets, sh.chunk, L.long_list,
                                                   L.long_count);
-            LAUNCHED();
+            H2V_LAUNCHED();
             msm_finish_long_kernel<<<148 * 2, 256, 0, st>>>(L.offsets, L.edges, L.buckets, sh.chunk, L.long_list, L.long_count);
-            LAUNCHED();
+            H2V_LAUNCHED();
         }
         if (tm) { tm->end(); tm->begin(5); }
         // reduction over each (column, group): serial radix levels while they fill the GPU, then one log-depth tree
@@ -643,7 +645,7 @@ int run_msm(cudaStream_t st, MsmWorkspace &ws, const fe *d_scalars, size_t col_s
             if (cnt <= H2V_TREE_MAX && !occ) {
                 const unsigned threads = std::max(32u, std::min(256u, cnt / 2));
                 msm_reduce_tree_kernel<<<n_inst, threads, 2 * cnt * sizeof(xyzz), st>>>(Sin, Ain, cnt, shift, L.S[pp], L.A[pp]);
-                LAUNCHED();
+                H2V_LAUNCHED();
                 Sin = L.S[pp];
                 Ain = L.A[pp];
                 cnt = 1;
@@ -657,7 +659,7 @@ int run_msm(cudaStream_t st, MsmWorkspace &ws, const fe *d_scalars, size_t col_s
             uint32_t cnt_out = (cnt + (1u << log_seg) - 1) >> log_seg;
             uint32_t total = n_inst * cnt_out;
             msm_reduce_kernel<<<(total + 127) / 128, 128, 0, st>>>(Sin, Ain, L.S[pp], L.A[pp], cnt, cnt_out, n_inst, shift, log_seg, occ);
-            LAUNCHED();
+            H2V_LAUNCHED();
             occ = nullptr;
             Sin = L.S[pp];
             Ain = L.A[pp];
@@ -667,14 +669,14 @@ int run_msm(cudaStream_t st, MsmWorkspace &ws, const fe *d_scalars, size_t col_s
         }
         if (!Ain) {   // nb == 1: a single bucket per group, its weight is 1 and there is no weighted part
             msm_reduce_kernel<<<(n_inst + 127) / 128, 128, 0, st>>>(Sin, nullptr, L.S[pp], L.A[pp], 1, 1, n_inst, 0, 3, occ);
-            LAUNCHED();
+            H2V_LAUNCHED();
             Sin = L.S[pp];
             Ain = L.A[pp];
         }
         if (tm) { tm->end(); tm->begin(6); }
         msm_final_kernel<<<cols, 32, 0, st>>>(Sin, Ain, cols, sh.G, sh.c, d_out_aff ? d_out_aff + c0 : nullptr,
                                                           d_out_jac ? d_out_jac + c0 : nullptr);
-        LAUNCHED();
+        H2V_LAUNCHED();
         if (tm) tm->end();
     }
     return H2V_OK;
@@ -715,8 +717,16 @@ struct SrsRep {
     std::atomic<unsigned> next_lane{0};
     int last_variant = 0;
 };
+struct h2v_srs {
+    std::vector<SrsRep *> rep;
+};
 
 namespace {
+SrsRep *srs_on(h2v_srs *h, int dev) {
+    for (SrsRep *r : h->rep)
+        if (r->dev == dev) return r;
+    return nullptr;
+}
 // Window choice per call: the share of non-zero digits under both window sizes is estimated from a strided sample of
 // the batch (one small kernel + a 16-byte read-back), then the cheaper plan wins under the cost model
 //   10 products per bucket addition (mixed add) + 28 per bucket of the reduction (two full additions).
@@ -734,13 +744,13 @@ int msm_srs(SrsRep *s, cudaStream_t st, MsmWorkspace &ws, int basis, const fe *d
             int rc = ws.buf.ensure(4096);
             if (rc) return rc;
             uint32_t *d_cnt = ws.buf.as<uint32_t>();
-            CU(cudaMemsetAsync(d_cnt, 0, 8, st));
+            H2V_CU(cudaMemsetAsync(d_cnt, 0, 8, st));
             MsmShape s0 = make_shape(len, s->cfg[0], s->n), s1 = make_shape(len, s->cfg[1], s->n);
             msm_density_kernel<<<(samples + 255) / 256, 256, 0, st>>>(d_scalars, col_stride, (uint32_t)n_cols, (uint32_t)len, samples, s0, s1, d_cnt);
-            LAUNCHED();
+            H2V_LAUNCHED();
             uint32_t h_cnt[2] = {0, 0};
-            CU(cudaMemcpyAsync(h_cnt, d_cnt, 8, cudaMemcpyDeviceToHost, st));
-            CU(cudaStreamSynchronize(st));
+            H2V_CU(cudaMemcpyAsync(h_cnt, d_cnt, 8, cudaMemcpyDeviceToHost, st));
+            H2V_CU(cudaStreamSynchronize(st));
             const double e0 = (double)h_cnt[0] / samples * len, e1 = (double)h_cnt[1] / samples * len;      // entries per column
             // the reduction is latency-bound when few columns share it: weigh it up for small batches
             const double inst_w = n_cols >= 32 ? 28.0 : 28.0 * (1.0 + 24.0 / (double)n_cols);
@@ -776,22 +786,22 @@ int h2v_device_count(void) {
 // single-column entry points run there).  Call before creating handles.  NULL / 0 = device 0.
 int h2v_init(const int *devices, int n_dev) {
     int n = h2v_device_count();
-    if (n <= 0) return fail(H2V_ECUDA, "no CUDA device visible (libh2v has no CPU fallback)");
+    if (n <= 0) return failf(H2V_ECUDA, "no CUDA device visible (libh2v has no CPU fallback)");
     std::vector<int> devs;
     if (!devices || n_dev <= 0) {
         devs.push_back(0);
     } else {
-        if (n_dev > H2V_MAX_DEV) return fail(H2V_EINVAL, "h2v_init: at most %d devices", H2V_MAX_DEV);
+        if (n_dev > H2V_MAX_DEV) return failf(H2V_EINVAL, "h2v_init: at most %d devices", H2V_MAX_DEV);
         for (int i = 0; i < n_dev; ++i) {
-            if (devices[i] < 0 || devices[i] >= n) return fail(H2V_EINVAL, "device %d out of range (have %d)", devices[i], n);
+            if (devices[i] < 0 || devices[i] >= n) return failf(H2V_EINVAL, "device %d out of range (have %d)", devices[i], n);
             for (int d : devs)
-                if (d == devices[i]) return fail(H2V_EINVAL, "h2v_init: device %d listed twice", d);
+                if (d == devices[i]) return failf(H2V_EINVAL, "h2v_init: device %d listed twice", d);
             devs.push_back(devices[i]);
         }
     }
     for (int d : devs) {
-        CU(cudaSetDevice(d));
-        CU(cudaFree(0));
+        H2V_CU(cudaSetDevice(d));
+        H2V_CU(cudaFree(0));
     }
     // peer access between all pairs (SRS replicas are copied device to device); failure just means staged copies
     for (int a : devs)
@@ -806,7 +816,7 @@ int h2v_init(const int *devices, int n_dev) {
         }
     g_devs = devs;
     t_dev = -1;
-    CU(cudaSetDevice(g_devs[0]));
+    H2V_CU(cudaSetDevice(g_devs[0]));
     return H2V_OK;
 }
 int h2v_device_list(int *out, int cap) {
@@ -817,7 +827,7 @@ int h2v_device_list(int *out, int cap) {
 // canonical x, little-endian, with the parity of canonical y in the top bit of byte 31 (poseidon.hpp); identity = 32 zero bytes.
 // Host-side (a proof holds ~10^3 commitments); uses the host instantiation of the field code.
 int h2v_g1_to_bytes(const uint64_t *affine_pts, size_t n, uint8_t *out) {
-    if (n && (!affine_pts || !out)) return fail(H2V_EINVAL, "g1_to_bytes: NULL buffer");
+    if (n && (!affine_pts || !out)) return failf(H2V_EINVAL, "g1_to_bytes: NULL buffer");
     for (size_t i = 0; i < n; ++i) {
         affine p;
         memcpy(&p, affine_pts + 8 * i, sizeof p);
@@ -832,7 +842,7 @@ int h2v_g1_to_bytes(const uint64_t *affine_pts, size_t n, uint8_t *out) {
 }
 // `Fr::to_repr()`: canonical little-endian bytes of Montgomery-form scalars
 int h2v_fr_to_repr(const uint64_t *fr_mont, size_t n, uint8_t *out) {
-    if (n && (!fr_mont || !out)) return fail(H2V_EINVAL, "fr_to_repr: NULL buffer");
+    if (n && (!fr_mont || !out)) return failf(H2V_EINVAL, "fr_to_repr: NULL buffer");
     for (size_t i = 0; i < n; ++i) {
         fe a;
         memcpy(a.v, fr_mont + 4 * i, 32);
@@ -845,11 +855,11 @@ int h2v_dev_alloc(size_t bytes, void **d_out) {
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
-    if (!d_out || !bytes) return fail(H2V_EINVAL, "dev_alloc: bad argument");
+    if (!d_out || !bytes) return failf(H2V_EINVAL, "dev_alloc: bad argument");
     cudaError_t e = cudaMalloc(d_out, bytes);
     if (e != cudaSuccess) {
         cudaGetLastError();
-        return fail(H2V_ENOMEM, "cudaMalloc(%zu bytes): %s", bytes, cudaGetErrorString(e));
+        return failf(H2V_ENOMEM, "cudaMalloc(%zu bytes): %s", bytes, cudaGetErrorString(e));
     }
     return H2V_OK;
 }
@@ -857,38 +867,38 @@ int h2v_dev_free(void *d_ptr) {
     t_dev = device_of(d_ptr);
     int rc = use_device();
     if (rc) return rc;
-    if (d_ptr) CU(cudaFree(d_ptr));
+    if (d_ptr) H2V_CU(cudaFree(d_ptr));
     return H2V_OK;
 }
 int h2v_dev_upload(void *d_dst, const void *src, size_t bytes) {
     t_dev = device_of(d_dst);
     int rc = use_device();
     if (rc) return rc;
-    if (bytes && (!d_dst || !src)) return fail(H2V_EINVAL, "dev_upload: NULL buffer");
-    CU(cudaMemcpy(d_dst, src, bytes, cudaMemcpyHostToDevice));
+    if (bytes && (!d_dst || !src)) return failf(H2V_EINVAL, "dev_upload: NULL buffer");
+    H2V_CU(cudaMemcpy(d_dst, src, bytes, cudaMemcpyHostToDevice));
     return H2V_OK;
 }
 int h2v_dev_download(void *dst, const void *d_src, size_t bytes) {
     t_dev = device_of(d_src);
     int rc = use_device();
     if (rc) return rc;
-    if (bytes && (!dst || !d_src)) return fail(H2V_EINVAL, "dev_download: NULL buffer");
-    CU(cudaMemcpy(dst, d_src, bytes, cudaMemcpyDeviceToHost));
+    if (bytes && (!dst || !d_src)) return failf(H2V_EINVAL, "dev_download: NULL buffer");
+    H2V_CU(cudaMemcpy(dst, d_src, bytes, cudaMemcpyDeviceToHost));
     return H2V_OK;
 }
 int h2v_host_register(void *ptr, size_t bytes) {
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
-    if (!ptr || !bytes) return fail(H2V_EINVAL, "host_register: bad argument");
-    CU(cudaHostRegister(ptr, bytes, cudaHostRegisterDefault));
+    if (!ptr || !bytes) return failf(H2V_EINVAL, "host_register: bad argument");
+    H2V_CU(cudaHostRegister(ptr, bytes, cudaHostRegisterDefault));
     return H2V_OK;
 }
 int h2v_host_unregister(void *ptr) {
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
-    CU(cudaHostUnregister(ptr));
+    H2V_CU(cudaHostUnregister(ptr));
     return H2V_OK;
 }
 int h2v_set_tuning(int chunk, int table) {
@@ -898,7 +908,7 @@ int h2v_set_tuning(int chunk, int table) {
 }
 uint64_t h2v_last_msm_entries(void) { return g_last_entries; }
 int h2v_last_kernel_ms(float out[8]) {
-    if (!out) return fail(H2V_EINVAL, "last_kernel_ms: NULL");
+    if (!out) return failf(H2V_EINVAL, "last_kernel_ms: NULL");
     memcpy(out, g_last_ms, sizeof g_last_ms);
     return H2V_OK;
 }
@@ -906,9 +916,9 @@ int h2v_last_kernel_ms(float out[8]) {
 // ---------------------------------------------------------------- SRS / commit
 static void rep_srs_free(SrsRep *s);
 static int rep_srs_load(uint32_t k, const uint64_t *g, const uint64_t *g_lagrange, SrsRep **out) {
-    if (!out) return fail(H2V_EINVAL, "h2v_srs_load: out is NULL");
+    if (!out) return failf(H2V_EINVAL, "h2v_srs_load: out is NULL");
     *out = nullptr;
-    if (k > 26) return fail(H2V_EINVAL, "h2v_srs_load: k = %u unsupported", k);
+    if (k > 26) return failf(H2V_EINVAL, "h2v_srs_load: k = %u unsupported", k);
     int rc = use_device();
     if (rc) return rc;
     SrsRep *s = new SrsRep();
@@ -935,7 +945,7 @@ static int rep_srs_load(uint32_t k, const uint64_t *g, const uint64_t *g_lagrang
     cudaError_t e = cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) {
         delete s;
-        return fail(H2V_ECUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
+        return failf(H2V_ECUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
     }
     const uint64_t *src[2] = {g, g_lagrange};
     for (int b = 0; b < 2; ++b) {
@@ -946,7 +956,7 @@ static int rep_srs_load(uint32_t k, const uint64_t *g, const uint64_t *g_lagrang
             if (rc) { rep_srs_free(s); return rc; }
             if (v == 0) e = cudaMemcpyAsync(tb.p, src[b], s->n * sizeof(affine), cudaMemcpyHostToDevice, s->stream);
             else e = cudaMemcpyAsync(tb.p, s->table[b][0].p, s->n * sizeof(affine), cudaMemcpyDeviceToDevice, s->stream);
-            if (e != cudaSuccess) { rep_srs_free(s); return fail(H2V_ECUDA, "SRS upload: %s", cudaGetErrorString(e)); }
+            if (e != cudaSuccess) { rep_srs_free(s); return failf(H2V_ECUDA, "SRS upload: %s", cudaGetErrorString(e)); }
             for (uint32_t lvl = 1; lvl < s->cfg[v].W; ++lvl) {
                 msm_precompute_kernel<<<(unsigned)((s->n + 127) / 128), 128, 0, s->stream>>>(tb.as<affine>(), (uint32_t)s->n, lvl, s->cfg[v].c);
                 g_launches.fetch_add(1);
@@ -956,12 +966,13 @@ static int rep_srs_load(uint32_t k, const uint64_t *g, const uint64_t *g_lagrang
     }
     e = cudaStreamSynchronize(s->stream);
     if (e == cudaSuccess) e = cudaGetLastError();
-    if (e != cudaSuccess) { rep_srs_free(s); return fail(H2V_ECUDA, "SRS table build: %s", cudaGetErrorString(e)); }
+    if (e != cudaSuccess) { rep_srs_free(s); return failf(H2V_ECUDA, "SRS table build: %s", cudaGetErrorString(e)); }
     *out = s;
     return H2V_OK;
 }
-static int rep_srs_info(SrsRep *s, uint32_t *window_bits, uint32_t *windows) {
-    if (!s) return fail(H2V_EINVAL, "srs_info: NULL srs");
+int h2v_srs_info(h2v_srs_t h, uint32_t *window_bits, uint32_t *windows) {
+    if (!h) return failf(H2V_EINVAL, "srs_info: NULL srs");
+    const SrsRep *s = h->rep[0];
     // the table the last commit on this handle used (the main one before any commit)
     if (window_bits) *window_bits = s->cfg[s->last_variant].c;
     if (windows) *windows = s->cfg[s->last_variant].W;
@@ -999,60 +1010,48 @@ static void rep_srs_free(SrsRep *s) {
 
 static int rep_commit_batch_dev(SrsRep *s, int basis, const void *d_polys, size_t col_stride, size_t n_polys, size_t len,
                          void *d_out_affine) {
-    if (!s) return fail(H2V_EINVAL, "commit: NULL srs");
-    if (basis != 0 && basis != 1) return fail(H2V_EINVAL, "commit: basis must be 0 or 1");
-    if (!s->have[basis]) return fail(H2V_EINVAL, "commit: basis %d was not loaded", basis);
-    if (len > s->n) return fail(H2V_EINVAL, "commit: poly length %zu exceeds n = %zu", len, s->n);
-    if (n_polys && (!d_polys || !d_out_affine)) return fail(H2V_EINVAL, "commit: NULL buffer");
-    int rc = use_device();
-    if (rc) return rc;
-    std::lock_guard<std::mutex> lk(s->mu);
-    Timer tm(s->stream);
+    if (!s) return failf(H2V_EINVAL, "commit: NULL srs");
+    if (basis != 0 && basis != 1) return failf(H2V_EINVAL, "commit: basis must be 0 or 1");
+    if (!s->have[basis]) return failf(H2V_EINVAL, "commit: basis %d was not loaded", basis);
+    if (len > s->n) return failf(H2V_EINVAL, "commit: poly length %zu exceeds n = %zu", len, s->n);
+    if (n_polys && (!d_polys || !d_out_affine)) return failf(H2V_EINVAL, "commit: NULL buffer");
+    H2V_TRY(use_device());
     t_entry_launches = 0;
-    rc = msm_srs(s, s->stream, s->ws, basis, (const fe *)d_polys, col_stride, n_polys, len, (affine *)d_out_affine, &tm);
-    cudaError_t e = cudaStreamSynchronize(s->stream);
-    tm.collect(true);
+    int rc = sync_call(s->mu, s->stream, -1, "commit", [&](Timer &tm) {
+        return msm_srs(s, s->stream, s->ws, basis, (const fe *)d_polys, col_stride, n_polys, len, (affine *)d_out_affine, &tm);
+    });
     g_last_entries = 0;
     for (int i = 0; i < t_entry_launches; ++i) g_last_entries += t_entry_counts[i];
-    if (rc) return rc;
-    if (e != cudaSuccess) return fail(H2V_ECUDA, "commit: %s", cudaGetErrorString(e));
-    return H2V_OK;
+    return rc;
 }
 
 static int rep_commit_batch(SrsRep *s, int basis, const uint64_t *const *polys, size_t n_polys, size_t len, uint64_t *out_affine) {
-    if (!s) return fail(H2V_EINVAL, "commit: NULL srs");
-    if (basis != 0 && basis != 1) return fail(H2V_EINVAL, "commit: basis must be 0 or 1");
-    if (!s->have[basis]) return fail(H2V_EINVAL, "commit: basis %d was not loaded", basis);
-    if (len > s->n) return fail(H2V_EINVAL, "commit: poly length %zu exceeds n = %zu", len, s->n);
+    if (!s) return failf(H2V_EINVAL, "commit: NULL srs");
+    if (basis != 0 && basis != 1) return failf(H2V_EINVAL, "commit: basis must be 0 or 1");
+    if (!s->have[basis]) return failf(H2V_EINVAL, "commit: basis %d was not loaded", basis);
+    if (len > s->n) return failf(H2V_EINVAL, "commit: poly length %zu exceeds n = %zu", len, s->n);
     if (n_polys == 0) return H2V_OK;
-    if (!polys || !out_affine) return fail(H2V_EINVAL, "commit: NULL buffer");
+    if (!polys || !out_affine) return failf(H2V_EINVAL, "commit: NULL buffer");
     int rc = use_device();
     if (rc) return rc;
     const size_t stride_small = std::max<size_t>(len, 1);
     if (n_polys * stride_small * sizeof(fe) <= ((size_t)48 << 20)) {
-        // one sub-batch: take a free lane (or wait for the next one in round-robin order)
-        // lowest free lane first (a single-threaded caller keeps reusing lane 0 and its buffers)
-        SrsRep::Lane *ln = nullptr;
-        for (int i = 0; i < SrsRep::H2V_LANES && !ln; ++i)
-            if (s->lanes[i].mu.try_lock()) ln = &s->lanes[i];
-        if (!ln) {
-            ln = &s->lanes[s->next_lane.fetch_add(1) % SrsRep::H2V_LANES];
-            ln->mu.lock();
-        }
+        // one sub-batch, on a lane
+        SrsRep::Lane *ln = lock_lane(s);
         std::lock_guard<std::mutex> lk(ln->mu, std::adopt_lock);
-        if (!ln->st) CU(cudaStreamCreateWithFlags(&ln->st, cudaStreamNonBlocking));
+        if (!ln->st) H2V_CU(cudaStreamCreateWithFlags(&ln->st, cudaStreamNonBlocking));
         if ((rc = ln->stage.ensure(n_polys * stride_small * sizeof(fe)))) return rc;
         if ((rc = ln->out.ensure(n_polys * sizeof(affine)))) return rc;
         for (size_t c = 0; c < n_polys; ++c)
-            if (!polys[c] && len) return fail(H2V_EINVAL, "commit: polys[%zu] is NULL", c);
-        CU(stage_columns(true, ln->stage.as<fe>(), stride_small, polys, n_polys, len, ln->st));
+            if (!polys[c] && len) return failf(H2V_EINVAL, "commit: polys[%zu] is NULL", c);
+        H2V_CU(stage_columns(true, ln->stage.as<fe>(), stride_small, polys, n_polys, len, ln->st));
         rc = msm_srs(s, ln->st, ln->ws, basis, ln->stage.as<fe>(), stride_small, n_polys, len, ln->out.as<affine>(), nullptr);
         if (rc) {
             cudaStreamSynchronize(ln->st);
             return rc;
         }
-        CU(cudaMemcpyAsync(out_affine, ln->out.p, n_polys * sizeof(affine), cudaMemcpyDeviceToHost, ln->st));
-        CU(cudaStreamSynchronize(ln->st));
+        H2V_CU(cudaMemcpyAsync(out_affine, ln->out.p, n_polys * sizeof(affine), cudaMemcpyDeviceToHost, ln->st));
+        H2V_CU(cudaStreamSynchronize(ln->st));
         return H2V_OK;
     }
     std::lock_guard<std::mutex> lk(s->mu);
@@ -1080,11 +1079,11 @@ static int rep_commit_batch(SrsRep *s, int basis, const uint64_t *const *polys, 
     if ((rc = s->stage.ensure(2 * sub * stride * sizeof(fe)))) return rc;
     if ((rc = s->out.ensure(n_polys * sizeof(affine)))) return rc;
     if (!s->copy_stream) {
-        CU(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
-        CU(cudaStreamCreateWithFlags(&s->stream2, cudaStreamNonBlocking));
+        H2V_CU(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
+        H2V_CU(cudaStreamCreateWithFlags(&s->stream2, cudaStreamNonBlocking));
         for (int b = 0; b < 2; ++b) {
-            CU(cudaEventCreateWithFlags(&s->copied[b], cudaEventDisableTiming));
-            CU(cudaEventCreateWithFlags(&s->computed[b], cudaEventDisableTiming));
+            H2V_CU(cudaEventCreateWithFlags(&s->copied[b], cudaEventDisableTiming));
+            H2V_CU(cudaEventCreateWithFlags(&s->computed[b], cudaEventDisableTiming));
         }
     }
     size_t it = 0;
@@ -1093,18 +1092,18 @@ static int rep_commit_batch(SrsRep *s, int basis, const uint64_t *const *polys, 
         const size_t cols = std::min(step, n_polys - c0);
         const int b = (int)(it & 1);
         fe *stg = s->stage.as<fe>() + (size_t)b * sub * stride;
-        if (it >= 2) CU(cudaStreamWaitEvent(s->copy_stream, s->computed[b], 0));
+        if (it >= 2) H2V_CU(cudaStreamWaitEvent(s->copy_stream, s->computed[b], 0));
         for (size_t c = 0; c < cols; ++c) {
             if (!polys[c0 + c] && len) {
                 cudaStreamSynchronize(s->stream);
                 cudaStreamSynchronize(s->copy_stream);
-                return fail(H2V_EINVAL, "commit: polys[%zu] is NULL", c0 + c);
+                return failf(H2V_EINVAL, "commit: polys[%zu] is NULL", c0 + c);
             }
         }
-        CU(stage_columns(true, stg, stride, polys + c0, cols, len, s->copy_stream));
-        CU(cudaEventRecord(s->copied[b], s->copy_stream));
+        H2V_CU(stage_columns(true, stg, stride, polys + c0, cols, len, s->copy_stream));
+        H2V_CU(cudaEventRecord(s->copied[b], s->copy_stream));
         cudaStream_t cst = b ? s->stream2 : s->stream;
-        CU(cudaStreamWaitEvent(cst, s->copied[b], 0));
+        H2V_CU(cudaStreamWaitEvent(cst, s->copied[b], 0));
         rc = msm_srs(s, cst, b ? s->ws2 : s->ws, basis, stg, stride, cols, len, s->out.as<affine>() + c0, nullptr);
         if (rc) {
             cudaStreamSynchronize(s->stream);
@@ -1112,16 +1111,12 @@ static int rep_commit_batch(SrsRep *s, int basis, const uint64_t *const *polys, 
             cudaStreamSynchronize(s->copy_stream);
             return rc;
         }
-        CU(cudaEventRecord(s->computed[b], cst));
+        H2V_CU(cudaEventRecord(s->computed[b], cst));
     }
-    if (it > 1) CU(cudaStreamWaitEvent(s->stream, s->computed[1], 0));
-    CU(cudaMemcpyAsync(out_affine, s->out.p, n_polys * sizeof(affine), cudaMemcpyDeviceToHost, s->stream));
-    CU(cudaStreamSynchronize(s->stream));
+    if (it > 1) H2V_CU(cudaStreamWaitEvent(s->stream, s->computed[1], 0));
+    H2V_CU(cudaMemcpyAsync(out_affine, s->out.p, n_polys * sizeof(affine), cudaMemcpyDeviceToHost, s->stream));
+    H2V_CU(cudaStreamSynchronize(s->stream));
     return H2V_OK;
-}
-static int rep_commit(SrsRep *s, int basis, const uint64_t *poly, size_t len, uint64_t out_affine[8]) {
-    const uint64_t *cols[1] = {poly};
-    return rep_commit_batch(s, basis, cols, 1, len, out_affine);
 }
 
 // one MSM over caller-supplied bases (no handle, no tables): Jacobian and / or affine result
@@ -1142,26 +1137,26 @@ static int multiexp_raw(const uint64_t *coeffs, const uint64_t *bases, size_t n,
     DevBuf &sc = cx.sc, &pts = cx.pts, &outb = cx.outb;
     cudaStream_t &st = cx.st;
     std::lock_guard<std::mutex> lk(mu);
-    if (!st) CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+    if (!st) H2V_CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
     if ((rc = sc.ensure(n * sizeof(fe)))) return rc;
     if ((rc = pts.ensure(n * sizeof(affine)))) return rc;
     if ((rc = outb.ensure(sizeof(jacobian) + sizeof(affine)))) return rc;
-    CU(cudaMemcpyAsync(sc.p, coeffs, n * sizeof(fe), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(pts.p, bases, n * sizeof(affine), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(sc.p, coeffs, n * sizeof(fe), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(pts.p, bases, n * sizeof(affine), cudaMemcpyHostToDevice, st));
     MsmCfg cfg = choose_cfg(n, false);
     jacobian *dj = outb.as<jacobian>();
     affine *da = reinterpret_cast<affine *>(dj + 1);
     rc = run_msm(st, ws, sc.as<fe>(), n, 1, n, pts.as<affine>(), cfg, n, out_affine ? da : nullptr, out_jacobian ? dj : nullptr, nullptr);
     if (rc) { cudaStreamSynchronize(st); return rc; }
-    if (out_jacobian) CU(cudaMemcpyAsync(out_jacobian, dj, sizeof(jacobian), cudaMemcpyDeviceToHost, st));
-    if (out_affine) CU(cudaMemcpyAsync(out_affine, da, sizeof(affine), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    if (out_jacobian) H2V_CU(cudaMemcpyAsync(out_jacobian, dj, sizeof(jacobian), cudaMemcpyDeviceToHost, st));
+    if (out_affine) H2V_CU(cudaMemcpyAsync(out_affine, da, sizeof(affine), cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaStreamSynchronize(st));
     return H2V_OK;
 }
 int h2v_best_multiexp(const uint64_t *coeffs, const uint64_t *bases, size_t n, uint64_t out_jacobian[12]) {
-    if (!out_jacobian) return fail(H2V_EINVAL, "best_multiexp: NULL output");
-    if (n && (!coeffs || !bases)) return fail(H2V_EINVAL, "best_multiexp: NULL input");
-    if (n >= ((size_t)1 << 27)) return fail(H2V_EINVAL, "best_multiexp: n = %zu unsupported", n);
+    if (!out_jacobian) return failf(H2V_EINVAL, "best_multiexp: NULL output");
+    if (n && (!coeffs || !bases)) return failf(H2V_EINVAL, "best_multiexp: NULL input");
+    if (n >= ((size_t)1 << 27)) return failf(H2V_EINVAL, "best_multiexp: n = %zu unsupported", n);
     if (n == 0) {
         t_dev = -1;
         int rc = use_device();
@@ -1174,9 +1169,9 @@ int h2v_best_multiexp(const uint64_t *coeffs, const uint64_t *bases, size_t n, u
     return multiexp_raw(coeffs, bases, n, out_jacobian, nullptr);
 }
 int h2v_g1_sum(const uint64_t *affine_pts, size_t n, uint64_t out_affine[8]) {
-    if (!out_affine) return fail(H2V_EINVAL, "g1_sum: NULL output");
-    if (n && !affine_pts) return fail(H2V_EINVAL, "g1_sum: NULL input");
-    if (n >= ((size_t)1 << 27)) return fail(H2V_EINVAL, "g1_sum: n = %zu unsupported", n);
+    if (!out_affine) return failf(H2V_EINVAL, "g1_sum: NULL output");
+    if (n && !affine_pts) return failf(H2V_EINVAL, "g1_sum: NULL input");
+    if (n >= ((size_t)1 << 27)) return failf(H2V_EINVAL, "g1_sum: n = %zu unsupported", n);
     if (n == 0) {
         int rc = use_device();
         if (rc) return rc;
@@ -1189,8 +1184,8 @@ int h2v_g1_sum(const uint64_t *affine_pts, size_t n, uint64_t out_affine[8]) {
 
 // ---------------------------------------------------------------- FFT / domain
 int h2v_best_fft(uint64_t *a, const uint64_t omega[4], uint32_t log_n) {
-    if (!a || !omega) return fail(H2V_EINVAL, "best_fft: NULL argument");
-    if (log_n > 27) return fail(H2V_EINVAL, "best_fft: log_n = %u unsupported", log_n);
+    if (!a || !omega) return failf(H2V_EINVAL, "best_fft: NULL argument");
+    if (log_n > 27) return failf(H2V_EINVAL, "best_fft: log_n = %u unsupported", log_n);
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
@@ -1209,7 +1204,7 @@ int h2v_best_fft(uint64_t *a, const uint64_t omega[4], uint32_t log_n) {
     fe &cached_omega = cx.cached_omega;
     int &cached_L = cx.cached_L;
     std::lock_guard<std::mutex> lk(mu);
-    if (!st) CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+    if (!st) H2V_CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
     size_t n = (size_t)1 << log_n;
     if ((rc = A.ensure(n * sizeof(fe)))) return rc;
     if ((rc = B.ensure(n * sizeof(fe)))) return rc;
@@ -1219,22 +1214,22 @@ int h2v_best_fft(uint64_t *a, const uint64_t omega[4], uint32_t log_n) {
         cached_L = (int)log_n;
         cached_omega = w;
     }
-    CU(cudaMemcpyAsync(A.p, a, n * sizeof(fe), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(A.p, a, n * sizeof(fe), cudaMemcpyHostToDevice, st));
     rc = run_ntt(st, A.as<fe>(), n, B.as<fe>(), n, (int)log_n, TW.as<fe>(), nullptr, 1, (uint32_t)n, nullptr, 1, (uint32_t)n, 1);
     if (rc) { cudaStreamSynchronize(st); return rc; }
-    CU(cudaMemcpyAsync(a, B.p, n * sizeof(fe), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    H2V_CU(cudaMemcpyAsync(a, B.p, n * sizeof(fe), cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaStreamSynchronize(st));
     return H2V_OK;
 }
 
 static void rep_domain_free(DomRep *d);
 static int rep_domain_new(uint32_t j, uint32_t k, DomRep **out) {
-    if (!out) return fail(H2V_EINVAL, "domain_new: out is NULL");
+    if (!out) return failf(H2V_EINVAL, "domain_new: out is NULL");
     *out = nullptr;
-    if (j < 2) return fail(H2V_EINVAL, "domain_new: j = %u (need j >= 2)", j);
+    if (j < 2) return failf(H2V_EINVAL, "domain_new: j = %u (need j >= 2)", j);
     uint32_t ek = k;
     while (((uint64_t)1 << ek) < ((uint64_t)1 << k) * (j - 1)) ++ek;
-    if (ek > 27 || ek - k > 6) return fail(H2V_EINVAL, "domain_new: extended_k = %u unsupported", ek);
+    if (ek > 27 || ek - k > 6) return failf(H2V_EINVAL, "domain_new: extended_k = %u unsupported", ek);
     int rc = use_device();
     if (rc) return rc;
     DomRep *d = new DomRep();
@@ -1282,7 +1277,7 @@ static int rep_domain_new(uint32_t j, uint32_t k, DomRep **out) {
     }
     if (e != cudaSuccess) {
         rep_domain_free(d);
-        return fail(H2V_ECUDA, "domain_new: %s", cudaGetErrorString(e));
+        return failf(H2V_ECUDA, "domain_new: %s", cudaGetErrorString(e));
     }
     *out = d;
     return H2V_OK;
@@ -1310,10 +1305,11 @@ static void rep_domain_free(DomRep *d) {
     if (d->stream) cudaStreamDestroy(d->stream);
     delete d;
 }
-static uint32_t rep_domain_k(DomRep *d) { return d ? d->k : 0; }
-static uint32_t rep_domain_extended_k(DomRep *d) { return d ? d->ek : 0; }
-static int rep_domain_constant(DomRep *d, int which, uint64_t out[4]) {
-    if (!d || !out) return fail(H2V_EINVAL, "domain_constant: NULL argument");
+uint32_t h2v_domain_k(h2v_domain_t h) { return h ? h->rep[0]->k : 0; }
+uint32_t h2v_domain_extended_k(h2v_domain_t h) { return h ? h->rep[0]->ek : 0; }
+int h2v_domain_constant(h2v_domain_t h, int which, uint64_t out[4]) {
+    if (!h || !out) return failf(H2V_EINVAL, "domain_constant: NULL argument");
+    const DomRep *d = h->rep[0];
     const fe *p = nullptr;
     switch (which) {
     case 0: p = &d->omega; break;
@@ -1327,23 +1323,25 @@ static int rep_domain_constant(DomRep *d, int which, uint64_t out[4]) {
     default:
         if (which >= 8 && (uint32_t)(which - 8) < d->nt) p = &d->t_eval[which - 8];
     }
-    if (!p) return fail(H2V_EINVAL, "domain_constant: index %d out of range", which);
+    if (!p) return failf(H2V_EINVAL, "domain_constant: index %d out of range", which);
     fe_to_u64x4(*p, out);
     return H2V_OK;
 }
 
 // ---- the scalar / index helpers of poly/domain.rs (SURVEY.md 8(a) row a12); host-side, no device work
 // EvaluationDomain::rotate_omega(value, rotation) = value * omega^rotation
-static int rep_domain_rotate_omega(DomRep *d, const uint64_t value[4], int32_t rotation, uint64_t out[4]) {
-    if (!d || !value || !out) return fail(H2V_EINVAL, "rotate_omega: NULL argument");
+int h2v_domain_rotate_omega(h2v_domain_t h, const uint64_t value[4], int32_t rotation, uint64_t out[4]) {
+    if (!h || !value || !out) return failf(H2V_EINVAL, "rotate_omega: NULL argument");
+    const DomRep *d = h->rep[0];
     fe w = rotation >= 0 ? fe_pow_u64<Fr>(d->omega, (uint64_t)rotation) : fe_pow_u64<Fr>(d->omega_inv, (uint64_t)(-(int64_t)rotation));
     fe_to_u64x4(fe_mul<Fr>(fe_from_u64x4(value), w), out);
     return H2V_OK;
 }
 // EvaluationDomain::rotate_extended(poly, rotation): cyclic shift of an extended-domain column by
 // rotation * 2^(extended_k - k) positions (out[i] = in[i + shift]); in != out
-static int rep_domain_rotate_extended(DomRep *d, const uint64_t *in, int32_t rotation, uint64_t *out) {
-    if (!d || !in || !out || in == out) return fail(H2V_EINVAL, "rotate_extended: NULL or aliased buffers");
+int h2v_domain_rotate_extended(h2v_domain_t h, const uint64_t *in, int32_t rotation, uint64_t *out) {
+    if (!h || !in || !out || in == out) return failf(H2V_EINVAL, "rotate_extended: NULL or aliased buffers");
+    const DomRep *d = h->rep[0];
     const size_t en = (size_t)1 << d->ek;
     const uint64_t per = (uint64_t)1 << (d->ek - d->k);
     const uint64_t mag = (uint64_t)(rotation < 0 ? -(int64_t)rotation : (int64_t)rotation) * per % en;
@@ -1354,9 +1352,10 @@ static int rep_domain_rotate_extended(DomRep *d, const uint64_t *in, int32_t rot
 }
 // EvaluationDomain::l_i_range(x, xn, rotations): out[t] = l_i(x) for i = rot_lo + t, rot_lo <= i < rot_hi, where
 // l_i(x) = omega^i (x^n - 1) / (n (x - omega^i)); xn = x^n is supplied as upstream's callers do.
-static int rep_domain_l_i_range(DomRep *d, const uint64_t x[4], const uint64_t xn[4], int32_t rot_lo, int32_t rot_hi, uint64_t *out) {
-    if (!d || !x || !xn || (rot_hi > rot_lo && !out)) return fail(H2V_EINVAL, "l_i_range: NULL argument");
-    if (rot_hi < rot_lo || (int64_t)rot_hi - rot_lo > (1 << 24)) return fail(H2V_EINVAL, "l_i_range: bad rotation range");
+int h2v_domain_l_i_range(h2v_domain_t h, const uint64_t x[4], const uint64_t xn[4], int32_t rot_lo, int32_t rot_hi, uint64_t *out) {
+    if (!h || !x || !xn || (rot_hi > rot_lo && !out)) return failf(H2V_EINVAL, "l_i_range: NULL argument");
+    const DomRep *d = h->rep[0];
+    if (rot_hi < rot_lo || (int64_t)rot_hi - rot_lo > (1 << 24)) return failf(H2V_EINVAL, "l_i_range: bad rotation range");
     const fe X = fe_from_u64x4(x), one = fe_one<Fr>();
     const fe common = fe_mul<Fr>(fe_sub<Fr>(fe_from_u64x4(xn), one), d->ifft_divisor);    // barycentric_weight = 1 / n
     const size_t cnt = (size_t)((int64_t)rot_hi - rot_lo);
@@ -1386,9 +1385,10 @@ static int rep_domain_l_i_range(DomRep *d, const uint64_t x[4], const uint64_t x
 }
 // EvaluationDomain::{empty_coeff, empty_lagrange, empty_extended, constant_lagrange, constant_extended}: a column of
 // the basis' length filled with `scalar` (NULL = zero).  basis: 0 coeff, 1 lagrange (both 2^k), 2 extended (2^extended_k)
-static int rep_domain_fill(DomRep *d, int basis, const uint64_t scalar[4], uint64_t *out) {
-    if (!d || !out) return fail(H2V_EINVAL, "domain_fill: NULL argument");
-    if (basis < 0 || basis > 2) return fail(H2V_EINVAL, "domain_fill: basis must be 0, 1 or 2");
+int h2v_domain_fill(h2v_domain_t h, int basis, const uint64_t scalar[4], uint64_t *out) {
+    if (!h || !out) return failf(H2V_EINVAL, "domain_fill: NULL argument");
+    const DomRep *d = h->rep[0];
+    if (basis < 0 || basis > 2) return failf(H2V_EINVAL, "domain_fill: basis must be 0, 1 or 2");
     const size_t len = (size_t)1 << (basis == 2 ? d->ek : d->k);
     if (!scalar) {
         memset(out, 0, len * 32);
@@ -1400,63 +1400,49 @@ static int rep_domain_fill(DomRep *d, int basis, const uint64_t scalar[4], uint6
 
 static int rep_domain_transform_dev(DomRep *d, int op, const void *d_in, size_t in_stride, void *d_out, size_t out_stride,
                              size_t n_cols) {
-    if (!d) return fail(H2V_EINVAL, "transform: NULL domain");
-    if (n_cols && (!d_in || !d_out)) return fail(H2V_EINVAL, "transform: NULL buffer");
-    if (op < 0 || op > H2V_OP_DIVIDE_BY_VANISHING) return fail(H2V_EINVAL, "unknown domain op %d", op);
+    if (!d) return failf(H2V_EINVAL, "transform: NULL domain");
+    if (n_cols && (!d_in || !d_out)) return failf(H2V_EINVAL, "transform: NULL buffer");
+    if (op < 0 || op > H2V_OP_DIVIDE_BY_VANISHING) return failf(H2V_EINVAL, "unknown domain op %d", op);
     // the output column doubles as the work buffer of the in-place passes: it needs the full transform size
     const size_t work_len = (size_t)1 << (op >= H2V_OP_COEFF_TO_EXTENDED ? d->ek : d->k);
     if (in_stride < op_in_len(d, op) || out_stride < work_len)
-        return fail(H2V_EINVAL, "transform: stride shorter than the column (out_stride must cover 2^%s)",
+        return failf(H2V_EINVAL, "transform: stride shorter than the column (out_stride must cover 2^%s)",
                     op >= H2V_OP_COEFF_TO_EXTENDED ? "extended_k" : "k");
-    int rc = use_device();
-    if (rc) return rc;
-    std::lock_guard<std::mutex> lk(d->mu);
-    Timer tm(d->stream);
-    tm.begin(7);
-    rc = domain_op_dev(d, d->stream, op, (const fe *)d_in, in_stride, (fe *)d_out, out_stride, n_cols);
-    tm.end();
-    cudaError_t e = cudaStreamSynchronize(d->stream);
-    tm.collect(true);
-    if (rc) return rc;
-    if (e != cudaSuccess) return fail(H2V_ECUDA, "transform: %s", cudaGetErrorString(e));
-    return H2V_OK;
+    H2V_TRY(use_device());
+    return sync_call(d->mu, d->stream, 7, "transform", [&](Timer &) {
+        return domain_op_dev(d, d->stream, op, (const fe *)d_in, in_stride, (fe *)d_out, out_stride, n_cols);
+    });
 }
 
 static int rep_domain_transform_batch(DomRep *d, int op, const uint64_t *const *in, uint64_t *const *out, size_t n_cols) {
-    if (!d) return fail(H2V_EINVAL, "transform: NULL domain");
-    if (op < 0 || op > H2V_OP_DIVIDE_BY_VANISHING) return fail(H2V_EINVAL, "unknown domain op %d", op);
+    if (!d) return failf(H2V_EINVAL, "transform: NULL domain");
+    if (op < 0 || op > H2V_OP_DIVIDE_BY_VANISHING) return failf(H2V_EINVAL, "unknown domain op %d", op);
     if (n_cols == 0) return H2V_OK;
-    if (!in || !out) return fail(H2V_EINVAL, "transform: NULL buffer");
+    if (!in || !out) return failf(H2V_EINVAL, "transform: NULL buffer");
     int rc = use_device();
     if (rc) return rc;
     const size_t nin = op_in_len(d, op), nout = op_out_len(d, op);
     const size_t out_stride = std::max(nout, (size_t)1 << (op >= H2V_OP_COEFF_TO_EXTENDED ? d->ek : d->k));
     if (n_cols * out_stride * sizeof(fe) <= ((size_t)8 << 20)) {
-        DomRep::Lane *ln = nullptr;
-        for (int i = 0; i < DomRep::H2V_LANES && !ln; ++i)
-            if (d->lanes[i].mu.try_lock()) ln = &d->lanes[i];
-        if (!ln) {
-            ln = &d->lanes[d->next_lane.fetch_add(1) % DomRep::H2V_LANES];
-            ln->mu.lock();
-        }
+        DomRep::Lane *ln = lock_lane(d);
         std::lock_guard<std::mutex> lk(ln->mu, std::adopt_lock);
-        if (!ln->st) CU(cudaStreamCreateWithFlags(&ln->st, cudaStreamNonBlocking));
+        if (!ln->st) H2V_CU(cudaStreamCreateWithFlags(&ln->st, cudaStreamNonBlocking));
         if ((rc = ln->stage_a.ensure(n_cols * nin * sizeof(fe)))) return rc;
         if ((rc = ln->stage_b.ensure(n_cols * out_stride * sizeof(fe)))) return rc;
         for (size_t c = 0; c < n_cols; ++c) {
             if (!in[c] || !out[c]) {
                 cudaStreamSynchronize(ln->st);
-                return fail(H2V_EINVAL, "transform: column %zu is NULL", c);
+                return failf(H2V_EINVAL, "transform: column %zu is NULL", c);
             }
         }
-        CU(stage_columns(true, ln->stage_a.as<fe>(), nin, in, n_cols, nin, ln->st));
+        H2V_CU(stage_columns(true, ln->stage_a.as<fe>(), nin, in, n_cols, nin, ln->st));
         rc = domain_op_dev(d, ln->st, op, ln->stage_a.as<fe>(), nin, ln->stage_b.as<fe>(), out_stride, n_cols);
         if (rc) {
             cudaStreamSynchronize(ln->st);
             return rc;
         }
-        CU(stage_columns(false, ln->stage_b.as<fe>(), out_stride, out, n_cols, nout, ln->st));
-        CU(cudaStreamSynchronize(ln->st));
+        H2V_CU(stage_columns(false, ln->stage_b.as<fe>(), out_stride, out, n_cols, nout, ln->st));
+        H2V_CU(cudaStreamSynchronize(ln->st));
         return H2V_OK;
     }
     // Pipelined batch: sub-batches rotate over three pipelines (stream + staging each) with no sync in between, so the
@@ -1471,8 +1457,8 @@ static int rep_domain_transform_batch(DomRep *d, int op, const uint64_t *const *
     per = std::min(per, n_cols);
     const int NP = 3;
     if (!d->pipe_stream) {
-        CU(cudaStreamCreateWithFlags(&d->pipe_stream, cudaStreamNonBlocking));
-        CU(cudaStreamCreateWithFlags(&d->pipe_stream2, cudaStreamNonBlocking));
+        H2V_CU(cudaStreamCreateWithFlags(&d->pipe_stream, cudaStreamNonBlocking));
+        H2V_CU(cudaStreamCreateWithFlags(&d->pipe_stream2, cudaStreamNonBlocking));
     }
     cudaStream_t pst[NP] = {d->stream, d->pipe_stream, d->pipe_stream2};
     DevBuf *pa[NP] = {&d->stage_a, &d->pipe_a, &d->pipe_a2}, *pb[NP] = {&d->stage_b, &d->pipe_b, &d->pipe_b2};
@@ -1490,14 +1476,14 @@ static int rep_domain_transform_batch(DomRep *d, int op, const uint64_t *const *
         for (size_t c = 0; c < cols; ++c) {
             if (!in[c0 + c] || !out[c0 + c]) {
                 sync_all();
-                return fail(H2V_EINVAL, "transform: column %zu is NULL", c0 + c);
+                return failf(H2V_EINVAL, "transform: column %zu is NULL", c0 + c);
             }
         }
         {
             cudaError_t e = stage_columns(true, pa[b]->as<fe>(), nin, in + c0, cols, nin, pst[b]);
             if (e != cudaSuccess) {
                 sync_all();
-                return fail(H2V_ECUDA, "transform: upload failed: %s", cudaGetErrorString(e));
+                return failf(H2V_ECUDA, "transform: upload failed: %s", cudaGetErrorString(e));
             }
         }
         rc = domain_op_dev(d, pst[b], op, pa[b]->as<fe>(), nin, pb[b]->as<fe>(), out_stride, cols);
@@ -1509,35 +1495,37 @@ static int rep_domain_transform_batch(DomRep *d, int op, const uint64_t *const *
             cudaError_t e = stage_columns(false, pb[b]->as<fe>(), out_stride, out + c0, cols, nout, pst[b]);
             if (e != cudaSuccess) {
                 sync_all();
-                return fail(H2V_ECUDA, "transform: download failed: %s", cudaGetErrorString(e));
+                return failf(H2V_ECUDA, "transform: download failed: %s", cudaGetErrorString(e));
             }
         }
     }
-    for (int b = 0; b < NP; ++b) CU(cudaStreamSynchronize(pst[b]));
+    for (int b = 0; b < NP; ++b) H2V_CU(cudaStreamSynchronize(pst[b]));
     return H2V_OK;
 }
-static int one_col(DomRep *d, int op, const uint64_t *in, uint64_t *out) {
-    const uint64_t *i1[1] = {in};
-    uint64_t *o1[1] = {out};
-    return rep_domain_transform_batch(d, op, i1, o1, 1);
+// one host column on the primary replica
+static int one_col(h2v_domain_t h, int op, const uint64_t *in, uint64_t *out) {
+    DomRep *d = dom_rep(h, nullptr);
+    return d ? rep_domain_transform_batch(d, op, &in, &out, 1) : H2V_EINVAL;
 }
-static int rep_lagrange_to_coeff(DomRep *d, uint64_t *a) { return one_col(d, H2V_OP_LAGRANGE_TO_COEFF, a, a); }
-static int rep_coeff_to_lagrange(DomRep *d, uint64_t *a) { return one_col(d, H2V_OP_COEFF_TO_LAGRANGE, a, a); }
-static int rep_coeff_to_extended(DomRep *d, const uint64_t *in, uint64_t *out) { return one_col(d, H2V_OP_COEFF_TO_EXTENDED, in, out); }
-static int rep_extended_to_coeff(DomRep *d, const uint64_t *in, uint64_t *out) { return one_col(d, H2V_OP_EXTENDED_TO_COEFF, in, out); }
-static int rep_divide_by_vanishing_poly(DomRep *d, uint64_t *a) {
-    if (!d || !a) return fail(H2V_EINVAL, "divide_by_vanishing_poly: NULL argument");
+int h2v_lagrange_to_coeff(h2v_domain_t h, uint64_t *a) { return one_col(h, H2V_OP_LAGRANGE_TO_COEFF, a, a); }
+int h2v_coeff_to_lagrange(h2v_domain_t h, uint64_t *a) { return one_col(h, H2V_OP_COEFF_TO_LAGRANGE, a, a); }
+int h2v_coeff_to_extended(h2v_domain_t h, const uint64_t *in, uint64_t *out) { return one_col(h, H2V_OP_COEFF_TO_EXTENDED, in, out); }
+int h2v_extended_to_coeff(h2v_domain_t h, const uint64_t *in, uint64_t *out) { return one_col(h, H2V_OP_EXTENDED_TO_COEFF, in, out); }
+int h2v_divide_by_vanishing_poly(h2v_domain_t h, uint64_t *a) {
+    DomRep *d = dom_rep(h, nullptr);
+    if (!d) return H2V_EINVAL;
+    if (!a) return failf(H2V_EINVAL, "divide_by_vanishing_poly: NULL argument");
     int rc = use_device();
     if (rc) return rc;
     std::lock_guard<std::mutex> lk(d->mu);
     size_t en = (size_t)1 << d->ek;
     if ((rc = d->stage_b.ensure(en * sizeof(fe)))) return rc;
-    CU(cudaMemcpyAsync(d->stage_b.p, a, en * sizeof(fe), cudaMemcpyHostToDevice, d->stream));
+    H2V_CU(cudaMemcpyAsync(d->stage_b.p, a, en * sizeof(fe), cudaMemcpyHostToDevice, d->stream));
     fr_scale_mod_kernel<<<dim3((unsigned)((en + 255) / 256), 1), 256, 0, d->stream>>>(d->stage_b.as<fe>(), en, d->dconst.as<fe>() + 8, d->nt,
                                                                                      (uint32_t)en);
-    LAUNCHED();
-    CU(cudaMemcpyAsync(a, d->stage_b.p, en * sizeof(fe), cudaMemcpyDeviceToHost, d->stream));
-    CU(cudaStreamSynchronize(d->stream));
+    H2V_LAUNCHED();
+    H2V_CU(cudaMemcpyAsync(a, d->stage_b.p, en * sizeof(fe), cudaMemcpyDeviceToHost, d->stream));
+    H2V_CU(cudaStreamSynchronize(d->stream));
     return H2V_OK;
 }
 
@@ -1553,7 +1541,7 @@ struct PolyCtx {
 PolyCtx g_poly_all[H2V_MAX_DEV];
 #define g_poly (g_poly_all[cur_dev()])
 int poly_ctx_ready() {
-    if (!g_poly.st) CU(cudaStreamCreateWithFlags(&g_poly.st, cudaStreamNonBlocking));
+    if (!g_poly.st) H2V_CU(cudaStreamCreateWithFlags(&g_poly.st, cudaStreamNonBlocking));
     return H2V_OK;
 }
 // I[i] = 1 / X[i] for n non-zero elements (one inversion in total); X and I are device arrays
@@ -1567,7 +1555,7 @@ template <class F> int run_batch_invert(cudaStream_t st, const fe *X, fe *I, uin
         v = (v + G - 1) / G;
         total += v;
     }
-    if (sizes[levels - 1] != 1) return fail(H2V_EINVAL, "batch_invert: n = %u unsupported", n);
+    if (sizes[levels - 1] != 1) return failf(H2V_EINVAL, "batch_invert: n = %u unsupported", n);
     // scratch: X_l (levels >= 1), P_l (all levels), I_l (levels >= 1)
     int rc = scratch.ensure((2 * total + n + total + 16) * sizeof(fe));
     if (rc) return rc;
@@ -1587,13 +1575,13 @@ template <class F> int run_batch_invert(cudaStream_t st, const fe *X, fe *I, uin
     }
     for (uint32_t l = 0; l + 1 < levels; ++l) {
         binv_up_kernel<F><<<(sizes[l + 1] + 127) / 128, 128, 0, st>>>(Xl[l], Pl[l], Xw[l + 1], sizes[l], G);
-        LAUNCHED();
+        H2V_LAUNCHED();
     }
     binv_top_kernel<F><<<1, 32, 0, st>>>(Xl[levels - 1], Il[levels - 1]);
-    LAUNCHED();
+    H2V_LAUNCHED();
     for (uint32_t l = levels - 1; l-- > 0;) {
         binv_down_kernel<F><<<(sizes[l + 1] + 127) / 128, 128, 0, st>>>(Xl[l], Pl[l], Il[l + 1], Il[l], sizes[l], G);
-        LAUNCHED();
+        H2V_LAUNCHED();
     }
     return H2V_OK;
 }
@@ -1603,28 +1591,22 @@ extern "C" {
 int h2v_eval_polynomial_dev(const void *d_polys, size_t stride, size_t n_polys, size_t len, const void *d_points, size_t n_points,
                             void *d_out) {
     if (!n_polys || !n_points) return H2V_OK;
-    if (!d_polys || !d_points || !d_out) return fail(H2V_EINVAL, "eval_polynomial: NULL buffer");
-    if (n_polys > 65535 || n_points > (1u << 20) || len >= ((size_t)1 << 31)) return fail(H2V_EINVAL, "eval_polynomial: batch too large");
+    if (!d_polys || !d_points || !d_out) return failf(H2V_EINVAL, "eval_polynomial: NULL buffer");
+    if (n_polys > 65535 || n_points > (1u << 20) || len >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "eval_polynomial: batch too large");
     t_dev = device_of(d_polys);
-    int rc = use_device();
-    if (rc) return rc;
-    std::lock_guard<std::mutex> lk(g_poly.mu);
-    if ((rc = poly_ctx_ready())) return rc;
-    Timer tm(g_poly.st);
-    tm.begin(7);
-    poly_eval_kernel<<<dim3((unsigned)n_points, (unsigned)n_polys), 256, 0, g_poly.st>>>((const fe *)d_polys, stride, (uint32_t)len,
-                                                                                       (const fe *)d_points, (uint32_t)n_points, (fe *)d_out);
-    LAUNCHED();
-    tm.end();
-    CU(cudaStreamSynchronize(g_poly.st));
-    tm.collect(true);
-    return H2V_OK;
+    H2V_TRY(use_device());
+    return sync_call(g_poly.mu, g_poly.st, 7, "eval_polynomial", [&](Timer &) {
+        poly_eval_kernel<<<dim3((unsigned)n_points, (unsigned)n_polys), 256, 0, g_poly.st>>>((const fe *)d_polys, stride, (uint32_t)len,
+                                                                                           (const fe *)d_points, (uint32_t)n_points, (fe *)d_out);
+        H2V_LAUNCHED();
+        return H2V_OK;
+    });
 }
 int h2v_eval_polynomial_batch(const uint64_t *const *polys, size_t n_polys, size_t len, const uint64_t *points, size_t n_points,
                               uint64_t *out) {
     if (!n_polys || !n_points) return H2V_OK;
-    if (!polys || !points || !out) return fail(H2V_EINVAL, "eval_polynomial: NULL buffer");
-    if (n_points > (1u << 20) || len >= ((size_t)1 << 31)) return fail(H2V_EINVAL, "eval_polynomial: batch too large");
+    if (!polys || !points || !out) return failf(H2V_EINVAL, "eval_polynomial: NULL buffer");
+    if (n_points > (1u << 20) || len >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "eval_polynomial: batch too large");
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
@@ -1637,25 +1619,25 @@ int h2v_eval_polynomial_batch(const uint64_t *const *polys, size_t n_polys, size
     if ((rc = g_poly.a.ensure(per * stride * sizeof(fe))) || (rc = g_poly.b.ensure(n_points * sizeof(fe))) ||
         (rc = g_poly.c.ensure(per * n_points * sizeof(fe))))
         return rc;
-    CU(cudaMemcpyAsync(g_poly.b.p, points, n_points * sizeof(fe), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(g_poly.b.p, points, n_points * sizeof(fe), cudaMemcpyHostToDevice, st));
     for (size_t c0 = 0; c0 < n_polys; c0 += per) {
         size_t cols = std::min(per, n_polys - c0);
         for (size_t c = 0; c < cols; ++c) {
-            if (!polys[c0 + c] && len) return fail(H2V_EINVAL, "eval_polynomial: polys[%zu] is NULL", c0 + c);
-            if (len) CU(cudaMemcpyAsync(g_poly.a.as<fe>() + c * stride, polys[c0 + c], len * sizeof(fe), cudaMemcpyHostToDevice, st));
+            if (!polys[c0 + c] && len) return failf(H2V_EINVAL, "eval_polynomial: polys[%zu] is NULL", c0 + c);
+            if (len) H2V_CU(cudaMemcpyAsync(g_poly.a.as<fe>() + c * stride, polys[c0 + c], len * sizeof(fe), cudaMemcpyHostToDevice, st));
         }
         poly_eval_kernel<<<dim3((unsigned)n_points, (unsigned)cols), 256, 0, st>>>(g_poly.a.as<fe>(), stride, (uint32_t)len, g_poly.b.as<fe>(),
                                                                                   (uint32_t)n_points, g_poly.c.as<fe>());
-        LAUNCHED();
-        CU(cudaMemcpyAsync(out + 4 * c0 * n_points, g_poly.c.p, cols * n_points * sizeof(fe), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
+        H2V_LAUNCHED();
+        H2V_CU(cudaMemcpyAsync(out + 4 * c0 * n_points, g_poly.c.p, cols * n_points * sizeof(fe), cudaMemcpyDeviceToHost, st));
+        H2V_CU(cudaStreamSynchronize(st));
     }
     return H2V_OK;
 }
 int h2v_batch_invert(uint64_t *a, size_t n) {
     if (!n) return H2V_OK;
-    if (!a) return fail(H2V_EINVAL, "batch_invert: NULL buffer");
-    if (n >= ((size_t)1 << 31)) return fail(H2V_EINVAL, "batch_invert: n too large");
+    if (!a) return failf(H2V_EINVAL, "batch_invert: NULL buffer");
+    if (n >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "batch_invert: n too large");
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
@@ -1663,15 +1645,15 @@ int h2v_batch_invert(uint64_t *a, size_t n) {
     if ((rc = poly_ctx_ready())) return rc;
     cudaStream_t st = g_poly.st;
     if ((rc = g_poly.a.ensure(n * sizeof(fe))) || (rc = g_poly.b.ensure(n * sizeof(fe))) || (rc = g_poly.c.ensure(n * sizeof(fe)))) return rc;
-    CU(cudaMemcpyAsync(g_poly.a.p, a, n * sizeof(fe), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(g_poly.a.p, a, n * sizeof(fe), cudaMemcpyHostToDevice, st));
     const unsigned gb = (unsigned)((n + 255) / 256);
     fr_zero_to_one_kernel<<<gb, 256, 0, st>>>(g_poly.a.as<fe>(), g_poly.b.as<fe>(), (uint32_t)n);
-    LAUNCHED();
+    H2V_LAUNCHED();
     if ((rc = run_batch_invert<FrP>(st, g_poly.b.as<fe>(), g_poly.c.as<fe>(), (uint32_t)n, g_poly.tree))) return rc;
     fr_select_inverse_kernel<<<gb, 256, 0, st>>>(g_poly.a.as<fe>(), g_poly.c.as<fe>(), g_poly.b.as<fe>(), (uint32_t)n);
-    LAUNCHED();
-    CU(cudaMemcpyAsync(a, g_poly.b.p, n * sizeof(fe), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    H2V_LAUNCHED();
+    H2V_CU(cudaMemcpyAsync(a, g_poly.b.p, n * sizeof(fe), cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaStreamSynchronize(st));
     return H2V_OK;
 }
 // out[c][0] = 1, out[c][i+1] = out[c][i] * num[c][i] / den[c][i] for `cols` contiguous columns of n elements (device)
@@ -1687,22 +1669,22 @@ static int run_grand_product(cudaStream_t st, const fe *num, const fe *den, uint
     // and does not disturb any other element of the batch.
     const unsigned gt = (unsigned)((tot + 255) / 256);
     fr_zero_to_one_kernel<<<gt, 256, 0, st>>>(den, g_poly.e.as<fe>(), (uint32_t)tot);
-    LAUNCHED();
+    H2V_LAUNCHED();
     if ((rc = run_batch_invert<FrP>(st, g_poly.e.as<fe>(), g_poly.c.as<fe>(), (uint32_t)tot, g_poly.tree))) return rc;
     fr_select_inverse_kernel<<<gt, 256, 0, st>>>(den, g_poly.c.as<fe>(), g_poly.e.as<fe>(), (uint32_t)tot);
-    LAUNCHED();
+    H2V_LAUNCHED();
     fr_prod_tiles_kernel<<<dim3(ntiles, cols), 256, 0, st>>>(num, g_poly.e.as<fe>(), n, g_poly.d.as<fe>());
-    LAUNCHED();
+    H2V_LAUNCHED();
     fr_scan_top_kernel<OpMul><<<dim3(1, cols), 256, 0, st>>>(g_poly.d.as<fe>(), ntiles);
-    LAUNCHED();
+    H2V_LAUNCHED();
     fr_prod_apply_kernel<<<dim3(ntiles, cols), 256, 0, st>>>(num, g_poly.e.as<fe>(), n, g_poly.d.as<fe>(), out);
-    LAUNCHED();
+    H2V_LAUNCHED();
     return H2V_OK;
 }
 int h2v_grand_product(const uint64_t *num, const uint64_t *den, size_t n, uint64_t *out) {
     if (!n) return H2V_OK;
-    if (!num || !den || !out) return fail(H2V_EINVAL, "grand_product: NULL buffer");
-    if (n >= ((size_t)1 << 31)) return fail(H2V_EINVAL, "grand_product: n too large");
+    if (!num || !den || !out) return failf(H2V_EINVAL, "grand_product: NULL buffer");
+    if (n >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "grand_product: n too large");
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
@@ -1710,35 +1692,26 @@ int h2v_grand_product(const uint64_t *num, const uint64_t *den, size_t n, uint64
     if ((rc = poly_ctx_ready())) return rc;
     cudaStream_t st = g_poly.st;
     if ((rc = g_poly.a.ensure(n * sizeof(fe))) || (rc = g_poly.b.ensure(n * sizeof(fe)))) return rc;
-    CU(cudaMemcpyAsync(g_poly.a.p, num, n * sizeof(fe), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(g_poly.b.p, den, n * sizeof(fe), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(g_poly.a.p, num, n * sizeof(fe), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(g_poly.b.p, den, n * sizeof(fe), cudaMemcpyHostToDevice, st));
     // the running product overwrites the staged denominators once their inverses exist
     if ((rc = run_grand_product(st, g_poly.a.as<fe>(), g_poly.b.as<fe>(), (uint32_t)n, 1, g_poly.b.as<fe>()))) {
         cudaStreamSynchronize(st);
         return rc;
     }
-    CU(cudaMemcpyAsync(out, g_poly.b.p, n * sizeof(fe), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    H2V_CU(cudaMemcpyAsync(out, g_poly.b.p, n * sizeof(fe), cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaStreamSynchronize(st));
     return H2V_OK;
 }
 int h2v_grand_product_dev(const void *d_num, const void *d_den, size_t n, size_t n_cols, void *d_out) {
     if (!n || !n_cols) return H2V_OK;
-    if (!d_num || !d_den || !d_out) return fail(H2V_EINVAL, "grand_product: NULL buffer");
-    if (n_cols > 65535 || n * n_cols >= ((size_t)1 << 31)) return fail(H2V_EINVAL, "grand_product: batch too large");
+    if (!d_num || !d_den || !d_out) return failf(H2V_EINVAL, "grand_product: NULL buffer");
+    if (n_cols > 65535 || n * n_cols >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "grand_product: batch too large");
     t_dev = device_of(d_num);
-    int rc = use_device();
-    if (rc) return rc;
-    std::lock_guard<std::mutex> lk(g_poly.mu);
-    if ((rc = poly_ctx_ready())) return rc;
-    Timer tm(g_poly.st);
-    tm.begin(7);
-    rc = run_grand_product(g_poly.st, (const fe *)d_num, (const fe *)d_den, (uint32_t)n, (uint32_t)n_cols, (fe *)d_out);
-    tm.end();
-    cudaError_t e = cudaStreamSynchronize(g_poly.st);
-    tm.collect(true);
-    if (rc) return rc;
-    if (e != cudaSuccess) return fail(H2V_ECUDA, "grand_product: %s", cudaGetErrorString(e));
-    return H2V_OK;
+    H2V_TRY(use_device());
+    return sync_call(g_poly.mu, g_poly.st, 7, "grand_product", [&](Timer &) {
+        return run_grand_product(g_poly.st, (const fe *)d_num, (const fe *)d_den, (uint32_t)n, (uint32_t)n_cols, (fe *)d_out);
+    });
 }
 // a, q device-resident (q: n - 1 coefficients, must not overlap a); g_poly.mu held by the caller
 static int run_kate_division(cudaStream_t st, const fe *a, uint32_t n, const fe &b, fe *q) {
@@ -1753,22 +1726,22 @@ static int run_kate_division(cudaStream_t st, const fe *a, uint32_t n, const fe 
     kp.tile = g_poly.d.as<fe>();
     if (fe_is_zero(kp.b)) {
         kate_shift_kernel<<<(n + 255) / 256, 256, 0, st>>>(kp.a, kp.q, kp.n);
-        LAUNCHED();
+        H2V_LAUNCHED();
     } else {
         kp.binv = fe_inv<Fr>(kp.b);      // one host-side inversion of the evaluation point
         kate_tiles_kernel<<<ntiles, 256, 0, st>>>(kp);
-        LAUNCHED();
+        H2V_LAUNCHED();
         fr_scan_top_kernel<OpAdd><<<1, 256, 0, st>>>(kp.tile, ntiles);
-        LAUNCHED();
+        H2V_LAUNCHED();
         kate_apply_kernel<<<ntiles, 256, 0, st>>>(kp);
-        LAUNCHED();
+        H2V_LAUNCHED();
     }
     return H2V_OK;
 }
 int h2v_kate_division_dev(const void *d_a, size_t n, const uint64_t b[4], void *d_out) {
     if (n <= 1) return H2V_OK;
-    if (!d_a || !b || !d_out) return fail(H2V_EINVAL, "kate_division: NULL buffer");
-    if (n >= ((size_t)1 << 31)) return fail(H2V_EINVAL, "kate_division: n too large");
+    if (!d_a || !b || !d_out) return failf(H2V_EINVAL, "kate_division: NULL buffer");
+    if (n >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "kate_division: n too large");
     t_dev = device_of(d_a);
     int rc = use_device();
     if (rc) return rc;
@@ -1777,13 +1750,13 @@ int h2v_kate_division_dev(const void *d_a, size_t n, const uint64_t b[4], void *
     rc = run_kate_division(g_poly.st, (const fe *)d_a, (uint32_t)n, fe_from_u64x4(b), (fe *)d_out);
     cudaError_t e = cudaStreamSynchronize(g_poly.st);
     if (rc) return rc;
-    if (e != cudaSuccess) return fail(H2V_ECUDA, "kate_division: %s", cudaGetErrorString(e));
+    if (e != cudaSuccess) return failf(H2V_ECUDA, "kate_division: %s", cudaGetErrorString(e));
     return H2V_OK;
 }
 int h2v_kate_division(const uint64_t *a, size_t n, const uint64_t b[4], uint64_t *out) {
     if (n <= 1) return H2V_OK;
-    if (!a || !b || !out) return fail(H2V_EINVAL, "kate_division: NULL buffer");
-    if (n >= ((size_t)1 << 31)) return fail(H2V_EINVAL, "kate_division: n too large");
+    if (!a || !b || !out) return failf(H2V_EINVAL, "kate_division: NULL buffer");
+    if (n >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "kate_division: n too large");
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
@@ -1791,13 +1764,13 @@ int h2v_kate_division(const uint64_t *a, size_t n, const uint64_t b[4], uint64_t
     if ((rc = poly_ctx_ready())) return rc;
     cudaStream_t st = g_poly.st;
     if ((rc = g_poly.a.ensure(n * sizeof(fe))) || (rc = g_poly.b.ensure(n * sizeof(fe)))) return rc;
-    CU(cudaMemcpyAsync(g_poly.a.p, a, n * sizeof(fe), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(g_poly.a.p, a, n * sizeof(fe), cudaMemcpyHostToDevice, st));
     if ((rc = run_kate_division(st, g_poly.a.as<fe>(), (uint32_t)n, fe_from_u64x4(b), g_poly.b.as<fe>()))) {
         cudaStreamSynchronize(st);
         return rc;
     }
-    CU(cudaMemcpyAsync(out, g_poly.b.p, (n - 1) * sizeof(fe), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    H2V_CU(cudaMemcpyAsync(out, g_poly.b.p, (n - 1) * sizeof(fe), cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaStreamSynchronize(st));
     return H2V_OK;
 }
 }  // extern "C"
@@ -1823,7 +1796,7 @@ int run_permute_batch(cudaStream_t st, const fe *const *inputs, const fe *const 
     }
     const uint32_t slices = (uint32_t)srcs.size();
     const size_t rows = (size_t)L * u;
-    if (rows >= ((size_t)1 << 31)) return fail(H2V_EINVAL, "permute_expression_pair: batch too large");
+    if (rows >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "permute_expression_pair: batch too large");
     const uint32_t ntiles = (uint32_t)((rows + H2V_SCAN_TILE - 1) / H2V_SCAN_TILE);
     const size_t ptr_words = ((size_t)slices * sizeof(void *) + 3) / 4;
     if ((rc = g_poly.a.ensure((size_t)slices * n_pad * sizeof(fe))) ||
@@ -1837,51 +1810,51 @@ int run_permute_batch(cudaStream_t st, const fe *const *inputs, const fe *const 
     uintptr_t pa = reinterpret_cast<uintptr_t>(d_tmap + L);
     pa = (pa + 7) & ~(uintptr_t)7;
     const fe **d_srcs = reinterpret_cast<const fe **>(pa);
-    CU(cudaMemsetAsync(err, 0, sizeof(int), st));
-    CU(cudaMemcpyAsync(d_tmap, tmap.data(), L * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_srcs, srcs.data(), slices * sizeof(void *), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemsetAsync(err, 0, sizeof(int), st));
+    H2V_CU(cudaMemcpyAsync(d_tmap, tmap.data(), L * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(d_srcs, srcs.data(), slices * sizeof(void *), cudaMemcpyHostToDevice, st));
     const unsigned gp = (n_pad + 255) / 256, gu = (u + 255) / 256;
     {
         lookup_canon_pad_batch_kernel<<<dim3(gp, slices), 256, 0, st>>>(d_srcs, keys, u, n_pad);
-        LAUNCHED();
+        H2V_LAUNCHED();
         const uint32_t tile = std::min<uint32_t>(H2V_SORT_TILE, n_pad);
         const unsigned tiles_n = n_pad / tile;
         const size_t smem = (size_t)tile * sizeof(fe);
         bitonic_tile_kernel<<<dim3(tiles_n, slices), H2V_SORT_TILE / 2, smem, st>>>(keys, n_pad, 0, 1);
-        LAUNCHED();
+        H2V_LAUNCHED();
         for (uint32_t k = 2 * tile; k <= n_pad && k; k <<= 1) {
             for (uint32_t j = k >> 1; j >= tile; j >>= 1) {
                 bitonic_global_kernel<<<dim3((n_pad / 2 + 255) / 256, slices), 256, 0, st>>>(keys, n_pad, k, j);
-                LAUNCHED();
+                H2V_LAUNCHED();
             }
             bitonic_tile_kernel<<<dim3(tiles_n, slices), H2V_SORT_TILE / 2, smem, st>>>(keys, n_pad, k, 0);
-            LAUNCHED();
+            H2V_LAUNCHED();
         }
     }
     lookup_fill_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(free_, 1u, (uint32_t)rows);
-    LAUNCHED();
+    H2V_LAUNCHED();
     lookup_flags_batch_kernel<<<dim3(gu, L), 256, 0, st>>>(keys, d_tmap, u, n_pad, rep, free_, err);
-    LAUNCHED();
+    H2V_LAUNCHED();
     for (int which = 0; which < 2; ++which) {
         const uint32_t *cnt = which ? free_ : rep;
         uint32_t *offs = which ? free_offs : rep_offs, *tl = tiles + which * ntiles;
         msm_scan_tiles_kernel<<<ntiles, 256, 0, st>>>(cnt, tl, (uint32_t)rows);
-        LAUNCHED();
+        H2V_LAUNCHED();
         msm_scan_top_kernel<<<1, 256, 0, st>>>(tl, ntiles, totals + which);
-        LAUNCHED();
+        H2V_LAUNCHED();
         msm_scan_apply_kernel<<<ntiles, 256, 0, st>>>(cnt, tl, offs, scratch, (uint32_t)rows);
-        LAUNCHED();
+        H2V_LAUNCHED();
     }
     lookup_emit_input_batch_kernel<<<dim3(gu, L), 256, 0, st>>>(keys, u, n_pad, rep, rep_offs, rep_rows, d_out_a, a_stride, d_out_s, s_stride);
-    LAUNCHED();
+    H2V_LAUNCHED();
     lookup_emit_table_batch_kernel<<<dim3(gu, L), 256, 0, st>>>(keys, d_tmap, L, u, n_pad, free_, free_offs, rep_offs, totals, rep_rows, d_out_s,
                                                                  s_stride, err);
-    LAUNCHED();
+    H2V_LAUNCHED();
     int herr = 0;
-    CU(cudaMemcpyAsync(&herr, err, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    if (herr == 1) return fail(H2V_EINVAL, "permute_expression_pair: an input value is not in the table (ConstraintSystemFailure)");
-    if (herr) return fail(H2V_ECUDA, "permute_expression_pair: leftover count mismatch");
+    H2V_CU(cudaMemcpyAsync(&herr, err, sizeof(int), cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaStreamSynchronize(st));
+    if (herr == 1) return failf(H2V_EINVAL, "permute_expression_pair: an input value is not in the table (ConstraintSystemFailure)");
+    if (herr) return failf(H2V_ECUDA, "permute_expression_pair: leftover count mismatch");
     return H2V_OK;
 }
 int run_permute_pair(cudaStream_t st, const fe *d_in_a, const fe *d_in_t, uint32_t u, fe *d_out_a, fe *d_out_s) {
@@ -1893,50 +1866,36 @@ extern "C" {
 int h2v_permute_expression_pair_dev(const void *d_input, const void *d_table, size_t usable_rows, void *d_permuted_input,
                                     void *d_permuted_table) {
     if (!usable_rows) return H2V_OK;
-    if (!d_input || !d_table || !d_permuted_input || !d_permuted_table) return fail(H2V_EINVAL, "permute_expression_pair: NULL buffer");
-    if (usable_rows > ((size_t)1 << 28)) return fail(H2V_EINVAL, "permute_expression_pair: too many rows");
+    if (!d_input || !d_table || !d_permuted_input || !d_permuted_table) return failf(H2V_EINVAL, "permute_expression_pair: NULL buffer");
+    if (usable_rows > ((size_t)1 << 28)) return failf(H2V_EINVAL, "permute_expression_pair: too many rows");
     t_dev = device_of(d_input);
-    int rc = use_device();
-    if (rc) return rc;
-    std::lock_guard<std::mutex> lk(g_poly.mu);
-    if ((rc = poly_ctx_ready())) return rc;
-    Timer tm(g_poly.st);
-    tm.begin(7);
-    rc = run_permute_pair(g_poly.st, (const fe *)d_input, (const fe *)d_table, (uint32_t)usable_rows, (fe *)d_permuted_input,
-                          (fe *)d_permuted_table);
-    tm.end();
-    cudaStreamSynchronize(g_poly.st);
-    tm.collect(true);
-    return rc;
+    H2V_TRY(use_device());
+    return sync_call(g_poly.mu, g_poly.st, 7, "permute_expression_pair", [&](Timer &) {
+        return run_permute_pair(g_poly.st, (const fe *)d_input, (const fe *)d_table, (uint32_t)usable_rows, (fe *)d_permuted_input,
+                                (fe *)d_permuted_table);
+    });
 }
 int h2v_permute_expression_pair_batch_dev(const void *const *d_inputs, const void *const *d_tables, size_t n_lookups, size_t usable_rows,
                                           void *d_permuted_inputs, size_t input_stride, void *d_permuted_tables, size_t table_stride) {
     if (!usable_rows || !n_lookups) return H2V_OK;
-    if (!d_inputs || !d_tables || !d_permuted_inputs || !d_permuted_tables) return fail(H2V_EINVAL, "permute_expression_pair: NULL buffer");
-    if (usable_rows > ((size_t)1 << 28) || n_lookups > 65535) return fail(H2V_EINVAL, "permute_expression_pair: too many rows / lookups");
+    if (!d_inputs || !d_tables || !d_permuted_inputs || !d_permuted_tables) return failf(H2V_EINVAL, "permute_expression_pair: NULL buffer");
+    if (usable_rows > ((size_t)1 << 28) || n_lookups > 65535) return failf(H2V_EINVAL, "permute_expression_pair: too many rows / lookups");
     if (n_lookups > 1 && (input_stride < usable_rows || table_stride < usable_rows))
-        return fail(H2V_EINVAL, "permute_expression_pair: output stride shorter than the usable rows");
+        return failf(H2V_EINVAL, "permute_expression_pair: output stride shorter than the usable rows");
     for (size_t l = 0; l < n_lookups; ++l)
-        if (!d_inputs[l] || !d_tables[l]) return fail(H2V_EINVAL, "permute_expression_pair: lookup %zu has a NULL column", l);
+        if (!d_inputs[l] || !d_tables[l]) return failf(H2V_EINVAL, "permute_expression_pair: lookup %zu has a NULL column", l);
     t_dev = device_of(d_inputs[0]);
-    int rc = use_device();
-    if (rc) return rc;
-    std::lock_guard<std::mutex> lk(g_poly.mu);
-    if ((rc = poly_ctx_ready())) return rc;
-    Timer tm(g_poly.st);
-    tm.begin(7);
-    rc = run_permute_batch(g_poly.st, (const fe *const *)d_inputs, (const fe *const *)d_tables, (uint32_t)n_lookups, (uint32_t)usable_rows,
-                           (fe *)d_permuted_inputs, input_stride, (fe *)d_permuted_tables, table_stride);
-    tm.end();
-    cudaStreamSynchronize(g_poly.st);
-    tm.collect(true);
-    return rc;
+    H2V_TRY(use_device());
+    return sync_call(g_poly.mu, g_poly.st, 7, "permute_expression_pair", [&](Timer &) {
+        return run_permute_batch(g_poly.st, (const fe *const *)d_inputs, (const fe *const *)d_tables, (uint32_t)n_lookups, (uint32_t)usable_rows,
+                                 (fe *)d_permuted_inputs, input_stride, (fe *)d_permuted_tables, table_stride);
+    });
 }
 int h2v_permute_expression_pair(const uint64_t *input, const uint64_t *table, size_t usable_rows, uint64_t *permuted_input,
                                 uint64_t *permuted_table) {
     if (!usable_rows) return H2V_OK;
-    if (!input || !table || !permuted_input || !permuted_table) return fail(H2V_EINVAL, "permute_expression_pair: NULL buffer");
-    if (usable_rows > ((size_t)1 << 28)) return fail(H2V_EINVAL, "permute_expression_pair: too many rows");
+    if (!input || !table || !permuted_input || !permuted_table) return failf(H2V_EINVAL, "permute_expression_pair: NULL buffer");
+    if (usable_rows > ((size_t)1 << 28)) return failf(H2V_EINVAL, "permute_expression_pair: too many rows");
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
@@ -1945,88 +1904,79 @@ int h2v_permute_expression_pair(const uint64_t *input, const uint64_t *table, si
     cudaStream_t st = g_poly.st;
     const size_t bytes = usable_rows * sizeof(fe);
     if ((rc = g_poly.c.ensure(bytes)) || (rc = g_poly.d.ensure(bytes))) return rc;
-    CU(cudaMemcpyAsync(g_poly.c.p, input, bytes, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(g_poly.d.p, table, bytes, cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(g_poly.c.p, input, bytes, cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(g_poly.d.p, table, bytes, cudaMemcpyHostToDevice, st));
     // the canonical copies are taken first, so the staging buffers double as the outputs
     if ((rc = run_permute_pair(st, g_poly.c.as<fe>(), g_poly.d.as<fe>(), (uint32_t)usable_rows, g_poly.c.as<fe>(), g_poly.d.as<fe>()))) {
         cudaStreamSynchronize(st);
         return rc;
     }
-    CU(cudaMemcpyAsync(permuted_input, g_poly.c.p, bytes, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(permuted_table, g_poly.d.p, bytes, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
+    H2V_CU(cudaMemcpyAsync(permuted_input, g_poly.c.p, bytes, cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaMemcpyAsync(permuted_table, g_poly.d.p, bytes, cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaStreamSynchronize(st));
     return H2V_OK;
 }
 }  // extern "C"
 
 // ================================================================== quotient evaluation ("next" row 1)
 namespace {
-int quotient_common(DomRep *d, const void *d_h, const uint64_t *y, QuotientCommon *c) {
-    if (!d) return fail(H2V_EINVAL, "quotient: NULL domain");
-    if (!d_h || !y) return fail(H2V_EINVAL, "quotient: NULL buffer");
+// the replica that holds d_h (made current) and the constants every quotient kernel takes
+int quotient_common(h2v_domain_t h, const void *d_h, const uint64_t *y, DomRep **d, QuotientCommon *c) {
+    if (!(*d = dom_rep(h, d_h))) return H2V_EINVAL;
+    if (!d_h || !y) return failf(H2V_EINVAL, "quotient: NULL buffer");
     c->y = fe_from_u64x4(y);
-    c->n_ext = 1u << d->ek;
-    c->rot = 1u << (d->ek - d->k);
+    c->n_ext = 1u << (*d)->ek;
+    c->rot = 1u << ((*d)->ek - (*d)->k);
     return use_device();
 }
-int quotient_finish(DomRep *d, Timer &tm) {
-    tm.end();
-    cudaError_t e = cudaStreamSynchronize(d->stream);
-    tm.collect(true);
-    if (e != cudaSuccess) return fail(H2V_ECUDA, "quotient: %s", cudaGetErrorString(e));
-    return H2V_OK;
+// the gate columns as strided arrays (ColsStrided) or device tables of column pointers (ColsTable)
+template <class Cols> int quotient_gates(h2v_domain_t h, void *d_h, const uint64_t y[4], size_t n_gates, Cols q, Cols a) {
+    DomRep *d;
+    QuotientCommon c;
+    int rc = quotient_common(h, d_h, y, &d, &c);
+    if (rc) return rc;
+    if (!n_gates) return H2V_OK;
+    if constexpr (std::is_same<Cols, ColsStrided>::value) {
+        if (!q.base || !a.base) return failf(H2V_EINVAL, "quotient_gates: NULL buffer");
+        if (q.stride < c.n_ext || a.stride < c.n_ext || n_gates > (1u << 20))
+            return failf(H2V_EINVAL, "quotient_gates: stride shorter than 2^extended_k, or too many gates");
+    } else {
+        if (!q.ptrs || !a.ptrs) return failf(H2V_EINVAL, "quotient_gates: NULL pointer table");
+        if (n_gates > (1u << 20)) return failf(H2V_EINVAL, "quotient_gates: too many gates");
+    }
+    return sync_call(d->mu, d->stream, 7, "quotient", [&](Timer &) {
+        quotient_gates_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, (uint32_t)n_gates, q, a);
+        H2V_LAUNCHED();
+        return H2V_OK;
+    });
 }
 }  // namespace
 
 extern "C" {
-static int rep_quotient_gates_dev(DomRep *d, void *d_h, const uint64_t y[4], size_t n_gates, const void *d_q, size_t q_stride,
-                           const void *d_a, size_t a_stride) {
-    QuotientCommon c;
-    int rc = quotient_common(d, d_h, y, &c);
-    if (rc) return rc;
-    if (!n_gates) return H2V_OK;
-    if (!d_q || !d_a) return fail(H2V_EINVAL, "quotient_gates: NULL buffer");
-    if (q_stride < c.n_ext || a_stride < c.n_ext || n_gates > (1u << 20))
-        return fail(H2V_EINVAL, "quotient_gates: stride shorter than 2^extended_k, or too many gates");
-    std::lock_guard<std::mutex> lk(d->mu);
-    Timer tm(d->stream);
-    tm.begin(7);
-    quotient_gates_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, (uint32_t)n_gates, ColsStrided{(const fe *)d_q, q_stride},
-                                                                        ColsStrided{(const fe *)d_a, a_stride});
-    LAUNCHED();
-    return quotient_finish(d, tm);
+int h2v_quotient_gates_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], size_t n_gates, const void *d_q, size_t q_stride, const void *d_a,
+                           size_t a_stride) {
+    return quotient_gates(h, d_h, y, n_gates, ColsStrided{(const fe *)d_q, q_stride}, ColsStrided{(const fe *)d_a, a_stride});
 }
-static int rep_quotient_gates_ptrs_dev(DomRep *d, void *d_h, const uint64_t y[4], size_t n_gates, const void *const *d_q_ptrs,
+int h2v_quotient_gates_ptrs_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], size_t n_gates, const void *const *d_q_ptrs,
                                 const void *const *d_a_ptrs) {
-    QuotientCommon c;
-    int rc = quotient_common(d, d_h, y, &c);
-    if (rc) return rc;
-    if (!n_gates) return H2V_OK;
-    if (!d_q_ptrs || !d_a_ptrs) return fail(H2V_EINVAL, "quotient_gates: NULL pointer table");
-    if (n_gates > (1u << 20)) return fail(H2V_EINVAL, "quotient_gates: too many gates");
-    std::lock_guard<std::mutex> lk(d->mu);
-    Timer tm(d->stream);
-    tm.begin(7);
-    quotient_gates_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, (uint32_t)n_gates, ColsTable{(const fe *const *)d_q_ptrs},
-                                                                        ColsTable{(const fe *const *)d_a_ptrs});
-    LAUNCHED();
-    return quotient_finish(d, tm);
+    return quotient_gates(h, d_h, y, n_gates, ColsTable{(const fe *const *)d_q_ptrs}, ColsTable{(const fe *const *)d_a_ptrs});
 }
-static int quotient_permutation_any(DomRep *d, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
+static int quotient_permutation_any(h2v_domain_t h, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
                                     size_t n_cols, size_t chunk_len, const void *d_cols, size_t cols_stride, const void *d_sigma,
                                     size_t sigma_stride, const void *d_z, size_t z_stride, const void *d_l0, const void *d_l_last,
                                     const void *d_l_active, uint32_t blinding_factors, bool tables, size_t set_begin = 0,
                                     size_t set_end = (size_t)-1, int with_head = 1) {
+    DomRep *d;
     QuotientCommon c;
-    int rc = quotient_common(d, d_h, y, &c);
+    int rc = quotient_common(h, d_h, y, &d, &c);
     if (rc) return rc;
     if (!n_cols) return H2V_OK;   // upstream: `if !sets.is_empty()`
     if (!beta || !gamma || !d_cols || !d_sigma || !d_z || !d_l0 || !d_l_last || !d_l_active)
-        return fail(H2V_EINVAL, "quotient_permutation: NULL buffer");
+        return failf(H2V_EINVAL, "quotient_permutation: NULL buffer");
     if (!chunk_len || n_cols > (1u << 20) || blinding_factors + 1 >= (1u << d->k))
-        return fail(H2V_EINVAL, "quotient_permutation: chunk_len = 0, too many columns, or blinding_factors >= n - 1");
+        return failf(H2V_EINVAL, "quotient_permutation: chunk_len = 0, too many columns, or blinding_factors >= n - 1");
     if ((!tables && (cols_stride < c.n_ext || sigma_stride < c.n_ext)) || z_stride < c.n_ext)
-        return fail(H2V_EINVAL, "quotient_permutation: stride shorter than 2^extended_k");
+        return failf(H2V_EINVAL, "quotient_permutation: stride shorter than 2^extended_k");
     QuotientPerm p;
     p.beta = fe_from_u64x4(beta);
     p.gamma = fe_from_u64x4(gamma);
@@ -2040,53 +1990,53 @@ static int quotient_permutation_any(DomRep *d, void *d_h, const uint64_t y[4], c
     p.z_stride = z_stride;
     p.l0 = (const fe *)d_l0; p.l_last = (const fe *)d_l_last; p.l_active = (const fe *)d_l_active;
     if (set_end == (size_t)-1) set_end = p.n_sets;
-    if (set_begin > set_end || set_end > p.n_sets) return fail(H2V_EINVAL, "quotient_permutation: set range [%zu, %zu) of %u sets", set_begin, set_end, p.n_sets);
+    if (set_begin > set_end || set_end > p.n_sets) return failf(H2V_EINVAL, "quotient_permutation: set range [%zu, %zu) of %u sets", set_begin, set_end, p.n_sets);
     p.set_begin = (uint32_t)set_begin;
     p.set_end = (uint32_t)set_end;
     p.head = with_head ? 1u : 0u;
     p.delta_begin = fe_pow_u64<Fr>(p.delta, (uint64_t)set_begin * p.chunk_len);
     if ((rc = domain_twiddles(d, 2, &p.tw))) return rc;
-    std::lock_guard<std::mutex> lk(d->mu);
-    Timer tm(d->stream);
-    tm.begin(7);
-    if (tables)
-        quotient_permutation_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, p, ColsTable{(const fe *const *)d_cols},
-                                                                                  ColsTable{(const fe *const *)d_sigma});
-    else
-        quotient_permutation_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, p, ColsStrided{(const fe *)d_cols, cols_stride},
-                                                                                  ColsStrided{(const fe *)d_sigma, sigma_stride});
-    LAUNCHED();
-    return quotient_finish(d, tm);
+    return sync_call(d->mu, d->stream, 7, "quotient", [&](Timer &) {
+        if (tables)
+            quotient_permutation_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, p, ColsTable{(const fe *const *)d_cols},
+                                                                                      ColsTable{(const fe *const *)d_sigma});
+        else
+            quotient_permutation_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, p, ColsStrided{(const fe *)d_cols, cols_stride},
+                                                                                      ColsStrided{(const fe *)d_sigma, sigma_stride});
+        H2V_LAUNCHED();
+        return H2V_OK;
+    });
 }
-static int rep_quotient_permutation_dev(DomRep *d, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
+int h2v_quotient_permutation_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
                                  size_t n_cols, size_t chunk_len, const void *d_cols, size_t cols_stride, const void *d_sigma,
                                  size_t sigma_stride, const void *d_z, size_t z_stride, const void *d_l0, const void *d_l_last,
                                  const void *d_l_active, uint32_t blinding_factors) {
-    return quotient_permutation_any(d, d_h, y, beta, gamma, n_cols, chunk_len, d_cols, cols_stride, d_sigma, sigma_stride, d_z, z_stride,
+    return quotient_permutation_any(h, d_h, y, beta, gamma, n_cols, chunk_len, d_cols, cols_stride, d_sigma, sigma_stride, d_z, z_stride,
                                     d_l0, d_l_last, d_l_active, blinding_factors, false);
 }
-static int rep_quotient_permutation_ptrs_dev(DomRep *d, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
+int h2v_quotient_permutation_ptrs_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
                                       size_t n_cols, size_t chunk_len, const void *const *d_col_ptrs, const void *const *d_sigma_ptrs,
                                       const void *d_z, size_t z_stride, const void *d_l0, const void *d_l_last, const void *d_l_active,
                                       uint32_t blinding_factors) {
-    return quotient_permutation_any(d, d_h, y, beta, gamma, n_cols, chunk_len, d_col_ptrs, 0, d_sigma_ptrs, 0, d_z, z_stride, d_l0, d_l_last,
+    return quotient_permutation_any(h, d_h, y, beta, gamma, n_cols, chunk_len, d_col_ptrs, 0, d_sigma_ptrs, 0, d_z, z_stride, d_l0, d_l_last,
                                     d_l_active, blinding_factors, true);
 }
-static int rep_quotient_permutation_range_ptrs_dev(DomRep *d, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
+int h2v_quotient_permutation_range_ptrs_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
                                             size_t n_cols, size_t chunk_len, size_t set_begin, size_t set_end, int with_head,
                                             const void *const *d_col_ptrs, const void *const *d_sigma_ptrs, const void *d_z, size_t z_stride,
                                             const void *d_l0, const void *d_l_last, const void *d_l_active, uint32_t blinding_factors) {
-    return quotient_permutation_any(d, d_h, y, beta, gamma, n_cols, chunk_len, d_col_ptrs, 0, d_sigma_ptrs, 0, d_z, z_stride, d_l0, d_l_last,
+    return quotient_permutation_any(h, d_h, y, beta, gamma, n_cols, chunk_len, d_col_ptrs, 0, d_sigma_ptrs, 0, d_z, z_stride, d_l0, d_l_last,
                                     d_l_active, blinding_factors, true, set_begin, set_end, with_head);
 }
-static int rep_quotient_lookup_dev(DomRep *d, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
-                            const void *d_input, const void *d_table, const void *d_perm_input, const void *d_perm_table,
-                            const void *d_z, const void *d_l0, const void *d_l_last, const void *d_l_active) {
+int h2v_quotient_lookup_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
+                            const void *d_input, const void *d_table, const void *d_perm_input, const void *d_perm_table, const void *d_z,
+                            const void *d_l0, const void *d_l_last, const void *d_l_active) {
+    DomRep *d;
     QuotientCommon c;
-    int rc = quotient_common(d, d_h, y, &c);
+    int rc = quotient_common(h, d_h, y, &d, &c);
     if (rc) return rc;
     if (!beta || !gamma || !d_input || !d_table || !d_perm_input || !d_perm_table || !d_z || !d_l0 || !d_l_last || !d_l_active)
-        return fail(H2V_EINVAL, "quotient_lookup: NULL buffer");
+        return failf(H2V_EINVAL, "quotient_lookup: NULL buffer");
     QuotientLookup p;
     p.beta = fe_from_u64x4(beta);
     p.gamma = fe_from_u64x4(gamma);
@@ -2094,12 +2044,11 @@ static int rep_quotient_lookup_dev(DomRep *d, void *d_h, const uint64_t y[4], co
     p.perm_input = (const fe *)d_perm_input; p.perm_table = (const fe *)d_perm_table;
     p.z = (const fe *)d_z;
     p.l0 = (const fe *)d_l0; p.l_last = (const fe *)d_l_last; p.l_active = (const fe *)d_l_active;
-    std::lock_guard<std::mutex> lk(d->mu);
-    Timer tm(d->stream);
-    tm.begin(7);
-    quotient_lookup_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, p);
-    LAUNCHED();
-    return quotient_finish(d, tm);
+    return sync_call(d->mu, d->stream, 7, "quotient", [&](Timer &) {
+        quotient_lookup_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, p);
+        H2V_LAUNCHED();
+        return H2V_OK;
+    });
 }
 }  // extern "C"
 
@@ -2254,17 +2203,17 @@ int h2v_selftest_field(int field, int op, const uint64_t *a, const uint64_t *b, 
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
-    if (!a || !out || n == 0) return fail(H2V_EINVAL, "selftest_field: bad argument");
+    if (!a || !out || n == 0) return failf(H2V_EINVAL, "selftest_field: bad argument");
     DevBuf A, B, O;
     if ((rc = A.ensure(n * 32)) || (rc = B.ensure(n * 32)) || (rc = O.ensure(n * 32))) return rc;
-    CU(cudaMemcpy(A.p, a, n * 32, cudaMemcpyHostToDevice));
-    if (b) CU(cudaMemcpy(B.p, b, n * 32, cudaMemcpyHostToDevice));
+    H2V_CU(cudaMemcpy(A.p, a, n * 32, cudaMemcpyHostToDevice));
+    if (b) H2V_CU(cudaMemcpy(B.p, b, n * 32, cudaMemcpyHostToDevice));
     unsigned g = (unsigned)((n + 127) / 128);
     if (field == 0) selftest_field_kernel<FrP><<<g, 128>>>(op, A.as<fe>(), b ? B.as<fe>() : nullptr, O.as<fe>(), n);
     else selftest_field_kernel<FqP><<<g, 128>>>(op, A.as<fe>(), b ? B.as<fe>() : nullptr, O.as<fe>(), n);
-    LAUNCHED();
-    CU(cudaDeviceSynchronize());
-    CU(cudaMemcpy(out, O.p, n * 32, cudaMemcpyDeviceToHost));
+    H2V_LAUNCHED();
+    H2V_CU(cudaDeviceSynchronize());
+    H2V_CU(cudaMemcpy(out, O.p, n * 32, cudaMemcpyDeviceToHost));
     A.release(); B.release(); O.release();
     return H2V_OK;
 }
@@ -2272,15 +2221,15 @@ int h2v_selftest_group(int mode, const uint64_t *p, const uint64_t *q, size_t n,
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
-    if (!p || !q || !out_affine || n == 0) return fail(H2V_EINVAL, "selftest_group: bad argument");
+    if (!p || !q || !out_affine || n == 0) return failf(H2V_EINVAL, "selftest_group: bad argument");
     DevBuf A, B, O;
     if ((rc = A.ensure(n * 64)) || (rc = B.ensure(n * 64)) || (rc = O.ensure(n * 64))) return rc;
-    CU(cudaMemcpy(A.p, p, n * 64, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(B.p, q, n * 64, cudaMemcpyHostToDevice));
+    H2V_CU(cudaMemcpy(A.p, p, n * 64, cudaMemcpyHostToDevice));
+    H2V_CU(cudaMemcpy(B.p, q, n * 64, cudaMemcpyHostToDevice));
     selftest_group_kernel<<<(unsigned)((n + 63) / 64), 64>>>(mode, A.as<affine>(), B.as<affine>(), O.as<affine>(), n);
-    LAUNCHED();
-    CU(cudaDeviceSynchronize());
-    CU(cudaMemcpy(out_affine, O.p, n * 64, cudaMemcpyDeviceToHost));
+    H2V_LAUNCHED();
+    H2V_CU(cudaDeviceSynchronize());
+    H2V_CU(cudaMemcpy(out_affine, O.p, n * 64, cudaMemcpyDeviceToHost));
     A.release(); B.release(); O.release();
     return H2V_OK;
 }
@@ -2288,8 +2237,8 @@ int h2v_srs_setup(uint32_t k, const uint64_t s_mont[4], uint64_t *g_out, uint64_
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
-    if (!s_mont || (!g_out && !g_lagrange_out)) return fail(H2V_EINVAL, "srs_setup: NULL argument");
-    if (k > 26) return fail(H2V_EINVAL, "srs_setup: k = %u unsupported", k);
+    if (!s_mont || (!g_out && !g_lagrange_out)) return failf(H2V_EINVAL, "srs_setup: NULL argument");
+    if (k > 26) return failf(H2V_EINVAL, "srs_setup: k = %u unsupported", k);
     const size_t n = (size_t)1 << k;
     SetupParams sp;
     sp.s = fe_from_u64x4(s_mont);
@@ -2301,16 +2250,16 @@ int h2v_srs_setup(uint32_t k, const uint64_t s_mont[4], uint64_t *g_out, uint64_
     fe sn = sp.s;
     for (uint32_t i = 0; i < k; ++i) sn = fe_sqr<Fr>(sn);                       // s^(2^k)
     sp.mult = fe_mul<Fr>(fe_sub<Fr>(sn, fe_one<Fr>()), fe_inv<Fr>(fr_from_small((uint64_t)n)));
-    if (fe_is_zero(fe_sub<Fr>(sn, fe_one<Fr>()))) return fail(H2V_EINVAL, "srs_setup: s is a 2^k-th root of unity");
+    if (fe_is_zero(fe_sub<Fr>(sn, fe_one<Fr>()))) return failf(H2V_EINVAL, "srs_setup: s is a 2^k-th root of unity");
     DevBuf O;
     if ((rc = O.ensure(n * sizeof(affine)))) return rc;
     uint64_t *dst[2] = {g_out, g_lagrange_out};
     for (int b = 0; b < 2; ++b) {
         if (!dst[b]) continue;
         srs_setup_kernel<<<(unsigned)((n + 127) / 128), 128>>>(sp, b, O.as<affine>());
-        LAUNCHED();
-        CU(cudaDeviceSynchronize());
-        CU(cudaMemcpy(dst[b], O.p, n * sizeof(affine), cudaMemcpyDeviceToHost));
+        H2V_LAUNCHED();
+        H2V_CU(cudaDeviceSynchronize());
+        H2V_CU(cudaMemcpy(dst[b], O.p, n * sizeof(affine), cudaMemcpyDeviceToHost));
     }
     O.release();
     return H2V_OK;
@@ -2319,14 +2268,14 @@ int h2v_synthetic_bases(uint64_t a, uint64_t b, size_t n, uint64_t *out_affine) 
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
-    if (!out_affine || n == 0) return fail(H2V_EINVAL, "synthetic_bases: bad argument");
-    if (a >> 62 || b >> 62 || n >> 32) return fail(H2V_EINVAL, "synthetic_bases: a, b < 2^62 and n < 2^32 required");
+    if (!out_affine || n == 0) return failf(H2V_EINVAL, "synthetic_bases: bad argument");
+    if (a >> 62 || b >> 62 || n >> 32) return failf(H2V_EINVAL, "synthetic_bases: a, b < 2^62 and n < 2^32 required");
     DevBuf O;
     if ((rc = O.ensure(n * 64))) return rc;
     synthetic_bases_kernel<<<(unsigned)((n + 127) / 128), 128>>>(O.as<affine>(), a, b, n);
-    LAUNCHED();
-    CU(cudaDeviceSynchronize());
-    CU(cudaMemcpy(out_affine, O.p, n * 64, cudaMemcpyDeviceToHost));
+    H2V_LAUNCHED();
+    H2V_CU(cudaDeviceSynchronize());
+    H2V_CU(cudaMemcpy(out_affine, O.p, n * 64, cudaMemcpyDeviceToHost));
     O.release();
     return H2V_OK;
 }
@@ -2336,18 +2285,18 @@ int h2v_selftest_op_rate(int which, double *out) {
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
-    if (!out || which < 0 || which > 2) return fail(H2V_EINVAL, "selftest_op_rate: bad argument");
+    if (!out || which < 0 || which > 2) return failf(H2V_EINVAL, "selftest_op_rate: bad argument");
     DevBuf O;
     if ((rc = O.ensure(256))) return rc;
     cudaDeviceProp prop;
-    CU(cudaGetDeviceProperties(&prop, cur_dev()));
+    H2V_CU(cudaGetDeviceProperties(&prop, cur_dev()));
     cudaEvent_t e0, e1;
-    CU(cudaEventCreate(&e0));
-    CU(cudaEventCreate(&e1));
+    H2V_CU(cudaEventCreate(&e0));
+    H2V_CU(cudaEventCreate(&e1));
     double best = 0;
     for (int rep = 0; rep < 4; ++rep) {
         double ops;
-        CU(cudaEventRecord(e0));
+        H2V_CU(cudaEventRecord(e0));
         if (which == 0) {
             unsigned blocks = prop.multiProcessorCount * 8, iters = 4096;
             mul_probe_kernel<1><<<blocks, 256>>>(O.as<fe>(), iters);
@@ -2361,11 +2310,11 @@ int h2v_selftest_op_rate(int which, double *out) {
             madd_probe_kernel<<<blocks, 128>>>(O.as<xyzz>(), iters);
             ops = (double)blocks * 128 * iters;
         }
-        LAUNCHED();
-        CU(cudaEventRecord(e1));
-        CU(cudaEventSynchronize(e1));
+        H2V_LAUNCHED();
+        H2V_CU(cudaEventRecord(e1));
+        H2V_CU(cudaEventSynchronize(e1));
         float ms = 0;
-        CU(cudaEventElapsedTime(&ms, e0, e1));
+        H2V_CU(cudaEventElapsedTime(&ms, e0, e1));
         if (rep > 0) best = std::max(best, ops / (ms * 1e-3));
     }
     cudaEventDestroy(e0);
@@ -2380,26 +2329,26 @@ int h2v_selftest_imad_probe(int which, double *out) {
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
-    if (!out || which < 0 || which > 1) return fail(H2V_EINVAL, "selftest_imad_probe: bad argument");
+    if (!out || which < 0 || which > 1) return failf(H2V_EINVAL, "selftest_imad_probe: bad argument");
     if (which == 0) return h2v_selftest_imad_peak(out);
     DevBuf O;
     if ((rc = O.ensure(64))) return rc;
     cudaDeviceProp prop;
-    CU(cudaGetDeviceProperties(&prop, cur_dev()));
+    H2V_CU(cudaGetDeviceProperties(&prop, cur_dev()));
     cudaEvent_t e0, e1;
-    CU(cudaEventCreate(&e0));
-    CU(cudaEventCreate(&e1));
+    H2V_CU(cudaEventCreate(&e0));
+    H2V_CU(cudaEventCreate(&e1));
     double best = 0;
     for (int occ = 2; occ <= 8; occ *= 2) {          // resident CTAs per SM: the rate must not depend on it once the pipe is full
         const unsigned blocks = prop.multiProcessorCount * occ, threads = 256, iters = 1 << 12;
         for (int rep = 0; rep < 3; ++rep) {
-            CU(cudaEventRecord(e0));
+            H2V_CU(cudaEventRecord(e0));
             imad_chain_probe_kernel<<<blocks, threads>>>(O.as<uint32_t>(), iters, 777u + rep);
-            LAUNCHED();
-            CU(cudaEventRecord(e1));
-            CU(cudaEventSynchronize(e1));
+            H2V_LAUNCHED();
+            H2V_CU(cudaEventRecord(e1));
+            H2V_CU(cudaEventSynchronize(e1));
             float ms = 0;
-            CU(cudaEventElapsedTime(&ms, e0, e1));
+            H2V_CU(cudaEventElapsedTime(&ms, e0, e1));
             const double rate = (double)blocks * threads * iters * 64.0 / (ms * 1e-3);      // 16 rows x 4 per iteration
             if (rep > 0 && rate > best) best = rate;
         }
@@ -2414,24 +2363,24 @@ int h2v_selftest_imad_peak(double *out) {
     t_dev = -1;
     int rc = use_device();
     if (rc) return rc;
-    if (!out) return fail(H2V_EINVAL, "selftest_imad_peak: NULL");
+    if (!out) return failf(H2V_EINVAL, "selftest_imad_peak: NULL");
     DevBuf O;
     if ((rc = O.ensure(64))) return rc;
     cudaDeviceProp prop;
-    CU(cudaGetDeviceProperties(&prop, cur_dev()));
+    H2V_CU(cudaGetDeviceProperties(&prop, cur_dev()));
     const unsigned blocks = prop.multiProcessorCount * 8, threads = 256, iters = 1 << 14;
     cudaEvent_t e0, e1;
-    CU(cudaEventCreate(&e0));
-    CU(cudaEventCreate(&e1));
+    H2V_CU(cudaEventCreate(&e0));
+    H2V_CU(cudaEventCreate(&e1));
     double best = 0;
     for (int rep = 0; rep < 5; ++rep) {
-        CU(cudaEventRecord(e0));
+        H2V_CU(cudaEventRecord(e0));
         imad_probe_kernel<<<blocks, threads>>>(O.as<uint64_t>(), iters, 12345u + rep);
-        LAUNCHED();
-        CU(cudaEventRecord(e1));
-        CU(cudaEventSynchronize(e1));
+        H2V_LAUNCHED();
+        H2V_CU(cudaEventRecord(e1));
+        H2V_CU(cudaEventSynchronize(e1));
         float ms = 0;
-        CU(cudaEventElapsedTime(&ms, e0, e1));
+        H2V_CU(cudaEventElapsedTime(&ms, e0, e1));
         double rate = (double)blocks * threads * iters * 8.0 / (ms * 1e-3);
         if (rep > 0 && rate > best) best = rate;
     }
@@ -2443,25 +2392,7 @@ int h2v_selftest_imad_peak(double *out) {
 }
 }
 
-// ================================================================== public handles: one replica per device
-struct h2v_srs {
-    std::vector<SrsRep *> rep;
-};
-struct h2v_domain {
-    std::vector<DomRep *> rep;
-};
-
 namespace {
-SrsRep *srs_on(h2v_srs *h, int dev) {
-    for (SrsRep *r : h->rep)
-        if (r->dev == dev) return r;
-    return nullptr;
-}
-DomRep *dom_on(h2v_domain *h, int dev) {
-    for (DomRep *r : h->rep)
-        if (r->dev == dev) return r;
-    return nullptr;
-}
 // a replica of `src` on the calling thread's current device: the window tables cross NVLink / PCIe once (peer copy)
 int rep_srs_clone(const SrsRep *src, SrsRep **out) {
     int rc = use_device();
@@ -2476,7 +2407,7 @@ int rep_srs_clone(const SrsRep *src, SrsRep **out) {
     cudaError_t e = cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking);
     if (e != cudaSuccess) {
         delete s;
-        return fail(H2V_ECUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
+        return failf(H2V_ECUDA, "cudaStreamCreate: %s", cudaGetErrorString(e));
     }
     for (int b = 0; b < 2; ++b) {
         if (!src->have[b]) continue;
@@ -2485,12 +2416,12 @@ int rep_srs_clone(const SrsRep *src, SrsRep **out) {
             rc = s->table[b][v].ensure(bytes);
             if (rc) { rep_srs_free(s); return rc; }
             e = cudaMemcpyPeerAsync(s->table[b][v].p, s->dev, src->table[b][v].p, src->dev, bytes, s->stream);
-            if (e != cudaSuccess) { rep_srs_free(s); return fail(H2V_ECUDA, "SRS replica copy: %s", cudaGetErrorString(e)); }
+            if (e != cudaSuccess) { rep_srs_free(s); return failf(H2V_ECUDA, "SRS replica copy: %s", cudaGetErrorString(e)); }
         }
         s->have[b] = true;
     }
     e = cudaStreamSynchronize(s->stream);
-    if (e != cudaSuccess) { rep_srs_free(s); return fail(H2V_ECUDA, "SRS replica copy: %s", cudaGetErrorString(e)); }
+    if (e != cudaSuccess) { rep_srs_free(s); return failf(H2V_ECUDA, "SRS replica copy: %s", cudaGetErrorString(e)); }
     *out = s;
     return H2V_OK;
 }
@@ -2521,22 +2452,22 @@ extern "C" {
 int h2v_dev_alloc_on(int device, size_t bytes, void **d_out) {
     bool known = false;
     for (int d : g_devs) known = known || d == device;
-    if (!known) return fail(H2V_EINVAL, "dev_alloc_on: device %d is not in the h2v_init list", device);
-    if (!d_out || !bytes) return fail(H2V_EINVAL, "dev_alloc: bad argument");
+    if (!known) return failf(H2V_EINVAL, "dev_alloc_on: device %d is not in the h2v_init list", device);
+    if (!d_out || !bytes) return failf(H2V_EINVAL, "dev_alloc: bad argument");
     t_dev = device;
     int rc = use_device();
     if (rc) return rc;
     cudaError_t e = cudaMalloc(d_out, bytes);
     if (e != cudaSuccess) {
         cudaGetLastError();
-        return fail(H2V_ENOMEM, "cudaMalloc(%zu bytes): %s", bytes, cudaGetErrorString(e));
+        return failf(H2V_ENOMEM, "cudaMalloc(%zu bytes): %s", bytes, cudaGetErrorString(e));
     }
     return H2V_OK;
 }
 
 // ---------------------------------------------------------------- SRS
 int h2v_srs_load(uint32_t k, const uint64_t *g, const uint64_t *g_lagrange, h2v_srs_t *out) {
-    if (!out) return fail(H2V_EINVAL, "h2v_srs_load: out is NULL");
+    if (!out) return failf(H2V_EINVAL, "h2v_srs_load: out is NULL");
     *out = nullptr;
     h2v_srs *h = new h2v_srs();
     for (size_t i = 0; i < g_devs.size(); ++i) {
@@ -2563,14 +2494,10 @@ void h2v_srs_free(h2v_srs_t h) {
     t_dev = -1;
     delete h;
 }
-int h2v_srs_info(h2v_srs_t h, uint32_t *window_bits, uint32_t *windows) {
-    if (!h) return fail(H2V_EINVAL, "srs_info: NULL srs");
-    return rep_srs_info(h->rep[0], window_bits, windows);
-}
 int h2v_commit_batch_dev(h2v_srs_t h, int basis, const void *d_polys, size_t col_stride, size_t n_polys, size_t len, void *d_out_affine) {
-    if (!h) return fail(H2V_EINVAL, "commit: NULL srs");
+    if (!h) return failf(H2V_EINVAL, "commit: NULL srs");
     SrsRep *r = srs_on(h, device_of(d_polys));
-    if (!r) return fail(H2V_EINVAL, "commit: the columns live on device %d, which is not in the h2v_init list", device_of(d_polys));
+    if (!r) return failf(H2V_EINVAL, "commit: the columns live on device %d, which is not in the h2v_init list", device_of(d_polys));
     const size_t G = h->rep.size();
     static const bool no_split = getenv("H2V_NO_PEER_SPLIT") != nullptr;
     if (G == 1 || no_split || n_polys < 8 * G || len == 0 || device_of(d_out_affine) != r->dev) {
@@ -2606,14 +2533,14 @@ int h2v_commit_batch_dev(h2v_srs_t h, int basis, const void *d_polys, size_t col
                                             len * sizeof(fe), rep->stream);
             }
             if (e == cudaSuccess) e = cudaStreamSynchronize(rep->stream);
-            if (e != cudaSuccess) return fail(H2V_ECUDA, "commit: peer copy %d -> %d: %s", r->dev, rep->dev, cudaGetErrorString(e));
+            if (e != cudaSuccess) return failf(H2V_ECUDA, "commit: peer copy %d -> %d: %s", r->dev, rep->dev, cudaGetErrorString(e));
         }
         if ((rc2 = rep_commit_batch_dev(rep, basis, rep->peer_stage.p, len, cnt, len, rep->peer_out.p))) return rc2;
         // (cudaMemcpyPeer returns before the copy has landed and does not order against non-blocking streams: copy on the
         // replica's stream and wait for it)
         cudaError_t e = cudaMemcpyPeerAsync(dst + c0, r->dev, rep->peer_out.p, rep->dev, cnt * sizeof(affine), rep->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(rep->stream);
-        if (e != cudaSuccess) return fail(H2V_ECUDA, "commit: peer copy of the results: %s", cudaGetErrorString(e));
+        if (e != cudaSuccess) return failf(H2V_ECUDA, "commit: peer copy of the results: %s", cudaGetErrorString(e));
         return H2V_OK;
     });
     t_dev = r->dev;
@@ -2625,14 +2552,14 @@ int h2v_commit_batch_dev(h2v_srs_t h, int basis, const void *d_polys, size_t col
 // owning device over NVLink; commitments land in the host array in column order.
 int h2v_commit_batch_resident(h2v_srs_t h, int basis, const uint64_t *const *polys, size_t n_polys, size_t len, const uint64_t *tails,
                               size_t row0, size_t n_rows, void *d_dst, size_t dst_stride, uint64_t *out_affine) {
-    if (!h) return fail(H2V_EINVAL, "commit: NULL srs");
+    if (!h) return failf(H2V_EINVAL, "commit: NULL srs");
     if (n_polys == 0) return H2V_OK;
-    if (!polys || !d_dst || !out_affine || (n_rows && !tails)) return fail(H2V_EINVAL, "commit_resident: NULL buffer");
-    if (len == 0 || dst_stride < len || row0 + n_rows > len) return fail(H2V_EINVAL, "commit_resident: bad length / stride / row range");
+    if (!polys || !d_dst || !out_affine || (n_rows && !tails)) return failf(H2V_EINVAL, "commit_resident: NULL buffer");
+    if (len == 0 || dst_stride < len || row0 + n_rows > len) return failf(H2V_EINVAL, "commit_resident: bad length / stride / row range");
     for (size_t c = 0; c < n_polys; ++c)
-        if (!polys[c]) return fail(H2V_EINVAL, "commit_resident: polys[%zu] is NULL", c);
+        if (!polys[c]) return failf(H2V_EINVAL, "commit_resident: polys[%zu] is NULL", c);
     SrsRep *r = srs_on(h, device_of(d_dst));
-    if (!r) return fail(H2V_EINVAL, "commit_resident: the destination lives on device %d, which is not in the h2v_init list", device_of(d_dst));
+    if (!r) return failf(H2V_EINVAL, "commit_resident: the destination lives on device %d, which is not in the h2v_init list", device_of(d_dst));
     const size_t G = (h->rep.size() > 1 && n_polys >= 8 * h->rep.size()) ? h->rep.size() : 1;
     const size_t per = (n_polys + G - 1) / G;
     fe *dst = (fe *)d_dst;
@@ -2647,10 +2574,12 @@ int h2v_commit_batch_resident(h2v_srs_t h, int basis, const uint64_t *const *pol
         std::lock_guard<std::mutex> plk(rep->peer_mu);
         if (!owner && (rc2 = rep->peer_stage.ensure(cnt * len * sizeof(fe)))) return rc2;
         if ((rc2 = rep->peer_out.ensure(cnt * sizeof(affine)))) return rc2;
-        if (!rep->up_stream) CU(cudaStreamCreateWithFlags(&rep->up_stream, cudaStreamNonBlocking));
+        if (!rep->up_stream) H2V_CU(cudaStreamCreateWithFlags(&rep->up_stream, cudaStreamNonBlocking));
         fe *stage = owner ? dst + c0 * dst_stride : rep->peer_stage.as<fe>();
         const size_t sstride = owner ? dst_stride : len;
-        const size_t nsub = std::min<size_t>(4, cnt), sub = (cnt + nsub - 1) / nsub;
+        // few sub-batches: every commit call ends in a latency-bound reduction tail (~1 ms) that only size amortises
+        const size_t sub = std::max<size_t>((cnt + 3) / 4, std::max<size_t>(1, ((size_t)64 << 20) / (len * sizeof(fe))));
+        const size_t nsub = (cnt + sub - 1) / sub;
         std::vector<cudaEvent_t> ev(nsub, nullptr);
         cudaError_t e = cudaSuccess;
         for (size_t b = 0; b < nsub && e == cudaSuccess; ++b) {
@@ -2683,7 +2612,7 @@ int h2v_commit_batch_resident(h2v_srs_t h, int basis, const uint64_t *const *pol
             if (x) cudaEventDestroy(x);
         if (rc2) return rc2;
         if (e != cudaSuccess || e2 != cudaSuccess)
-            return fail(H2V_ECUDA, "commit_resident: %s", cudaGetErrorString(e != cudaSuccess ? e : e2));
+            return failf(H2V_ECUDA, "commit_resident: %s", cudaGetErrorString(e != cudaSuccess ? e : e2));
         return H2V_OK;
     });
     t_dev = r->dev;
@@ -2692,7 +2621,7 @@ int h2v_commit_batch_resident(h2v_srs_t h, int basis, const uint64_t *const *pol
 // Host columns: with several devices column j goes to device j mod G (each device has its own PCIe link and SRS
 // replica, no collective); the commitments come back in column order.
 int h2v_commit_batch(h2v_srs_t h, int basis, const uint64_t *const *polys, size_t n_polys, size_t len, uint64_t *out_affine) {
-    if (!h) return fail(H2V_EINVAL, "commit: NULL srs");
+    if (!h) return failf(H2V_EINVAL, "commit: NULL srs");
     const size_t G = h->rep.size();
     if (G == 1 || n_polys < 2 * G || !polys || !out_affine) {
         t_dev = h->rep[0]->dev;
@@ -2712,14 +2641,14 @@ int h2v_commit_batch(h2v_srs_t h, int basis, const uint64_t *const *polys, size_
     return H2V_OK;
 }
 int h2v_commit(h2v_srs_t h, int basis, const uint64_t *poly, size_t len, uint64_t out_affine[8]) {
-    if (!h) return fail(H2V_EINVAL, "commit: NULL srs");
+    if (!h) return failf(H2V_EINVAL, "commit: NULL srs");
     t_dev = h->rep[0]->dev;
-    return rep_commit(h->rep[0], basis, poly, len, out_affine);
+    return rep_commit_batch(h->rep[0], basis, &poly, 1, len, out_affine);
 }
 
 // ---------------------------------------------------------------- EvaluationDomain
 int h2v_domain_new(uint32_t j, uint32_t k, h2v_domain_t *out) {
-    if (!out) return fail(H2V_EINVAL, "domain_new: out is NULL");
+    if (!out) return failf(H2V_EINVAL, "domain_new: out is NULL");
     *out = nullptr;
     h2v_domain *h = new h2v_domain();
     for (size_t i = 0; i < g_devs.size(); ++i) {
@@ -2746,28 +2675,9 @@ void h2v_domain_free(h2v_domain_t h) {
     t_dev = -1;
     delete h;
 }
-uint32_t h2v_domain_k(h2v_domain_t h) { return h ? rep_domain_k(h->rep[0]) : 0; }
-uint32_t h2v_domain_extended_k(h2v_domain_t h) { return h ? rep_domain_extended_k(h->rep[0]) : 0; }
-int h2v_domain_constant(h2v_domain_t h, int which, uint64_t out[4]) { return rep_domain_constant(h ? h->rep[0] : nullptr, which, out); }
-int h2v_domain_rotate_omega(h2v_domain_t h, const uint64_t value[4], int32_t rotation, uint64_t out[4]) {
-    return rep_domain_rotate_omega(h ? h->rep[0] : nullptr, value, rotation, out);
-}
-int h2v_domain_rotate_extended(h2v_domain_t h, const uint64_t *in, int32_t rotation, uint64_t *out) {
-    return rep_domain_rotate_extended(h ? h->rep[0] : nullptr, in, rotation, out);
-}
-int h2v_domain_l_i_range(h2v_domain_t h, const uint64_t x[4], const uint64_t xn[4], int32_t rot_lo, int32_t rot_hi, uint64_t *out) {
-    return rep_domain_l_i_range(h ? h->rep[0] : nullptr, x, xn, rot_lo, rot_hi, out);
-}
-int h2v_domain_fill(h2v_domain_t h, int basis, const uint64_t scalar[4], uint64_t *out) {
-    return rep_domain_fill(h ? h->rep[0] : nullptr, basis, scalar, out);
-}
-#define H2V_DOM_ON(ptr)                                                                                                        \
-    if (!h) return fail(H2V_EINVAL, "NULL domain");                                                                            \
-    DomRep *r = dom_on(h, device_of(ptr));                                                                                     \
-    if (!r) return fail(H2V_EINVAL, "the columns live on device %d, which is not in the h2v_init list", device_of(ptr));      \
-    t_dev = r->dev;
 int h2v_domain_transform_dev(h2v_domain_t h, int op, const void *d_in, size_t in_stride, void *d_out, size_t out_stride, size_t n_cols) {
-    H2V_DOM_ON(d_in)
+    DomRep *r = dom_rep(h, d_in);
+    if (!r) return H2V_EINVAL;
     const size_t G = h->rep.size();
     static const bool no_split = getenv("H2V_NO_PEER_SPLIT") != nullptr;
     // worth splitting when every device gets about 2^21 points of transform: 8 columns of a 2^18-point extended domain
@@ -2808,7 +2718,7 @@ int h2v_domain_transform_dev(h2v_domain_t h, int op, const void *d_in, size_t in
                                             rep->stream);
             }
             if (e == cudaSuccess) e = cudaStreamSynchronize(rep->stream);
-            if (e != cudaSuccess) return fail(H2V_ECUDA, "transform: peer copy %d -> %d: %s", r->dev, rep->dev, cudaGetErrorString(e));
+            if (e != cudaSuccess) return failf(H2V_ECUDA, "transform: peer copy %d -> %d: %s", r->dev, rep->dev, cudaGetErrorString(e));
         }
         if ((rc2 = rep_domain_transform_dev(rep, op, rep->peer_in.p, nin, rep->peer_out.p, work_len, cnt))) return rc2;
         if (out_stride == work_len && nout == work_len) {
@@ -2819,14 +2729,14 @@ int h2v_domain_transform_dev(h2v_domain_t h, int op, const void *d_in, size_t in
                                         nout * sizeof(fe), rep->stream);
         }
         if (e == cudaSuccess) e = cudaStreamSynchronize(rep->stream);
-        if (e != cudaSuccess) return fail(H2V_ECUDA, "transform: peer copy of the results: %s", cudaGetErrorString(e));
+        if (e != cudaSuccess) return failf(H2V_ECUDA, "transform: peer copy of the results: %s", cudaGetErrorString(e));
         return H2V_OK;
     });
     t_dev = r->dev;
     return rc;
 }
 int h2v_domain_transform_batch(h2v_domain_t h, int op, const uint64_t *const *in, uint64_t *const *out, size_t n_cols) {
-    if (!h) return fail(H2V_EINVAL, "transform: NULL domain");
+    if (!h) return failf(H2V_EINVAL, "transform: NULL domain");
     const size_t G = h->rep.size();
     if (G == 1 || n_cols < 2 * G || !in || !out) {
         t_dev = h->rep[0]->dev;
@@ -2844,54 +2754,6 @@ int h2v_domain_transform_batch(h2v_domain_t h, int op, const uint64_t *const *in
     });
     t_dev = -1;
     return rc;
-}
-#define H2V_DOM_PRIMARY                                   \
-    if (!h) return fail(H2V_EINVAL, "NULL domain");       \
-    t_dev = h->rep[0]->dev;
-int h2v_lagrange_to_coeff(h2v_domain_t h, uint64_t *a) { H2V_DOM_PRIMARY return rep_lagrange_to_coeff(h->rep[0], a); }
-int h2v_coeff_to_lagrange(h2v_domain_t h, uint64_t *a) { H2V_DOM_PRIMARY return rep_coeff_to_lagrange(h->rep[0], a); }
-int h2v_coeff_to_extended(h2v_domain_t h, const uint64_t *in, uint64_t *out) { H2V_DOM_PRIMARY return rep_coeff_to_extended(h->rep[0], in, out); }
-int h2v_extended_to_coeff(h2v_domain_t h, const uint64_t *in, uint64_t *out) { H2V_DOM_PRIMARY return rep_extended_to_coeff(h->rep[0], in, out); }
-int h2v_divide_by_vanishing_poly(h2v_domain_t h, uint64_t *a) { H2V_DOM_PRIMARY return rep_divide_by_vanishing_poly(h->rep[0], a); }
-int h2v_quotient_gates_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], size_t n_gates, const void *d_q, size_t q_stride, const void *d_a,
-                           size_t a_stride) {
-    H2V_DOM_ON(d_h)
-    return rep_quotient_gates_dev(r, d_h, y, n_gates, d_q, q_stride, d_a, a_stride);
-}
-int h2v_quotient_gates_ptrs_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], size_t n_gates, const void *const *d_q_ptrs,
-                                const void *const *d_a_ptrs) {
-    H2V_DOM_ON(d_h)
-    return rep_quotient_gates_ptrs_dev(r, d_h, y, n_gates, d_q_ptrs, d_a_ptrs);
-}
-int h2v_quotient_permutation_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
-                                 size_t n_cols, size_t chunk_len, const void *d_cols, size_t cols_stride, const void *d_sigma,
-                                 size_t sigma_stride, const void *d_z, size_t z_stride, const void *d_l0, const void *d_l_last,
-                                 const void *d_l_active, uint32_t blinding_factors) {
-    H2V_DOM_ON(d_h)
-    return rep_quotient_permutation_dev(r, d_h, y, beta, gamma, n_cols, chunk_len, d_cols, cols_stride, d_sigma, sigma_stride, d_z, z_stride,
-                                        d_l0, d_l_last, d_l_active, blinding_factors);
-}
-int h2v_quotient_permutation_ptrs_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
-                                      size_t n_cols, size_t chunk_len, const void *const *d_col_ptrs, const void *const *d_sigma_ptrs,
-                                      const void *d_z, size_t z_stride, const void *d_l0, const void *d_l_last, const void *d_l_active,
-                                      uint32_t blinding_factors) {
-    H2V_DOM_ON(d_h)
-    return rep_quotient_permutation_ptrs_dev(r, d_h, y, beta, gamma, n_cols, chunk_len, d_col_ptrs, d_sigma_ptrs, d_z, z_stride, d_l0,
-                                             d_l_last, d_l_active, blinding_factors);
-}
-int h2v_quotient_permutation_range_ptrs_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
-                                            size_t n_cols, size_t chunk_len, size_t set_begin, size_t set_end, int with_head,
-                                            const void *const *d_col_ptrs, const void *const *d_sigma_ptrs, const void *d_z, size_t z_stride,
-                                            const void *d_l0, const void *d_l_last, const void *d_l_active, uint32_t blinding_factors) {
-    H2V_DOM_ON(d_h)
-    return rep_quotient_permutation_range_ptrs_dev(r, d_h, y, beta, gamma, n_cols, chunk_len, set_begin, set_end, with_head, d_col_ptrs,
-                                                   d_sigma_ptrs, d_z, z_stride, d_l0, d_l_last, d_l_active, blinding_factors);
-}
-int h2v_quotient_lookup_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
-                            const void *d_input, const void *d_table, const void *d_perm_input, const void *d_perm_table, const void *d_z,
-                            const void *d_l0, const void *d_l_last, const void *d_l_active) {
-    H2V_DOM_ON(d_h)
-    return rep_quotient_lookup_dev(r, d_h, y, beta, gamma, d_input, d_table, d_perm_input, d_perm_table, d_z, d_l0, d_l_last, d_l_active);
 }
 
 }  // extern "C"

@@ -20,6 +20,30 @@ inline int failf(int code, const char *fmt, ...) {
     va_end(ap);
     return set_error(code, buf);
 }
+
+// a device allocation that grows on demand and keeps its size between calls
+struct DevBuf {
+    void *p = nullptr;
+    size_t cap = 0;
+    int ensure(size_t bytes) {
+        if (bytes <= cap) return H2V_OK;
+        release();
+        cudaError_t e = cudaMalloc(&p, bytes);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            p = nullptr;
+            return failf(H2V_ENOMEM, "cudaMalloc(%zu bytes): %s", bytes, cudaGetErrorString(e));
+        }
+        cap = bytes;
+        return H2V_OK;
+    }
+    void release() {
+        if (p) cudaFree(p);
+        p = nullptr;
+        cap = 0;
+    }
+    template <class T> T *as() const { return reinterpret_cast<T *>(p); }
+};
 }  // namespace h2v
 
 #define H2V_CU(x)                                                                                                  \

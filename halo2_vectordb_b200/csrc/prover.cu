@@ -47,29 +47,6 @@ namespace {
 
 typedef FrP Fr;
 
-struct DevBuf {
-    void *p = nullptr;
-    size_t cap = 0;
-    int ensure(size_t bytes) {
-        if (bytes <= cap) return H2V_OK;
-        release();
-        cudaError_t e = cudaMalloc(&p, bytes);
-        if (e != cudaSuccess) {
-            cudaGetLastError();
-            p = nullptr;
-            return failf(H2V_ENOMEM, "cudaMalloc(%zu bytes): %s", bytes, cudaGetErrorString(e));
-        }
-        cap = bytes;
-        return H2V_OK;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
-    fe *f() const { return reinterpret_cast<fe *>(p); }
-};
-
 // ------------------------------------------------------------------ column kernels
 __device__ __forceinline__ fe ld(const fe *p) {
     const uint4 *q = reinterpret_cast<const uint4 *>(p);
@@ -442,7 +419,7 @@ int h2v_pk_load(h2v_srs_t srs, const h2v_circuit_t *cs, const uint64_t *const *f
             if (!pk->stream_ext) H2V_TRY(g.E->ensure(g.cnt * ne * sizeof(fe)));
             for (size_t c = 0; c < g.cnt; ++c) {
                 if (!g.src[c]) return failf(H2V_EINVAL, "pk_load: column %zu is NULL", c);
-                H2V_CU(cudaMemcpyAsync(g.L->f() + c * n, g.src[c], n * sizeof(fe), cudaMemcpyHostToDevice, pk->st));
+                H2V_CU(cudaMemcpyAsync(g.L->as<fe>() + c * n, g.src[c], n * sizeof(fe), cudaMemcpyHostToDevice, pk->st));
             }
             H2V_TRY(sync(pk));
             H2V_TRY(h2v_domain_transform_dev(pk->dom, H2V_OP_LAGRANGE_TO_COEFF, g.L->p, n, g.C->p, n, g.cnt));
@@ -542,62 +519,24 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
     H2V_TRY(pk->adv_C.ensure((size_t)A * n * sizeof(fe)));
     for (uint32_t c = 0; c < A; ++c)
         if (!advice[c]) return failf(H2V_EINVAL, "create_proof: advice[%u] is NULL", c);
-    std::vector<affine> pts;
-    if (h2v_device_list(nullptr, 0) > 1 && A >= 8u * (uint32_t)h2v_device_list(nullptr, 0)) {
-        // several devices: every device uploads its block of the columns over its own PCIe link, blinds and commits it, and
-        // forwards it to adv_L over NVLink (h2v_commit_batch_resident); same draws, same bytes
-        std::vector<Fr64> tails((size_t)A * (bf + 1));
-        for (auto &t : tails) t = rng.fr_random();                       // column by column, rows u .. n-1
-        for (uint32_t c = 0; c < A; ++c) (void)rng.fr_random();          // one Blind per column (unused by KZG, but drawn)
-        pts.resize(A);
-        H2V_TRY(h2v_commit_batch_resident(pk->srs, H2V_BASIS_LAGRANGE, advice, A, n, (const uint64_t *)tails.data(), u, bf + 1, pk->adv_L.p, n,
-                                          (uint64_t *)pts.data()));
-        H2V_CU(cudaSetDevice(pk->dev));
-    } else
-    {
-        // the columns cross PCIe in sub-batches on the proof's stream while the previous sub-batch is being committed
-        // (the commit entry point blocks the host, the copies were queued before it)
-        std::vector<Fr64> tails((size_t)A * (bf + 1));
-        for (auto &t : tails) t = rng.fr_random();                       // column by column, rows u .. n-1
-        for (uint32_t c = 0; c < A; ++c) (void)rng.fr_random();          // one Blind per column (unused by KZG, but drawn)
-        // few sub-batches: every commit call ends in a latency-bound reduction tail (~1 ms) that only size amortises
-        const uint32_t sub = std::max<uint32_t>((A + 3) / 4, (uint32_t)std::max<size_t>(1, ((size_t)64 << 20) / (n * sizeof(fe))));
-        const uint32_t nsub = (A + sub - 1) / sub;
-        std::vector<cudaEvent_t> ev(nsub, nullptr);
-        int rc = H2V_OK;
-        for (uint32_t b = 0; b < nsub && !rc; ++b) {
-            const uint32_t c0 = b * sub, c1 = std::min(A, c0 + sub);
-            for (uint32_t c = c0; c < c1; ++c)
-                if (cudaMemcpyAsync(pk->adv_L.f() + (size_t)c * n, advice[c], n * sizeof(fe), cudaMemcpyHostToDevice, st) != cudaSuccess) rc = H2V_ECUDA;
-            if (cudaMemcpy2DAsync(pk->adv_L.f() + (size_t)c0 * n + u, n * sizeof(fe), tails.data() + (size_t)c0 * (bf + 1), (bf + 1) * sizeof(fe),
-                                  (bf + 1) * sizeof(fe), c1 - c0, cudaMemcpyHostToDevice, st) != cudaSuccess)
-                rc = H2V_ECUDA;
-            if (cudaEventCreateWithFlags(&ev[b], cudaEventDisableTiming) != cudaSuccess || cudaEventRecord(ev[b], st) != cudaSuccess) rc = H2V_ECUDA;
-        }
-        pts.resize(A);
-        if (!rc) rc = pk->commits.ensure((size_t)A * sizeof(affine));
-        for (uint32_t b = 0; b < nsub && !rc; ++b) {
-            const uint32_t c0 = b * sub, c1 = std::min(A, c0 + sub);
-            if (cudaEventSynchronize(ev[b]) != cudaSuccess) { rc = H2V_ECUDA; break; }
-            rc = h2v_commit_batch_dev(pk->srs, H2V_BASIS_LAGRANGE, pk->adv_L.f() + (size_t)c0 * n, n, c1 - c0, n, (affine *)pk->commits.p + c0);
-            cudaSetDevice(pk->dev);
-        }
-        cudaStreamSynchronize(st);
-        for (cudaEvent_t e : ev)
-            if (e) cudaEventDestroy(e);
-        if (rc == H2V_ECUDA) return failf(H2V_ECUDA, "create_proof: advice upload failed: %s", cudaGetErrorString(cudaGetLastError()));
-        if (rc) return rc;
-        H2V_CU(cudaMemcpy(pts.data(), pk->commits.p, (size_t)A * sizeof(affine), cudaMemcpyDeviceToHost));
-    }
+    // h2v_commit_batch_resident: each device uploads its block of the columns in sub-batches (the next one crosses while the
+    // previous one is committed), writes the tails, commits the block and leaves it in adv_L
+    std::vector<Fr64> tails((size_t)A * (bf + 1));
+    for (auto &t : tails) t = rng.fr_random();                       // column by column, rows u .. n-1
+    for (uint32_t c = 0; c < A; ++c) (void)rng.fr_random();          // one Blind per column (unused by KZG, but drawn)
+    std::vector<affine> pts(A);
+    H2V_TRY(h2v_commit_batch_resident(pk->srs, H2V_BASIS_LAGRANGE, advice, A, n, (const uint64_t *)tails.data(), u, bf + 1, pk->adv_L.p, n,
+                                      (uint64_t *)pts.data()));
+    H2V_CU(cudaSetDevice(pk->dev));
     H2V_TRY(write_points(T, pts));
     T.absorb_async();      // the advice commitments are hashed on a worker thread while the lookup permutations run
     lap();   // phase 0: upload + advice commitments
     // column pointer helpers
     auto col_L = [&](uint8_t kind, uint32_t idx) -> const fe * {
-        return kind == 0 ? pk->adv_L.f() + (size_t)idx * n : kind == 1 ? pk->fixed_L.f() + (size_t)idx * n : pk->inst_L.f() + (size_t)idx * n;
+        return kind == 0 ? pk->adv_L.as<fe>() + (size_t)idx * n : kind == 1 ? pk->fixed_L.as<fe>() + (size_t)idx * n : pk->inst_L.as<fe>() + (size_t)idx * n;
     };
     auto col_E = [&](uint8_t kind, uint32_t idx) -> const fe * {
-        return kind == 0 ? pk->adv_E.f() + (size_t)idx * ne : kind == 1 ? pk->fixed_E.f() + (size_t)idx * ne : pk->inst_E.f() + (size_t)idx * ne;
+        return kind == 0 ? pk->adv_E.as<fe>() + (size_t)idx * ne : kind == 1 ? pk->fixed_E.as<fe>() + (size_t)idx * ne : pk->inst_E.as<fe>() + (size_t)idx * ne;
     };
     // ---- 5. theta; lookups: permuted input / table columns                   (lookup/prover.rs commit_permuted)
     // theta is squeezed at its place in the transcript (below, before A' / S' are written); single-expression lookups
@@ -612,7 +551,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
                 li[l] = col_L(0, pk->lookup_input[l]);
                 lt[l] = col_L(1, pk->lookup_table[l]);
             }
-            H2V_TRY(h2v_permute_expression_pair_batch_dev(li.data(), lt.data(), L, u, pk->pa_L.f(), n, pk->ps_L.f(), n));
+            H2V_TRY(h2v_permute_expression_pair_batch_dev(li.data(), lt.data(), L, u, pk->pa_L.as<fe>(), n, pk->ps_L.as<fe>(), n));
             H2V_CU(cudaSetDevice(pk->dev));
         }
         for (uint32_t l = 0; l < L; ++l) {
@@ -621,11 +560,11 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
             (void)rng.fr_random();     // permuted input blind
             (void)rng.fr_random();     // permuted table blind
         }
-        H2V_TRY(write_rows(pk, pk->pa_L.f(), n, u, bf + 1, L, ta));
-        H2V_TRY(write_rows(pk, pk->ps_L.f(), n, u, bf + 1, L, ts));
+        H2V_TRY(write_rows(pk, pk->pa_L.as<fe>(), n, u, bf + 1, L, ta));
+        H2V_TRY(write_rows(pk, pk->ps_L.as<fe>(), n, u, bf + 1, L, ts));
         std::vector<affine> ca, cs_;
-        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->pa_L.f(), L, ca));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->ps_L.f(), L, cs_));
+        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->pa_L.as<fe>(), L, ca));
+        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->ps_L.as<fe>(), L, cs_));
         (void)T.squeeze_challenge();      // theta
         for (uint32_t l = 0; l < L; ++l) {
             if (!T.write_point(ca[l]) || !T.write_point(cs_[l]))
@@ -645,7 +584,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         std::vector<const fe *> hp(2 * NP);
         for (uint32_t c = 0; c < NP; ++c) {
             hp[c] = col_L(pk->perm_kind[c], pk->perm_index[c]);
-            hp[NP + c] = pk->sigma_L.f() + (size_t)c * n;
+            hp[NP + c] = pk->sigma_L.as<fe>() + (size_t)c * n;
         }
         H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), hp.size() * sizeof(void *)));
         std::vector<Fr64> dstart(NS);
@@ -659,32 +598,32 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         PermArgs pa;
         pa.cols = (const fe *const *)pk->ptrs.p;
         pa.sigma = pa.cols + NP;
-        pa.omega_pows = pk->omega_pows.f();
-        pa.delta_start = pk->scal.f();
+        pa.omega_pows = pk->omega_pows.as<fe>();
+        pa.delta_start = pk->scal.as<fe>();
         pa.beta = frh::to_fe(beta); pa.gamma = frh::to_fe(gamma); pa.delta = frh::to_fe(pk->delta);
         pa.n_cols = NP; pa.chunk = pk->chunk; pa.n = (uint32_t)n;
-        perm_numden_kernel<<<dim3(gn, NS), 256, 0, st>>>(pa, pk->num.f(), pk->den.f());
+        perm_numden_kernel<<<dim3(gn, NS), 256, 0, st>>>(pa, pk->num.as<fe>(), pk->den.as<fe>());
         H2V_LAUNCHED();
         H2V_TRY(sync(pk));
         // z_s with z_s[0] = 1; then chain: z_s *= z_{s-1}[u] (upstream carries `last_z` from set to set)
         H2V_TRY(h2v_grand_product_dev(pk->num.p, pk->den.p, n, NS, pk->z_L.p));
         std::vector<Fr64> last(NS), scale(NS);
-        H2V_CU(cudaMemcpy2D(last.data(), sizeof(fe), pk->z_L.f() + u, n * sizeof(fe), sizeof(fe), NS, cudaMemcpyDeviceToHost));
+        H2V_CU(cudaMemcpy2D(last.data(), sizeof(fe), pk->z_L.as<fe>() + u, n * sizeof(fe), sizeof(fe), NS, cudaMemcpyDeviceToHost));
         cur = frh::ONE;
         for (uint32_t s = 0; s < NS; ++s) {
             scale[s] = cur;
             cur = frh::mul(cur, last[s]);
         }
         H2V_TRY(upload(pk, pk->scal, 0, scale.data(), NS * sizeof(fe)));
-        scale_cols_kernel<<<dim3(gn, NS), 256, 0, st>>>(pk->z_L.f(), (uint32_t)n, pk->scal.f());
+        scale_cols_kernel<<<dim3(gn, NS), 256, 0, st>>>(pk->z_L.as<fe>(), (uint32_t)n, pk->scal.as<fe>());
         H2V_LAUNCHED();
         std::vector<Fr64> tails((size_t)NS * bf);
         for (uint32_t s = 0; s < NS; ++s) {
             for (uint32_t i = 0; i < bf; ++i) tails[(size_t)s * bf + i] = rng.fr_random();     // rows n - bf .. n - 1
             (void)rng.fr_random();                                                             // product blind
         }
-        H2V_TRY(write_rows(pk, pk->z_L.f(), n, n - bf, bf, NS, tails));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->z_L.f(), NS, pts));
+        H2V_TRY(write_rows(pk, pk->z_L.as<fe>(), n, n - bf, bf, NS, tails));
+        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->z_L.as<fe>(), NS, pts));
         H2V_TRY(write_points(T, pts));
         T.absorb_async();      // hashed while the lookup products are built and committed
     }
@@ -697,8 +636,8 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
             hp[L + l] = col_L(1, pk->lookup_table[l]);
         }
         H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), hp.size() * sizeof(void *)));
-        lookup_numden_kernel<<<dim3(gn, L), 256, 0, st>>>((const fe *const *)pk->ptrs.p, (const fe *const *)pk->ptrs.p + L, pk->pa_L.f(),
-                                                        pk->ps_L.f(), frh::to_fe(beta), frh::to_fe(gamma), (uint32_t)n, pk->num.f(), pk->den.f());
+        lookup_numden_kernel<<<dim3(gn, L), 256, 0, st>>>((const fe *const *)pk->ptrs.p, (const fe *const *)pk->ptrs.p + L, pk->pa_L.as<fe>(),
+                                                        pk->ps_L.as<fe>(), frh::to_fe(beta), frh::to_fe(gamma), (uint32_t)n, pk->num.as<fe>(), pk->den.as<fe>());
         H2V_LAUNCHED();
         H2V_TRY(sync(pk));
         H2V_TRY(h2v_grand_product_dev(pk->num.p, pk->den.p, n, L, pk->zl_L.p));
@@ -707,8 +646,8 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
             for (uint32_t i = 0; i < bf; ++i) tails[(size_t)l * bf + i] = rng.fr_random();
             (void)rng.fr_random();
         }
-        H2V_TRY(write_rows(pk, pk->zl_L.f(), n, n - bf, bf, L, tails));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->zl_L.f(), L, pts));
+        H2V_TRY(write_rows(pk, pk->zl_L.as<fe>(), n, n - bf, bf, L, tails));
+        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->zl_L.as<fe>(), L, pts));
         H2V_TRY(write_points(T, pts));
         T.absorb_async();
     }
@@ -719,12 +658,12 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         // n consecutive Fr::random draws = n consecutive key-stream blocks: produced on the device
         ChaChaKey key;
         memcpy(key.k, rng.key, 32);
-        chacha_fr_kernel<<<gn, 256, 0, st>>>(key, rng.next_block(), (uint32_t)n, pk->rnd_C.f());
+        chacha_fr_kernel<<<gn, 256, 0, st>>>(key, rng.next_block(), (uint32_t)n, pk->rnd_C.as<fe>());
         H2V_LAUNCHED();
         rng.skip_fr(n);
         (void)rng.fr_random();      // random_blind
         H2V_TRY(sync(pk));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, pk->rnd_C.f(), 1, pts));
+        H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, pk->rnd_C.as<fe>(), 1, pts));
         H2V_TRY(write_points(T, pts));
         T.absorb_async();
     }
@@ -750,10 +689,10 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
     const Fr64 y = T.squeeze_challenge();
     lap();   // phase 3: random poly + transforms
     H2V_TRY(pk->hq.ensure(2 * ne * sizeof(fe)));
-    fe *h_ext = pk->hq.f(), *h_out = pk->hq.f() + ne;
+    fe *h_ext = pk->hq.as<fe>(), *h_out = pk->hq.as<fe>() + ne;
     H2V_CU(cudaMemsetAsync(h_ext, 0, ne * sizeof(fe), st));
     H2V_TRY(sync(pk));
-    const fe *l0 = pk->lrows_E.f(), *ll = l0 + ne, *la = l0 + 2 * ne;
+    const fe *l0 = pk->lrows_E.as<fe>(), *ll = l0 + ne, *la = l0 + 2 * ne;
     if (!stream) {
         std::vector<const fe *> hp(2 * G + 2 * NP);
         for (uint32_t j = 0; j < G; ++j) {
@@ -762,7 +701,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         }
         for (uint32_t c = 0; c < NP; ++c) {
             hp[2 * G + c] = col_E(pk->perm_kind[c], pk->perm_index[c]);
-            hp[2 * G + NP + c] = pk->sigma_E.f() + (size_t)c * ne;
+            hp[2 * G + NP + c] = pk->sigma_E.as<fe>() + (size_t)c * ne;
         }
         if (!hp.empty()) H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), hp.size() * sizeof(void *)));
         const void *const *tab = (const void *const *)pk->ptrs.p;
@@ -772,16 +711,16 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
                                                       tab + 2 * G + NP, pk->z_E.p, ne, l0, ll, la, bf));
         for (uint32_t l = 0; l < L; ++l)
             H2V_TRY(h2v_quotient_lookup_dev(pk->dom, h_ext, u64(y), u64(beta), u64(gamma), col_E(0, pk->lookup_input[l]),
-                                            col_E(1, pk->lookup_table[l]), pk->pa_E.f() + (size_t)l * ne, pk->ps_E.f() + (size_t)l * ne,
-                                            pk->zl_E.f() + (size_t)l * ne, l0, ll, la));
+                                            col_E(1, pk->lookup_table[l]), pk->pa_E.as<fe>() + (size_t)l * ne, pk->ps_E.as<fe>() + (size_t)l * ne,
+                                            pk->zl_E.as<fe>() + (size_t)l * ne, l0, ll, la));
     } else {
         // the same folds, in upstream's order, over slices of columns whose extended forms are rebuilt into `scr_E` from
         // the resident coefficient forms (every term reads columns of its own gate / set / lookup only)
         const size_t SC = pk->scr_cols;
         H2V_TRY(pk->scr_E.ensure(SC * ne * sizeof(fe)));
-        fe *scr = pk->scr_E.f();
+        fe *scr = pk->scr_E.as<fe>();
         auto col_C = [&](uint8_t kind, uint32_t idx) -> const fe * {
-            return kind == 0 ? pk->adv_C.f() + (size_t)idx * n : kind == 1 ? pk->fixed_C.f() + (size_t)idx * n : pk->inst_C.f() + (size_t)idx * n;
+            return kind == 0 ? pk->adv_C.as<fe>() + (size_t)idx * n : kind == 1 ? pk->fixed_C.as<fe>() + (size_t)idx * n : pk->inst_C.as<fe>() + (size_t)idx * n;
         };
         // coeff_to_extended of a list of coefficient columns into consecutive scratch slots; neighbours share one launch
         const bool timing = getenv("H2V_PROVE_TIMING") != nullptr;
@@ -847,9 +786,9 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
                 }
                 for (size_t c = c0; c < c1; ++c) {
                     if (c < pk->cached_sigma) {
-                        sg.push_back(pk->ext_cache.f() + c * ne);
+                        sg.push_back(pk->ext_cache.as<fe>() + c * ne);
                     } else {
-                        src.push_back(pk->sigma_C.f() + c * n);
+                        src.push_back(pk->sigma_C.as<fe>() + c * n);
                         sg.push_back(scr + slot++ * ne);
                     }
                 }
@@ -878,7 +817,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
             const Fr64 cf[2] = {frh::pow_u64(y, 2ull * NS + 1), frh::ONE};
             H2V_TRY(upload(pk, pk->ptrs, 0, two, sizeof two));
             H2V_TRY(upload(pk, pk->scal, 0, cf, sizeof cf));
-            lincomb_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.f(), 2, (uint32_t)ne, h_ext);
+            lincomb_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.as<fe>(), 2, (uint32_t)ne, h_ext);
             H2V_LAUNCHED();
             H2V_TRY(sync(pk));
             mark(t_fold);
@@ -903,7 +842,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
             src.clear();
             hp.assign(2 * cnt, nullptr);
             for (size_t c = c0; c < c1; ++c) src.push_back(col_C(pk->perm_kind[c], pk->perm_index[c]));
-            for (size_t c = c0; c < c1; ++c) src.push_back(pk->sigma_C.f() + c * n);
+            for (size_t c = c0; c < c1; ++c) src.push_back(pk->sigma_C.as<fe>() + c * n);
             H2V_TRY(extend(src, scr));
             mark(t_ext);
             for (size_t j = 0; j < 2 * cnt; ++j) hp[j] = scr + j * ne;
@@ -928,7 +867,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
             mark(t_ext);
             for (uint32_t l = l0_; l < l1_; ++l)
                 H2V_TRY(h2v_quotient_lookup_dev(pk->dom, h_ext, u64(y), u64(beta), u64(gamma), scr + (size_t)(1 + l - l0_) * ne, scr,
-                                                pk->pa_E.f() + (size_t)l * ne, pk->ps_E.f() + (size_t)l * ne, pk->zl_E.f() + (size_t)l * ne, l0, ll, la));
+                                                pk->pa_E.as<fe>() + (size_t)l * ne, pk->ps_E.as<fe>() + (size_t)l * ne, pk->zl_E.as<fe>() + (size_t)l * ne, l0, ll, la));
             mark(t_fold);
             l0_ = l1_;
         }
@@ -957,7 +896,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
     const uint32_t p_cur = point_of(0), p_next = point_of(1), p_prev = point_of(-1), p_last = point_of(-(int32_t)(bf + 1));
     // h(X) = sum_i xn^i h_i(X)
     H2V_TRY(pk->sh_h.ensure(2 * n * sizeof(fe)));
-    fe *h_poly = pk->sh_h.f(), *hx_dev = pk->sh_h.f() + n;
+    fe *h_poly = pk->sh_h.as<fe>(), *hx_dev = pk->sh_h.as<fe>() + n;
     {
         std::vector<const fe *> hp(NH);
         std::vector<Fr64> cf(NH);
@@ -969,29 +908,29 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         }
         H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), NH * sizeof(void *)));
         H2V_TRY(upload(pk, pk->scal, 0, cf.data(), NH * sizeof(fe)));
-        lincomb_kernel<<<gn, 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.f(), NH, (uint32_t)n, h_poly);
+        lincomb_kernel<<<gn, 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.as<fe>(), NH, (uint32_t)n, h_poly);
         H2V_LAUNCHED();
     }
     // every (polynomial, point) pair that is evaluated, in transcript order first, then the two the transcript skips
     std::vector<EvalPair> pairs;
     auto push = [&](const fe *poly, uint32_t pt) { pairs.push_back(EvalPair{poly, pt}); return (uint32_t)(pairs.size() - 1); };
-    for (size_t q = 0; q < pk->aq_col.size(); ++q) push(pk->adv_C.f() + (size_t)pk->aq_col[q] * n, point_of(pk->aq_rot[q]));
-    for (size_t q = 0; q < pk->fq_col.size(); ++q) push(pk->fixed_C.f() + (size_t)pk->fq_col[q] * n, point_of(pk->fq_rot[q]));
-    const uint32_t e_random = push(pk->rnd_C.f(), p_cur);
-    for (uint32_t c = 0; c < NP; ++c) push(pk->sigma_C.f() + (size_t)c * n, p_cur);
+    for (size_t q = 0; q < pk->aq_col.size(); ++q) push(pk->adv_C.as<fe>() + (size_t)pk->aq_col[q] * n, point_of(pk->aq_rot[q]));
+    for (size_t q = 0; q < pk->fq_col.size(); ++q) push(pk->fixed_C.as<fe>() + (size_t)pk->fq_col[q] * n, point_of(pk->fq_rot[q]));
+    const uint32_t e_random = push(pk->rnd_C.as<fe>(), p_cur);
+    for (uint32_t c = 0; c < NP; ++c) push(pk->sigma_C.as<fe>() + (size_t)c * n, p_cur);
     const uint32_t e_perm = (uint32_t)pairs.size();
     for (uint32_t s = 0; s < NS; ++s) {
-        push(pk->z_C.f() + (size_t)s * n, p_cur);
-        push(pk->z_C.f() + (size_t)s * n, p_next);
-        if (s + 1 < NS) push(pk->z_C.f() + (size_t)s * n, p_last);
+        push(pk->z_C.as<fe>() + (size_t)s * n, p_cur);
+        push(pk->z_C.as<fe>() + (size_t)s * n, p_next);
+        if (s + 1 < NS) push(pk->z_C.as<fe>() + (size_t)s * n, p_last);
     }
     const uint32_t e_lookup = (uint32_t)pairs.size();
     for (uint32_t l = 0; l < L; ++l) {
-        push(pk->zl_C.f() + (size_t)l * n, p_cur);
-        push(pk->zl_C.f() + (size_t)l * n, p_next);
-        push(pk->pa_C.f() + (size_t)l * n, p_cur);
-        push(pk->pa_C.f() + (size_t)l * n, p_prev);
-        push(pk->ps_C.f() + (size_t)l * n, p_cur);
+        push(pk->zl_C.as<fe>() + (size_t)l * n, p_cur);
+        push(pk->zl_C.as<fe>() + (size_t)l * n, p_next);
+        push(pk->pa_C.as<fe>() + (size_t)l * n, p_cur);
+        push(pk->pa_C.as<fe>() + (size_t)l * n, p_prev);
+        push(pk->ps_C.as<fe>() + (size_t)l * n, p_cur);
     }
     const uint32_t n_written = (uint32_t)pairs.size();
     const uint32_t e_h = push(h_poly, p_cur);       // h(x): opened by the multi-open argument, not written
@@ -1002,7 +941,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         H2V_TRY(pk->pts.ensure((points.size() + 8) * sizeof(fe)));
         H2V_TRY(upload(pk, pk->pairs, 0, pairs.data(), pairs.size() * sizeof(EvalPair)));
         H2V_TRY(upload(pk, pk->pts, 0, points.data(), points.size() * sizeof(fe)));
-        eval_pairs_kernel<<<(unsigned)pairs.size(), 256, 0, st>>>((const EvalPair *)pk->pairs.p, pk->pts.f(), (uint32_t)n, pk->evals.f());
+        eval_pairs_kernel<<<(unsigned)pairs.size(), 256, 0, st>>>((const EvalPair *)pk->pairs.p, pk->pts.as<fe>(), (uint32_t)n, pk->evals.as<fe>());
         H2V_LAUNCHED();
         H2V_CU(cudaMemcpyAsync(evals.data(), pk->evals.p, pairs.size() * sizeof(fe), cudaMemcpyDeviceToHost, st));
         H2V_TRY(sync(pk));
@@ -1048,7 +987,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         queries.insert(queries.end(), fix_q.begin(), fix_q.end());
         queries.insert(queries.end(), sig_q.begin(), sig_q.end());
         queries.push_back(Query{h_poly, p_cur, evals[e_h]});
-        queries.push_back(Query{pk->rnd_C.f(), p_cur, evals[e_random]});
+        queries.push_back(Query{pk->rnd_C.as<fe>(), p_cur, evals[e_random]});
     }
     // construct_intermediate_sets: point sets are ordered sets of field elements (BTreeSet<Fr>: numeric order of the
     // canonical values); commitments and rotation sets keep their order of first appearance
@@ -1105,7 +1044,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
     H2V_TRY(pk->scal.ensure((max_polys + NR + 16) * sizeof(fe)));
     std::vector<std::vector<Fr64>> r_comb(NR);           // sum_j y^j R_ij(X), low degree
     std::vector<std::vector<std::vector<Fr64>>> r_ij(NR);
-    fe *Q = pk->sh_B.f();                                // quotient contributions Q_i, n coefficients each
+    fe *Q = pk->sh_B.as<fe>();                                // quotient contributions Q_i, n coefficients each
     for (size_t i = 0; i < NR; ++i) {
         const std::vector<Fr64> ps = pts_of(rsets[i].mask);
         const size_t m = ps.size(), nc = rsets[i].polys.size();
@@ -1126,14 +1065,14 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         // S_i(X) = sum_j y^j P_ij(X)
         H2V_TRY(upload(pk, pk->ptrs, 0, rsets[i].polys.data(), nc * sizeof(void *)));
         H2V_TRY(upload(pk, pk->scal, 0, ypow.data(), nc * sizeof(fe)));
-        fe *S = pk->sh_S.f() + i * n;
-        lincomb_kernel<<<gn, 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.f(), (uint32_t)nc, (uint32_t)n, S);
+        fe *S = pk->sh_S.as<fe>() + i * n;
+        lincomb_kernel<<<gn, 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.as<fe>(), (uint32_t)nc, (uint32_t)n, S);
         H2V_LAUNCHED();
         // N_i = S_i - sum_j y^j R_ij, then Q_i = N_i / prod (X - p)
-        fe *cur_buf = Q + i * n, *oth = pk->sh_A.f();
+        fe *cur_buf = Q + i * n, *oth = pk->sh_A.as<fe>();
         H2V_CU(cudaMemcpyAsync(cur_buf, S, n * sizeof(fe), cudaMemcpyDeviceToDevice, st));
         H2V_TRY(upload(pk, pk->scal, 0, r_comb[i].data(), m * sizeof(fe)));
-        sub_low_kernel<<<1, 32, 0, st>>>(cur_buf, pk->scal.f(), (uint32_t)m);
+        sub_low_kernel<<<1, 32, 0, st>>>(cur_buf, pk->scal.as<fe>(), (uint32_t)m);
         H2V_LAUNCHED();
         H2V_TRY(sync(pk));
         size_t len = n;
@@ -1158,7 +1097,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         }
         H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), NR * sizeof(void *)));
         H2V_TRY(upload(pk, pk->scal, 0, cf.data(), NR * sizeof(fe)));
-        lincomb_kernel<<<gn, 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.f(), (uint32_t)NR, (uint32_t)n, hx_dev);
+        lincomb_kernel<<<gn, 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.as<fe>(), (uint32_t)NR, (uint32_t)n, hx_dev);
         H2V_LAUNCHED();
         H2V_TRY(sync(pk));
         H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, hx_dev, 1, pts));
@@ -1181,7 +1120,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
                 ri = frh::add(ri, frh::mul(yp, eval_small(r_ij[i][j], uc)));
                 yp = frh::mul(yp, ys);
             }
-            hp[i] = pk->sh_S.f() + i * n;
+            hp[i] = pk->sh_S.as<fe>() + i * n;
             cf[i] = frh::mul(vp, zi);
             konst = frh::add(konst, frh::mul(cf[i], ri));
             vp = frh::mul(vp, vs);
@@ -1192,11 +1131,11 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         cf[NR] = frh::neg(zt);
         H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), (NR + 1) * sizeof(void *)));
         H2V_TRY(upload(pk, pk->scal, 0, cf.data(), (NR + 1) * sizeof(fe)));
-        fe *Lx = pk->sh_A.f();
-        lincomb_kernel<<<gn, 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.f(), (uint32_t)(NR + 1), (uint32_t)n, Lx);
+        fe *Lx = pk->sh_A.as<fe>();
+        lincomb_kernel<<<gn, 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.as<fe>(), (uint32_t)(NR + 1), (uint32_t)n, Lx);
         H2V_LAUNCHED();
         H2V_TRY(upload(pk, pk->scal, 0, &konst, sizeof(fe)));
-        sub_low_kernel<<<1, 32, 0, st>>>(Lx, pk->scal.f(), 1);
+        sub_low_kernel<<<1, 32, 0, st>>>(Lx, pk->scal.as<fe>(), 1);
         H2V_LAUNCHED();
         H2V_TRY(sync(pk));
         fe *W = Q;        // the quotient contributions are no longer needed
@@ -1204,7 +1143,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         H2V_CU(cudaMemsetAsync(W + (n - 1), 0, sizeof(fe), st));
         const Fr64 z0inv = frh::inv(z0);
         H2V_TRY(upload(pk, pk->scal, 0, &z0inv, sizeof(fe)));
-        scale_cols_kernel<<<dim3(gn, 1), 256, 0, st>>>(W, (uint32_t)n, pk->scal.f());
+        scale_cols_kernel<<<dim3(gn, 1), 256, 0, st>>>(W, (uint32_t)n, pk->scal.as<fe>());
         H2V_LAUNCHED();
         H2V_TRY(sync(pk));
         H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, W, 1, pts));

@@ -152,16 +152,19 @@ def test_proof_bytes_do_not_depend_on_the_device_count(h2v):
     assert proofs[0] == PL.create_proof(params, t.cs, t.fixed, t.sigma, t.vk_repr, t.advice, t.instances, seed)
 
 
-@pytest.mark.parametrize("devices", [1, 2])
-def test_commit_batch_resident(h2v, devices):
+@pytest.mark.parametrize("devices,k,cols_n", [pytest.param(1, 9, 19, id="1"), pytest.param(2, 9, 19, id="2"),
+                                              pytest.param(1, 16, 40, id="1-k16")])
+def test_commit_batch_resident(h2v, devices, k, cols_n):
     """h2v_commit_batch_resident: host columns are blinded, committed and left on the device (the advice phase of
-    create_proof); with two devices each uploads and commits a block and forwards it to the owner."""
+    create_proof); with two devices each uploads and commits a block and forwards it to the owner.  At k = 16 the 40
+    columns go up in two sub-batches of 32 and 8 (a full one holds 64 MiB of columns): the second crosses while the
+    first is committed."""
     import torch
     if h2v.device_count() < devices:
         pytest.skip("needs 2 GPUs")
     h2v.init(list(range(devices)) if devices > 1 else 0)
     try:
-        k, n, cols_n, rows = 9, 1 << 9, 19, 6
+        n, rows = 1 << k, 6
         bases = O.gen_bases(n)
         srs = h2v.ParamsKZG(k, None, bases)
         cols = [O.fr_fill(n, 700 + i, mode=i % 2) for i in range(cols_n)]
