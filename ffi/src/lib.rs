@@ -99,6 +99,8 @@ extern "C" {
     pub fn h2v_proof_size(pk: *mut H2vPk) -> usize;
     pub fn h2v_create_proof(pk: *mut H2vPk, advice: *const *const u64, instances: *const *const u64, instance_len: *const u32,
                             rng_seed: *const u8, proof_out: *mut u8, proof_cap: usize, proof_len: *mut usize) -> c_int;
+    pub fn h2v_create_proofs(pk: *mut H2vPk, n_proofs: usize, advice: *const *const *const u64, instances: *const *const *const u64,
+                             instance_len: *const *const u32, rng_seeds: *const u8, proofs_out: *mut u8, proof_stride: usize) -> c_int;
     pub fn h2v_quotient_gates_dev(dom: *mut H2vDomain, d_h: *mut c_void, y: *const u64, n_gates: usize, d_q: *const c_void,
                                   q_stride: usize, d_a: *const c_void, a_stride: usize) -> c_int;
     pub fn h2v_quotient_permutation_dev(dom: *mut H2vDomain, d_h: *mut c_void, y: *const u64, beta: *const u64, gamma: *const u64,
@@ -312,6 +314,26 @@ impl DeviceProvingKey {
         ok(unsafe { h2v_create_proof(self.0, a.as_ptr(), i.as_ptr(), il.as_ptr(), rng_seed.as_ptr(), out.as_mut_ptr(), out.len(), &mut len) });
         out.truncate(len);
         out
+    }
+    /// proof p = `create_proof(n, advice[p], instances[p], &rng_seeds[p])`, byte for byte; the proofs run in groups on the
+    /// device, phase by phase (one vector-database query answered per proof)
+    pub fn create_proofs(&self, n: usize, advice: &[&[&[Fr]]], instances: &[&[&[Fr]]], rng_seeds: &[[u8; 32]]) -> Vec<Vec<u8>> {
+        let b = advice.len();
+        assert!(instances.len() == b && rng_seeds.len() == b);
+        assert!(advice.iter().all(|a| a.iter().all(|c| c.len() == n)));
+        let a: Vec<Vec<*const u64>> = advice.iter().map(|a| a.iter().map(|c| c.as_ptr() as *const u64).collect()).collect();
+        let i: Vec<Vec<*const u64>> = instances.iter().map(|a| a.iter().map(|c| c.as_ptr() as *const u64).collect()).collect();
+        let il: Vec<Vec<u32>> = instances.iter().map(|a| a.iter().map(|c| c.len() as u32).collect()).collect();
+        let ap: Vec<*const *const u64> = a.iter().map(|v| v.as_ptr()).collect();
+        let ip: Vec<*const *const u64> = i.iter().map(|v| v.as_ptr()).collect();
+        let lp: Vec<*const u32> = il.iter().map(|v| v.as_ptr()).collect();
+        let seeds: Vec<u8> = rng_seeds.iter().flatten().copied().collect();
+        let size = unsafe { h2v_proof_size(self.0) };
+        let mut out = vec![0u8; b * size];
+        if b > 0 {
+            ok(unsafe { h2v_create_proofs(self.0, b, ap.as_ptr(), ip.as_ptr(), lp.as_ptr(), seeds.as_ptr(), out.as_mut_ptr(), size) });
+        }
+        out.chunks(size.max(1)).take(b).map(|c| c.to_vec()).collect()
     }
 }
 impl Drop for DeviceProvingKey {

@@ -36,7 +36,7 @@ ABI_SYMBOLS = [
     "h2v_g1_to_bytes", "h2v_fr_to_repr",
     "h2v_domain_rotate_omega", "h2v_domain_rotate_extended", "h2v_domain_l_i_range", "h2v_domain_fill", "h2v_kate_division_dev",
     "h2v_quotient_gates_ptrs_dev", "h2v_quotient_permutation_ptrs_dev", "h2v_quotient_permutation_range_ptrs_dev", "h2v_commit_batch_resident",
-    "h2v_pk_load", "h2v_pk_free", "h2v_create_proof", "h2v_proof_size", "h2v_pk_last_phase_ms",
+    "h2v_pk_load", "h2v_pk_free", "h2v_create_proof", "h2v_create_proofs", "h2v_proof_size", "h2v_pk_last_phase_ms",
     "h2v_transcript_new", "h2v_transcript_free", "h2v_transcript_common_point", "h2v_transcript_common_scalar",
     "h2v_transcript_write_point", "h2v_transcript_write_scalar", "h2v_transcript_squeeze_challenge", "h2v_transcript_bytes",
     "h2v_poseidon_permutation", "h2v_poseidon_permutation_variant", "h2v_chacha20_fr_random", "h2v_chacha20_block",
@@ -147,6 +147,8 @@ def lib():
         L.h2v_pk_free.restype = None
         L.h2v_create_proof.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_size_t, C.POINTER(C.c_size_t)]
+        L.h2v_create_proofs.argtypes = [C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_char_p,
+                                        C.c_void_p, C.c_size_t]
         L.h2v_proof_size.argtypes = [C.c_void_p]
         L.h2v_proof_size.restype = C.c_size_t
         L.h2v_pk_last_phase_ms.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
@@ -874,6 +876,37 @@ class ProvingKey:
         ln = C.c_size_t()
         _check(lib().h2v_create_proof(self._h, aa, ia, _ptr(il), bytes(rng_seed), _ptr(out), cap, C.byref(ln)))
         return bytes(out[:ln.value])
+
+    def create_proofs(self, advice_list, instances_list, rng_seeds):
+        """Many proofs on this key in one call: proof p = create_proof(advice_list[p], instances_list[p], rng_seeds[p]),
+        byte for byte.  The proofs run in groups, phase by phase (h2v_create_proofs) -> list of proof bytes"""
+        B = len(advice_list)
+        if len(instances_list) != B or len(rng_seeds) != B:
+            raise ValueError("create_proofs: advice_list, instances_list and rng_seeds differ in length")
+        if not B:
+            return []
+        n = 1 << self.cs["k"]
+        keep, adv_ptrs, inst_ptrs, len_ptrs = [], [], [], []
+        for p, (advice, instances, seed) in enumerate(zip(advice_list, instances_list, rng_seeds)):
+            adv = [_fr(c, n) for c in advice]
+            if len(adv) != self.cs["n_advice"] or len(instances) != self.cs["n_instance"]:
+                raise ValueError(f"create_proofs: proof {p}: advice / instance column count does not match the constraint system")
+            if len(bytes(seed)) != 32:
+                raise ValueError(f"create_proofs: proof {p}: the rng seed is not 32 bytes")
+            inst = [_fr(np.asarray(c, dtype=np.uint64).reshape(-1, 4)) for c in instances]
+            aa = (C.c_void_p * max(1, len(adv)))(*[c.ctypes.data for c in adv])
+            ia = (C.c_void_p * max(1, len(inst)))(*[c.ctypes.data for c in inst])
+            il = np.ascontiguousarray([c.shape[0] for c in inst] or [0], dtype=np.uint32)
+            keep += [adv, inst, aa, ia, il]
+            adv_ptrs.append(C.cast(aa, C.c_void_p))
+            inst_ptrs.append(C.cast(ia, C.c_void_p))
+            len_ptrs.append(il.ctypes.data)
+        seeds = b"".join(bytes(s_) for s_ in rng_seeds)
+        size = self.proof_size()
+        out = np.zeros(B * size, dtype=np.uint8)
+        arr = lambda xs: (C.c_void_p * B)(*xs)
+        _check(lib().h2v_create_proofs(self._h, B, arr(adv_ptrs), arr(inst_ptrs), arr(len_ptrs), seeds, _ptr(out), size))
+        return [bytes(out[p * size:(p + 1) * size]) for p in range(B)]
 
     def last_phase_ms(self):
         buf = (C.c_double * 8)()

@@ -282,6 +282,7 @@ struct DomRep {
     bool tw_ready[4] = {false, false, false, false};
     DevBuf stage_a, stage_b, pipe_a, pipe_b, pipe_a2, pipe_b2;
     DevBuf peer_in, peer_out;      // columns of another device's batch (h2v_domain_transform_dev with several devices)
+    DevBuf qargs;                  // a quotient entry point's per-proof scalars and column table (under mu)
     cudaStream_t stream = nullptr, pipe_stream = nullptr, pipe_stream2 = nullptr;
     std::mutex mu, tw_mu, peer_mu;
     struct Lane {            // small host-facing transforms from concurrent caller threads (see SrsRep::Lane)
@@ -1713,45 +1714,67 @@ int h2v_grand_product_dev(const void *d_num, const void *d_den, size_t n, size_t
         return run_grand_product(g_poly.st, (const fe *)d_num, (const fe *)d_den, (uint32_t)n, (uint32_t)n_cols, (fe *)d_out);
     });
 }
-// a, q device-resident (q: n - 1 coefficients, must not overlap a); g_poly.mu held by the caller
-static int run_kate_division(cudaStream_t st, const fe *a, uint32_t n, const fe &b, fe *q) {
+// every job's division in one set of launches (poly.cuh KateCol); a, q device-resident (q: n - 1 coefficients, must not
+// overlap a); g_poly.mu held by the caller
+static int run_kate_division(cudaStream_t st, const KateJob *jobs, size_t n_jobs) {
     int rc;
-    const uint32_t ntiles = (n + H2V_FR_TILE - 1) / H2V_FR_TILE;
-    if ((rc = g_poly.d.ensure(((size_t)ntiles + 1) * sizeof(fe)))) return rc;
-    KateParams kp;
-    kp.a = a;
-    kp.q = q;
-    kp.n = n;
-    kp.b = b;
-    kp.tile = g_poly.d.as<fe>();
-    if (fe_is_zero(kp.b)) {
-        kate_shift_kernel<<<(n + 255) / 256, 256, 0, st>>>(kp.a, kp.q, kp.n);
-        H2V_LAUNCHED();
-    } else {
-        kp.binv = fe_inv<Fr>(kp.b);      // one host-side inversion of the evaluation point
-        kate_tiles_kernel<<<ntiles, 256, 0, st>>>(kp);
-        H2V_LAUNCHED();
-        fr_scan_top_kernel<OpAdd><<<1, 256, 0, st>>>(kp.tile, ntiles);
-        H2V_LAUNCHED();
-        kate_apply_kernel<<<ntiles, 256, 0, st>>>(kp);
-        H2V_LAUNCHED();
+    std::vector<KateCol> cols;
+    uint32_t nmax = 0;
+    for (size_t j = 0; j < n_jobs; ++j) {
+        if (jobs[j].n <= 1) continue;
+        KateCol c;
+        c.a = (const fe *)jobs[j].a;
+        c.q = (fe *)jobs[j].q;
+        c.n = (uint32_t)jobs[j].n;
+        c.b = fe_from_u64x4(jobs[j].b);
+        c.binv = fe_is_zero(c.b) ? fe_zero() : fe_inv<Fr>(c.b);      // one host-side inversion per point
+        cols.push_back(c);
+        nmax = std::max(nmax, c.n);
     }
+    if (cols.empty()) return H2V_OK;
+    if (cols.size() > 65535) return failf(H2V_EINVAL, "kate_division: %zu columns in one call", cols.size());
+    const uint32_t ntiles = (nmax + H2V_FR_TILE - 1) / H2V_FR_TILE;
+    if ((rc = g_poly.d.ensure((cols.size() * ntiles + 1) * sizeof(fe))) || (rc = g_poly.e.ensure(cols.size() * sizeof(KateCol)))) return rc;
+    H2V_CU(cudaMemcpyAsync(g_poly.e.p, cols.data(), cols.size() * sizeof(KateCol), cudaMemcpyHostToDevice, st));
+    const KateCol *d_cols = g_poly.e.as<KateCol>();
+    fe *tile = g_poly.d.as<fe>();
+    const dim3 grid(ntiles, (unsigned)cols.size());
+    kate_tiles_kernel<<<grid, 256, 0, st>>>(d_cols, tile, ntiles);
+    H2V_LAUNCHED();
+    fr_scan_top_kernel<OpAdd><<<dim3(1, (unsigned)cols.size()), 256, 0, st>>>(tile, ntiles);
+    H2V_LAUNCHED();
+    kate_apply_kernel<<<grid, 256, 0, st>>>(d_cols, tile, ntiles);
+    H2V_LAUNCHED();
     return H2V_OK;
 }
-int h2v_kate_division_dev(const void *d_a, size_t n, const uint64_t b[4], void *d_out) {
-    if (n <= 1) return H2V_OK;
-    if (!d_a || !b || !d_out) return failf(H2V_EINVAL, "kate_division: NULL buffer");
-    if (n >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "kate_division: n too large");
-    t_dev = device_of(d_a);
+}  // extern "C"
+namespace h2v {
+int kate_division_batch_dev(const KateJob *jobs, size_t n_jobs) {
+    if (!n_jobs) return H2V_OK;
+    if (!jobs) return failf(H2V_EINVAL, "kate_division: NULL job list");
+    for (size_t j = 0; j < n_jobs; ++j) {
+        if (jobs[j].n <= 1) continue;
+        if (!jobs[j].a || !jobs[j].q) return failf(H2V_EINVAL, "kate_division: NULL buffer");
+        if (jobs[j].n >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "kate_division: n too large");
+    }
+    t_dev = device_of(jobs[0].a);
     int rc = use_device();
     if (rc) return rc;
     std::lock_guard<std::mutex> lk(g_poly.mu);
     if ((rc = poly_ctx_ready())) return rc;
-    rc = run_kate_division(g_poly.st, (const fe *)d_a, (uint32_t)n, fe_from_u64x4(b), (fe *)d_out);
+    rc = run_kate_division(g_poly.st, jobs, n_jobs);
     cudaError_t e = cudaStreamSynchronize(g_poly.st);
     if (rc) return rc;
     if (e != cudaSuccess) return failf(H2V_ECUDA, "kate_division: %s", cudaGetErrorString(e));
     return H2V_OK;
+}
+}  // namespace h2v
+extern "C" {
+int h2v_kate_division_dev(const void *d_a, size_t n, const uint64_t b[4], void *d_out) {
+    if (n <= 1) return H2V_OK;
+    if (!d_a || !b || !d_out) return failf(H2V_EINVAL, "kate_division: NULL buffer");
+    KateJob job{d_a, d_out, n, {b[0], b[1], b[2], b[3]}};
+    return kate_division_batch_dev(&job, 1);
 }
 int h2v_kate_division(const uint64_t *a, size_t n, const uint64_t b[4], uint64_t *out) {
     if (n <= 1) return H2V_OK;
@@ -1765,7 +1788,8 @@ int h2v_kate_division(const uint64_t *a, size_t n, const uint64_t b[4], uint64_t
     cudaStream_t st = g_poly.st;
     if ((rc = g_poly.a.ensure(n * sizeof(fe))) || (rc = g_poly.b.ensure(n * sizeof(fe)))) return rc;
     H2V_CU(cudaMemcpyAsync(g_poly.a.p, a, n * sizeof(fe), cudaMemcpyHostToDevice, st));
-    if ((rc = run_kate_division(st, g_poly.a.as<fe>(), (uint32_t)n, fe_from_u64x4(b), g_poly.b.as<fe>()))) {
+    const KateJob job{g_poly.a.p, g_poly.b.p, n, {b[0], b[1], b[2], b[3]}};
+    if ((rc = run_kate_division(st, &job, 1))) {
         cudaStreamSynchronize(st);
         return rc;
     }
@@ -1921,20 +1945,33 @@ int h2v_permute_expression_pair(const uint64_t *input, const uint64_t *table, si
 // ================================================================== quotient evaluation ("next" row 1)
 namespace {
 // the replica that holds d_h (made current) and the constants every quotient kernel takes
-int quotient_common(h2v_domain_t h, const void *d_h, const uint64_t *y, DomRep **d, QuotientCommon *c) {
+int quotient_common(h2v_domain_t h, const void *d_h, DomRep **d, QuotientCommon *c) {
     if (!(*d = dom_rep(h, d_h))) return H2V_EINVAL;
-    if (!d_h || !y) return failf(H2V_EINVAL, "quotient: NULL buffer");
-    c->y = fe_from_u64x4(y);
+    if (!d_h) return failf(H2V_EINVAL, "quotient: NULL buffer");
     c->n_ext = 1u << (*d)->ek;
     c->rot = 1u << ((*d)->ek - (*d)->k);
     return use_device();
+}
+// one proof's y, beta, gamma (and `extra_bytes` behind them) into the replica's argument buffer, on its stream: the
+// public entry points are groups of one; d->mu held by the caller
+int quotient_args(DomRep *d, const uint64_t *y, const uint64_t *beta, const uint64_t *gamma, const void *extra, size_t extra_bytes,
+                  QuotientGroup *g, const void **extra_dev) {
+    const fe host[3] = {fe_from_u64x4(y), beta ? fe_from_u64x4(beta) : fe_zero(), gamma ? fe_from_u64x4(gamma) : fe_zero()};
+    H2V_TRY(d->qargs.ensure(sizeof host + extra_bytes));
+    H2V_CU(cudaMemcpyAsync(d->qargs.p, host, sizeof host, cudaMemcpyHostToDevice, d->stream));
+    if (extra_bytes)
+        H2V_CU(cudaMemcpyAsync((char *)d->qargs.p + sizeof host, extra, extra_bytes, cudaMemcpyHostToDevice, d->stream));
+    g->scal = d->qargs.as<fe>();
+    if (extra_dev) *extra_dev = (const char *)d->qargs.p + sizeof host;
+    return H2V_OK;
 }
 // the gate columns as strided arrays (ColsStrided) or device tables of column pointers (ColsTable)
 template <class Cols> int quotient_gates(h2v_domain_t h, void *d_h, const uint64_t y[4], size_t n_gates, Cols q, Cols a) {
     DomRep *d;
     QuotientCommon c;
-    int rc = quotient_common(h, d_h, y, &d, &c);
+    int rc = quotient_common(h, d_h, &d, &c);
     if (rc) return rc;
+    if (!y) return failf(H2V_EINVAL, "quotient: NULL buffer");
     if (!n_gates) return H2V_OK;
     if constexpr (std::is_same<Cols, ColsStrided>::value) {
         if (!q.base || !a.base) return failf(H2V_EINVAL, "quotient_gates: NULL buffer");
@@ -1945,21 +1982,45 @@ template <class Cols> int quotient_gates(h2v_domain_t h, void *d_h, const uint64
         if (n_gates > (1u << 20)) return failf(H2V_EINVAL, "quotient_gates: too many gates");
     }
     return sync_call(d->mu, d->stream, 7, "quotient", [&](Timer &) {
-        quotient_gates_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, (uint32_t)n_gates, q, a);
+        QuotientGroup g{(fe *)d_h, 0, nullptr};
+        H2V_TRY(quotient_args(d, y, nullptr, nullptr, nullptr, 0, &g, nullptr));
+        quotient_gates_kernel<<<dim3((c.n_ext + 255) / 256, 1), 256, 0, d->stream>>>(g, c, (uint32_t)n_gates, q, a);
         H2V_LAUNCHED();
         return H2V_OK;
     });
+}
+// the permutation argument's constants for the sets [set_begin, set_end)
+int perm_params(DomRep *d, size_t n_cols, size_t chunk_len, const void *d_z, size_t z_stride, const void *d_l0, const void *d_l_last,
+                const void *d_l_active, uint32_t blinding_factors, size_t set_begin, size_t set_end, int with_head, QuotientPerm *p) {
+    p->delta = fe_pow_u64<Fr>(fr_from_small(7), (uint64_t)1 << 28);   // Fr::DELTA = MULTIPLICATIVE_GENERATOR^(2^S)
+    p->g_coset = d->g_coset;
+    p->n_cols = (uint32_t)n_cols;
+    p->chunk_len = (uint32_t)std::min<size_t>(chunk_len, n_cols);
+    p->n_sets = (p->n_cols + p->chunk_len - 1) / p->chunk_len;
+    p->last_rot = -(int)(blinding_factors + 1);
+    p->z = (const fe *)d_z;
+    p->z_stride = z_stride;
+    p->z_pstride = 0;
+    p->l0 = (const fe *)d_l0; p->l_last = (const fe *)d_l_last; p->l_active = (const fe *)d_l_active;
+    if (set_end == (size_t)-1) set_end = p->n_sets;
+    if (set_begin > set_end || set_end > p->n_sets)
+        return failf(H2V_EINVAL, "quotient_permutation: set range [%zu, %zu) of %u sets", set_begin, set_end, p->n_sets);
+    p->set_begin = (uint32_t)set_begin;
+    p->set_end = (uint32_t)set_end;
+    p->head = with_head ? 1u : 0u;
+    p->delta_begin = fe_pow_u64<Fr>(p->delta, (uint64_t)set_begin * p->chunk_len);
+    return domain_twiddles(d, 2, &p->tw);
 }
 }  // namespace
 
 extern "C" {
 int h2v_quotient_gates_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], size_t n_gates, const void *d_q, size_t q_stride, const void *d_a,
                            size_t a_stride) {
-    return quotient_gates(h, d_h, y, n_gates, ColsStrided{(const fe *)d_q, q_stride}, ColsStrided{(const fe *)d_a, a_stride});
+    return quotient_gates(h, d_h, y, n_gates, ColsStrided{(const fe *)d_q, q_stride, 0}, ColsStrided{(const fe *)d_a, a_stride, 0});
 }
 int h2v_quotient_gates_ptrs_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], size_t n_gates, const void *const *d_q_ptrs,
                                 const void *const *d_a_ptrs) {
-    return quotient_gates(h, d_h, y, n_gates, ColsTable{(const fe *const *)d_q_ptrs}, ColsTable{(const fe *const *)d_a_ptrs});
+    return quotient_gates(h, d_h, y, n_gates, ColsTable{(const fe *const *)d_q_ptrs, 0}, ColsTable{(const fe *const *)d_a_ptrs, 0});
 }
 static int quotient_permutation_any(h2v_domain_t h, void *d_h, const uint64_t y[4], const uint64_t beta[4], const uint64_t gamma[4],
                                     size_t n_cols, size_t chunk_len, const void *d_cols, size_t cols_stride, const void *d_sigma,
@@ -1968,8 +2029,9 @@ static int quotient_permutation_any(h2v_domain_t h, void *d_h, const uint64_t y[
                                     size_t set_end = (size_t)-1, int with_head = 1) {
     DomRep *d;
     QuotientCommon c;
-    int rc = quotient_common(h, d_h, y, &d, &c);
+    int rc = quotient_common(h, d_h, &d, &c);
     if (rc) return rc;
+    if (!y) return failf(H2V_EINVAL, "quotient: NULL buffer");
     if (!n_cols) return H2V_OK;   // upstream: `if !sets.is_empty()`
     if (!beta || !gamma || !d_cols || !d_sigma || !d_z || !d_l0 || !d_l_last || !d_l_active)
         return failf(H2V_EINVAL, "quotient_permutation: NULL buffer");
@@ -1978,31 +2040,18 @@ static int quotient_permutation_any(h2v_domain_t h, void *d_h, const uint64_t y[
     if ((!tables && (cols_stride < c.n_ext || sigma_stride < c.n_ext)) || z_stride < c.n_ext)
         return failf(H2V_EINVAL, "quotient_permutation: stride shorter than 2^extended_k");
     QuotientPerm p;
-    p.beta = fe_from_u64x4(beta);
-    p.gamma = fe_from_u64x4(gamma);
-    p.delta = fe_pow_u64<Fr>(fr_from_small(7), (uint64_t)1 << 28);   // Fr::DELTA = MULTIPLICATIVE_GENERATOR^(2^S)
-    p.beta_zeta = fe_mul<Fr>(p.beta, d->g_coset);
-    p.n_cols = (uint32_t)n_cols;
-    p.chunk_len = (uint32_t)std::min<size_t>(chunk_len, n_cols);
-    p.n_sets = (p.n_cols + p.chunk_len - 1) / p.chunk_len;
-    p.last_rot = -(int)(blinding_factors + 1);
-    p.z = (const fe *)d_z;
-    p.z_stride = z_stride;
-    p.l0 = (const fe *)d_l0; p.l_last = (const fe *)d_l_last; p.l_active = (const fe *)d_l_active;
-    if (set_end == (size_t)-1) set_end = p.n_sets;
-    if (set_begin > set_end || set_end > p.n_sets) return failf(H2V_EINVAL, "quotient_permutation: set range [%zu, %zu) of %u sets", set_begin, set_end, p.n_sets);
-    p.set_begin = (uint32_t)set_begin;
-    p.set_end = (uint32_t)set_end;
-    p.head = with_head ? 1u : 0u;
-    p.delta_begin = fe_pow_u64<Fr>(p.delta, (uint64_t)set_begin * p.chunk_len);
-    if ((rc = domain_twiddles(d, 2, &p.tw))) return rc;
+    if ((rc = perm_params(d, n_cols, chunk_len, d_z, z_stride, d_l0, d_l_last, d_l_active, blinding_factors, set_begin, set_end, with_head, &p)))
+        return rc;
     return sync_call(d->mu, d->stream, 7, "quotient", [&](Timer &) {
+        QuotientGroup g{(fe *)d_h, 0, nullptr};
+        H2V_TRY(quotient_args(d, y, beta, gamma, nullptr, 0, &g, nullptr));
+        const dim3 grid((c.n_ext + 255) / 256, 1);
         if (tables)
-            quotient_permutation_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, p, ColsTable{(const fe *const *)d_cols},
-                                                                                      ColsTable{(const fe *const *)d_sigma});
+            quotient_permutation_kernel<<<grid, 256, 0, d->stream>>>(g, c, p, ColsTable{(const fe *const *)d_cols, 0},
+                                                                    ColsTable{(const fe *const *)d_sigma, 0});
         else
-            quotient_permutation_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, p, ColsStrided{(const fe *)d_cols, cols_stride},
-                                                                                      ColsStrided{(const fe *)d_sigma, sigma_stride});
+            quotient_permutation_kernel<<<grid, 256, 0, d->stream>>>(g, c, p, ColsStrided{(const fe *)d_cols, cols_stride, 0},
+                                                                    ColsStrided{(const fe *)d_sigma, sigma_stride, 0});
         H2V_LAUNCHED();
         return H2V_OK;
     });
@@ -2033,24 +2082,61 @@ int h2v_quotient_lookup_dev(h2v_domain_t h, void *d_h, const uint64_t y[4], cons
                             const void *d_l0, const void *d_l_last, const void *d_l_active) {
     DomRep *d;
     QuotientCommon c;
-    int rc = quotient_common(h, d_h, y, &d, &c);
+    int rc = quotient_common(h, d_h, &d, &c);
     if (rc) return rc;
-    if (!beta || !gamma || !d_input || !d_table || !d_perm_input || !d_perm_table || !d_z || !d_l0 || !d_l_last || !d_l_active)
+    if (!y || !beta || !gamma || !d_input || !d_table || !d_perm_input || !d_perm_table || !d_z || !d_l0 || !d_l_last || !d_l_active)
         return failf(H2V_EINVAL, "quotient_lookup: NULL buffer");
-    QuotientLookup p;
-    p.beta = fe_from_u64x4(beta);
-    p.gamma = fe_from_u64x4(gamma);
-    p.input = (const fe *)d_input; p.table = (const fe *)d_table;
-    p.perm_input = (const fe *)d_perm_input; p.perm_table = (const fe *)d_perm_table;
-    p.z = (const fe *)d_z;
-    p.l0 = (const fe *)d_l0; p.l_last = (const fe *)d_l_last; p.l_active = (const fe *)d_l_active;
+    const void *tab[5] = {d_input, d_table, d_perm_input, d_perm_table, d_z};
     return sync_call(d->mu, d->stream, 7, "quotient", [&](Timer &) {
-        quotient_lookup_kernel<<<(c.n_ext + 255) / 256, 256, 0, d->stream>>>((fe *)d_h, c, p);
+        QuotientGroup g{(fe *)d_h, 0, nullptr};
+        const void *d_tab = nullptr;
+        H2V_TRY(quotient_args(d, y, beta, gamma, tab, sizeof tab, &g, &d_tab));
+        QuotientLookup p{(const fe *const *)d_tab, 0, 1, (const fe *)d_l0, (const fe *)d_l_last, (const fe *)d_l_active};
+        quotient_lookup_kernel<<<dim3((c.n_ext + 255) / 256, 1), 256, 0, d->stream>>>(g, c, p);
         H2V_LAUNCHED();
         return H2V_OK;
     });
 }
 }  // extern "C"
+
+namespace h2v {
+// evaluate_h's three folds for a group of proofs, one launch each (gates, permutation, lookups: upstream's order)
+int quotient_batch_dev(h2v_domain_t h, const QuotientBatch &b) {
+    DomRep *d;
+    QuotientCommon c;
+    int rc = quotient_common(h, b.h, &d, &c);
+    if (rc) return rc;
+    if (!b.n_proofs) return H2V_OK;
+    if (!b.scal || b.n_proofs > 65535) return failf(H2V_EINVAL, "quotient: no per-proof scalars, or more than 65535 proofs");
+    QuotientPerm p;
+    if (b.n_perm) {
+        if ((rc = perm_params(d, b.n_perm, b.chunk, b.z, b.z_stride, b.l0, b.l_last, b.l_active, b.blinding_factors, 0, (size_t)-1, 1, &p)))
+            return rc;
+        p.z_pstride = b.z_pstride;
+    }
+    return sync_call(d->mu, d->stream, 7, "quotient", [&](Timer &) {
+        const QuotientGroup g{(fe *)b.h, b.h_stride, (const fe *)b.scal};
+        const dim3 grid((c.n_ext + 255) / 256, (unsigned)b.n_proofs);
+        const fe *const *gt = (const fe *const *)b.gate_tab, *const *pt = (const fe *const *)b.perm_tab;
+        if (b.n_gates) {
+            quotient_gates_kernel<<<grid, 256, 0, d->stream>>>(g, c, (uint32_t)b.n_gates, ColsTable{gt, b.gate_pstride},
+                                                              ColsTable{gt + b.n_gates, b.gate_pstride});
+            H2V_LAUNCHED();
+        }
+        if (b.n_perm) {
+            quotient_permutation_kernel<<<grid, 256, 0, d->stream>>>(g, c, p, ColsTable{pt, b.perm_pstride}, ColsTable{pt + b.n_perm, b.perm_pstride});
+            H2V_LAUNCHED();
+        }
+        if (b.n_lookups) {
+            const QuotientLookup q{(const fe *const *)b.lookup_tab, b.lookup_pstride, (uint32_t)b.n_lookups, (const fe *)b.l0,
+                                   (const fe *)b.l_last, (const fe *)b.l_active};
+            quotient_lookup_kernel<<<grid, 256, 0, d->stream>>>(g, c, q);
+            H2V_LAUNCHED();
+        }
+        return H2V_OK;
+    });
+}
+}  // namespace h2v
 
 // ================================================================== self-tests
 namespace {

@@ -44,6 +44,41 @@ struct DevBuf {
     }
     template <class T> T *as() const { return reinterpret_cast<T *>(p); }
 };
+
+// Entry points of the group prover (prover.cu), not part of the C ABI.
+// Kate division of many device columns in one set of launches: job j divides a[0 .. n) by (X - b) into q[0 .. n - 1)
+// (b: Montgomery limbs, as h2v_kate_division_dev takes it).  Synchronous.
+struct KateJob {
+    const void *a;
+    void *q;
+    size_t n;
+    uint64_t b[4];
+};
+int kate_division_batch_dev(const KateJob *jobs, size_t n_jobs);
+// evaluate_h's folds for n_proofs proofs, one launch per argument: proof p folds into h + p * h_stride with y, beta, gamma
+// = scal[3p .. 3p + 2] (device); its gate table is n_gates selectors then n_gates advice columns at gate_tab + p * gate_pstride,
+// its permutation table n_perm columns then n_perm sigma columns at perm_tab + p * perm_pstride, its products at
+// z + p * z_pstride, its lookups 5 columns each (input, table, A', S', z) at lookup_tab + p * lookup_pstride.  Synchronous.
+struct QuotientBatch {
+    void *h;
+    size_t h_stride;
+    const void *scal;
+    size_t n_proofs;
+    size_t n_gates;
+    const void *const *gate_tab;
+    size_t gate_pstride;
+    size_t n_perm, chunk;
+    const void *const *perm_tab;
+    size_t perm_pstride;
+    const void *z;
+    size_t z_stride, z_pstride;
+    uint32_t blinding_factors;
+    size_t n_lookups;
+    const void *const *lookup_tab;
+    size_t lookup_pstride;
+    const void *l0, *l_last, *l_active;
+};
+int quotient_batch_dev(h2v_domain_t h, const QuotientBatch &b);
 }  // namespace h2v
 
 #define H2V_CU(x)                                                                                                  \

@@ -202,16 +202,17 @@ __global__ void __launch_bounds__(256) fr_prod_apply_kernel(const fe *__restrict
 }
 
 // ------------------------------------------------------------------ kate_division
-// q[i] = b^-(i+1) * S[i+1],  S[k] = sum_{j >= k} a[j] b^j  (b != 0).  Forward index k <-> j = n-1-k:
-// t_k = a[n-1-k] b^(n-1-k), inclusive prefix sums P_k = S[n-1-k], q[n-2-k] = P_k * binv^(n-1-k).
-struct KateParams {
+// Many columns at once (grid.y = column), each with its own length and point: column j divides a[0 .. n) by (X - b)
+// into q[0 .. n - 1).  q[i] = b^-(i+1) * S[i+1],  S[k] = sum_{j >= k} a[j] b^j  (b != 0).  Forward index k <-> j = n-1-k:
+// t_k = a[n-1-k] b^(n-1-k), inclusive prefix sums P_k = S[n-1-k], q[n-2-k] = P_k * binv^(n-1-k).  b == 0: q[i] = a[i+1].
+// The tile sums of column j lie at tile + j * ntiles (ntiles covers the longest column).
+struct KateCol {
     const fe *a;
     fe *q;
     uint32_t n;
-    fe b, binv;
-    fe *tile;
+    fe b, binv;      // binv: unused when b == 0
 };
-__device__ __forceinline__ void kate_thread(const KateParams &p, uint32_t base, fe (&t)[8], fe &sum) {
+__device__ __forceinline__ void kate_thread(const KateCol &p, uint32_t base, fe (&t)[8], fe &sum) {
     // powers b^(n-1-base), then multiply by binv per step
     fe pw = (base < p.n) ? fe_pow_small<Fr>(p.b, p.n - 1 - base) : fe_zero();
     sum = fe_zero();
@@ -226,19 +227,27 @@ __device__ __forceinline__ void kate_thread(const KateParams &p, uint32_t base, 
         sum = fe_add<Fr>(sum, t[k]);
     }
 }
-__global__ void __launch_bounds__(256) kate_tiles_kernel(KateParams p) {
+__global__ void __launch_bounds__(256) kate_tiles_kernel(const KateCol *cols, fe *tile, uint32_t ntiles) {
     __shared__ fe sm8[8];
+    const KateCol p = cols[blockIdx.y];
+    if (fe_is_zero(p.b)) return;          // the shift needs no tile sums (uniform over the CTA)
     fe t[8], s, tot;
     kate_thread(p, blockIdx.x * H2V_FR_TILE + threadIdx.x * 8, t, s);
     block_excl_scan_256<OpAdd>(s, &tot, sm8);
-    if (threadIdx.x == 0) pl_st(p.tile + blockIdx.x, tot);
+    if (threadIdx.x == 0) pl_st(tile + (size_t)blockIdx.y * ntiles + blockIdx.x, tot);
 }
-__global__ void __launch_bounds__(256) kate_apply_kernel(KateParams p) {
+__global__ void __launch_bounds__(256) kate_apply_kernel(const KateCol *cols, const fe *tile, uint32_t ntiles) {
     __shared__ fe sm8[8];
+    const KateCol p = cols[blockIdx.y];
     const uint32_t base = blockIdx.x * H2V_FR_TILE + threadIdx.x * 8;
+    if (fe_is_zero(p.b)) {
+        for (uint32_t i = base; i < base + 8; ++i)
+            if (i + 1 < p.n) pl_st(p.q + i, pl_ld(p.a + i + 1));
+        return;
+    }
     fe t[8], s, tot;
     kate_thread(p, base, t, s);
-    fe run = fe_add<Fr>(block_excl_scan_256<OpAdd>(s, &tot, sm8), pl_ld(p.tile + blockIdx.x));
+    fe run = fe_add<Fr>(block_excl_scan_256<OpAdd>(s, &tot, sm8), pl_ld(tile + (size_t)blockIdx.y * ntiles + blockIdx.x));
     // output factor binv^(n-1-k), stepping up by b
     fe f = (base < p.n) ? fe_pow_small<Fr>(p.binv, p.n - 1 - base) : fe_zero();
 #pragma unroll 1
@@ -248,11 +257,6 @@ __global__ void __launch_bounds__(256) kate_apply_kernel(KateParams p) {
         if (kk + 1 < p.n) pl_st(p.q + (p.n - 2 - kk), fe_mul<Fr>(run, f));
         f = fe_mul<Fr>(f, p.b);
     }
-}
-// b == 0: q[i] = a[i+1]
-__global__ void __launch_bounds__(256) kate_shift_kernel(const fe *__restrict__ a, fe *__restrict__ q, uint32_t n) {
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i + 1 < n) pl_st(q + i, pl_ld(a + i + 1));
 }
 
 }  // namespace h2v

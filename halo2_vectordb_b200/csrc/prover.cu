@@ -23,7 +23,10 @@
 
 #include <algorithm>
 #include <map>
+#include <memory>
 #include <mutex>
+#include <string>
+#include <thread>
 #include <vector>
 
 #include "h2v.h"
@@ -62,39 +65,50 @@ __device__ __forceinline__ void st(fe *p, const fe &x) {
     q[1] = make_uint4(x.v[4], x.v[5], x.v[6], x.v[7]);
 }
 
-// permutation argument, plonk/permutation/prover.rs `Argument::commit`: for set s (grid.y) and row i
+// A group of B proofs on one key runs phase by phase: proof p's columns of one kind lie after proof p-1's, and the
+// kernels below take the proof on grid.z (grid.y where there is no other dimension) with its challenges from a small
+// device array (beta_gamma[2p] = beta, beta_gamma[2p + 1] = gamma of proof p).
+
+// permutation argument, plonk/permutation/prover.rs `Argument::commit`: for proof p (grid.z), set s (grid.y) and row i
 //   den[s][i] = prod_{c in set} (v_c[i] + beta sigma_c[i] + gamma),  num[s][i] = prod (v_c[i] + beta delta^c w^i + gamma)
 struct PermArgs {
-    const fe *const *cols;      // n_cols Lagrange columns in permutation order
-    const fe *const *sigma;     // their sigma polynomials, Lagrange
+    const fe *const *cols;      // n_cols Lagrange columns in permutation order, per proof (n_cols apart)
+    const fe *const *sigma;     // their sigma polynomials, Lagrange (the key's: shared by the proofs)
     const fe *omega_pows;       // w^i
     const fe *delta_start;      // per set: delta^(s * chunk)
-    fe beta, gamma, delta;
+    const fe *beta_gamma;       // per proof
+    fe delta;
     uint32_t n_cols, chunk, n;
 };
 __global__ void __launch_bounds__(256) perm_numden_kernel(PermArgs a, fe *num, fe *den) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x, s = blockIdx.y;
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x, s = blockIdx.y, p = blockIdx.z;
     if (i >= a.n) return;
+    const fe *const *cols = a.cols + (size_t)p * a.n_cols;
+    const fe beta = ld(a.beta_gamma + 2 * p), gamma = ld(a.beta_gamma + 2 * p + 1);
     const uint32_t c0 = s * a.chunk, c1 = min(c0 + a.chunk, a.n_cols);
-    fe cur = fe_mul<Fr>(fe_mul<Fr>(a.beta, ld(a.omega_pows + i)), ld(a.delta_start + s));
+    fe cur = fe_mul<Fr>(fe_mul<Fr>(beta, ld(a.omega_pows + i)), ld(a.delta_start + s));
     fe nu = fe_one<Fr>(), de = fe_one<Fr>();
     for (uint32_t c = c0; c < c1; ++c) {
-        const fe v = fe_add<Fr>(ld(a.cols[c] + i), a.gamma);
-        de = fe_mul<Fr>(de, fe_add<Fr>(v, fe_mul<Fr>(a.beta, ld(a.sigma[c] + i))));
+        const fe v = fe_add<Fr>(ld(cols[c] + i), gamma);
+        de = fe_mul<Fr>(de, fe_add<Fr>(v, fe_mul<Fr>(beta, ld(a.sigma[c] + i))));
         nu = fe_mul<Fr>(nu, fe_add<Fr>(v, cur));
         cur = fe_mul<Fr>(cur, a.delta);
     }
-    st(num + (size_t)s * a.n + i, nu);
-    st(den + (size_t)s * a.n + i, de);
+    const size_t o = ((size_t)p * gridDim.y + s) * a.n + i;
+    st(num + o, nu);
+    st(den + o, de);
 }
-// lookup argument, plonk/lookup/prover.rs `Permuted::commit_product`: for lookup l (grid.y) and row i
+// lookup argument, plonk/lookup/prover.rs `Permuted::commit_product`: for proof p (grid.z), lookup l (grid.y) and row i
 //   den = (a'[i] + beta)(s'[i] + gamma),  num = (a[i] + beta)(t[i] + gamma)
+// inputs: per proof (L apart), tables: the key's; perm_in / perm_tab / num / den: column p * L + l
 __global__ void __launch_bounds__(256) lookup_numden_kernel(const fe *const *inputs, const fe *const *tables, const fe *perm_in,
-                                                            const fe *perm_tab, fe beta, fe gamma, uint32_t n, fe *num, fe *den) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x, l = blockIdx.y;
+                                                            const fe *perm_tab, const fe *beta_gamma, uint32_t n, fe *num, fe *den) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x, l = blockIdx.y, p = blockIdx.z;
     if (i >= n) return;
-    const size_t o = (size_t)l * n + i;
-    st(num + o, fe_mul<Fr>(fe_add<Fr>(ld(inputs[l] + i), beta), fe_add<Fr>(ld(tables[l] + i), gamma)));
+    const uint32_t col = p * gridDim.y + l;
+    const fe beta = ld(beta_gamma + 2 * p), gamma = ld(beta_gamma + 2 * p + 1);
+    const size_t o = (size_t)col * n + i;
+    st(num + o, fe_mul<Fr>(fe_add<Fr>(ld(inputs[col] + i), beta), fe_add<Fr>(ld(tables[l] + i), gamma)));
     st(den + o, fe_mul<Fr>(fe_add<Fr>(ld(perm_in + o), beta), fe_add<Fr>(ld(perm_tab + o), gamma)));
 }
 // cols[c][i] *= scalars[c]   (n_cols contiguous columns of n)
@@ -104,18 +118,21 @@ __global__ void __launch_bounds__(256) scale_cols_kernel(fe *cols, uint32_t n, c
     fe *p = cols + (size_t)blockIdx.y * n + i;
     st(p, fe_mul<Fr>(ld(p), ld(scalars + blockIdx.y)));
 }
-// out[i] = sum_j coef[j] * cols[j][i]
-__global__ void __launch_bounds__(256) lincomb_kernel(const fe *const *cols, const fe *coef, uint32_t n_cols, uint32_t n, fe *out) {
+// job j (grid.y): out[j * out_stride + i] = sum_{t in [off[j], off[j+1])} coef[t] * cols[t][i]
+__global__ void __launch_bounds__(256) lincomb_kernel(const fe *const *cols, const fe *coef, const uint32_t *off, uint32_t n, fe *out,
+                                                     size_t out_stride) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
+    const uint32_t t0 = off[blockIdx.y], t1 = off[blockIdx.y + 1];
     fe acc = fe_zero();
-    for (uint32_t j = 0; j < n_cols; ++j) acc = fe_add<Fr>(acc, fe_mul<Fr>(ld(cols[j] + i), ld(coef + j)));
-    st(out + i, acc);
+    for (uint32_t t = t0; t < t1; ++t) acc = fe_add<Fr>(acc, fe_mul<Fr>(ld(cols[t] + i), ld(coef + t)));
+    st(out + (size_t)blockIdx.y * out_stride + i, acc);
 }
-// a[i] -= low[i], i < cnt   (subtracting a low-degree polynomial)
-__global__ void sub_low_kernel(fe *a, const fe *low, uint32_t cnt) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < cnt) st(a + i, fe_sub<Fr>(ld(a + i), ld(low + i)));
+// job j (grid.x): a[j * stride + i] -= low[j * cnt + i], i < cnt   (subtracting a low-degree polynomial; a job with fewer
+// coefficients pads them with zeros, which leave a unchanged)
+__global__ void sub_low_kernel(fe *a, size_t stride, const fe *low, uint32_t cnt) {
+    fe *aj = a + (size_t)blockIdx.x * stride;
+    for (uint32_t i = threadIdx.x; i < cnt; i += blockDim.x) st(aj + i, fe_sub<Fr>(ld(aj + i), ld(low + (size_t)blockIdx.x * cnt + i)));
 }
 // arithmetic.rs eval_polynomial for a list of (polynomial, point) pairs: one CTA per pair, Horner over 256 slices
 struct EvalPair {
@@ -175,10 +192,17 @@ __device__ __forceinline__ fe canon_below_2_256(fe v) {      // v < 2^256 < 6r  
     }
     return v;
 }
-__global__ void __launch_bounds__(256) chacha_fr_kernel(ChaChaKey key, uint64_t counter0, uint32_t n, fe *out) {
+// proof p (grid.y) draws from its own key and block counter into out + p * n
+struct ChaChaStream {
+    ChaChaKey key;
+    uint64_t counter0;
+};
+__global__ void __launch_bounds__(256) chacha_fr_kernel(const ChaChaStream *streams, uint32_t n, fe *out) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const uint64_t ctr = counter0 + i;
+    const ChaChaKey key = streams[blockIdx.y].key;
+    const uint64_t ctr = streams[blockIdx.y].counter0 + i;
+    out += (size_t)blockIdx.y * n;
     uint32_t x0 = 0x61707865u, x1 = 0x3320646eu, x2 = 0x79622d32u, x3 = 0x6b206574u;
     uint32_t x4 = key.k[0], x5 = key.k[1], x6 = key.k[2], x7 = key.k[3], x8 = key.k[4], x9 = key.k[5], x10 = key.k[6], x11 = key.k[7];
     uint32_t x12 = (uint32_t)ctr, x13 = (uint32_t)(ctr >> 32), x14 = 0, x15 = 0;
@@ -253,9 +277,9 @@ struct h2v_pk {
     uint32_t u = 0, chunk = 0, n_sets = 0;
     Fr64 vk_repr, omega, omega_inv, delta;
     DevBuf fixed_L, fixed_C, fixed_E, sigma_L, sigma_C, sigma_E, lrows_E, omega_pows;
-    // per-proof workspace, kept between proofs
+    // workspace of a group of proofs (B times what one proof needs), kept between calls
     DevBuf adv_L, adv_C, adv_E, inst_L, inst_C, inst_E, pa_L, ps_L, pa_C, ps_C, pa_E, ps_E, z_L, z_C, z_E, zl_L, zl_C, zl_E;
-    DevBuf num, den, tails, ptrs, scal, pts, rnd_C, hq, hx_pieces, evals, pairs, sh_S, sh_A, sh_B, sh_h, commits;
+    DevBuf num, den, tails, ptrs, scal, offs, streams, pts, rnd_C, hq, hx_pieces, evals, pairs, sh_S, sh_A, sh_B, sh_T, sh_h, commits;
     // k = 20-sized keys: the extended-coset forms of the fixed / sigma / advice columns (4n each) are not kept -- the
     // quotient step rebuilds them from the coefficient forms in slices of `scr_cols` columns of `scr_E`
     bool stream_ext = false;
@@ -269,7 +293,7 @@ struct h2v_pk {
     cudaStream_t st = nullptr;
     int dev = 0;                 // the proof runs on the primary device (columns and key resident there)
     std::mutex mu;
-    double last_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // wall-clock per phase of the last create_proof
+    double last_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // wall-clock per phase of the last call, summed over its groups
 };
 
 namespace {
@@ -301,9 +325,9 @@ int commit_dev(h2v_pk *pk, int basis, const fe *cols, size_t n_cols, std::vector
     H2V_CU(cudaMemcpy(out.data(), pk->commits.p, n_cols * sizeof(affine), cudaMemcpyDeviceToHost));
     return H2V_OK;
 }
-int write_points(PoseidonTranscript &T, const std::vector<affine> &pts) {
-    for (const affine &p : pts)
-        if (!T.write_point(p)) return failf(H2V_EINVAL, "create_proof: Cannot write points at infinity to the transcript");
+int write_points(PoseidonTranscript &T, const affine *pts, size_t cnt) {
+    for (size_t i = 0; i < cnt; ++i)
+        if (!T.write_point(pts[i])) return failf(H2V_EINVAL, "create_proof: Cannot write points at infinity to the transcript");
     return H2V_OK;
 }
 struct PhaseClock {
@@ -326,8 +350,8 @@ void h2v_pk_free(h2v_pk_t pk) {
     DevBuf *all[] = {&pk->fixed_L, &pk->fixed_C, &pk->fixed_E, &pk->sigma_L, &pk->sigma_C, &pk->sigma_E, &pk->lrows_E, &pk->omega_pows,
                      &pk->adv_L, &pk->adv_C, &pk->adv_E, &pk->inst_L, &pk->inst_C, &pk->inst_E, &pk->pa_L, &pk->ps_L, &pk->pa_C, &pk->ps_C,
                      &pk->pa_E, &pk->ps_E, &pk->z_L, &pk->z_C, &pk->z_E, &pk->zl_L, &pk->zl_C, &pk->zl_E, &pk->num, &pk->den, &pk->tails,
-                     &pk->ptrs, &pk->scal, &pk->pts, &pk->rnd_C, &pk->hq, &pk->hx_pieces, &pk->evals, &pk->pairs, &pk->sh_S, &pk->sh_A,
-                     &pk->sh_B, &pk->sh_h, &pk->commits, &pk->scr_E, &pk->ext_cache};
+                     &pk->ptrs, &pk->scal, &pk->offs, &pk->streams, &pk->pts, &pk->rnd_C, &pk->hq, &pk->hx_pieces, &pk->evals, &pk->pairs, &pk->sh_S, &pk->sh_A,
+                     &pk->sh_B, &pk->sh_T, &pk->sh_h, &pk->commits, &pk->scr_E, &pk->ext_cache};
     for (DevBuf *b : all) b->release();
     if (pk->dom) h2v_domain_free(pk->dom);
     if (pk->st) cudaStreamDestroy(pk->st);
@@ -470,7 +494,7 @@ int h2v_pk_last_phase_ms(h2v_pk_t pk, double out[8]) {
 
 }  // extern "C"
 
-// ================================================================== create_proof
+// ================================================================== create_proof over a group of proofs
 namespace {
 
 struct Query {
@@ -479,206 +503,332 @@ struct Query {
     Fr64 eval;
 };
 
-int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_t *const *instances, const uint32_t *instance_len,
-                        const uint8_t rng_seed[32], std::vector<uint8_t> &proof) {
+// the arguments of one h2v_create_proof
+struct ProofIn {
+    const uint64_t *const *advice;
+    const uint64_t *const *instances;
+    const uint32_t *instance_len;
+    const uint8_t *seed;
+};
+// what one proof of a group carries from phase to phase: its own RNG, transcript and challenges
+struct ProofState {
+    PoseidonTranscript T;
+    ChaCha20Rng rng;
+    Fr64 beta, gamma, y, x, xn, ys, vs, uc;
+    explicit ProofState(const uint8_t *seed) : rng(seed) {}
+};
+
+// f(p) for every proof p < B, on up to B host threads (the proofs' transcripts and point-set arithmetic are independent).
+// h2v_last_error() is per thread: a worker's error text is carried back to the caller's thread.
+template <class F> int par_proofs(size_t B, F f) {
+    if (B == 1) return f(0);
+    const size_t W = std::min<size_t>(B, std::max(1u, std::thread::hardware_concurrency()));
+    std::vector<int> rc(B, H2V_OK);
+    std::vector<std::string> msg(B);
+    std::vector<std::thread> th;
+    for (size_t w = 0; w < W; ++w)
+        th.emplace_back([&, w] {
+            for (size_t p = w; p < B; p += W)
+                if ((rc[p] = f(p))) msg[p] = h2v_last_error();
+        });
+    for (auto &t : th) t.join();
+    for (size_t p = 0; p < B; ++p)
+        if (rc[p]) return set_error(rc[p], msg[p].c_str());
+    return H2V_OK;
+}
+
+// the host vector into a device buffer that grows to fit it (the stream is idle when this returns)
+template <class T> int put(h2v_pk *pk, DevBuf &b, const std::vector<T> &v) {
+    if (v.empty()) return H2V_OK;
+    if (v.size() * sizeof(T) > b.cap) H2V_TRY(sync(pk));      // nothing queued may still read the buffer that is replaced
+    H2V_TRY(b.ensure(v.size() * sizeof(T)));
+    return upload(pk, b, 0, v.data(), v.size() * sizeof(T));
+}
+// out + j * out_stride = sum_{t in [off[j], off[j+1])} coef[t] * cols[t] over `len` rows, one launch for every job
+int lincomb(h2v_pk *pk, const std::vector<const fe *> &cols, const std::vector<Fr64> &coef, const std::vector<uint32_t> &off, fe *out,
+            size_t out_stride, size_t len) {
+    H2V_TRY(put(pk, pk->ptrs, cols));
+    H2V_TRY(put(pk, pk->scal, coef));
+    H2V_TRY(put(pk, pk->offs, off));
+    lincomb_kernel<<<dim3((unsigned)((len + 255) / 256), (unsigned)(off.size() - 1)), 256, 0, pk->st>>>(
+        (const fe *const *)pk->ptrs.p, pk->scal.as<fe>(), pk->offs.as<uint32_t>(), (uint32_t)len, out, out_stride);
+    H2V_LAUNCHED();
+    return H2V_OK;
+}
+// a[j * stride + i] -= low[j][i] for every job j (low: the same number of coefficients per job, zero-padded)
+int sub_low(h2v_pk *pk, fe *a, size_t stride, const std::vector<Fr64> &low, size_t jobs) {
+    const uint32_t cnt = (uint32_t)(low.size() / jobs);
+    H2V_TRY(put(pk, pk->scal, low));
+    sub_low_kernel<<<(unsigned)jobs, 32, 0, pk->st>>>(a, stride, pk->scal.as<fe>(), cnt);
+    H2V_LAUNCHED();
+    return H2V_OK;
+}
+
+// The prover.  Proofs in[0 .. B) run in lockstep, phase by phase: every commit, transform, grand product and column
+// kernel of a phase is one call over the B proofs' columns (proof p's columns of a kind after proof p-1's), while each proof
+// keeps its own RNG (upstream's draw order) and transcript (its own challenges).  The caller holds pk->mu and has checked
+// the inputs; on a failure traced to one proof, `bad` is that proof (else it stays SIZE_MAX).
+int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector<uint8_t>> &proofs, size_t &bad) {
     const size_t n = pk->n, ne = pk->ne;
     const uint32_t A = pk->n_advice, F = pk->n_fixed, I = pk->n_instance, L = (uint32_t)pk->lookup_input.size(),
                    G = (uint32_t)pk->gate_advice.size(), NP = (uint32_t)pk->perm_kind.size(), NS = pk->n_sets, bf = pk->bf, u = pk->u;
+    const size_t BA = B * A, BI = B * I, BL = B * L, BS = B * NS;
     const unsigned gn = (unsigned)((n + 255) / 256);
     cudaStream_t st = pk->st;
     double t_phase = PhaseClock::now();
     int phase = 0;
     auto lap = [&]() {
         double t = PhaseClock::now();
-        if (phase < 8) pk->last_ms[phase++] = t - t_phase;
+        if (phase < 7) pk->last_ms[phase++] += t - t_phase;
         t_phase = t;
     };
-    for (double &v : pk->last_ms) v = 0;
+    bad = SIZE_MAX;
+    std::vector<std::unique_ptr<ProofState>> P;
+    for (size_t p = 0; p < B; ++p) P.emplace_back(new ProofState(in[p].seed));
 
-    PoseidonTranscript T;
-    ChaCha20Rng rng(rng_seed);
     // ---- 1. vk, instances                                                   (prover.rs: hash_into, common_scalar)
-    T.common_scalar(pk->vk_repr);
-    H2V_TRY(pk->inst_L.ensure(std::max<size_t>(1, I) * n * sizeof(fe)));
-    H2V_TRY(pk->inst_C.ensure(std::max<size_t>(1, I) * n * sizeof(fe)));
-    H2V_TRY(pk->inst_E.ensure(std::max<size_t>(1, I) * ne * sizeof(fe)));
+    for (auto &s : P) s->T.common_scalar(pk->vk_repr);
+    H2V_TRY(pk->inst_L.ensure(std::max<size_t>(1, BI) * n * sizeof(fe)));
+    H2V_TRY(pk->inst_C.ensure(std::max<size_t>(1, BI) * n * sizeof(fe)));
+    H2V_TRY(pk->inst_E.ensure(std::max<size_t>(1, BI) * ne * sizeof(fe)));
     if (I) {
-        std::vector<Fr64> inst(I * n, frh::zero());
-        for (uint32_t c = 0; c < I; ++c) {
-            if (instance_len[c] > u) return failf(H2V_EINVAL, "create_proof: InstanceTooLarge (%u values, %u usable rows)", instance_len[c], u);
-            for (uint32_t i = 0; i < instance_len[c]; ++i) {
-                inst[c * n + i] = frh::load(instances[c] + 4 * i);
-                T.common_scalar(inst[c * n + i]);
-            }
-        }
-        H2V_TRY(upload(pk, pk->inst_L, 0, inst.data(), I * n * sizeof(fe)));
-        H2V_TRY(h2v_domain_transform_dev(pk->dom, H2V_OP_LAGRANGE_TO_COEFF, pk->inst_L.p, n, pk->inst_C.p, n, I));
+        std::vector<Fr64> inst(BI * n, frh::zero());
+        for (size_t p = 0; p < B; ++p)
+            for (uint32_t c = 0; c < I; ++c)
+                for (uint32_t i = 0; i < in[p].instance_len[c]; ++i) {
+                    Fr64 &v = inst[(p * I + c) * n + i];
+                    v = frh::load(in[p].instances[c] + 4 * i);
+                    P[p]->T.common_scalar(v);
+                }
+        H2V_TRY(upload(pk, pk->inst_L, 0, inst.data(), BI * n * sizeof(fe)));
+        H2V_TRY(h2v_domain_transform_dev(pk->dom, H2V_OP_LAGRANGE_TO_COEFF, pk->inst_L.p, n, pk->inst_C.p, n, BI));
     }
     // ---- 2-4. advice columns: upload, blind the last blinding_factors + 1 rows, commit
-    H2V_TRY(pk->adv_L.ensure((size_t)A * n * sizeof(fe)));
-    H2V_TRY(pk->adv_C.ensure((size_t)A * n * sizeof(fe)));
-    for (uint32_t c = 0; c < A; ++c)
-        if (!advice[c]) return failf(H2V_EINVAL, "create_proof: advice[%u] is NULL", c);
-    // h2v_commit_batch_resident: each device uploads its block of the columns in sub-batches (the next one crosses while the
-    // previous one is committed), writes the tails, commits the block and leaves it in adv_L
-    std::vector<Fr64> tails((size_t)A * (bf + 1));
-    for (auto &t : tails) t = rng.fr_random();                       // column by column, rows u .. n-1
-    for (uint32_t c = 0; c < A; ++c) (void)rng.fr_random();          // one Blind per column (unused by KZG, but drawn)
-    std::vector<affine> pts(A);
-    H2V_TRY(h2v_commit_batch_resident(pk->srs, H2V_BASIS_LAGRANGE, advice, A, n, (const uint64_t *)tails.data(), u, bf + 1, pk->adv_L.p, n,
+    H2V_TRY(pk->adv_L.ensure(BA * n * sizeof(fe)));
+    H2V_TRY(pk->adv_C.ensure(BA * n * sizeof(fe)));
+    // h2v_commit_batch_resident: each device uploads its block of the B x A columns in sub-batches (the next one crosses
+    // while the previous one is committed), writes the tails, commits the block and leaves it in adv_L
+    std::vector<Fr64> tails(BA * (bf + 1));
+    std::vector<const uint64_t *> adv(BA);
+    for (size_t p = 0; p < B; ++p) {
+        ChaCha20Rng &rng = P[p]->rng;
+        for (size_t t = 0; t < (size_t)A * (bf + 1); ++t) tails[p * A * (bf + 1) + t] = rng.fr_random();   // column by column, rows u .. n-1
+        for (uint32_t c = 0; c < A; ++c) (void)rng.fr_random();          // one Blind per column (unused by KZG, but drawn)
+        for (uint32_t c = 0; c < A; ++c) adv[p * A + c] = in[p].advice[c];
+    }
+    std::vector<affine> pts(BA);
+    H2V_TRY(h2v_commit_batch_resident(pk->srs, H2V_BASIS_LAGRANGE, adv.data(), BA, n, (const uint64_t *)tails.data(), u, bf + 1, pk->adv_L.p, n,
                                       (uint64_t *)pts.data()));
     H2V_CU(cudaSetDevice(pk->dev));
-    H2V_TRY(write_points(T, pts));
-    T.absorb_async();      // the advice commitments are hashed on a worker thread while the lookup permutations run
+    for (size_t p = 0; p < B; ++p) {
+        if (int rc = write_points(P[p]->T, pts.data() + p * A, A)) {
+            bad = p;
+            return rc;
+        }
+        P[p]->T.absorb_async();      // the advice commitments are hashed on worker threads while the lookup permutations run
+    }
     lap();   // phase 0: upload + advice commitments
-    // column pointer helpers
-    auto col_L = [&](uint8_t kind, uint32_t idx) -> const fe * {
-        return kind == 0 ? pk->adv_L.as<fe>() + (size_t)idx * n : kind == 1 ? pk->fixed_L.as<fe>() + (size_t)idx * n : pk->inst_L.as<fe>() + (size_t)idx * n;
+    // column pointer helpers: column idx of a kind of proof p
+    auto col_L = [&](size_t p, uint8_t kind, uint32_t idx) -> const fe * {
+        return kind == 0 ? pk->adv_L.as<fe>() + (p * A + idx) * n : kind == 1 ? pk->fixed_L.as<fe>() + (size_t)idx * n
+                                                                                : pk->inst_L.as<fe>() + (p * I + idx) * n;
     };
-    auto col_E = [&](uint8_t kind, uint32_t idx) -> const fe * {
-        return kind == 0 ? pk->adv_E.as<fe>() + (size_t)idx * ne : kind == 1 ? pk->fixed_E.as<fe>() + (size_t)idx * ne : pk->inst_E.as<fe>() + (size_t)idx * ne;
+    auto col_E = [&](size_t p, uint8_t kind, uint32_t idx) -> const fe * {
+        return kind == 0 ? pk->adv_E.as<fe>() + (p * A + idx) * ne : kind == 1 ? pk->fixed_E.as<fe>() + (size_t)idx * ne
+                                                                                 : pk->inst_E.as<fe>() + (p * I + idx) * ne;
     };
     // ---- 5. theta; lookups: permuted input / table columns                   (lookup/prover.rs commit_permuted)
     // theta is squeezed at its place in the transcript (below, before A' / S' are written); single-expression lookups
     // have nothing to compress, so the permutations do not wait for it
-    H2V_TRY(pk->pa_L.ensure(std::max<size_t>(1, L) * n * sizeof(fe)));
-    H2V_TRY(pk->ps_L.ensure(std::max<size_t>(1, L) * n * sizeof(fe)));
+    H2V_TRY(pk->pa_L.ensure(std::max<size_t>(1, BL) * n * sizeof(fe)));
+    H2V_TRY(pk->ps_L.ensure(std::max<size_t>(1, BL) * n * sizeof(fe)));
     if (L) {
-        std::vector<Fr64> ta((size_t)L * (bf + 1)), ts((size_t)L * (bf + 1));
+        std::vector<Fr64> ta(BL * (bf + 1)), ts(BL * (bf + 1));
         {
-            std::vector<const void *> li(L), lt(L);
-            for (uint32_t l = 0; l < L; ++l) {
-                li[l] = col_L(0, pk->lookup_input[l]);
-                lt[l] = col_L(1, pk->lookup_table[l]);
+            std::vector<const void *> li(BL), lt(BL);
+            for (size_t p = 0; p < B; ++p)
+                for (uint32_t l = 0; l < L; ++l) {
+                    li[p * L + l] = col_L(p, 0, pk->lookup_input[l]);
+                    lt[p * L + l] = col_L(p, 1, pk->lookup_table[l]);      // the key's table: sorted once for the group
+                }
+            int rc = h2v_permute_expression_pair_batch_dev(li.data(), lt.data(), BL, u, pk->pa_L.as<fe>(), n, pk->ps_L.as<fe>(), n);
+            if (rc == H2V_EINVAL && B > 1) {
+                // an input value outside its table: find the proof it belongs to
+                for (size_t p = 0; p < B; ++p) {
+                    const int rc_p = h2v_permute_expression_pair_batch_dev(li.data() + p * L, lt.data() + p * L, L, u, pk->pa_L.as<fe>(), n,
+                                                                           pk->ps_L.as<fe>(), n);
+                    if (rc_p) {
+                        bad = p;
+                        return rc_p;
+                    }
+                }
             }
-            H2V_TRY(h2v_permute_expression_pair_batch_dev(li.data(), lt.data(), L, u, pk->pa_L.as<fe>(), n, pk->ps_L.as<fe>(), n));
+            if (rc) return rc;
             H2V_CU(cudaSetDevice(pk->dev));
         }
-        for (uint32_t l = 0; l < L; ++l) {
-            for (uint32_t i = 0; i <= bf; ++i) ta[(size_t)l * (bf + 1) + i] = rng.fr_random();
-            for (uint32_t i = 0; i <= bf; ++i) ts[(size_t)l * (bf + 1) + i] = rng.fr_random();
-            (void)rng.fr_random();     // permuted input blind
-            (void)rng.fr_random();     // permuted table blind
+        for (size_t p = 0; p < B; ++p) {
+            ChaCha20Rng &rng = P[p]->rng;
+            for (uint32_t l = 0; l < L; ++l) {
+                const size_t col = p * L + l;
+                for (uint32_t i = 0; i <= bf; ++i) ta[col * (bf + 1) + i] = rng.fr_random();
+                for (uint32_t i = 0; i <= bf; ++i) ts[col * (bf + 1) + i] = rng.fr_random();
+                (void)rng.fr_random();     // permuted input blind
+                (void)rng.fr_random();     // permuted table blind
+            }
         }
-        H2V_TRY(write_rows(pk, pk->pa_L.as<fe>(), n, u, bf + 1, L, ta));
-        H2V_TRY(write_rows(pk, pk->ps_L.as<fe>(), n, u, bf + 1, L, ts));
+        H2V_TRY(write_rows(pk, pk->pa_L.as<fe>(), n, u, bf + 1, BL, ta));
+        H2V_TRY(write_rows(pk, pk->ps_L.as<fe>(), n, u, bf + 1, BL, ts));
         std::vector<affine> ca, cs_;
-        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->pa_L.as<fe>(), L, ca));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->ps_L.as<fe>(), L, cs_));
-        (void)T.squeeze_challenge();      // theta
-        for (uint32_t l = 0; l < L; ++l) {
-            if (!T.write_point(ca[l]) || !T.write_point(cs_[l]))
-                return failf(H2V_EINVAL, "create_proof: Cannot write points at infinity to the transcript");
+        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->pa_L.as<fe>(), BL, ca));
+        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->ps_L.as<fe>(), BL, cs_));
+        for (size_t p = 0; p < B; ++p) {
+            (void)P[p]->T.squeeze_challenge();      // theta
+            for (uint32_t l = 0; l < L; ++l)
+                if (!P[p]->T.write_point(ca[p * L + l]) || !P[p]->T.write_point(cs_[p * L + l])) {
+                    bad = p;
+                    return failf(H2V_EINVAL, "create_proof: Cannot write points at infinity to the transcript");
+                }
         }
+    } else {
+        for (auto &s : P) (void)s->T.squeeze_challenge();     // theta
     }
-    else (void)T.squeeze_challenge();     // theta
     lap();   // phase 1: lookup permutations
     // ---- 6. beta, gamma; permutation grand products                          (permutation/prover.rs commit)
-    const Fr64 beta = T.squeeze_challenge(), gamma = T.squeeze_challenge();
-    H2V_TRY(pk->z_L.ensure(std::max<size_t>(1, NS) * n * sizeof(fe)));
-    H2V_TRY(pk->num.ensure(std::max<size_t>(1, std::max(NS, L)) * n * sizeof(fe)));
-    H2V_TRY(pk->den.ensure(std::max<size_t>(1, std::max(NS, L)) * n * sizeof(fe)));
-    H2V_TRY(pk->ptrs.ensure((size_t)(4 * (NP + G + L) + 4096) * sizeof(void *)));
-    H2V_TRY(pk->scal.ensure((size_t)(NS + A + F + NP + 3 * NS + 5 * L + 64) * sizeof(fe) + 4096));
+    std::vector<Fr64> beta_gamma(2 * B);
+    for (size_t p = 0; p < B; ++p) {
+        P[p]->beta = beta_gamma[2 * p] = P[p]->T.squeeze_challenge();
+        P[p]->gamma = beta_gamma[2 * p + 1] = P[p]->T.squeeze_challenge();
+    }
+    H2V_TRY(pk->z_L.ensure(std::max<size_t>(1, BS) * n * sizeof(fe)));
+    H2V_TRY(pk->num.ensure(std::max<size_t>(1, B * std::max(NS, L)) * n * sizeof(fe)));
+    H2V_TRY(pk->den.ensure(std::max<size_t>(1, B * std::max(NS, L)) * n * sizeof(fe)));
+    H2V_TRY(pk->ptrs.ensure((size_t)(4 * (NP + G + L) * B + 4096) * sizeof(void *)));
+    H2V_TRY(pk->scal.ensure((size_t)(NS + A + F + NP + 3 * NS + 5 * L + 64) * B * sizeof(fe) + 4096));
     if (NS) {
-        std::vector<const fe *> hp(2 * NP);
-        for (uint32_t c = 0; c < NP; ++c) {
-            hp[c] = col_L(pk->perm_kind[c], pk->perm_index[c]);
-            hp[NP + c] = pk->sigma_L.as<fe>() + (size_t)c * n;
-        }
-        H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), hp.size() * sizeof(void *)));
-        std::vector<Fr64> dstart(NS);
+        std::vector<const fe *> hp((B + 1) * NP);
+        for (size_t p = 0; p < B; ++p)
+            for (uint32_t c = 0; c < NP; ++c) hp[p * NP + c] = col_L(p, pk->perm_kind[c], pk->perm_index[c]);
+        for (uint32_t c = 0; c < NP; ++c) hp[B * NP + c] = pk->sigma_L.as<fe>() + (size_t)c * n;
+        H2V_TRY(put(pk, pk->ptrs, hp));
+        std::vector<Fr64> sc(NS);                       // delta^(s * chunk), then beta, gamma of every proof
         const Fr64 dchunk = frh::pow_u64(pk->delta, pk->chunk);
         Fr64 cur = frh::ONE;
         for (uint32_t s = 0; s < NS; ++s) {
-            dstart[s] = cur;
+            sc[s] = cur;
             cur = frh::mul(cur, dchunk);
         }
-        H2V_TRY(upload(pk, pk->scal, 0, dstart.data(), NS * sizeof(fe)));
+        sc.insert(sc.end(), beta_gamma.begin(), beta_gamma.end());
+        H2V_TRY(put(pk, pk->scal, sc));
         PermArgs pa;
         pa.cols = (const fe *const *)pk->ptrs.p;
-        pa.sigma = pa.cols + NP;
+        pa.sigma = pa.cols + B * NP;
         pa.omega_pows = pk->omega_pows.as<fe>();
         pa.delta_start = pk->scal.as<fe>();
-        pa.beta = frh::to_fe(beta); pa.gamma = frh::to_fe(gamma); pa.delta = frh::to_fe(pk->delta);
+        pa.beta_gamma = pk->scal.as<fe>() + NS;
+        pa.delta = frh::to_fe(pk->delta);
         pa.n_cols = NP; pa.chunk = pk->chunk; pa.n = (uint32_t)n;
-        perm_numden_kernel<<<dim3(gn, NS), 256, 0, st>>>(pa, pk->num.as<fe>(), pk->den.as<fe>());
+        perm_numden_kernel<<<dim3(gn, NS, (unsigned)B), 256, 0, st>>>(pa, pk->num.as<fe>(), pk->den.as<fe>());
         H2V_LAUNCHED();
         H2V_TRY(sync(pk));
         // z_s with z_s[0] = 1; then chain: z_s *= z_{s-1}[u] (upstream carries `last_z` from set to set)
-        H2V_TRY(h2v_grand_product_dev(pk->num.p, pk->den.p, n, NS, pk->z_L.p));
-        std::vector<Fr64> last(NS), scale(NS);
-        H2V_CU(cudaMemcpy2D(last.data(), sizeof(fe), pk->z_L.as<fe>() + u, n * sizeof(fe), sizeof(fe), NS, cudaMemcpyDeviceToHost));
-        cur = frh::ONE;
-        for (uint32_t s = 0; s < NS; ++s) {
-            scale[s] = cur;
-            cur = frh::mul(cur, last[s]);
+        H2V_TRY(h2v_grand_product_dev(pk->num.p, pk->den.p, n, BS, pk->z_L.p));
+        std::vector<Fr64> last(BS), scale(BS);
+        H2V_CU(cudaMemcpy2D(last.data(), sizeof(fe), pk->z_L.as<fe>() + u, n * sizeof(fe), sizeof(fe), BS, cudaMemcpyDeviceToHost));
+        for (size_t p = 0; p < B; ++p) {
+            cur = frh::ONE;
+            for (uint32_t s = 0; s < NS; ++s) {
+                scale[p * NS + s] = cur;
+                cur = frh::mul(cur, last[p * NS + s]);
+            }
         }
-        H2V_TRY(upload(pk, pk->scal, 0, scale.data(), NS * sizeof(fe)));
-        scale_cols_kernel<<<dim3(gn, NS), 256, 0, st>>>(pk->z_L.as<fe>(), (uint32_t)n, pk->scal.as<fe>());
+        H2V_TRY(put(pk, pk->scal, scale));
+        scale_cols_kernel<<<dim3(gn, (unsigned)BS), 256, 0, st>>>(pk->z_L.as<fe>(), (uint32_t)n, pk->scal.as<fe>());
         H2V_LAUNCHED();
-        std::vector<Fr64> tails((size_t)NS * bf);
-        for (uint32_t s = 0; s < NS; ++s) {
-            for (uint32_t i = 0; i < bf; ++i) tails[(size_t)s * bf + i] = rng.fr_random();     // rows n - bf .. n - 1
-            (void)rng.fr_random();                                                             // product blind
+        std::vector<Fr64> zt(BS * bf);
+        for (size_t p = 0; p < B; ++p)
+            for (uint32_t s = 0; s < NS; ++s) {
+                for (uint32_t i = 0; i < bf; ++i) zt[(p * NS + s) * bf + i] = P[p]->rng.fr_random();     // rows n - bf .. n - 1
+                (void)P[p]->rng.fr_random();                                                           // product blind
+            }
+        H2V_TRY(write_rows(pk, pk->z_L.as<fe>(), n, n - bf, bf, BS, zt));
+        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->z_L.as<fe>(), BS, pts));
+        for (size_t p = 0; p < B; ++p) {
+            if (int rc = write_points(P[p]->T, pts.data() + p * NS, NS)) {
+                bad = p;
+                return rc;
+            }
+            P[p]->T.absorb_async();      // hashed while the lookup products are built and committed
         }
-        H2V_TRY(write_rows(pk, pk->z_L.as<fe>(), n, n - bf, bf, NS, tails));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->z_L.as<fe>(), NS, pts));
-        H2V_TRY(write_points(T, pts));
-        T.absorb_async();      // hashed while the lookup products are built and committed
     }
     // ---- 7. lookup grand products                                             (lookup/prover.rs commit_product)
-    H2V_TRY(pk->zl_L.ensure(std::max<size_t>(1, L) * n * sizeof(fe)));
+    H2V_TRY(pk->zl_L.ensure(std::max<size_t>(1, BL) * n * sizeof(fe)));
     if (L) {
-        std::vector<const fe *> hp(2 * L);
-        for (uint32_t l = 0; l < L; ++l) {
-            hp[l] = col_L(0, pk->lookup_input[l]);
-            hp[L + l] = col_L(1, pk->lookup_table[l]);
-        }
-        H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), hp.size() * sizeof(void *)));
-        lookup_numden_kernel<<<dim3(gn, L), 256, 0, st>>>((const fe *const *)pk->ptrs.p, (const fe *const *)pk->ptrs.p + L, pk->pa_L.as<fe>(),
-                                                        pk->ps_L.as<fe>(), frh::to_fe(beta), frh::to_fe(gamma), (uint32_t)n, pk->num.as<fe>(), pk->den.as<fe>());
+        std::vector<const fe *> hp(BL + L);
+        for (size_t p = 0; p < B; ++p)
+            for (uint32_t l = 0; l < L; ++l) hp[p * L + l] = col_L(p, 0, pk->lookup_input[l]);
+        for (uint32_t l = 0; l < L; ++l) hp[BL + l] = col_L(0, 1, pk->lookup_table[l]);
+        H2V_TRY(put(pk, pk->ptrs, hp));
+        H2V_TRY(put(pk, pk->scal, beta_gamma));
+        lookup_numden_kernel<<<dim3(gn, L, (unsigned)B), 256, 0, st>>>((const fe *const *)pk->ptrs.p, (const fe *const *)pk->ptrs.p + BL,
+                                                                      pk->pa_L.as<fe>(), pk->ps_L.as<fe>(), pk->scal.as<fe>(), (uint32_t)n,
+                                                                      pk->num.as<fe>(), pk->den.as<fe>());
         H2V_LAUNCHED();
         H2V_TRY(sync(pk));
-        H2V_TRY(h2v_grand_product_dev(pk->num.p, pk->den.p, n, L, pk->zl_L.p));
-        std::vector<Fr64> tails((size_t)L * bf);
-        for (uint32_t l = 0; l < L; ++l) {
-            for (uint32_t i = 0; i < bf; ++i) tails[(size_t)l * bf + i] = rng.fr_random();
-            (void)rng.fr_random();
+        H2V_TRY(h2v_grand_product_dev(pk->num.p, pk->den.p, n, BL, pk->zl_L.p));
+        std::vector<Fr64> lt(BL * bf);
+        for (size_t p = 0; p < B; ++p)
+            for (uint32_t l = 0; l < L; ++l) {
+                for (uint32_t i = 0; i < bf; ++i) lt[(p * L + l) * bf + i] = P[p]->rng.fr_random();
+                (void)P[p]->rng.fr_random();
+            }
+        H2V_TRY(write_rows(pk, pk->zl_L.as<fe>(), n, n - bf, bf, BL, lt));
+        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->zl_L.as<fe>(), BL, pts));
+        for (size_t p = 0; p < B; ++p) {
+            if (int rc = write_points(P[p]->T, pts.data() + p * L, L)) {
+                bad = p;
+                return rc;
+            }
+            P[p]->T.absorb_async();
         }
-        H2V_TRY(write_rows(pk, pk->zl_L.as<fe>(), n, n - bf, bf, L, tails));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->zl_L.as<fe>(), L, pts));
-        H2V_TRY(write_points(T, pts));
-        T.absorb_async();
     }
     lap();   // phase 2: grand products
     // ---- 8. vanishing argument: random polynomial                             (vanishing/prover.rs commit)
-    H2V_TRY(pk->rnd_C.ensure(n * sizeof(fe)));
+    H2V_TRY(pk->rnd_C.ensure(B * n * sizeof(fe)));
     {
-        // n consecutive Fr::random draws = n consecutive key-stream blocks: produced on the device
-        ChaChaKey key;
-        memcpy(key.k, rng.key, 32);
-        chacha_fr_kernel<<<gn, 256, 0, st>>>(key, rng.next_block(), (uint32_t)n, pk->rnd_C.as<fe>());
+        // n consecutive Fr::random draws = n consecutive key-stream blocks: produced on the device, every proof's in one launch
+        std::vector<ChaChaStream> cs(B);
+        for (size_t p = 0; p < B; ++p) {
+            ChaCha20Rng &rng = P[p]->rng;
+            memcpy(cs[p].key.k, rng.key, 32);
+            cs[p].counter0 = rng.next_block();
+            rng.skip_fr(n);
+            (void)rng.fr_random();      // random_blind
+        }
+        H2V_TRY(put(pk, pk->streams, cs));
+        chacha_fr_kernel<<<dim3(gn, (unsigned)B), 256, 0, st>>>(pk->streams.as<ChaChaStream>(), (uint32_t)n, pk->rnd_C.as<fe>());
         H2V_LAUNCHED();
-        rng.skip_fr(n);
-        (void)rng.fr_random();      // random_blind
         H2V_TRY(sync(pk));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, pk->rnd_C.as<fe>(), 1, pts));
-        H2V_TRY(write_points(T, pts));
-        T.absorb_async();
+        H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, pk->rnd_C.as<fe>(), B, pts));
+        for (size_t p = 0; p < B; ++p) {
+            if (int rc = write_points(P[p]->T, pts.data() + p, 1)) {
+                bad = p;
+                return rc;
+            }
+            P[p]->T.absorb_async();
+        }
     }
     // ---- 9-11. coefficient and extended forms (no challenge involved: they run while the commitments above are hashed);
     //            then y, evaluate_h, quotient pieces
     const int L2C = H2V_OP_LAGRANGE_TO_COEFF, C2E = H2V_OP_COEFF_TO_EXTENDED;
-    const bool stream = pk->stream_ext;
+    const bool stream = pk->stream_ext;      // (a streamed key proves in groups of one)
     // (the per-proof buffers are kept between proofs, also in streamed mode: with peer access enabled, freeing and
     // re-allocating gigabytes every proof costs more than the transforms themselves -- measured on two devices)
-    if (!stream) H2V_TRY(pk->adv_E.ensure((size_t)A * ne * sizeof(fe)));
-    H2V_TRY(h2v_domain_transform_dev(pk->dom, L2C, pk->adv_L.p, n, pk->adv_C.p, n, A));
-    if (!stream) H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, pk->adv_C.p, n, pk->adv_E.p, ne, A));
-    if (I) H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, pk->inst_C.p, n, pk->inst_E.p, ne, I));
-    struct Tr { DevBuf *Lb, *Cb, *Eb; size_t cnt; } trs[4] = {{&pk->pa_L, &pk->pa_C, &pk->pa_E, L}, {&pk->ps_L, &pk->ps_C, &pk->ps_E, L},
-                                                            {&pk->z_L, &pk->z_C, &pk->z_E, NS}, {&pk->zl_L, &pk->zl_C, &pk->zl_E, L}};
+    if (!stream) H2V_TRY(pk->adv_E.ensure(BA * ne * sizeof(fe)));
+    H2V_TRY(h2v_domain_transform_dev(pk->dom, L2C, pk->adv_L.p, n, pk->adv_C.p, n, BA));
+    if (!stream) H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, pk->adv_C.p, n, pk->adv_E.p, ne, BA));
+    if (I) H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, pk->inst_C.p, n, pk->inst_E.p, ne, BI));
+    struct Tr { DevBuf *Lb, *Cb, *Eb; size_t cnt; } trs[4] = {{&pk->pa_L, &pk->pa_C, &pk->pa_E, BL}, {&pk->ps_L, &pk->ps_C, &pk->ps_E, BL},
+                                                            {&pk->z_L, &pk->z_C, &pk->z_E, BS}, {&pk->zl_L, &pk->zl_C, &pk->zl_E, BL}};
     for (auto &t : trs) {
         H2V_TRY(t.Cb->ensure(std::max<size_t>(1, t.cnt) * n * sizeof(fe)));
         H2V_TRY(t.Eb->ensure(std::max<size_t>(1, t.cnt) * ne * sizeof(fe)));
@@ -686,36 +836,59 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         H2V_TRY(h2v_domain_transform_dev(pk->dom, L2C, t.Lb->p, n, t.Cb->p, n, t.cnt));
         H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, t.Cb->p, n, t.Eb->p, ne, t.cnt));
     }
-    const Fr64 y = T.squeeze_challenge();
+    for (auto &s : P) s->y = s->T.squeeze_challenge();
     lap();   // phase 3: random poly + transforms
-    H2V_TRY(pk->hq.ensure(2 * ne * sizeof(fe)));
-    fe *h_ext = pk->hq.as<fe>(), *h_out = pk->hq.as<fe>() + ne;
-    H2V_CU(cudaMemsetAsync(h_ext, 0, ne * sizeof(fe), st));
+    // h_ext of proof p at hq + p ne, its quotient after the division at hq + (B + p) ne
+    H2V_TRY(pk->hq.ensure(2 * B * ne * sizeof(fe)));
+    fe *h_ext0 = pk->hq.as<fe>(), *h_out0 = pk->hq.as<fe>() + B * ne;
+    H2V_CU(cudaMemsetAsync(h_ext0, 0, B * ne * sizeof(fe), st));
     H2V_TRY(sync(pk));
     const fe *l0 = pk->lrows_E.as<fe>(), *ll = l0 + ne, *la = l0 + 2 * ne;
     if (!stream) {
-        std::vector<const fe *> hp(2 * G + 2 * NP);
-        for (uint32_t j = 0; j < G; ++j) {
-            hp[j] = col_E(1, pk->gate_selector[j]);
-            hp[G + j] = col_E(0, pk->gate_advice[j]);
+        const size_t per = 2 * (size_t)G + 2 * (size_t)NP;
+        std::vector<const fe *> hp(B * per);
+        for (size_t p = 0; p < B; ++p) {
+            const fe **t = hp.data() + p * per;
+            for (uint32_t j = 0; j < G; ++j) {
+                t[j] = col_E(p, 1, pk->gate_selector[j]);
+                t[G + j] = col_E(p, 0, pk->gate_advice[j]);
+            }
+            for (uint32_t c = 0; c < NP; ++c) {
+                t[2 * G + c] = col_E(p, pk->perm_kind[c], pk->perm_index[c]);
+                t[2 * G + NP + c] = pk->sigma_E.as<fe>() + (size_t)c * ne;
+            }
         }
-        for (uint32_t c = 0; c < NP; ++c) {
-            hp[2 * G + c] = col_E(pk->perm_kind[c], pk->perm_index[c]);
-            hp[2 * G + NP + c] = pk->sigma_E.as<fe>() + (size_t)c * ne;
+        // the lookups' five columns per lookup after the gate and permutation tables; every proof's y, beta, gamma
+        const size_t lper = 5 * (size_t)L;
+        for (size_t p = 0; p < B; ++p)
+            for (uint32_t l = 0; l < L; ++l) {
+                const size_t col = p * L + l;
+                const fe *five[5] = {col_E(p, 0, pk->lookup_input[l]), col_E(p, 1, pk->lookup_table[l]), pk->pa_E.as<fe>() + col * ne,
+                                     pk->ps_E.as<fe>() + col * ne, pk->zl_E.as<fe>() + col * ne};
+                hp.insert(hp.end(), five, five + 5);
+            }
+        H2V_TRY(put(pk, pk->ptrs, hp));
+        std::vector<Fr64> ybg(3 * B);
+        for (size_t p = 0; p < B; ++p) {
+            ybg[3 * p] = P[p]->y;
+            ybg[3 * p + 1] = P[p]->beta;
+            ybg[3 * p + 2] = P[p]->gamma;
         }
-        if (!hp.empty()) H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), hp.size() * sizeof(void *)));
+        H2V_TRY(put(pk, pk->scal, ybg));
         const void *const *tab = (const void *const *)pk->ptrs.p;
-        H2V_TRY(h2v_quotient_gates_ptrs_dev(pk->dom, h_ext, u64(y), G, tab, tab + G));
-        if (NP)
-            H2V_TRY(h2v_quotient_permutation_ptrs_dev(pk->dom, h_ext, u64(y), u64(beta), u64(gamma), NP, pk->chunk, tab + 2 * G,
-                                                      tab + 2 * G + NP, pk->z_E.p, ne, l0, ll, la, bf));
-        for (uint32_t l = 0; l < L; ++l)
-            H2V_TRY(h2v_quotient_lookup_dev(pk->dom, h_ext, u64(y), u64(beta), u64(gamma), col_E(0, pk->lookup_input[l]),
-                                            col_E(1, pk->lookup_table[l]), pk->pa_E.as<fe>() + (size_t)l * ne, pk->ps_E.as<fe>() + (size_t)l * ne,
-                                            pk->zl_E.as<fe>() + (size_t)l * ne, l0, ll, la));
+        QuotientBatch qb;
+        qb.h = h_ext0; qb.h_stride = ne; qb.scal = pk->scal.p; qb.n_proofs = B;
+        qb.n_gates = G; qb.gate_tab = tab; qb.gate_pstride = per;
+        qb.n_perm = NP; qb.chunk = pk->chunk; qb.perm_tab = tab + 2 * G; qb.perm_pstride = per;
+        qb.z = pk->z_E.p; qb.z_stride = ne; qb.z_pstride = (size_t)NS * ne; qb.blinding_factors = bf;
+        qb.n_lookups = L; qb.lookup_tab = tab + B * per; qb.lookup_pstride = lper;
+        qb.l0 = l0; qb.l_last = ll; qb.l_active = la;
+        H2V_TRY(quotient_batch_dev(pk->dom, qb));
     } else {
         // the same folds, in upstream's order, over slices of columns whose extended forms are rebuilt into `scr_E` from
-        // the resident coefficient forms (every term reads columns of its own gate / set / lookup only)
+        // the resident coefficient forms (every term reads columns of its own gate / set / lookup only); one proof
+        fe *h_ext = h_ext0, *h_out = h_out0;
+        const Fr64 &y = P[0]->y, &beta = P[0]->beta, &gamma = P[0]->gamma;
         const size_t SC = pk->scr_cols;
         H2V_TRY(pk->scr_E.ensure(SC * ne * sizeof(fe)));
         fe *scr = pk->scr_E.as<fe>();
@@ -813,12 +986,7 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
                 mark(t_fold);
             }
             // h <- h y^T + hp, T = the permutation argument's terms: 2 + (NS - 1) + NS
-            const fe *two[2] = {h_ext, hp_acc};
-            const Fr64 cf[2] = {frh::pow_u64(y, 2ull * NS + 1), frh::ONE};
-            H2V_TRY(upload(pk, pk->ptrs, 0, two, sizeof two));
-            H2V_TRY(upload(pk, pk->scal, 0, cf, sizeof cf));
-            lincomb_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.as<fe>(), 2, (uint32_t)ne, h_ext);
-            H2V_LAUNCHED();
+            H2V_TRY(lincomb(pk, {h_ext, hp_acc}, {frh::pow_u64(y, 2ull * NS + 1), frh::ONE}, {0, 2}, h_ext, ne, ne));
             H2V_TRY(sync(pk));
             mark(t_fold);
         } else {
@@ -873,284 +1041,469 @@ int create_proof_locked(h2v_pk *pk, const uint64_t *const *advice, const uint64_
         }
         if (timing) fprintf(stderr, "evaluate_h (streamed): coeff_to_extended of the slices %.1f ms, folds %.1f ms\n", t_ext, t_fold);
     }
-    H2V_TRY(h2v_domain_transform_dev(pk->dom, H2V_OP_DIVIDE_BY_VANISHING, h_ext, ne, h_out, ne, 1));
+    H2V_TRY(h2v_domain_transform_dev(pk->dom, H2V_OP_DIVIDE_BY_VANISHING, h_ext0, ne, h_out0, ne, B));
     const uint32_t NH = pk->degree - 1;          // quotient pieces of n coefficients each
-    for (uint32_t i = 0; i < NH; ++i) (void)rng.fr_random();     // h_blinds
-    H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, h_out, NH, pts));
-    H2V_TRY(write_points(T, pts));
+    for (auto &s : P)
+        for (uint32_t i = 0; i < NH; ++i) (void)s->rng.fr_random();     // h_blinds
+    // the B x NH pieces as contiguous columns of n (they already are when NH n = ne, and for one proof)
+    fe *pieces = h_out0;
+    if (B > 1 && NH * n != ne) {
+        H2V_TRY(pk->hx_pieces.ensure(B * NH * n * sizeof(fe)));
+        pieces = pk->hx_pieces.as<fe>();
+        H2V_CU(cudaMemcpy2DAsync(pieces, NH * n * sizeof(fe), h_out0, ne * sizeof(fe), NH * n * sizeof(fe), B, cudaMemcpyDeviceToDevice, st));
+        H2V_TRY(sync(pk));
+    }
+    H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, pieces, B * NH, pts));
+    for (size_t p = 0; p < B; ++p) {
+        if (int rc = write_points(P[p]->T, pts.data() + p * NH, NH)) {
+            bad = p;
+            return rc;
+        }
+    }
     lap();   // phase 4: evaluate_h + quotient commitments
     // ---- 12. x; evaluations
-    const Fr64 x = T.squeeze_challenge();
-    Fr64 xn = x;
-    for (uint32_t i = 0; i < pk->k; ++i) xn = frh::sqr(xn);
-    // distinct evaluation points x * w^rot
+    for (auto &s : P) {
+        s->x = s->T.squeeze_challenge();
+        s->xn = s->x;
+        for (uint32_t i = 0; i < pk->k; ++i) s->xn = frh::sqr(s->xn);
+    }
+    // distinct evaluation points x * w^rot: the same rotations for every proof, in order of first use
     std::vector<int32_t> rots;
-    std::vector<Fr64> points;
     auto point_of = [&](int32_t rot) -> uint32_t {
         for (size_t i = 0; i < rots.size(); ++i)
             if (rots[i] == rot) return (uint32_t)i;
         rots.push_back(rot);
-        points.push_back(frh::rotate(x, pk->omega, pk->omega_inv, rot));
         return (uint32_t)(rots.size() - 1);
     };
     const uint32_t p_cur = point_of(0), p_next = point_of(1), p_prev = point_of(-1), p_last = point_of(-(int32_t)(bf + 1));
-    // h(X) = sum_i xn^i h_i(X)
-    H2V_TRY(pk->sh_h.ensure(2 * n * sizeof(fe)));
-    fe *h_poly = pk->sh_h.as<fe>(), *hx_dev = pk->sh_h.as<fe>() + n;
+    // h(X) = sum_i xn^i h_i(X); proof p's at sh_h + p n
+    H2V_TRY(pk->sh_h.ensure(2 * B * n * sizeof(fe)));
+    fe *h_poly0 = pk->sh_h.as<fe>(), *hx0 = pk->sh_h.as<fe>() + B * n;
     {
-        std::vector<const fe *> hp(NH);
-        std::vector<Fr64> cf(NH);
-        Fr64 cur = frh::ONE;
-        for (uint32_t i = 0; i < NH; ++i) {
-            hp[i] = h_out + (size_t)i * n;
-            cf[i] = cur;
-            cur = frh::mul(cur, xn);
+        std::vector<const fe *> hp(B * NH);
+        std::vector<Fr64> cf(B * NH);
+        std::vector<uint32_t> off(B + 1);
+        for (size_t p = 0; p < B; ++p) {
+            Fr64 cur = frh::ONE;
+            off[p] = (uint32_t)(p * NH);
+            for (uint32_t i = 0; i < NH; ++i) {
+                hp[p * NH + i] = pieces + (p * NH + i) * n;
+                cf[p * NH + i] = cur;
+                cur = frh::mul(cur, P[p]->xn);
+            }
         }
-        H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), NH * sizeof(void *)));
-        H2V_TRY(upload(pk, pk->scal, 0, cf.data(), NH * sizeof(fe)));
-        lincomb_kernel<<<gn, 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.as<fe>(), NH, (uint32_t)n, h_poly);
-        H2V_LAUNCHED();
+        off[B] = (uint32_t)(B * NH);
+        H2V_TRY(lincomb(pk, hp, cf, off, h_poly0, n, n));
     }
-    // every (polynomial, point) pair that is evaluated, in transcript order first, then the two the transcript skips
+    // every (polynomial, point) pair that is evaluated, in transcript order first, then the two the transcript skips; the
+    // same list for every proof, over its own columns
     std::vector<EvalPair> pairs;
-    auto push = [&](const fe *poly, uint32_t pt) { pairs.push_back(EvalPair{poly, pt}); return (uint32_t)(pairs.size() - 1); };
-    for (size_t q = 0; q < pk->aq_col.size(); ++q) push(pk->adv_C.as<fe>() + (size_t)pk->aq_col[q] * n, point_of(pk->aq_rot[q]));
-    for (size_t q = 0; q < pk->fq_col.size(); ++q) push(pk->fixed_C.as<fe>() + (size_t)pk->fq_col[q] * n, point_of(pk->fq_rot[q]));
-    const uint32_t e_random = push(pk->rnd_C.as<fe>(), p_cur);
-    for (uint32_t c = 0; c < NP; ++c) push(pk->sigma_C.as<fe>() + (size_t)c * n, p_cur);
-    const uint32_t e_perm = (uint32_t)pairs.size();
-    for (uint32_t s = 0; s < NS; ++s) {
-        push(pk->z_C.as<fe>() + (size_t)s * n, p_cur);
-        push(pk->z_C.as<fe>() + (size_t)s * n, p_next);
-        if (s + 1 < NS) push(pk->z_C.as<fe>() + (size_t)s * n, p_last);
+    uint32_t e_random = 0, e_perm = 0, e_lookup = 0, n_written = 0, e_h = 0;
+    for (size_t p = 0; p < B; ++p) {
+        const size_t base = pairs.size();
+        auto push = [&](const fe *poly, uint32_t pt) { pairs.push_back(EvalPair{poly, pt}); return (uint32_t)(pairs.size() - 1 - base); };
+        const fe *adv_C = pk->adv_C.as<fe>() + p * A * n, *z_C = pk->z_C.as<fe>() + p * NS * n, *zl_C = pk->zl_C.as<fe>() + p * L * n,
+                 *pa_C = pk->pa_C.as<fe>() + p * L * n, *ps_C = pk->ps_C.as<fe>() + p * L * n;
+        for (size_t q = 0; q < pk->aq_col.size(); ++q) push(adv_C + (size_t)pk->aq_col[q] * n, point_of(pk->aq_rot[q]));
+        for (size_t q = 0; q < pk->fq_col.size(); ++q) push(pk->fixed_C.as<fe>() + (size_t)pk->fq_col[q] * n, point_of(pk->fq_rot[q]));
+        e_random = push(pk->rnd_C.as<fe>() + p * n, p_cur);
+        for (uint32_t c = 0; c < NP; ++c) push(pk->sigma_C.as<fe>() + (size_t)c * n, p_cur);
+        e_perm = e_random + 1 + NP;
+        for (uint32_t s = 0; s < NS; ++s) {
+            push(z_C + (size_t)s * n, p_cur);
+            push(z_C + (size_t)s * n, p_next);
+            if (s + 1 < NS) push(z_C + (size_t)s * n, p_last);
+        }
+        e_lookup = e_perm + (NS ? 3 * NS - 1 : 0);
+        for (uint32_t l = 0; l < L; ++l) {
+            push(zl_C + (size_t)l * n, p_cur);
+            push(zl_C + (size_t)l * n, p_next);
+            push(pa_C + (size_t)l * n, p_cur);
+            push(pa_C + (size_t)l * n, p_prev);
+            push(ps_C + (size_t)l * n, p_cur);
+        }
+        n_written = e_lookup + 5 * L;
+        e_h = push(h_poly0 + p * n, p_cur);       // h(x): opened by the multi-open argument, not written
     }
-    const uint32_t e_lookup = (uint32_t)pairs.size();
-    for (uint32_t l = 0; l < L; ++l) {
-        push(pk->zl_C.as<fe>() + (size_t)l * n, p_cur);
-        push(pk->zl_C.as<fe>() + (size_t)l * n, p_next);
-        push(pk->pa_C.as<fe>() + (size_t)l * n, p_cur);
-        push(pk->pa_C.as<fe>() + (size_t)l * n, p_prev);
-        push(pk->ps_C.as<fe>() + (size_t)l * n, p_cur);
-    }
-    const uint32_t n_written = (uint32_t)pairs.size();
-    const uint32_t e_h = push(h_poly, p_cur);       // h(x): opened by the multi-open argument, not written
+    const size_t NE = e_h + 1, NPT = rots.size();        // pairs and distinct points per proof
+    std::vector<Fr64> points(B * NPT);                   // proof p's points at p NPT
+    for (size_t p = 0; p < B; ++p)
+        for (size_t i = 0; i < NPT; ++i) points[p * NPT + i] = frh::rotate(P[p]->x, pk->omega, pk->omega_inv, rots[i]);
+    std::vector<EvalPair> dev_pairs(pairs);
+    for (size_t e = 0; e < dev_pairs.size(); ++e) dev_pairs[e].point += (uint32_t)((e / NE) * NPT);
     std::vector<Fr64> evals(pairs.size());
     {
-        H2V_TRY(pk->pairs.ensure(pairs.size() * sizeof(EvalPair)));
+        H2V_TRY(put(pk, pk->pairs, dev_pairs));
+        H2V_TRY(put(pk, pk->pts, points));
         H2V_TRY(pk->evals.ensure(pairs.size() * sizeof(fe)));
-        H2V_TRY(pk->pts.ensure((points.size() + 8) * sizeof(fe)));
-        H2V_TRY(upload(pk, pk->pairs, 0, pairs.data(), pairs.size() * sizeof(EvalPair)));
-        H2V_TRY(upload(pk, pk->pts, 0, points.data(), points.size() * sizeof(fe)));
         eval_pairs_kernel<<<(unsigned)pairs.size(), 256, 0, st>>>((const EvalPair *)pk->pairs.p, pk->pts.as<fe>(), (uint32_t)n, pk->evals.as<fe>());
         H2V_LAUNCHED();
         H2V_CU(cudaMemcpyAsync(evals.data(), pk->evals.p, pairs.size() * sizeof(fe), cudaMemcpyDeviceToHost, st));
         H2V_TRY(sync(pk));
     }
-    for (uint32_t i = 0; i < n_written; ++i) T.write_scalar(evals[i]);
+    for (size_t p = 0; p < B; ++p)
+        for (uint32_t i = 0; i < n_written; ++i) P[p]->T.write_scalar(evals[p * NE + i]);
     lap();   // phase 5: evaluations
     // ---- 13. multi-open argument (SHPLONK)
-    // the prover's queries, in upstream's order: advice, permutation products, lookups, fixed, sigma, vanishing
-    std::vector<Query> queries;
-    {
-        size_t e = 0;
-        std::vector<Query> adv_q, fix_q, sig_q;
-        for (size_t q = 0; q < pk->aq_col.size(); ++q, ++e) adv_q.push_back(Query{pairs[e].poly, pairs[e].point, evals[e]});
-        for (size_t q = 0; q < pk->fq_col.size(); ++q, ++e) fix_q.push_back(Query{pairs[e].poly, pairs[e].point, evals[e]});
-        ++e;   // random_eval
-        for (uint32_t c = 0; c < NP; ++c, ++e) sig_q.push_back(Query{pairs[e].poly, pairs[e].point, evals[e]});
-        queries = adv_q;
-        // permutation::prover::Evaluated::open: (x, z_s), (wx, z_s) for every set, then (w^last x, z_s) for all but the
-        // last set taken in reverse order
-        {
-            std::vector<uint32_t> at(NS);
-            uint32_t pos = e_perm;
-            for (uint32_t s = 0; s < NS; ++s) {
-                at[s] = pos;
-                queries.push_back(Query{pairs[pos].poly, p_cur, evals[pos]});
-                queries.push_back(Query{pairs[pos + 1].poly, p_next, evals[pos + 1]});
-                pos += (s + 1 < NS) ? 3 : 2;
-            }
-            for (uint32_t s = NS; s-- > 0;) {
-                if (s + 1 == NS) continue;
-                queries.push_back(Query{pairs[at[s] + 2].poly, p_last, evals[at[s] + 2]});
-            }
-        }
-        // lookup::prover::Evaluated::open: (x, z), (x, a'), (x, s'), (w^-1 x, a'), (wx, z)
-        for (uint32_t l = 0; l < L; ++l) {
-            const uint32_t b = e_lookup + 5 * l;
-            queries.push_back(Query{pairs[b].poly, p_cur, evals[b]});
-            queries.push_back(Query{pairs[b + 2].poly, p_cur, evals[b + 2]});
-            queries.push_back(Query{pairs[b + 4].poly, p_cur, evals[b + 4]});
-            queries.push_back(Query{pairs[b + 3].poly, p_prev, evals[b + 3]});
-            queries.push_back(Query{pairs[b + 1].poly, p_next, evals[b + 1]});
-        }
-        queries.insert(queries.end(), fix_q.begin(), fix_q.end());
-        queries.insert(queries.end(), sig_q.begin(), sig_q.end());
-        queries.push_back(Query{h_poly, p_cur, evals[e_h]});
-        queries.push_back(Query{pk->rnd_C.as<fe>(), p_cur, evals[e_random]});
-    }
-    // construct_intermediate_sets: point sets are ordered sets of field elements (BTreeSet<Fr>: numeric order of the
-    // canonical values); commitments and rotation sets keep their order of first appearance
-    const size_t NPT = points.size();
-    std::vector<uint32_t> rank(NPT);      // rank[p] = position of point p in the numeric order
-    {
-        std::vector<uint32_t> ord(NPT);
-        for (size_t i = 0; i < NPT; ++i) ord[i] = (uint32_t)i;
-        std::sort(ord.begin(), ord.end(), [&](uint32_t a, uint32_t b) { return frh::less_canonical(points[a], points[b]); });
-        for (size_t i = 0; i < NPT; ++i) rank[ord[i]] = (uint32_t)i;
-    }
-    struct Com { const fe *poly; uint64_t mask; };       // mask over ranks
-    std::vector<Com> coms;
-    std::map<const fe *, size_t> com_of;
-    std::map<std::pair<const fe *, uint32_t>, Fr64> eval_of;
-    uint64_t super_mask = 0;
-    for (const Query &q : queries) {
-        const uint64_t bit = (uint64_t)1 << rank[q.pt];
-        super_mask |= bit;
-        auto it = com_of.find(q.poly);
-        if (it == com_of.end()) {
-            com_of[q.poly] = coms.size();
-            coms.push_back(Com{q.poly, bit});
-        } else {
-            coms[it->second].mask |= bit;
-        }
-        eval_of[{q.poly, rank[q.pt]}] = q.eval;
-    }
+    // Host side per proof, on B threads: the queries, construct_intermediate_sets, y / v, the Lagrange bases and the
+    // interpolated R_ij.  Every proof has the same rotation sets (commitments grouped by the rotations they are opened
+    // at, in order of first appearance); only the numeric order of the points inside a set differs.
     struct RSet { uint64_t mask; std::vector<const fe *> polys; };
-    std::vector<RSet> rsets;
-    for (const Com &c : coms) {
-        size_t i = 0;
-        for (; i < rsets.size(); ++i)
-            if (rsets[i].mask == c.mask) break;
-        if (i == rsets.size()) rsets.push_back(RSet{c.mask, {}});
-        rsets[i].polys.push_back(c.poly);
-    }
-    std::vector<Fr64> sorted_pts(NPT);
-    for (size_t i = 0; i < NPT; ++i) sorted_pts[rank[i]] = points[i];
-    auto pts_of = [&](uint64_t mask) {
-        std::vector<Fr64> v;
-        for (size_t r = 0; r < NPT; ++r)
-            if ((mask >> r) & 1) v.push_back(sorted_pts[r]);
-        return v;
+    struct MultiOpen {
+        std::vector<RSet> rsets;
+        std::vector<Fr64> sorted_pts;
+        uint64_t super_mask = 0;
+        std::vector<std::vector<Fr64>> r_comb;                 // sum_j y^j R_ij(X), low degree
+        std::vector<std::vector<std::vector<Fr64>>> r_ij;
+        std::vector<std::vector<Fr64>> set_pts;                // the points of set i, numeric order
+        std::vector<std::vector<Fr64>> ypow;
+        std::vector<Fr64> pts_of(uint64_t mask) const {
+            std::vector<Fr64> v;
+            for (size_t r = 0; r < sorted_pts.size(); ++r)
+                if ((mask >> r) & 1) v.push_back(sorted_pts[r]);
+            return v;
+        }
     };
-    const Fr64 ys = T.squeeze_challenge(), vs = T.squeeze_challenge();
-    const size_t NR = rsets.size();
-    H2V_TRY(pk->sh_S.ensure(NR * n * sizeof(fe)));
-    H2V_TRY(pk->sh_A.ensure((n + 8) * sizeof(fe)));
-    H2V_TRY(pk->sh_B.ensure(std::max<size_t>(NR, 1) * n * sizeof(fe)));
-    size_t max_polys = 0;
-    for (auto &rs : rsets) max_polys = std::max(max_polys, rs.polys.size());
-    H2V_TRY(pk->ptrs.ensure((max_polys + NR + 8) * sizeof(void *)));
-    H2V_TRY(pk->scal.ensure((max_polys + NR + 16) * sizeof(fe)));
-    std::vector<std::vector<Fr64>> r_comb(NR);           // sum_j y^j R_ij(X), low degree
-    std::vector<std::vector<std::vector<Fr64>>> r_ij(NR);
-    fe *Q = pk->sh_B.as<fe>();                                // quotient contributions Q_i, n coefficients each
-    for (size_t i = 0; i < NR; ++i) {
-        const std::vector<Fr64> ps = pts_of(rsets[i].mask);
-        const size_t m = ps.size(), nc = rsets[i].polys.size();
-        const std::vector<std::vector<Fr64>> basis = lagrange_basis(ps);
-        std::vector<Fr64> ypow(nc);
-        Fr64 cur = frh::ONE;
-        r_comb[i].assign(m, frh::zero());
-        r_ij[i].resize(nc);
-        for (size_t j = 0; j < nc; ++j) {
-            ypow[j] = cur;
-            std::vector<Fr64> ev;
-            for (size_t r = 0; r < NPT; ++r)
-                if ((rsets[i].mask >> r) & 1) ev.push_back(eval_of[{rsets[i].polys[j], (uint32_t)r}]);
-            r_ij[i][j] = lagrange_interpolate(basis, ev);
-            for (size_t t = 0; t < m; ++t) r_comb[i][t] = frh::add(r_comb[i][t], frh::mul(r_ij[i][j][t], cur));
-            cur = frh::mul(cur, ys);
+    std::vector<MultiOpen> MO(B);
+    H2V_TRY(par_proofs(B, [&](size_t p) -> int {
+        MultiOpen &mo = MO[p];
+        const EvalPair *pr = pairs.data() + p * NE;
+        const Fr64 *ev = evals.data() + p * NE, *pt = points.data() + p * NPT;
+        // the prover's queries, in upstream's order: advice, permutation products, lookups, fixed, sigma, vanishing
+        std::vector<Query> queries;
+        {
+            size_t e = 0;
+            std::vector<Query> adv_q, fix_q, sig_q;
+            for (size_t q = 0; q < pk->aq_col.size(); ++q, ++e) adv_q.push_back(Query{pr[e].poly, pr[e].point, ev[e]});
+            for (size_t q = 0; q < pk->fq_col.size(); ++q, ++e) fix_q.push_back(Query{pr[e].poly, pr[e].point, ev[e]});
+            ++e;   // random_eval
+            for (uint32_t c = 0; c < NP; ++c, ++e) sig_q.push_back(Query{pr[e].poly, pr[e].point, ev[e]});
+            queries = adv_q;
+            // permutation::prover::Evaluated::open: (x, z_s), (wx, z_s) for every set, then (w^last x, z_s) for all but the
+            // last set taken in reverse order
+            {
+                std::vector<uint32_t> at(NS);
+                uint32_t pos = e_perm;
+                for (uint32_t s = 0; s < NS; ++s) {
+                    at[s] = pos;
+                    queries.push_back(Query{pr[pos].poly, p_cur, ev[pos]});
+                    queries.push_back(Query{pr[pos + 1].poly, p_next, ev[pos + 1]});
+                    pos += (s + 1 < NS) ? 3 : 2;
+                }
+                for (uint32_t s = NS; s-- > 0;) {
+                    if (s + 1 == NS) continue;
+                    queries.push_back(Query{pr[at[s] + 2].poly, p_last, ev[at[s] + 2]});
+                }
+            }
+            // lookup::prover::Evaluated::open: (x, z), (x, a'), (x, s'), (w^-1 x, a'), (wx, z)
+            for (uint32_t l = 0; l < L; ++l) {
+                const uint32_t b = e_lookup + 5 * l;
+                queries.push_back(Query{pr[b].poly, p_cur, ev[b]});
+                queries.push_back(Query{pr[b + 2].poly, p_cur, ev[b + 2]});
+                queries.push_back(Query{pr[b + 4].poly, p_cur, ev[b + 4]});
+                queries.push_back(Query{pr[b + 3].poly, p_prev, ev[b + 3]});
+                queries.push_back(Query{pr[b + 1].poly, p_next, ev[b + 1]});
+            }
+            queries.insert(queries.end(), fix_q.begin(), fix_q.end());
+            queries.insert(queries.end(), sig_q.begin(), sig_q.end());
+            queries.push_back(Query{pr[e_h].poly, p_cur, ev[e_h]});
+            queries.push_back(Query{pr[e_random].poly, p_cur, ev[e_random]});
         }
-        // S_i(X) = sum_j y^j P_ij(X)
-        H2V_TRY(upload(pk, pk->ptrs, 0, rsets[i].polys.data(), nc * sizeof(void *)));
-        H2V_TRY(upload(pk, pk->scal, 0, ypow.data(), nc * sizeof(fe)));
-        fe *S = pk->sh_S.as<fe>() + i * n;
-        lincomb_kernel<<<gn, 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.as<fe>(), (uint32_t)nc, (uint32_t)n, S);
-        H2V_LAUNCHED();
-        // N_i = S_i - sum_j y^j R_ij, then Q_i = N_i / prod (X - p)
-        fe *cur_buf = Q + i * n, *oth = pk->sh_A.as<fe>();
-        H2V_CU(cudaMemcpyAsync(cur_buf, S, n * sizeof(fe), cudaMemcpyDeviceToDevice, st));
-        H2V_TRY(upload(pk, pk->scal, 0, r_comb[i].data(), m * sizeof(fe)));
-        sub_low_kernel<<<1, 32, 0, st>>>(cur_buf, pk->scal.as<fe>(), (uint32_t)m);
-        H2V_LAUNCHED();
-        H2V_TRY(sync(pk));
-        size_t len = n;
-        for (size_t t = 0; t < m; ++t) {
-            H2V_TRY(h2v_kate_division_dev(cur_buf, len, u64(ps[t]), oth));
-            --len;
-            std::swap(cur_buf, oth);
+        // construct_intermediate_sets: point sets are ordered sets of field elements (BTreeSet<Fr>: numeric order of the
+        // canonical values); commitments and rotation sets keep their order of first appearance
+        std::vector<uint32_t> rank(NPT);      // rank[i] = position of point i in the numeric order
+        {
+            std::vector<uint32_t> ord(NPT);
+            for (size_t i = 0; i < NPT; ++i) ord[i] = (uint32_t)i;
+            std::sort(ord.begin(), ord.end(), [&](uint32_t a, uint32_t b) { return frh::less_canonical(pt[a], pt[b]); });
+            for (size_t i = 0; i < NPT; ++i) rank[ord[i]] = (uint32_t)i;
         }
-        if (cur_buf != Q + i * n) H2V_CU(cudaMemcpyAsync(Q + i * n, cur_buf, len * sizeof(fe), cudaMemcpyDeviceToDevice, st));
-        H2V_CU(cudaMemsetAsync(Q + i * n + len, 0, (n - len) * sizeof(fe), st));
+        struct Com { const fe *poly; uint64_t mask; };       // mask over ranks
+        std::vector<Com> coms;
+        std::map<const fe *, size_t> com_of;
+        std::map<std::pair<const fe *, uint32_t>, Fr64> eval_of;
+        for (const Query &q : queries) {
+            const uint64_t bit = (uint64_t)1 << rank[q.pt];
+            mo.super_mask |= bit;
+            auto it = com_of.find(q.poly);
+            if (it == com_of.end()) {
+                com_of[q.poly] = coms.size();
+                coms.push_back(Com{q.poly, bit});
+            } else {
+                coms[it->second].mask |= bit;
+            }
+            eval_of[{q.poly, rank[q.pt]}] = q.eval;
+        }
+        for (const Com &c : coms) {
+            size_t i = 0;
+            for (; i < mo.rsets.size(); ++i)
+                if (mo.rsets[i].mask == c.mask) break;
+            if (i == mo.rsets.size()) mo.rsets.push_back(RSet{c.mask, {}});
+            mo.rsets[i].polys.push_back(c.poly);
+        }
+        mo.sorted_pts.resize(NPT);
+        for (size_t i = 0; i < NPT; ++i) mo.sorted_pts[rank[i]] = pt[i];
+        ProofState &S = *P[p];
+        S.ys = S.T.squeeze_challenge();
+        S.vs = S.T.squeeze_challenge();
+        const size_t NR = mo.rsets.size();
+        mo.r_comb.resize(NR);
+        mo.r_ij.resize(NR);
+        mo.set_pts.resize(NR);
+        mo.ypow.resize(NR);
+        for (size_t i = 0; i < NR; ++i) {
+            const std::vector<Fr64> ps = mo.pts_of(mo.rsets[i].mask);
+            const size_t m = ps.size(), nc = mo.rsets[i].polys.size();
+            const std::vector<std::vector<Fr64>> basis = lagrange_basis(ps);
+            Fr64 cur = frh::ONE;
+            mo.r_comb[i].assign(m, frh::zero());
+            mo.r_ij[i].resize(nc);
+            mo.ypow[i].resize(nc);
+            for (size_t j = 0; j < nc; ++j) {
+                mo.ypow[i][j] = cur;
+                std::vector<Fr64> evj;
+                for (size_t r = 0; r < NPT; ++r)
+                    if ((mo.rsets[i].mask >> r) & 1) evj.push_back(eval_of[{mo.rsets[i].polys[j], (uint32_t)r}]);
+                mo.r_ij[i][j] = lagrange_interpolate(basis, evj);
+                for (size_t t = 0; t < m; ++t) mo.r_comb[i][t] = frh::add(mo.r_comb[i][t], frh::mul(mo.r_ij[i][j][t], cur));
+                cur = frh::mul(cur, S.ys);
+            }
+            mo.set_pts[i] = ps;
+        }
+        return H2V_OK;
+    }));
+    const size_t NR = MO[0].rsets.size();
+    for (const MultiOpen &mo : MO)
+        if (mo.rsets.size() != NR) return failf(H2V_EINVAL, "create_proof: rotation sets differ between the proofs of a group");
+    size_t max_m = 1;
+    for (size_t i = 0; i < NR; ++i) max_m = std::max(max_m, MO[0].set_pts[i].size());
+    H2V_TRY(pk->sh_S.ensure(B * NR * n * sizeof(fe)));
+    H2V_TRY(pk->sh_A.ensure((B * n + 8) * sizeof(fe)));
+    H2V_TRY(pk->sh_B.ensure(std::max<size_t>(B * NR, B) * n * sizeof(fe)));
+    fe *S0 = pk->sh_S.as<fe>(), *Q = pk->sh_B.as<fe>();       // S_i and the quotient contributions Q_i of proof p: (p NR + i) n
+    {
+        // S_i(X) = sum_j y^j P_ij(X) for every proof and set in one launch; N_i = S_i - sum_j y^j R_ij
+        std::vector<const fe *> hp;
+        std::vector<Fr64> cf, low(B * NR * max_m, frh::zero());
+        std::vector<uint32_t> off;
+        for (size_t p = 0; p < B; ++p)
+            for (size_t i = 0; i < NR; ++i) {
+                off.push_back((uint32_t)hp.size());
+                hp.insert(hp.end(), MO[p].rsets[i].polys.begin(), MO[p].rsets[i].polys.end());
+                cf.insert(cf.end(), MO[p].ypow[i].begin(), MO[p].ypow[i].end());
+                std::copy(MO[p].r_comb[i].begin(), MO[p].r_comb[i].end(), low.begin() + (p * NR + i) * max_m);
+            }
+        off.push_back((uint32_t)hp.size());
+        H2V_TRY(lincomb(pk, hp, cf, off, S0, n, n));
+        H2V_CU(cudaMemcpyAsync(Q, S0, B * NR * n * sizeof(fe), cudaMemcpyDeviceToDevice, st));
+        H2V_TRY(sub_low(pk, Q, n, low, B * NR));
         H2V_TRY(sync(pk));
+    }
+    // Q_i = N_i / prod (X - p): one division per point of the set, every (proof, set) with a t-th point in one batched
+    // pass; each column ping-pongs between its home in Q and its own slot in sh_T
+    H2V_TRY(pk->sh_T.ensure(B * NR * n * sizeof(fe)));
+    {
+        std::vector<KateJob> jobs;
+        for (size_t t = 0; t < max_m; ++t) {
+            jobs.clear();
+            for (size_t p = 0; p < B; ++p)
+                for (size_t i = 0; i < NR; ++i) {
+                    const std::vector<Fr64> &ps = MO[p].set_pts[i];
+                    if (t >= ps.size()) continue;
+                    fe *home = Q + (p * NR + i) * n, *slot = pk->sh_T.as<fe>() + (p * NR + i) * n;
+                    KateJob j{t % 2 ? slot : home, t % 2 ? home : slot, n - t, {}};
+                    memcpy(j.b, u64(ps[t]), sizeof j.b);
+                    jobs.push_back(j);
+                }
+            H2V_TRY(kate_division_batch_dev(jobs.data(), jobs.size()));
+        }
+        for (size_t p = 0; p < B; ++p)
+            for (size_t i = 0; i < NR; ++i) {
+                const size_t m = MO[p].set_pts[i].size(), len = n - m;
+                fe *home = Q + (p * NR + i) * n;
+                if (m % 2) H2V_CU(cudaMemcpyAsync(home, pk->sh_T.as<fe>() + (p * NR + i) * n, len * sizeof(fe), cudaMemcpyDeviceToDevice, st));
+                H2V_CU(cudaMemsetAsync(home + len, 0, m * sizeof(fe), st));
+            }
     }
     // h(X) = sum_i v^i Q_i(X)
     {
-        std::vector<const fe *> hp(NR);
-        std::vector<Fr64> cf(NR);
-        Fr64 cur = frh::ONE;
-        for (size_t i = 0; i < NR; ++i) {
-            hp[i] = Q + i * n;
-            cf[i] = cur;
-            cur = frh::mul(cur, vs);
+        std::vector<const fe *> hp(B * NR);
+        std::vector<Fr64> cf(B * NR);
+        std::vector<uint32_t> off(B + 1);
+        for (size_t p = 0; p < B; ++p) {
+            Fr64 cur = frh::ONE;
+            off[p] = (uint32_t)(p * NR);
+            for (size_t i = 0; i < NR; ++i) {
+                hp[p * NR + i] = Q + (p * NR + i) * n;
+                cf[p * NR + i] = cur;
+                cur = frh::mul(cur, P[p]->vs);
+            }
         }
-        H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), NR * sizeof(void *)));
-        H2V_TRY(upload(pk, pk->scal, 0, cf.data(), NR * sizeof(fe)));
-        lincomb_kernel<<<gn, 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.as<fe>(), (uint32_t)NR, (uint32_t)n, hx_dev);
-        H2V_LAUNCHED();
+        off[B] = (uint32_t)(B * NR);
+        H2V_TRY(lincomb(pk, hp, cf, off, hx0, n, n));
         H2V_TRY(sync(pk));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, hx_dev, 1, pts));
-        H2V_TRY(write_points(T, pts));
+        H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, hx0, B, pts));
+        for (size_t p = 0; p < B; ++p) {
+            if (int rc = write_points(P[p]->T, pts.data() + p, 1)) {
+                bad = p;
+                return rc;
+            }
+        }
     }
-    const Fr64 uc = T.squeeze_challenge();
+    for (auto &s : P) s->uc = s->T.squeeze_challenge();
     {
         // L(X) = sum_i v^i z_i (S_i(X) - sum_j y^j R_ij(u)) - Z_T(u) h(X);  second opening proof = L / (X - u) / z_0
-        const std::vector<Fr64> sup = pts_of(super_mask);
-        std::vector<const fe *> hp(NR + 1);
-        std::vector<Fr64> cf(NR + 1);
-        Fr64 vp = frh::ONE, konst = frh::zero(), z0 = frh::ONE;
-        for (size_t i = 0; i < NR; ++i) {
-            Fr64 zi = frh::ONE;
-            for (size_t r = 0; r < NPT; ++r)
-                if (((super_mask & ~rsets[i].mask) >> r) & 1) zi = frh::mul(zi, frh::sub(uc, sorted_pts[r]));
-            if (i == 0) z0 = zi;
-            Fr64 ri = frh::zero(), yp = frh::ONE;
-            for (size_t j = 0; j < rsets[i].polys.size(); ++j) {
-                ri = frh::add(ri, frh::mul(yp, eval_small(r_ij[i][j], uc)));
-                yp = frh::mul(yp, ys);
+        std::vector<const fe *> hp(B * (NR + 1));
+        std::vector<Fr64> cf(B * (NR + 1)), konst(B), z0inv(B);
+        std::vector<uint32_t> off(B + 1);
+        H2V_TRY(par_proofs(B, [&](size_t p) -> int {
+            const MultiOpen &mo = MO[p];
+            const Fr64 &uc = P[p]->uc;
+            Fr64 vp = frh::ONE, z0 = frh::ONE;
+            konst[p] = frh::zero();
+            for (size_t i = 0; i < NR; ++i) {
+                Fr64 zi = frh::ONE;
+                for (size_t r = 0; r < NPT; ++r)
+                    if (((mo.super_mask & ~mo.rsets[i].mask) >> r) & 1) zi = frh::mul(zi, frh::sub(uc, mo.sorted_pts[r]));
+                if (i == 0) z0 = zi;
+                Fr64 ri = frh::zero(), yp = frh::ONE;
+                for (size_t j = 0; j < mo.rsets[i].polys.size(); ++j) {
+                    ri = frh::add(ri, frh::mul(yp, eval_small(mo.r_ij[i][j], uc)));
+                    yp = frh::mul(yp, P[p]->ys);
+                }
+                hp[p * (NR + 1) + i] = S0 + (p * NR + i) * n;
+                cf[p * (NR + 1) + i] = frh::mul(vp, zi);
+                konst[p] = frh::add(konst[p], frh::mul(cf[p * (NR + 1) + i], ri));
+                vp = frh::mul(vp, P[p]->vs);
             }
-            hp[i] = pk->sh_S.as<fe>() + i * n;
-            cf[i] = frh::mul(vp, zi);
-            konst = frh::add(konst, frh::mul(cf[i], ri));
-            vp = frh::mul(vp, vs);
+            Fr64 zt = frh::ONE;
+            for (const Fr64 &x : mo.pts_of(mo.super_mask)) zt = frh::mul(zt, frh::sub(uc, x));
+            hp[p * (NR + 1) + NR] = hx0 + p * n;
+            cf[p * (NR + 1) + NR] = frh::neg(zt);
+            off[p] = (uint32_t)(p * (NR + 1));
+            z0inv[p] = frh::inv(z0);
+            return H2V_OK;
+        }));
+        off[B] = (uint32_t)(B * (NR + 1));
+        fe *Lx = pk->sh_A.as<fe>();           // proof p's L at Lx + p n
+        H2V_TRY(lincomb(pk, hp, cf, off, Lx, n, n));
+        H2V_TRY(sub_low(pk, Lx, n, konst, B));
+        H2V_TRY(sync(pk));
+        fe *W = Q;        // the quotient contributions are no longer needed; proof p's W at W + p n
+        std::vector<KateJob> jobs(B);
+        for (size_t p = 0; p < B; ++p) {
+            jobs[p] = KateJob{Lx + p * n, W + p * n, n, {}};
+            memcpy(jobs[p].b, u64(P[p]->uc), sizeof jobs[p].b);
         }
-        Fr64 zt = frh::ONE;
-        for (const Fr64 &p : sup) zt = frh::mul(zt, frh::sub(uc, p));
-        hp[NR] = hx_dev;
-        cf[NR] = frh::neg(zt);
-        H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), (NR + 1) * sizeof(void *)));
-        H2V_TRY(upload(pk, pk->scal, 0, cf.data(), (NR + 1) * sizeof(fe)));
-        fe *Lx = pk->sh_A.as<fe>();
-        lincomb_kernel<<<gn, 256, 0, st>>>((const fe *const *)pk->ptrs.p, pk->scal.as<fe>(), (uint32_t)(NR + 1), (uint32_t)n, Lx);
-        H2V_LAUNCHED();
-        H2V_TRY(upload(pk, pk->scal, 0, &konst, sizeof(fe)));
-        sub_low_kernel<<<1, 32, 0, st>>>(Lx, pk->scal.as<fe>(), 1);
+        H2V_TRY(kate_division_batch_dev(jobs.data(), B));
+        for (size_t p = 0; p < B; ++p) H2V_CU(cudaMemsetAsync(W + p * n + (n - 1), 0, sizeof(fe), st));
+        H2V_TRY(put(pk, pk->scal, z0inv));
+        scale_cols_kernel<<<dim3(gn, (unsigned)B), 256, 0, st>>>(W, (uint32_t)n, pk->scal.as<fe>());
         H2V_LAUNCHED();
         H2V_TRY(sync(pk));
-        fe *W = Q;        // the quotient contributions are no longer needed
-        H2V_TRY(h2v_kate_division_dev(Lx, n, u64(uc), W));
-        H2V_CU(cudaMemsetAsync(W + (n - 1), 0, sizeof(fe), st));
-        const Fr64 z0inv = frh::inv(z0);
-        H2V_TRY(upload(pk, pk->scal, 0, &z0inv, sizeof(fe)));
-        scale_cols_kernel<<<dim3(gn, 1), 256, 0, st>>>(W, (uint32_t)n, pk->scal.as<fe>());
-        H2V_LAUNCHED();
-        H2V_TRY(sync(pk));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, W, 1, pts));
-        H2V_TRY(write_points(T, pts));
+        H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, W, B, pts));
+        for (size_t p = 0; p < B; ++p) {
+            if (int rc = write_points(P[p]->T, pts.data() + p, 1)) {
+                bad = p;
+                return rc;
+            }
+        }
     }
     lap();   // phase 6: multi-open argument
-    proof.swap(T.out);
+    proofs.resize(B);
+    for (size_t p = 0; p < B; ++p) proofs[p].swap(P[p]->T.out);
+    return H2V_OK;
+}
+
+// ---------------------------------------------------------------- groups
+// The per-proof workspace; a group of B proofs holds B times the buffers of one.
+DevBuf *workspace(h2v_pk *pk, size_t i) {
+    DevBuf *all[] = {&pk->adv_L, &pk->adv_C, &pk->adv_E, &pk->inst_L, &pk->inst_C, &pk->inst_E, &pk->pa_L, &pk->ps_L, &pk->pa_C, &pk->ps_C,
+                     &pk->pa_E, &pk->ps_E, &pk->z_L, &pk->z_C, &pk->z_E, &pk->zl_L, &pk->zl_C, &pk->zl_E, &pk->num, &pk->den,
+                     &pk->tails, &pk->ptrs, &pk->scal, &pk->offs, &pk->streams, &pk->pts, &pk->rnd_C, &pk->hq, &pk->hx_pieces,
+                     &pk->evals, &pk->pairs, &pk->sh_S, &pk->sh_A, &pk->sh_B, &pk->sh_T, &pk->sh_h, &pk->commits};
+    return i < sizeof all / sizeof all[0] ? all[i] : nullptr;
+}
+// device bytes one proof of a group adds (the rotation sets of the multi-open argument are counted as 8)
+size_t proof_bytes(const h2v_pk *pk) {
+    const size_t n = pk->n, ne = pk->ne, L = pk->lookup_input.size(), NS = pk->n_sets;
+    const size_t cols = pk->n_advice + pk->n_instance + 3 * L + NS;              // Lagrange, coefficient and extended forms
+    const size_t ncols = 2 * std::max(NS, L) + 1 + (pk->degree - 1) + 2 + 2 * 8 + 1;   // num / den, random, pieces, h, S / Q, L
+    return sizeof(fe) * (cols * (2 * n + (pk->stream_ext ? 0 : ne)) + 2 * ne + ncols * n) + 4096;
+}
+// The group size for n_proofs proofs: H2V_PROOF_GROUP if set, else as many as fit in the device memory left after the
+// key, with 8 GB kept free as the extended-sigma cache keeps it; capped so that every grid dimension and batch call
+// stays within its limits.  Streamed keys prove one at a time.
+size_t group_size(h2v_pk *pk, size_t n_proofs) {
+    if (pk->stream_ext || n_proofs <= 1) return 1;
+    const size_t cmax = std::max<size_t>({pk->n_sets, pk->lookup_input.size(), 16});
+    size_t cap = std::min<size_t>(65535 / cmax, (((size_t)1 << 31) - 1) / (pk->n * cmax));
+    cap = std::max<size_t>(1, std::min(cap, n_proofs));
+    if (const char *e = getenv("H2V_PROOF_GROUP")) {
+        const long g = atol(e);
+        if (g > 0) return std::min<size_t>((size_t)g, cap);
+    }
+    size_t free_b = 0, total_b = 0;
+    cudaMemGetInfo(&free_b, &total_b);
+    size_t held = 0;
+    for (size_t i = 0; DevBuf *b = workspace(pk, i); ++i) held += b->cap;
+    const size_t margin = (size_t)8 << 30, avail = free_b + held;
+    const size_t fit = avail > margin ? (avail - margin) / proof_bytes(pk) : 1;
+    return std::max<size_t>(1, std::min(fit, cap));
+}
+
+// Inputs of proof `idx` (who: the prefix of the error text)
+int check_inputs(const h2v_pk *pk, const ProofIn &in, const std::string &who) {
+    if (!in.seed) return failf(H2V_EINVAL, "%s: NULL rng seed", who.c_str());
+    if ((pk->n_advice && !in.advice) || (pk->n_instance && (!in.instances || !in.instance_len)))
+        return failf(H2V_EINVAL, "%s: NULL column list", who.c_str());
+    for (uint32_t c = 0; c < pk->n_advice; ++c)
+        if (!in.advice[c]) return failf(H2V_EINVAL, "%s: advice[%u] is NULL", who.c_str(), c);
+    for (uint32_t c = 0; c < pk->n_instance; ++c) {
+        if (in.instance_len[c] > pk->u)
+            return failf(H2V_EINVAL, "%s: InstanceTooLarge (%u values, %u usable rows)", who.c_str(), in.instance_len[c], pk->u);
+        if (in.instance_len[c] && !in.instances[c]) return failf(H2V_EINVAL, "%s: instances[%u] is NULL", who.c_str(), c);
+    }
+    return H2V_OK;
+}
+
+// n_proofs proofs in groups; emit(i, bytes) receives proof i.  A group that runs out of device memory is halved and run
+// again (a group of one needs what one proof always needed).  `batch`: prefix error texts with the proof they concern.
+template <class Emit> int run_proofs(h2v_pk *pk, size_t n_proofs, const ProofIn *in, bool batch, Emit emit) {
+    for (double &v : pk->last_ms) v = 0;
+    size_t G = group_size(pk, n_proofs);
+    for (size_t p0 = 0; p0 < n_proofs;) {
+        const size_t b = std::min(G, n_proofs - p0);
+        std::vector<std::vector<uint8_t>> out;
+        size_t bad = SIZE_MAX;
+        int rc = prove_group(pk, b, in + p0, out, bad);
+        if (rc == H2V_ENOMEM && pk->cached_sigma) {
+            // the key's opportunistic cache of extended sigma columns (streamed mode) took memory something else now needs:
+            // give it back for good and run the group again
+            cudaStreamSynchronize(pk->st);
+            pk->ext_cache.release();
+            pk->cached_sigma = 0;
+            continue;
+        }
+        if (rc == H2V_ENOMEM && b > 1) {
+            cudaStreamSynchronize(pk->st);
+            for (size_t i = 0; DevBuf *w = workspace(pk, i); ++i) w->release();
+            G = b / 2;
+            continue;
+        }
+        if (rc) {
+            cudaStreamSynchronize(pk->st);
+            if (batch) {
+                const std::string msg = h2v_last_error();
+                if (bad != SIZE_MAX) return failf(rc, "create_proofs: proof %zu: %s", p0 + bad, msg.c_str());
+                return failf(rc, "create_proofs: group of proofs %zu .. %zu: %s", p0, p0 + b - 1, msg.c_str());
+            }
+            return rc;
+        }
+        for (size_t p = 0; p < b; ++p) H2V_TRY(emit(p0 + p, out[p]));
+        pk->last_ms[7] += 1;      // groups run
+        p0 += b;
+    }
     return H2V_OK;
 }
 
@@ -1161,31 +1514,47 @@ extern "C" {
 int h2v_create_proof(h2v_pk_t pk, const uint64_t *const *advice, const uint64_t *const *instances, const uint32_t *instance_len,
                      const uint8_t rng_seed[32], uint8_t *proof_out, size_t proof_cap, size_t *proof_len) {
     if (!pk || !rng_seed || !proof_len) return failf(H2V_EINVAL, "create_proof: NULL argument");
-    if ((pk->n_advice && !advice) || (pk->n_instance && (!instances || !instance_len))) return failf(H2V_EINVAL, "create_proof: NULL column list");
+    const ProofIn in{advice, instances, instance_len, rng_seed};
+    H2V_TRY(check_inputs(pk, in, "create_proof"));
     if (cudaSetDevice(pk->dev) != cudaSuccess) {
         cudaGetLastError();
         return failf(H2V_ECUDA, "create_proof: no CUDA device (libh2v has no CPU fallback)");
     }
     std::lock_guard<std::mutex> lk(pk->mu);
-    std::vector<uint8_t> proof;
-    int rc = create_proof_locked(pk, advice, instances, instance_len, rng_seed, proof);
-    if (rc == H2V_ENOMEM && pk->cached_sigma) {
-        // the key's opportunistic cache of extended sigma columns (streamed mode) took memory something else now needs:
-        // give it back for good and run the proof again
-        cudaStreamSynchronize(pk->st);
-        pk->ext_cache.release();
-        pk->cached_sigma = 0;
-        proof.clear();
-        rc = create_proof_locked(pk, advice, instances, instance_len, rng_seed, proof);
+    return run_proofs(pk, 1, &in, false, [&](size_t, const std::vector<uint8_t> &proof) -> int {
+        *proof_len = proof.size();
+        if (proof.size() > proof_cap || !proof_out)
+            return failf(H2V_EINVAL, "create_proof: proof needs %zu bytes, buffer has %zu", proof.size(), proof_cap);
+        memcpy(proof_out, proof.data(), proof.size());
+        return H2V_OK;
+    });
+}
+int h2v_create_proofs(h2v_pk_t pk, size_t n_proofs, const uint64_t *const *const *advice, const uint64_t *const *const *instances,
+                      const uint32_t *const *instance_len, const uint8_t *rng_seeds, uint8_t *proofs_out, size_t proof_stride) {
+    if (!pk) return failf(H2V_EINVAL, "create_proofs: NULL key");
+    if (!n_proofs) return H2V_OK;
+    if (!rng_seeds || !proofs_out || (pk->n_advice && !advice) || (pk->n_instance && (!instances || !instance_len)))
+        return failf(H2V_EINVAL, "create_proofs: NULL argument");
+    const size_t size = h2v_proof_size(pk);
+    if (proof_stride < size) return failf(H2V_EINVAL, "create_proofs: proof_stride %zu is shorter than a proof (%zu bytes)", proof_stride, size);
+    std::vector<ProofIn> in(n_proofs);
+    for (size_t p = 0; p < n_proofs; ++p) {
+        in[p] = ProofIn{pk->n_advice ? advice[p] : nullptr, pk->n_instance ? instances[p] : nullptr, pk->n_instance ? instance_len[p] : nullptr,
+                        rng_seeds + 32 * p};
+        char who[64];
+        snprintf(who, sizeof who, "create_proofs: proof %zu", p);
+        H2V_TRY(check_inputs(pk, in[p], who));
     }
-    if (rc) {
-        cudaStreamSynchronize(pk->st);
-        return rc;
+    if (cudaSetDevice(pk->dev) != cudaSuccess) {
+        cudaGetLastError();
+        return failf(H2V_ECUDA, "create_proofs: no CUDA device (libh2v has no CPU fallback)");
     }
-    *proof_len = proof.size();
-    if (proof.size() > proof_cap || !proof_out) return failf(H2V_EINVAL, "create_proof: proof needs %zu bytes, buffer has %zu", proof.size(), proof_cap);
-    memcpy(proof_out, proof.data(), proof.size());
-    return H2V_OK;
+    std::lock_guard<std::mutex> lk(pk->mu);
+    return run_proofs(pk, n_proofs, in.data(), true, [&](size_t p, const std::vector<uint8_t> &proof) -> int {
+        if (proof.size() != size) return failf(H2V_EINVAL, "create_proofs: proof %zu has %zu bytes, expected %zu", p, proof.size(), size);
+        memcpy(proofs_out + p * proof_stride, proof.data(), size);
+        return H2V_OK;
+    });
 }
 size_t h2v_proof_size(h2v_pk_t pk) {
     if (!pk) return 0;

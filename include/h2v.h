@@ -267,10 +267,20 @@ void h2v_pk_free(h2v_pk_t pk);
  * byte stream, exactly h2v_proof_size(pk) bytes) to proof_out. */
 int h2v_create_proof(h2v_pk_t pk, const uint64_t *const *advice, const uint64_t *const *instances, const uint32_t *instance_len,
                      const uint8_t rng_seed[32], uint8_t *proof_out, size_t proof_cap, size_t *proof_len);
+/* n_proofs proofs on one key: proof p = h2v_create_proof(pk, advice[p], instances[p], instance_len[p], rng_seeds + 32 p),
+ * written to proofs_out + p * proof_stride (proof_stride >= h2v_proof_size(pk)).  Byte for byte the proofs of n_proofs
+ * h2v_create_proof calls; the proofs run in groups, phase by phase, so that each launch, commit and synchronisation is
+ * paid once per group.  Group size: H2V_PROOF_GROUP if set, else as many proofs as fit in the device memory the key
+ * leaves (8 GB kept free); a group that runs out of memory is halved; streamed keys prove one at a time.  Every proof's
+ * inputs are checked before any device work; an error text names the proof it concerns ("create_proofs: proof 2: ...")
+ * and the key stays usable.  n_proofs = 0 does nothing.  Calls on one key serialise. */
+int h2v_create_proofs(h2v_pk_t pk, size_t n_proofs, const uint64_t *const *const *advice, const uint64_t *const *const *instances,
+                      const uint32_t *const *instance_len, const uint8_t *rng_seeds, uint8_t *proofs_out, size_t proof_stride);
 size_t h2v_proof_size(h2v_pk_t pk);
-/* wall-clock milliseconds per phase of the last create_proof on this key: 0 upload + advice commitments, 1 lookup
- * permutations, 2 grand products, 3 random polynomial + transforms, 4 evaluate_h + quotient commitments, 5 evaluations,
- * 6 multi-open argument */
+/* wall-clock milliseconds per phase of the last h2v_create_proof / h2v_create_proofs call on this key, summed over the
+ * call's groups: 0 upload + advice commitments, 1 lookup permutations, 2 grand products, 3 random polynomial +
+ * transforms, 4 evaluate_h + quotient commitments, 5 evaluations, 6 multi-open argument; out[7]: the number of groups
+ * the call ran in */
 int h2v_pk_last_phase_ms(h2v_pk_t pk, double out[8]);
 
 /* ---- circuit builder ("next": SURVEY.md 8(f) row 4; host-side, no device needed) -----------------------------------

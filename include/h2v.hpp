@@ -7,6 +7,7 @@
 // Upstream panics (assert!) become std::invalid_argument; CUDA failures std::runtime_error (no CPU fallback).
 // The reference reaches these through src/scaffold/mod.rs:273 (create_pk) and :296 (gen_snark_shplonk).
 #pragma once
+#include <algorithm>
 #include <array>
 #include <cstdint>
 #include <stdexcept>
@@ -260,6 +261,34 @@ class ProvingKey {
         check(h2v_create_proof(h_, reinterpret_cast<const uint64_t *const *>(advice.data()), ip.data(), il.data(), rng_seed.data(), out.data(),
                                out.size(), &len));
         out.resize(len);
+        return out;
+    }
+    // proof p = create_proof(advice[p], instances[p], rng_seeds[p]), the proofs run in groups (h2v_create_proofs)
+    std::vector<std::vector<uint8_t>> create_proofs(const std::vector<std::vector<const Fr *>> &advice,
+                                                    const std::vector<std::vector<std::vector<Fr>>> &instances,
+                                                    const std::vector<std::array<uint8_t, 32>> &rng_seeds) const {
+        const size_t B = advice.size();
+        if (instances.size() != B || rng_seeds.size() != B) throw std::invalid_argument("create_proofs: list lengths differ");
+        std::vector<std::vector<const uint64_t *>> ip(B);
+        std::vector<std::vector<uint32_t>> il(B);
+        std::vector<const uint64_t *const *> ap(B), ipp(B);
+        std::vector<const uint32_t *> ilp(B);
+        std::vector<uint8_t> seeds(32 * B);
+        for (size_t p = 0; p < B; ++p) {
+            for (const auto &c : instances[p]) {
+                ip[p].push_back(reinterpret_cast<const uint64_t *>(c.data()));
+                il[p].push_back((uint32_t)c.size());
+            }
+            ap[p] = reinterpret_cast<const uint64_t *const *>(advice[p].data());
+            ipp[p] = ip[p].data();
+            ilp[p] = il[p].data();
+            std::copy(rng_seeds[p].begin(), rng_seeds[p].end(), seeds.begin() + 32 * p);
+        }
+        const size_t size = h2v_proof_size(h_);
+        std::vector<uint8_t> flat(B * size);
+        check(h2v_create_proofs(h_, B, ap.data(), ipp.data(), ilp.data(), seeds.data(), flat.data(), size));
+        std::vector<std::vector<uint8_t>> out(B);
+        for (size_t p = 0; p < B; ++p) out[p].assign(flat.begin() + p * size, flat.begin() + (p + 1) * size);
         return out;
     }
 
