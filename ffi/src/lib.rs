@@ -30,6 +30,17 @@ pub struct H2vCircuit {
     pub n_advice_queries: u32, pub advice_query_col: *const u32, pub advice_query_rot: *const i32,
     pub n_fixed_queries: u32, pub fixed_query_col: *const u32, pub fixed_query_rot: *const i32,
 }
+/// `h2v_mock_failure_t`: one failed constraint of `h2v_mock_prover` (kind = H2V_MOCK_*)
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default, PartialEq, Eq)]
+pub struct H2vMockFailure { pub kind: u32, pub column: u32, pub row: u32, pub other_column: u32, pub other_row: u32 }
+pub const H2V_MOCK_GATE: u32 = 1;
+pub const H2V_MOCK_GATE_UNUSABLE: u32 = 2;
+pub const H2V_MOCK_LOOKUP: u32 = 3;
+pub const H2V_MOCK_SIGMA_NOT_DELTA_OMEGA: u32 = 4;
+pub const H2V_MOCK_SIGMA_NOT_PERMUTATION: u32 = 5;
+pub const H2V_MOCK_COPY_UNUSABLE: u32 = 6;
+pub const H2V_MOCK_COPY: u32 = 7;
 pub const H2V_BASIS_MONOMIAL: c_int = 0;
 pub const H2V_BASIS_LAGRANGE: c_int = 1;
 pub const H2V_OP_LAGRANGE_TO_COEFF: c_int = 0;
@@ -101,6 +112,9 @@ extern "C" {
                             rng_seed: *const u8, proof_out: *mut u8, proof_cap: usize, proof_len: *mut usize) -> c_int;
     pub fn h2v_create_proofs(pk: *mut H2vPk, n_proofs: usize, advice: *const *const *const u64, instances: *const *const *const u64,
                              instance_len: *const *const u32, rng_seeds: *const u8, proofs_out: *mut u8, proof_stride: usize) -> c_int;
+    pub fn h2v_mock_prover(cs: *const H2vCircuit, fixed: *const *const u64, sigma: *const *const u64, advice: *const *const u64,
+                           instances: *const *const u64, instance_len: *const u32, failures_out: *mut H2vMockFailure, cap: usize,
+                           n_failures: *mut u64) -> c_int;
     pub fn h2v_quotient_gates_dev(dom: *mut H2vDomain, d_h: *mut c_void, y: *const u64, n_gates: usize, d_q: *const c_void,
                                   q_stride: usize, d_a: *const c_void, a_stride: usize) -> c_int;
     pub fn h2v_quotient_permutation_dev(dom: *mut H2vDomain, d_h: *mut c_void, y: *const u64, beta: *const u64, gamma: *const u64,
@@ -117,6 +131,24 @@ extern "C" {
                                    d_input: *const c_void, d_table: *const c_void, d_perm_input: *const c_void,
                                    d_perm_table: *const c_void, d_z: *const c_void, d_l0: *const c_void, d_l_last: *const c_void,
                                    d_l_active: *const c_void) -> c_int;
+}
+
+/// `MockProver::run(k, circuit, instances)` on the device: (the first `max_failures` failures in the order gates, lookups,
+/// permutation; their total).  Columns are Lagrange, 2^k values each; no SRS and no key.
+pub fn mock_prover(cs: &H2vCircuit, fixed: &[&[Fr]], sigma: &[&[Fr]], advice: &[&[Fr]], instances: &[&[Fr]],
+                   max_failures: usize) -> (Vec<H2vMockFailure>, u64) {
+    let n = 1usize << cs.k;
+    assert!(fixed.len() == cs.n_fixed as usize && sigma.len() == cs.n_perm as usize && advice.len() == cs.n_advice as usize
+            && instances.len() == cs.n_instance as usize);
+    assert!(fixed.iter().chain(sigma).chain(advice).all(|c| c.len() == n));
+    let ptrs = |cols: &[&[Fr]]| -> Vec<*const u64> { cols.iter().map(|c| c.as_ptr() as *const u64).collect() };
+    let (f, s, a, i) = (ptrs(fixed), ptrs(sigma), ptrs(advice), ptrs(instances));
+    let il: Vec<u32> = instances.iter().map(|c| c.len() as u32).collect();
+    let mut out = vec![H2vMockFailure::default(); max_failures];
+    let mut total = 0u64;
+    ok(unsafe { h2v_mock_prover(cs, f.as_ptr(), s.as_ptr(), a.as_ptr(), i.as_ptr(), il.as_ptr(), out.as_mut_ptr(), max_failures, &mut total) });
+    out.truncate((total as usize).min(max_failures));
+    (out, total)
 }
 
 /// `plonk::lookup::prover::permute_expression_pair` on the usable rows; `Err(())` = `Error::ConstraintSystemFailure`

@@ -13,6 +13,7 @@ Fr (n, 4), G1Affine (n, 8), G1 Jacobian (12,).
 """
 import ctypes as C
 import os
+from collections import namedtuple
 
 import numpy as np
 
@@ -37,6 +38,7 @@ ABI_SYMBOLS = [
     "h2v_domain_rotate_omega", "h2v_domain_rotate_extended", "h2v_domain_l_i_range", "h2v_domain_fill", "h2v_kate_division_dev",
     "h2v_quotient_gates_ptrs_dev", "h2v_quotient_permutation_ptrs_dev", "h2v_quotient_permutation_range_ptrs_dev", "h2v_commit_batch_resident",
     "h2v_pk_load", "h2v_pk_free", "h2v_create_proof", "h2v_create_proofs", "h2v_proof_size", "h2v_pk_last_phase_ms",
+    "h2v_mock_prover", "h2v_mock_last_ms",
     "h2v_transcript_new", "h2v_transcript_free", "h2v_transcript_common_point", "h2v_transcript_common_scalar",
     "h2v_transcript_write_point", "h2v_transcript_write_scalar", "h2v_transcript_squeeze_challenge", "h2v_transcript_bytes",
     "h2v_poseidon_permutation", "h2v_poseidon_permutation_variant", "h2v_chacha20_fr_random", "h2v_chacha20_block",
@@ -152,6 +154,8 @@ def lib():
         L.h2v_proof_size.argtypes = [C.c_void_p]
         L.h2v_proof_size.restype = C.c_size_t
         L.h2v_pk_last_phase_ms.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
+        L.h2v_mock_prover.argtypes = [C.c_void_p] * 7 + [C.c_size_t, C.POINTER(C.c_uint64)]
+        L.h2v_mock_last_ms.argtypes = [C.POINTER(C.c_double)]
         L.h2v_transcript_new.argtypes = [C.POINTER(C.c_void_p)]
         L.h2v_transcript_free.argtypes = [C.c_void_p]
         L.h2v_transcript_free.restype = None
@@ -815,6 +819,23 @@ class _CircuitT(C.Structure):
                 ("n_fixed_queries", C.c_uint32), ("fixed_query_col", C.c_void_p), ("fixed_query_rot", C.c_void_p)]
 
 
+def _circuit_struct(cs):
+    """cs dict (see ProvingKey) -> (h2v_circuit_t, the index arrays it points into: keep them alive while it is used)"""
+    u32 = lambda xs: np.ascontiguousarray(xs, dtype=np.uint32)
+    a = dict(
+        ga=u32([g[0] for g in cs["gates"]]), gs=u32([g[1] for g in cs["gates"]]),
+        li=u32([l[0] for l in cs["lookups"]]), lt=u32([l[1] for l in cs["lookups"]]),
+        pk=np.ascontiguousarray([p[0] for p in cs["permutation"]], dtype=np.uint8), pi=u32([p[1] for p in cs["permutation"]]),
+        aqc=u32([q[0] for q in cs["advice_queries"]]), aqr=np.ascontiguousarray([q[1] for q in cs["advice_queries"]], dtype=np.int32),
+        fqc=u32([q[0] for q in cs["fixed_queries"]]), fqr=np.ascontiguousarray([q[1] for q in cs["fixed_queries"]], dtype=np.int32))
+    p = lambda x: x.ctypes.data if x.size else None
+    ct = _CircuitT(cs["k"], cs["degree"], cs["blinding_factors"], cs["n_advice"], cs["n_fixed"], cs["n_instance"],
+                   len(cs["gates"]), p(a["ga"]), p(a["gs"]), len(cs["lookups"]), p(a["li"]), p(a["lt"]),
+                   len(cs["permutation"]), p(a["pk"]), p(a["pi"]), len(cs["advice_queries"]), p(a["aqc"]), p(a["aqr"]),
+                   len(cs["fixed_queries"]), p(a["fqc"]), p(a["fqr"]))
+    return ct, a
+
+
 class ProvingKey:
     """halo2 `ProvingKey` for a halo2-base-shaped constraint system, resident on the device.
 
@@ -824,19 +845,7 @@ class ProvingKey:
 
     def __init__(self, params, cs, fixed, sigma, vk_transcript_repr):
         self.params, self.cs = params, cs
-        u32 = lambda xs: np.ascontiguousarray(xs, dtype=np.uint32)
-        self._arrs = dict(
-            ga=u32([g[0] for g in cs["gates"]]), gs=u32([g[1] for g in cs["gates"]]),
-            li=u32([l[0] for l in cs["lookups"]]), lt=u32([l[1] for l in cs["lookups"]]),
-            pk=np.ascontiguousarray([p[0] for p in cs["permutation"]], dtype=np.uint8), pi=u32([p[1] for p in cs["permutation"]]),
-            aqc=u32([q[0] for q in cs["advice_queries"]]), aqr=np.ascontiguousarray([q[1] for q in cs["advice_queries"]], dtype=np.int32),
-            fqc=u32([q[0] for q in cs["fixed_queries"]]), fqr=np.ascontiguousarray([q[1] for q in cs["fixed_queries"]], dtype=np.int32))
-        a = self._arrs
-        p = lambda x: x.ctypes.data if x.size else None
-        ct = _CircuitT(cs["k"], cs["degree"], cs["blinding_factors"], cs["n_advice"], cs["n_fixed"], cs["n_instance"],
-                       len(cs["gates"]), p(a["ga"]), p(a["gs"]), len(cs["lookups"]), p(a["li"]), p(a["lt"]),
-                       len(cs["permutation"]), p(a["pk"]), p(a["pi"]), len(cs["advice_queries"]), p(a["aqc"]), p(a["aqr"]),
-                       len(cs["fixed_queries"]), p(a["fqc"]), p(a["fqr"]))
+        ct, self._arrs = _circuit_struct(cs)
         n = 1 << cs["k"]
         fx = [_fr(c, n) for c in fixed]
         sg = [_fr(c, n) for c in sigma]
@@ -913,6 +922,57 @@ class ProvingKey:
         _check(lib().h2v_pk_last_phase_ms(self._h, buf))
         names = ["advice_commit", "lookup_permute", "grand_products", "transforms", "quotient", "evaluations", "multiopen"]
         return dict(zip(names, [float(x) for x in buf]))
+
+
+# ----------------------------------------------------------------------------- dev/mock.rs MockProver
+MOCK_GATE, MOCK_GATE_UNUSABLE, MOCK_LOOKUP, MOCK_SIGMA_NOT_DELTA_OMEGA, MOCK_SIGMA_NOT_PERMUTATION, MOCK_COPY_UNUSABLE, MOCK_COPY = range(1, 8)
+MOCK_KINDS = {MOCK_GATE: "gate", MOCK_GATE_UNUSABLE: "gate_unusable", MOCK_LOOKUP: "lookup",
+              MOCK_SIGMA_NOT_DELTA_OMEGA: "sigma_not_delta_omega", MOCK_SIGMA_NOT_PERMUTATION: "sigma_not_permutation",
+              MOCK_COPY_UNUSABLE: "copy_unusable", MOCK_COPY: "copy"}
+MockFailure = namedtuple("MockFailure", "kind column row other_column other_row")
+
+
+class _MockFailureT(C.Structure):
+    _fields_ = [(f, C.c_uint32) for f in MockFailure._fields]
+
+
+class MockProver:
+    """halo2 `MockProver::run(k, circuit, instances)` on the device (h2v_mock_prover): every gate, lookup and copy
+    constraint of a laid-out circuit.  `failures`: the first max_failures failures (MockFailure, kind = MOCK_*) in the
+    order gates, lookups, permutation; `n_failures`: how many there are in all; `upload_ms` / `check_ms`: the call's
+    wall-clock time moving the columns to the device and checking them."""
+
+    def __init__(self, failures, n_failures, upload_ms, check_ms):
+        self.failures, self.n_failures, self.upload_ms, self.check_ms = failures, n_failures, upload_ms, check_ms
+
+    @classmethod
+    def run(cls, cs, fixed, sigma, advice, instances, max_failures=64):
+        """cs as ProvingKey takes it; fixed / sigma / advice: Lagrange columns of 2^k Fr (Montgomery limbs, shape (n, 4));
+        instances: one array of public inputs per instance column"""
+        ct, _keep = _circuit_struct(cs)      # the index arrays ct points into
+        n = 1 << cs["k"]
+        fx, sg, adv = [_fr(c, n) for c in fixed], [_fr(c, n) for c in sigma], [_fr(c, n) for c in advice]
+        inst = [_fr(np.asarray(c, dtype=np.uint64).reshape(-1, 4)) for c in instances]
+        if (len(fx), len(sg), len(adv), len(inst)) != (cs["n_fixed"], len(cs["permutation"]), cs["n_advice"], cs["n_instance"]):
+            raise ValueError("MockProver: fixed / sigma / advice / instance column count does not match the constraint system")
+        arr = lambda cols: (C.c_void_p * max(1, len(cols)))(*[c.ctypes.data for c in cols])
+        il = np.ascontiguousarray([c.shape[0] for c in inst] or [0], dtype=np.uint32)
+        out = (_MockFailureT * max(1, max_failures))()
+        total = C.c_uint64()
+        _check(lib().h2v_mock_prover(C.byref(ct), arr(fx), arr(sg), arr(adv), arr(inst), _ptr(il), out, max_failures, C.byref(total)))
+        ms = (C.c_double * 2)()
+        _check(lib().h2v_mock_last_ms(ms))
+        got = min(max_failures, total.value)
+        fails = [MockFailure(*(getattr(out[i], f) for f in MockFailure._fields)) for i in range(got)]
+        return cls(fails, total.value, ms[0], ms[1])
+
+    def assert_satisfied(self):
+        if self.n_failures:
+            lines = [f"{MOCK_KINDS.get(f.kind, f.kind)}: column {f.column} row {f.row} (other: column {f.other_column} row {f.other_row})"
+                     for f in self.failures[:16]]
+            more = self.n_failures - len(lines)
+            raise AssertionError(f"{self.n_failures} constraint(s) not satisfied:\n  " + "\n  ".join(lines)
+                                 + (f"\n  ... and {more} more" if more > 0 else ""))
 
 
 # ----------------------------------------------------------------------------- device self-tests

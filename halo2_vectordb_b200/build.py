@@ -30,7 +30,7 @@ def build(force=False, verbose=False):
     srcs = _sources()
     nvcc = os.environ.get("NVCC", "nvcc")
     if force or _newer(LIB, srcs):
-        # two translation units (kernels + ABI, prover) compiled side by side; -split-compile 0: ptxas works on the
+        # the translation units (kernels + ABI, prover, circuit builder, mock prover) compiled side by side; -split-compile 0: ptxas works on the
         # kernels of one unit in parallel (4.5 min -> 2 min on 8 cores), same code
         common = [nvcc, "-Xcompiler", "-fPIC", "-O3", "-std=c++17", "-lineinfo", "-split-compile", "0", *ARCH,
                   "-I" + os.path.join(ROOT, "include"), "-I" + CSRC]
@@ -38,7 +38,7 @@ def build(force=False, verbose=False):
             common.insert(1, "-Xptxas=-v")
         os.makedirs(os.path.join(PKG, "build"), exist_ok=True)
         procs, objs = [], []
-        for unit in ("h2v", "prover", "circuit"):
+        for unit in ("h2v", "prover", "circuit", "mock"):
             src, obj = os.path.join(CSRC, unit + ".cu"), os.path.join(PKG, "build", unit + ".o")
             objs.append(obj)
             deps = [s_ for s_ in srcs if not s_.endswith(".cu")] + [src]

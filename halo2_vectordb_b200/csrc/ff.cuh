@@ -96,6 +96,21 @@ H2V_HD bool fe_eq(const fe &a, const fe &b) {
     for (int i = 0; i < 8; ++i) o |= a.v[i] ^ b.v[i];
     return o == 0;
 }
+#ifdef __CUDACC__
+// order and equality of sort keys (canonical integers, 8 limbs)
+__device__ __forceinline__ bool key_less(const fe &a, const fe &b) {
+#pragma unroll
+    for (int i = 7; i >= 0; --i)
+        if (a.v[i] != b.v[i]) return a.v[i] < b.v[i];
+    return false;
+}
+__device__ __forceinline__ bool key_eq(const fe &a, const fe &b) {
+    uint32_t d = 0;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) d |= a.v[i] ^ b.v[i];
+    return d == 0;
+}
+#endif
 
 // ------------------------------------------------------------------ add / sub
 #ifdef __CUDA_ARCH__

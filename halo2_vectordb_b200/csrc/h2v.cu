@@ -1800,6 +1800,36 @@ int h2v_kate_division(const uint64_t *a, size_t n, const uint64_t b[4], uint64_t
 }  // extern "C"
 
 // ================================================================== lookup argument: permuted columns
+namespace h2v {
+int sort_canonical_dev(cudaStream_t st, const fe *const *d_srcs, uint32_t slices, uint32_t u, uint32_t n_pad, fe *keys) {
+    lookup_canon_pad_batch_kernel<<<dim3((n_pad + 255) / 256, slices), 256, 0, st>>>(d_srcs, keys, u, n_pad);
+    H2V_LAUNCHED();
+    const uint32_t tile = std::min<uint32_t>(H2V_SORT_TILE, n_pad);
+    const unsigned tiles_n = n_pad / tile;
+    const size_t smem = (size_t)tile * sizeof(fe);
+    bitonic_tile_kernel<<<dim3(tiles_n, slices), H2V_SORT_TILE / 2, smem, st>>>(keys, n_pad, 0, 1);
+    H2V_LAUNCHED();
+    for (uint32_t k = 2 * tile; k <= n_pad && k; k <<= 1) {
+        for (uint32_t j = k >> 1; j >= tile; j >>= 1) {
+            bitonic_global_kernel<<<dim3((n_pad / 2 + 255) / 256, slices), 256, 0, st>>>(keys, n_pad, k, j);
+            H2V_LAUNCHED();
+        }
+        bitonic_tile_kernel<<<dim3(tiles_n, slices), H2V_SORT_TILE / 2, smem, st>>>(keys, n_pad, k, 0);
+        H2V_LAUNCHED();
+    }
+    return H2V_OK;
+}
+int scan_u32_dev(cudaStream_t st, const uint32_t *cnt, uint32_t len, uint32_t *offs, uint32_t *tiles, uint32_t *scratch, uint32_t *total) {
+    const uint32_t ntiles = (len + H2V_SCAN_TILE - 1) / H2V_SCAN_TILE;
+    msm_scan_tiles_kernel<<<ntiles, 256, 0, st>>>(cnt, tiles, len);
+    H2V_LAUNCHED();
+    msm_scan_top_kernel<<<1, 256, 0, st>>>(tiles, ntiles, total);
+    H2V_LAUNCHED();
+    msm_scan_apply_kernel<<<ntiles, 256, 0, st>>>(cnt, tiles, offs, scratch, len);
+    H2V_LAUNCHED();
+    return H2V_OK;
+}
+}  // namespace h2v
 namespace {
 // A', S' of `u` usable rows from device-resident input / table expressions (Montgomery); g_poly.mu held by the caller
 // All lookup arguments of one proof phase in one set of launches (lookup.cuh): inputs[l] / tables[l] are device columns,
@@ -1837,38 +1867,14 @@ int run_permute_batch(cudaStream_t st, const fe *const *inputs, const fe *const 
     H2V_CU(cudaMemsetAsync(err, 0, sizeof(int), st));
     H2V_CU(cudaMemcpyAsync(d_tmap, tmap.data(), L * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
     H2V_CU(cudaMemcpyAsync(d_srcs, srcs.data(), slices * sizeof(void *), cudaMemcpyHostToDevice, st));
-    const unsigned gp = (n_pad + 255) / 256, gu = (u + 255) / 256;
-    {
-        lookup_canon_pad_batch_kernel<<<dim3(gp, slices), 256, 0, st>>>(d_srcs, keys, u, n_pad);
-        H2V_LAUNCHED();
-        const uint32_t tile = std::min<uint32_t>(H2V_SORT_TILE, n_pad);
-        const unsigned tiles_n = n_pad / tile;
-        const size_t smem = (size_t)tile * sizeof(fe);
-        bitonic_tile_kernel<<<dim3(tiles_n, slices), H2V_SORT_TILE / 2, smem, st>>>(keys, n_pad, 0, 1);
-        H2V_LAUNCHED();
-        for (uint32_t k = 2 * tile; k <= n_pad && k; k <<= 1) {
-            for (uint32_t j = k >> 1; j >= tile; j >>= 1) {
-                bitonic_global_kernel<<<dim3((n_pad / 2 + 255) / 256, slices), 256, 0, st>>>(keys, n_pad, k, j);
-                H2V_LAUNCHED();
-            }
-            bitonic_tile_kernel<<<dim3(tiles_n, slices), H2V_SORT_TILE / 2, smem, st>>>(keys, n_pad, k, 0);
-            H2V_LAUNCHED();
-        }
-    }
+    const unsigned gu = (u + 255) / 256;
+    H2V_TRY(sort_canonical_dev(st, d_srcs, slices, u, n_pad, keys));
     lookup_fill_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(free_, 1u, (uint32_t)rows);
     H2V_LAUNCHED();
     lookup_flags_batch_kernel<<<dim3(gu, L), 256, 0, st>>>(keys, d_tmap, u, n_pad, rep, free_, err);
     H2V_LAUNCHED();
-    for (int which = 0; which < 2; ++which) {
-        const uint32_t *cnt = which ? free_ : rep;
-        uint32_t *offs = which ? free_offs : rep_offs, *tl = tiles + which * ntiles;
-        msm_scan_tiles_kernel<<<ntiles, 256, 0, st>>>(cnt, tl, (uint32_t)rows);
-        H2V_LAUNCHED();
-        msm_scan_top_kernel<<<1, 256, 0, st>>>(tl, ntiles, totals + which);
-        H2V_LAUNCHED();
-        msm_scan_apply_kernel<<<ntiles, 256, 0, st>>>(cnt, tl, offs, scratch, (uint32_t)rows);
-        H2V_LAUNCHED();
-    }
+    for (int which = 0; which < 2; ++which)
+        H2V_TRY(scan_u32_dev(st, which ? free_ : rep, (uint32_t)rows, which ? free_offs : rep_offs, tiles + which * ntiles, scratch, totals + which));
     lookup_emit_input_batch_kernel<<<dim3(gu, L), 256, 0, st>>>(keys, u, n_pad, rep, rep_offs, rep_rows, d_out_a, a_stride, d_out_s, s_stride);
     H2V_LAUNCHED();
     lookup_emit_table_batch_kernel<<<dim3(gu, L), 256, 0, st>>>(keys, d_tmap, L, u, n_pad, free_, free_offs, rep_offs, totals, rep_rows, d_out_s,

@@ -79,6 +79,18 @@ struct QuotientBatch {
     const void *l0, *l_last, *l_active;
 };
 int quotient_batch_dev(h2v_domain_t h, const QuotientBatch &b);
+
+// The constraint-system checks of h2v_pk_load, in its order: degree, k, blinding factors, then "NULL column list" when
+// have_column_lists is false, then every column index.  Errors name `who`.
+int check_circuit(const h2v_circuit_t *cs, bool have_column_lists, const char *who);
+
+// Launch helpers of h2v.cu over the lookup argument's kernels (lookup.cuh, msm.cuh), asynchronous on `st`.
+struct fe;
+// keys + s * n_pad <- the first u values of column d_srcs[s] (device pointer table), canonical and sorted ascending, padded
+// with all-ones keys to n_pad (a power of two >= u), for s < slices
+int sort_canonical_dev(cudaStream_t st, const fe *const *d_srcs, uint32_t slices, uint32_t u, uint32_t n_pad, fe *keys);
+// offs = exclusive prefix sums of cnt[0 .. len), *total = their sum (device); tiles: ceil(len / 2048) words, scratch: len words
+int scan_u32_dev(cudaStream_t st, const uint32_t *cnt, uint32_t len, uint32_t *offs, uint32_t *tiles, uint32_t *scratch, uint32_t *total);
 }  // namespace h2v
 
 #define H2V_CU(x)                                                                                                  \

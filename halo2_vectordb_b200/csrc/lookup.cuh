@@ -18,18 +18,6 @@ namespace h2v {
 typedef FrP FrL;
 #define H2V_SORT_TILE 1024u          // elements per shared-memory tile (32 KiB)
 
-__device__ __forceinline__ bool key_less(const fe &a, const fe &b) {
-#pragma unroll
-    for (int i = 7; i >= 0; --i)
-        if (a.v[i] != b.v[i]) return a.v[i] < b.v[i];
-    return false;
-}
-__device__ __forceinline__ bool key_eq(const fe &a, const fe &b) {
-    uint32_t d = 0;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) d |= a.v[i] ^ b.v[i];
-    return d == 0;
-}
 
 // out[i] = canonical(in[i]) for i < n, all-ones (greater than any field element) for n <= i < n_pad
 // (grid.y = 0: input -> keys[0 .. n_pad), grid.y = 1: table -> keys[n_pad .. 2 n_pad): both sorts share every launch)

@@ -342,6 +342,29 @@ struct PhaseClock {
 
 }  // namespace
 
+namespace h2v {
+int check_circuit(const h2v_circuit_t *cs, bool have_column_lists, const char *who) {
+    if (cs->degree < 3 || cs->degree > 9) return failf(H2V_EINVAL, "%s: cs.degree() = %u unsupported", who, cs->degree);
+    if (cs->k < 2 || cs->k > 24) return failf(H2V_EINVAL, "%s: k = %u unsupported", who, cs->k);
+    const size_t n = (size_t)1 << cs->k;
+    if ((size_t)cs->blinding_factors + 2 >= n) return failf(H2V_EINVAL, "%s: blinding_factors too large for k", who);
+    if (!have_column_lists) return failf(H2V_EINVAL, "%s: NULL column list", who);
+    for (uint32_t j = 0; j < cs->n_gates; ++j)
+        if (cs->gate_advice[j] >= cs->n_advice || cs->gate_selector[j] >= cs->n_fixed) return failf(H2V_EINVAL, "%s: gate %u out of range", who, j);
+    for (uint32_t j = 0; j < cs->n_lookups; ++j)
+        if (cs->lookup_input[j] >= cs->n_advice || cs->lookup_table[j] >= cs->n_fixed) return failf(H2V_EINVAL, "%s: lookup %u out of range", who, j);
+    for (uint32_t j = 0; j < cs->n_perm; ++j) {
+        const uint32_t lim = cs->perm_kind[j] == 0 ? cs->n_advice : cs->perm_kind[j] == 1 ? cs->n_fixed : cs->n_instance;
+        if (cs->perm_kind[j] > 2 || cs->perm_index[j] >= lim) return failf(H2V_EINVAL, "%s: permutation column %u out of range", who, j);
+    }
+    for (uint32_t j = 0; j < cs->n_advice_queries; ++j)
+        if (cs->advice_query_col[j] >= cs->n_advice) return failf(H2V_EINVAL, "%s: advice query %u out of range", who, j);
+    for (uint32_t j = 0; j < cs->n_fixed_queries; ++j)
+        if (cs->fixed_query_col[j] >= cs->n_fixed) return failf(H2V_EINVAL, "%s: fixed query %u out of range", who, j);
+    return H2V_OK;
+}
+}  // namespace h2v
+
 extern "C" {
 
 void h2v_pk_free(h2v_pk_t pk) {
@@ -363,23 +386,8 @@ int h2v_pk_load(h2v_srs_t srs, const h2v_circuit_t *cs, const uint64_t *const *f
     if (!out) return failf(H2V_EINVAL, "pk_load: out is NULL");
     *out = nullptr;
     if (!srs || !cs || !vk_transcript_repr) return failf(H2V_EINVAL, "pk_load: NULL argument");
-    if (cs->degree < 3 || cs->degree > 9) return failf(H2V_EINVAL, "pk_load: cs.degree() = %u unsupported", cs->degree);
-    if (cs->k < 2 || cs->k > 24) return failf(H2V_EINVAL, "pk_load: k = %u unsupported", cs->k);
+    H2V_TRY(check_circuit(cs, !(cs->n_fixed && !fixed) && !(cs->n_perm && !sigma), "pk_load"));
     const size_t n = (size_t)1 << cs->k;
-    if ((size_t)cs->blinding_factors + 2 >= n) return failf(H2V_EINVAL, "pk_load: blinding_factors too large for k");
-    if ((cs->n_fixed && !fixed) || (cs->n_perm && !sigma)) return failf(H2V_EINVAL, "pk_load: NULL column list");
-    for (uint32_t j = 0; j < cs->n_gates; ++j)
-        if (cs->gate_advice[j] >= cs->n_advice || cs->gate_selector[j] >= cs->n_fixed) return failf(H2V_EINVAL, "pk_load: gate %u out of range", j);
-    for (uint32_t j = 0; j < cs->n_lookups; ++j)
-        if (cs->lookup_input[j] >= cs->n_advice || cs->lookup_table[j] >= cs->n_fixed) return failf(H2V_EINVAL, "pk_load: lookup %u out of range", j);
-    for (uint32_t j = 0; j < cs->n_perm; ++j) {
-        const uint32_t lim = cs->perm_kind[j] == 0 ? cs->n_advice : cs->perm_kind[j] == 1 ? cs->n_fixed : cs->n_instance;
-        if (cs->perm_kind[j] > 2 || cs->perm_index[j] >= lim) return failf(H2V_EINVAL, "pk_load: permutation column %u out of range", j);
-    }
-    for (uint32_t j = 0; j < cs->n_advice_queries; ++j)
-        if (cs->advice_query_col[j] >= cs->n_advice) return failf(H2V_EINVAL, "pk_load: advice query %u out of range", j);
-    for (uint32_t j = 0; j < cs->n_fixed_queries; ++j)
-        if (cs->fixed_query_col[j] >= cs->n_fixed) return failf(H2V_EINVAL, "pk_load: fixed query %u out of range", j);
     uint32_t srs_c = 0;
     H2V_TRY(h2v_srs_info(srs, &srs_c, nullptr));
 

@@ -283,6 +283,44 @@ size_t h2v_proof_size(h2v_pk_t pk);
  * the call ran in */
 int h2v_pk_last_phase_ms(h2v_pk_t pk, double out[8]);
 
+/* ---- mock prover: check a laid-out circuit's constraints -------------------------------------------------------
+ * halo2 `MockProver::run(k, circuit, instances).assert_satisfied()` (the reference's `mock` command, scaffold mod.rs:263)
+ * for the constraint-system shape above, on the primary device.  The inputs are those of h2v_pk_load + h2v_create_proof:
+ * Lagrange columns of 2^k in Montgomery form; no SRS and no key.  Values are compared as field elements (limbs that are
+ * not reduced compare equal to their reduced form).
+ *   gates        gate j, every row with fixed[gate_selector[j]][row] != 0: GATE_UNUSABLE if row + 3 >= usable rows
+ *                (2^k - blinding_factors - 1), else GATE if a + a(w) a(w^2) - a(w^3) != 0.  column = j, other_column = the
+ *                gate's advice column, other_row = row.
+ *   lookups      lookup l, every usable row: advice[lookup_input[l]][row] must occur among the usable rows of
+ *                fixed[lookup_table[l]]; else LOOKUP with column = l, other_column = the input column, other_row = row.
+ *   permutation  permutation column c, every row: sigma[c][row] must be delta^c2 * w^r2 with c2 < n_perm, else
+ *                SIGMA_NOT_DELTA_OMEGA (other_column = other_row = 0xFFFFFFFF) and the cell's other checks are skipped;
+ *                SIGMA_NOT_PERMUTATION when a cell earlier in (column, row) order has the same image; when the image is
+ *                another cell, COPY_UNUSABLE if either row is unusable and COPY if the two cell values differ.  Instance
+ *                column c holds instances[c] in its first instance_len[c] rows and zeros below.  column / row = (c, row),
+ *                other_column / other_row = (c2, r2).
+ * failures_out receives the first min(cap, total) failures in this order: gates, lookups, permutation; then by gate,
+ * lookup or permutation column; then by row; within one cell SIGMA_NOT_DELTA_OMEGA, SIGMA_NOT_PERMUTATION,
+ * COPY_UNUSABLE, COPY.  *n_failures = the exact total.  The same inputs always give the same output.
+ * Every argument is checked before any device work (H2V_EINVAL: NULL pointers, the column indices of cs as h2v_pk_load
+ * checks them, instance_len[c] > 2^k, more than 65535 gates / lookups / permutation columns, more than 2^32 flags).
+ * Device memory: the columns (32 bytes per cell of every advice, fixed, sigma and instance column), 4 bytes per
+ * permutation cell, one bit per gate row, lookup row and 4 per permutation cell, and the table of the 2^k values w^r
+ * (40 bytes per row): about 29.8 GB for the SIFT-shaped k = 20 circuit (28.3 GB of columns, 290 permutation columns). */
+typedef struct {
+    uint32_t kind, column, row, other_column, other_row;
+} h2v_mock_failure_t;
+enum {
+    H2V_MOCK_GATE = 1, H2V_MOCK_GATE_UNUSABLE, H2V_MOCK_LOOKUP, H2V_MOCK_SIGMA_NOT_DELTA_OMEGA, H2V_MOCK_SIGMA_NOT_PERMUTATION,
+    H2V_MOCK_COPY_UNUSABLE, H2V_MOCK_COPY
+};
+int h2v_mock_prover(const h2v_circuit_t *cs, const uint64_t *const *fixed, const uint64_t *const *sigma, const uint64_t *const *advice,
+                    const uint64_t *const *instances, const uint32_t *instance_len, h2v_mock_failure_t *failures_out, size_t cap,
+                    uint64_t *n_failures);
+/* wall-clock milliseconds of the calling thread's last h2v_mock_prover call: out[0] the upload of the columns, out[1] the
+ * checks (every kernel, the compaction and the download of the failures) */
+int h2v_mock_last_ms(double out[2]);
+
 /* ---- circuit builder ("next": SURVEY.md 8(f) row 4; host-side, no device needed) -----------------------------------
  * The step before the hot path: the reference's chips produce the execution trace whose columns create_proof commits.
  * One builder = halo2-base's GateThreadBuilder with the single Context the scaffold uses (`builder.main(0)`,

@@ -296,4 +296,40 @@ class ProvingKey {
     h2v_pk_t h_ = nullptr;
 };
 
+// halo2 MockProver::run(k, circuit, instances) on the device (h2v_mock_prover): the first max_failures failures in the order
+// gates, lookups, permutation, and how many there are in all
+struct MockProver {
+    std::vector<h2v_mock_failure_t> failures;
+    uint64_t n_failures = 0;
+
+    static MockProver run(const h2v_circuit_t &cs, const std::vector<const Fr *> &fixed, const std::vector<const Fr *> &sigma,
+                          const std::vector<const Fr *> &advice, const std::vector<std::vector<Fr>> &instances, size_t max_failures = 64) {
+        if (fixed.size() != cs.n_fixed || sigma.size() != cs.n_perm || advice.size() != cs.n_advice || instances.size() != cs.n_instance)
+            throw std::invalid_argument("MockProver: column count does not match the constraint system");
+        std::vector<const uint64_t *> ip;
+        std::vector<uint32_t> il;
+        for (const auto &c : instances) {
+            ip.push_back(reinterpret_cast<const uint64_t *>(c.data()));
+            il.push_back((uint32_t)c.size());
+        }
+        MockProver m;
+        m.failures.resize(max_failures);
+        check(h2v_mock_prover(&cs, reinterpret_cast<const uint64_t *const *>(fixed.data()), reinterpret_cast<const uint64_t *const *>(sigma.data()),
+                              reinterpret_cast<const uint64_t *const *>(advice.data()), ip.data(), il.data(), m.failures.data(), max_failures,
+                              &m.n_failures));
+        m.failures.resize((size_t)std::min<uint64_t>(max_failures, m.n_failures));
+        return m;
+    }
+    // MockProver::assert_satisfied: throws std::logic_error naming the first failures
+    void assert_satisfied() const {
+        if (!n_failures) return;
+        static const char *kinds[] = {"?", "gate", "gate_unusable", "lookup", "sigma_not_delta_omega", "sigma_not_permutation", "copy_unusable", "copy"};
+        std::string msg = std::to_string(n_failures) + " constraint(s) not satisfied";
+        for (const auto &f : failures)
+            msg += "\n  " + std::string(kinds[f.kind < 8 ? f.kind : 0]) + ": column " + std::to_string(f.column) + " row " + std::to_string(f.row) +
+                   " (other: column " + std::to_string(f.other_column) + " row " + std::to_string(f.other_row) + ")";
+        throw std::logic_error(msg);
+    }
+};
+
 }  // namespace h2v_host
