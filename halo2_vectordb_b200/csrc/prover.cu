@@ -277,9 +277,9 @@ struct h2v_pk {
     uint32_t u = 0, chunk = 0, n_sets = 0;
     Fr64 vk_repr, omega, omega_inv, delta;
     DevBuf fixed_L, fixed_C, fixed_E, sigma_L, sigma_C, sigma_E, lrows_E, omega_pows;
-    // workspace of a group of proofs (B times what one proof needs), kept between calls
+    // workspace of a group of proofs (B times what one proof needs), kept between calls; listed by workspace()
     DevBuf adv_L, adv_C, adv_E, inst_L, inst_C, inst_E, pa_L, ps_L, pa_C, ps_C, pa_E, ps_E, z_L, z_C, z_E, zl_L, zl_C, zl_E;
-    DevBuf num, den, tails, ptrs, scal, offs, streams, pts, rnd_C, hq, hx_pieces, evals, pairs, sh_S, sh_A, sh_B, sh_T, sh_h, commits;
+    DevBuf num, den, ptrs, scal, offs, streams, pts, rnd_C, hq, hx_pieces, evals, pairs, sh_S, sh_A, sh_B, sh_T, sh_h, commits;
     // k = 20-sized keys: the extended-coset forms of the fixed / sigma / advice columns (4n each) are not kept -- the
     // quotient step rebuilds them from the coefficient forms in slices of `scr_cols` columns of `scr_E`
     bool stream_ext = false;
@@ -298,6 +298,11 @@ struct h2v_pk {
 
 namespace {
 
+int set_device(int dev, const char *who) {
+    if (cudaSetDevice(dev) == cudaSuccess) return H2V_OK;
+    cudaGetLastError();
+    return failf(H2V_ECUDA, "%s: no CUDA device (libh2v has no CPU fallback)", who);
+}
 int sync(h2v_pk *pk) {
     H2V_CU(cudaStreamSynchronize(pk->st));
     return H2V_OK;
@@ -305,16 +310,14 @@ int sync(h2v_pk *pk) {
 // upload a host array of device pointers / scalars into a (reused) device buffer at byte offset `off`
 int upload(h2v_pk *pk, DevBuf &b, size_t off, const void *src, size_t bytes) {
     H2V_CU(cudaMemcpyAsync((char *)b.p + off, src, bytes, cudaMemcpyHostToDevice, pk->st));
-    H2V_CU(cudaStreamSynchronize(pk->st));      // the host staging vectors are short-lived
-    return H2V_OK;
+    return sync(pk);      // the host staging vectors are short-lived
 }
 // rows [row0, row0 + rows) of `n_cols` contiguous columns of n <- tails (n_cols x rows, host)
 int write_rows(h2v_pk *pk, fe *cols, size_t n, size_t row0, size_t rows, size_t n_cols, const std::vector<Fr64> &tails) {
     if (!rows || !n_cols) return H2V_OK;
     H2V_CU(cudaMemcpy2DAsync(cols + row0, n * sizeof(fe), tails.data(), rows * sizeof(fe), rows * sizeof(fe), n_cols,
                              cudaMemcpyHostToDevice, pk->st));
-    H2V_CU(cudaStreamSynchronize(pk->st));
-    return H2V_OK;
+    return sync(pk);
 }
 int commit_dev(h2v_pk *pk, int basis, const fe *cols, size_t n_cols, std::vector<affine> &out) {
     out.resize(n_cols);
@@ -325,20 +328,19 @@ int commit_dev(h2v_pk *pk, int basis, const fe *cols, size_t n_cols, std::vector
     H2V_CU(cudaMemcpy(out.data(), pk->commits.p, n_cols * sizeof(affine), cudaMemcpyDeviceToHost));
     return H2V_OK;
 }
-int write_points(PoseidonTranscript &T, const affine *pts, size_t cnt) {
-    for (size_t i = 0; i < cnt; ++i)
-        if (!T.write_point(pts[i])) return failf(H2V_EINVAL, "create_proof: Cannot write points at infinity to the transcript");
-    return H2V_OK;
+double now_ms() {
+    timespec ts;
+    clock_gettime(CLOCK_MONOTONIC, &ts);
+    return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6;
 }
-struct PhaseClock {
-    cudaEvent_t dummy;
-    double t0;
-    static double now() {
-        timespec ts;
-        clock_gettime(CLOCK_MONOTONIC, &ts);
-        return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6;
-    }
-};
+// The per-proof workspace; a group of B proofs holds B times the buffers of one.
+DevBuf *workspace(h2v_pk *pk, size_t i) {
+    DevBuf *all[] = {&pk->adv_L, &pk->adv_C, &pk->adv_E, &pk->inst_L, &pk->inst_C, &pk->inst_E, &pk->pa_L, &pk->ps_L, &pk->pa_C, &pk->ps_C,
+                     &pk->pa_E, &pk->ps_E, &pk->z_L, &pk->z_C, &pk->z_E, &pk->zl_L, &pk->zl_C, &pk->zl_E, &pk->num, &pk->den,
+                     &pk->ptrs, &pk->scal, &pk->offs, &pk->streams, &pk->pts, &pk->rnd_C, &pk->hq, &pk->hx_pieces,
+                     &pk->evals, &pk->pairs, &pk->sh_S, &pk->sh_A, &pk->sh_B, &pk->sh_T, &pk->sh_h, &pk->commits};
+    return i < sizeof all / sizeof all[0] ? all[i] : nullptr;
+}
 
 }  // namespace
 
@@ -370,12 +372,9 @@ extern "C" {
 void h2v_pk_free(h2v_pk_t pk) {
     if (!pk) return;
     cudaSetDevice(pk->dev);
-    DevBuf *all[] = {&pk->fixed_L, &pk->fixed_C, &pk->fixed_E, &pk->sigma_L, &pk->sigma_C, &pk->sigma_E, &pk->lrows_E, &pk->omega_pows,
-                     &pk->adv_L, &pk->adv_C, &pk->adv_E, &pk->inst_L, &pk->inst_C, &pk->inst_E, &pk->pa_L, &pk->ps_L, &pk->pa_C, &pk->ps_C,
-                     &pk->pa_E, &pk->ps_E, &pk->z_L, &pk->z_C, &pk->z_E, &pk->zl_L, &pk->zl_C, &pk->zl_E, &pk->num, &pk->den, &pk->tails,
-                     &pk->ptrs, &pk->scal, &pk->offs, &pk->streams, &pk->pts, &pk->rnd_C, &pk->hq, &pk->hx_pieces, &pk->evals, &pk->pairs, &pk->sh_S, &pk->sh_A,
-                     &pk->sh_B, &pk->sh_T, &pk->sh_h, &pk->commits, &pk->scr_E, &pk->ext_cache};
-    for (DevBuf *b : all) b->release();
+    for (DevBuf *b : {&pk->fixed_L, &pk->fixed_C, &pk->fixed_E, &pk->sigma_L, &pk->sigma_C, &pk->sigma_E, &pk->lrows_E, &pk->omega_pows, &pk->scr_E,
+                      &pk->ext_cache}) b->release();
+    for (size_t i = 0; DevBuf *b = workspace(pk, i); ++i) b->release();
     if (pk->dom) h2v_domain_free(pk->dom);
     if (pk->st) cudaStreamDestroy(pk->st);
     delete pk;
@@ -391,10 +390,7 @@ int h2v_pk_load(h2v_srs_t srs, const h2v_circuit_t *cs, const uint64_t *const *f
     uint32_t srs_c = 0;
     H2V_TRY(h2v_srs_info(srs, &srs_c, nullptr));
 
-    if (cudaSetDevice(current_device()) != cudaSuccess) {
-        cudaGetLastError();
-        return failf(H2V_ECUDA, "pk_load: no CUDA device (libh2v has no CPU fallback)");
-    }
+    H2V_TRY(set_device(current_device(), "pk_load"));
     h2v_pk *pk = new h2v_pk();
     pk->dev = current_device();
     pk->srs = srs;
@@ -505,12 +501,6 @@ int h2v_pk_last_phase_ms(h2v_pk_t pk, double out[8]) {
 // ================================================================== create_proof over a group of proofs
 namespace {
 
-struct Query {
-    const fe *poly;     // device-resident coefficients (n): the commitment's identity, as upstream's PolynomialPointer
-    uint32_t pt;        // index into the distinct evaluation points
-    Fr64 eval;
-};
-
 // the arguments of one h2v_create_proof
 struct ProofIn {
     const uint64_t *const *advice;
@@ -524,6 +514,52 @@ struct ProofState {
     ChaCha20Rng rng;
     Fr64 beta, gamma, y, x, xn, ys, vs, uc;
     explicit ProofState(const uint8_t *seed) : rng(seed) {}
+};
+
+enum ColForm { LAGRANGE, COEFF, EXTENDED };
+
+// What the phases of one group of proofs share.  Proofs in[0 .. B) run in lockstep: every commit, transform, grand
+// product and column kernel of a phase is one call over the B proofs' columns (proof p's columns of a kind after proof
+// p - 1's), while each proof keeps its own RNG (upstream's draw order) and transcript (its own challenges) in P[p].
+struct Group {
+    h2v_pk *pk;
+    size_t B;
+    const ProofIn *in;
+    std::vector<std::unique_ptr<ProofState>> P;
+    size_t n, ne;
+    uint32_t A, F, I, L, G, NP, NS, NH, bf, u;      // NH: quotient pieces of n coefficients each
+    unsigned gn;                                    // blocks of 256 rows
+    size_t &bad;                                    // on a failure traced to one proof, that proof (else SIZE_MAX)
+    std::vector<affine> pts;                        // commitments of the current step
+    fe *pieces = nullptr;                           // the B x NH quotient pieces, contiguous columns of n (commit_quotient)
+    double t_phase = now_ms();
+    int phase = 0;
+
+    Group(h2v_pk *pk_, size_t B_, const ProofIn *in_, size_t &bad_)
+        : pk(pk_), B(B_), in(in_), n(pk_->n), ne(pk_->ne), A(pk_->n_advice), F(pk_->n_fixed), I(pk_->n_instance),
+          L((uint32_t)pk_->lookup_input.size()), G((uint32_t)pk_->gate_advice.size()), NP((uint32_t)pk_->perm_kind.size()),
+          NS(pk_->n_sets), NH(pk_->degree - 1), bf(pk_->bf), u(pk_->u), gn((unsigned)((pk_->n + 255) / 256)), bad(bad_) {
+        bad = SIZE_MAX;
+        for (size_t p = 0; p < B; ++p) P.emplace_back(new ProofState(in[p].seed));
+    }
+    // column idx of a kind (0 advice, 1 fixed, 2 instance) of proof p; the fixed columns are the key's, shared by the proofs
+    const fe *col(ColForm form, size_t p, uint8_t kind, uint32_t idx) const {
+        const DevBuf *bufs[3][3] = {{&pk->adv_L, &pk->adv_C, &pk->adv_E}, {&pk->fixed_L, &pk->fixed_C, &pk->fixed_E},
+                                    {&pk->inst_L, &pk->inst_C, &pk->inst_E}};
+        const size_t at = kind == 0 ? p * A + idx : kind == 1 ? idx : p * I + idx;
+        return bufs[kind][form]->as<fe>() + at * (form == EXTENDED ? ne : n);
+    }
+    std::vector<Fr64> beta_gamma() const {      // beta, gamma of every proof, as the column kernels read them
+        std::vector<Fr64> v;
+        for (auto &s : P) v.insert(v.end(), {s->beta, s->gamma});
+        return v;
+    }
+    // ends the current phase of h2v_pk_last_phase_ms
+    void lap() {
+        const double t = now_ms();
+        if (phase < 7) pk->last_ms[phase++] += t - t_phase;
+        t_phase = t;
+    }
 };
 
 // f(p) for every proof p < B, on up to B host threads (the proofs' transcripts and point-set arithmetic are independent).
@@ -571,47 +607,73 @@ int sub_low(h2v_pk *pk, fe *a, size_t stride, const std::vector<Fr64> &low, size
     H2V_LAUNCHED();
     return H2V_OK;
 }
+// out + p n = sum_i c^i cols[(p m + i) n] for every proof p, with c = the proof's challenge `c`; one launch
+int sum_powers(Group &g, const fe *cols, size_t m, Fr64 ProofState::*c, fe *out) {
+    std::vector<const fe *> hp(g.B * m);
+    std::vector<Fr64> cf(g.B * m);
+    std::vector<uint32_t> off(g.B + 1);
+    for (size_t p = 0; p < g.B; ++p) {
+        Fr64 cur = frh::ONE;
+        off[p] = (uint32_t)(p * m);
+        for (size_t i = 0; i < m; ++i) {
+            hp[p * m + i] = cols + (p * m + i) * g.n;
+            cf[p * m + i] = cur;
+            cur = frh::mul(cur, (*g.P[p]).*c);
+        }
+    }
+    off[g.B] = (uint32_t)(g.B * m);
+    return lincomb(g.pk, hp, cf, off, out, g.n, g.n);
+}
+// proof p's commitments pts[p per_proof .. (p + 1) per_proof) into its transcript, for every proof; a point at infinity
+// fails the proof it belongs to.  absorb: hash them on the transcripts' worker threads while the next kernels run.
+int write_commitments(Group &g, const std::vector<affine> &pts, size_t per_proof, bool absorb) {
+    for (size_t p = 0; p < g.B; ++p) {
+        for (size_t i = 0; i < per_proof; ++i)
+            if (!g.P[p]->T.write_point(pts[p * per_proof + i])) {
+                g.bad = p;
+                return failf(H2V_EINVAL, "create_proof: Cannot write points at infinity to the transcript");
+            }
+        if (absorb) g.P[p]->T.absorb_async();
+    }
+    return H2V_OK;
+}
+// the end of a grand-product step (permutation/prover.rs commit, lookup/prover.rs commit_product): per proof and
+// column, bf random rows at n - bf and one blind; then the columns of z are committed and written
+int commit_products(Group &g, DevBuf &z, size_t cols_per_proof) {
+    const size_t cols = g.B * cols_per_proof;
+    std::vector<Fr64> zt(cols * g.bf);
+    for (size_t p = 0; p < g.B; ++p)
+        for (size_t c = 0; c < cols_per_proof; ++c) {
+            for (uint32_t i = 0; i < g.bf; ++i) zt[(p * cols_per_proof + c) * g.bf + i] = g.P[p]->rng.fr_random();   // rows n - bf .. n - 1
+            (void)g.P[p]->rng.fr_random();                                                                        // product blind
+        }
+    H2V_TRY(write_rows(g.pk, z.as<fe>(), g.n, g.n - g.bf, g.bf, cols, zt));
+    H2V_TRY(commit_dev(g.pk, H2V_BASIS_LAGRANGE, z.as<fe>(), cols, g.pts));
+    return write_commitments(g, g.pts, cols_per_proof, true);
+}
 
-// The prover.  Proofs in[0 .. B) run in lockstep, phase by phase: every commit, transform, grand product and column
-// kernel of a phase is one call over the B proofs' columns (proof p's columns of a kind after proof p-1's), while each proof
-// keeps its own RNG (upstream's draw order) and transcript (its own challenges).  The caller holds pk->mu and has checked
-// the inputs; on a failure traced to one proof, `bad` is that proof (else it stays SIZE_MAX).
-int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector<uint8_t>> &proofs, size_t &bad) {
-    const size_t n = pk->n, ne = pk->ne;
-    const uint32_t A = pk->n_advice, F = pk->n_fixed, I = pk->n_instance, L = (uint32_t)pk->lookup_input.size(),
-                   G = (uint32_t)pk->gate_advice.size(), NP = (uint32_t)pk->perm_kind.size(), NS = pk->n_sets, bf = pk->bf, u = pk->u;
-    const size_t BA = B * A, BI = B * I, BL = B * L, BS = B * NS;
-    const unsigned gn = (unsigned)((n + 255) / 256);
-    cudaStream_t st = pk->st;
-    double t_phase = PhaseClock::now();
-    int phase = 0;
-    auto lap = [&]() {
-        double t = PhaseClock::now();
-        if (phase < 7) pk->last_ms[phase++] += t - t_phase;
-        t_phase = t;
-    };
-    bad = SIZE_MAX;
-    std::vector<std::unique_ptr<ProofState>> P;
-    for (size_t p = 0; p < B; ++p) P.emplace_back(new ProofState(in[p].seed));
-
-    // ---- 1. vk, instances                                                   (prover.rs: hash_into, common_scalar)
-    for (auto &s : P) s->T.common_scalar(pk->vk_repr);
+// ---- phase 0.  plonk/prover.rs create_proof steps 1-4: vk and instances into the transcripts (hash_into, common_scalar);
+//      the advice columns uploaded, blinded in their last bf + 1 rows and committed
+int instances_and_advice(Group &g) {
+    h2v_pk *pk = g.pk;
+    const size_t B = g.B, n = g.n, BA = B * g.A, BI = B * g.I;
+    const uint32_t A = g.A, bf = g.bf;
+    for (auto &s : g.P) s->T.common_scalar(pk->vk_repr);
     H2V_TRY(pk->inst_L.ensure(std::max<size_t>(1, BI) * n * sizeof(fe)));
     H2V_TRY(pk->inst_C.ensure(std::max<size_t>(1, BI) * n * sizeof(fe)));
-    H2V_TRY(pk->inst_E.ensure(std::max<size_t>(1, BI) * ne * sizeof(fe)));
-    if (I) {
+    H2V_TRY(pk->inst_E.ensure(std::max<size_t>(1, BI) * g.ne * sizeof(fe)));
+    if (g.I) {
         std::vector<Fr64> inst(BI * n, frh::zero());
         for (size_t p = 0; p < B; ++p)
-            for (uint32_t c = 0; c < I; ++c)
-                for (uint32_t i = 0; i < in[p].instance_len[c]; ++i) {
-                    Fr64 &v = inst[(p * I + c) * n + i];
-                    v = frh::load(in[p].instances[c] + 4 * i);
-                    P[p]->T.common_scalar(v);
+            for (uint32_t c = 0; c < g.I; ++c)
+                for (uint32_t i = 0; i < g.in[p].instance_len[c]; ++i) {
+                    Fr64 &v = inst[(p * g.I + c) * n + i];
+                    v = frh::load(g.in[p].instances[c] + 4 * i);
+                    g.P[p]->T.common_scalar(v);
                 }
         H2V_TRY(upload(pk, pk->inst_L, 0, inst.data(), BI * n * sizeof(fe)));
         H2V_TRY(h2v_domain_transform_dev(pk->dom, H2V_OP_LAGRANGE_TO_COEFF, pk->inst_L.p, n, pk->inst_C.p, n, BI));
     }
-    // ---- 2-4. advice columns: upload, blind the last blinding_factors + 1 rows, commit
     H2V_TRY(pk->adv_L.ensure(BA * n * sizeof(fe)));
     H2V_TRY(pk->adv_C.ensure(BA * n * sizeof(fe)));
     // h2v_commit_batch_resident: each device uploads its block of the B x A columns in sub-batches (the next one crosses
@@ -619,63 +681,52 @@ int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector
     std::vector<Fr64> tails(BA * (bf + 1));
     std::vector<const uint64_t *> adv(BA);
     for (size_t p = 0; p < B; ++p) {
-        ChaCha20Rng &rng = P[p]->rng;
+        ChaCha20Rng &rng = g.P[p]->rng;
         for (size_t t = 0; t < (size_t)A * (bf + 1); ++t) tails[p * A * (bf + 1) + t] = rng.fr_random();   // column by column, rows u .. n-1
         for (uint32_t c = 0; c < A; ++c) (void)rng.fr_random();          // one Blind per column (unused by KZG, but drawn)
-        for (uint32_t c = 0; c < A; ++c) adv[p * A + c] = in[p].advice[c];
+        for (uint32_t c = 0; c < A; ++c) adv[p * A + c] = g.in[p].advice[c];
     }
-    std::vector<affine> pts(BA);
-    H2V_TRY(h2v_commit_batch_resident(pk->srs, H2V_BASIS_LAGRANGE, adv.data(), BA, n, (const uint64_t *)tails.data(), u, bf + 1, pk->adv_L.p, n,
-                                      (uint64_t *)pts.data()));
+    g.pts.resize(BA);
+    H2V_TRY(h2v_commit_batch_resident(pk->srs, H2V_BASIS_LAGRANGE, adv.data(), BA, n, (const uint64_t *)tails.data(), g.u, bf + 1, pk->adv_L.p, n,
+                                      (uint64_t *)g.pts.data()));
     H2V_CU(cudaSetDevice(pk->dev));
-    for (size_t p = 0; p < B; ++p) {
-        if (int rc = write_points(P[p]->T, pts.data() + p * A, A)) {
-            bad = p;
-            return rc;
-        }
-        P[p]->T.absorb_async();      // the advice commitments are hashed on worker threads while the lookup permutations run
-    }
-    lap();   // phase 0: upload + advice commitments
-    // column pointer helpers: column idx of a kind of proof p
-    auto col_L = [&](size_t p, uint8_t kind, uint32_t idx) -> const fe * {
-        return kind == 0 ? pk->adv_L.as<fe>() + (p * A + idx) * n : kind == 1 ? pk->fixed_L.as<fe>() + (size_t)idx * n
-                                                                                : pk->inst_L.as<fe>() + (p * I + idx) * n;
-    };
-    auto col_E = [&](size_t p, uint8_t kind, uint32_t idx) -> const fe * {
-        return kind == 0 ? pk->adv_E.as<fe>() + (p * A + idx) * ne : kind == 1 ? pk->fixed_E.as<fe>() + (size_t)idx * ne
-                                                                                 : pk->inst_E.as<fe>() + (p * I + idx) * ne;
-    };
-    // ---- 5. theta; lookups: permuted input / table columns                   (lookup/prover.rs commit_permuted)
-    // theta is squeezed at its place in the transcript (below, before A' / S' are written); single-expression lookups
-    // have nothing to compress, so the permutations do not wait for it
+    return write_commitments(g, g.pts, A, true);      // hashed while the lookup permutations run
+}
+
+// ---- phase 1.  lookup/prover.rs commit_permuted (step 5): the permuted input and table columns A', S' of every lookup,
+//      blinded and committed.  theta is squeezed at its place in the transcript, just before A' / S' are written:
+//      single-expression lookups have nothing to compress, so the permutations do not wait for it
+int permuted_lookups(Group &g) {
+    h2v_pk *pk = g.pk;
+    const size_t B = g.B, n = g.n, L = g.L, BL = B * L;
+    const uint32_t bf = g.bf;
     H2V_TRY(pk->pa_L.ensure(std::max<size_t>(1, BL) * n * sizeof(fe)));
     H2V_TRY(pk->ps_L.ensure(std::max<size_t>(1, BL) * n * sizeof(fe)));
+    std::vector<affine> written(2 * BL);      // A'_l, S'_l of each lookup of each proof, in transcript order
     if (L) {
-        std::vector<Fr64> ta(BL * (bf + 1)), ts(BL * (bf + 1));
-        {
-            std::vector<const void *> li(BL), lt(BL);
-            for (size_t p = 0; p < B; ++p)
-                for (uint32_t l = 0; l < L; ++l) {
-                    li[p * L + l] = col_L(p, 0, pk->lookup_input[l]);
-                    lt[p * L + l] = col_L(p, 1, pk->lookup_table[l]);      // the key's table: sorted once for the group
-                }
-            int rc = h2v_permute_expression_pair_batch_dev(li.data(), lt.data(), BL, u, pk->pa_L.as<fe>(), n, pk->ps_L.as<fe>(), n);
-            if (rc == H2V_EINVAL && B > 1) {
-                // an input value outside its table: find the proof it belongs to
-                for (size_t p = 0; p < B; ++p) {
-                    const int rc_p = h2v_permute_expression_pair_batch_dev(li.data() + p * L, lt.data() + p * L, L, u, pk->pa_L.as<fe>(), n,
-                                                                           pk->ps_L.as<fe>(), n);
-                    if (rc_p) {
-                        bad = p;
-                        return rc_p;
-                    }
+        std::vector<const void *> li(BL), lt(BL);
+        for (size_t p = 0; p < B; ++p)
+            for (uint32_t l = 0; l < L; ++l) {
+                li[p * L + l] = g.col(LAGRANGE, p, 0, pk->lookup_input[l]);
+                lt[p * L + l] = g.col(LAGRANGE, p, 1, pk->lookup_table[l]);      // the key's table: sorted once for the group
+            }
+        int rc = h2v_permute_expression_pair_batch_dev(li.data(), lt.data(), BL, g.u, pk->pa_L.as<fe>(), n, pk->ps_L.as<fe>(), n);
+        if (rc == H2V_EINVAL && B > 1) {
+            // an input value outside its table: find the proof it belongs to
+            for (size_t p = 0; p < B; ++p) {
+                const int rc_p = h2v_permute_expression_pair_batch_dev(li.data() + p * L, lt.data() + p * L, L, g.u, pk->pa_L.as<fe>(), n,
+                                                                       pk->ps_L.as<fe>(), n);
+                if (rc_p) {
+                    g.bad = p;
+                    return rc_p;
                 }
             }
-            if (rc) return rc;
-            H2V_CU(cudaSetDevice(pk->dev));
         }
+        if (rc) return rc;
+        H2V_CU(cudaSetDevice(pk->dev));
+        std::vector<Fr64> ta(BL * (bf + 1)), ts(BL * (bf + 1));
         for (size_t p = 0; p < B; ++p) {
-            ChaCha20Rng &rng = P[p]->rng;
+            ChaCha20Rng &rng = g.P[p]->rng;
             for (uint32_t l = 0; l < L; ++l) {
                 const size_t col = p * L + l;
                 for (uint32_t i = 0; i <= bf; ++i) ta[col * (bf + 1) + i] = rng.fr_random();
@@ -684,149 +735,125 @@ int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector
                 (void)rng.fr_random();     // permuted table blind
             }
         }
-        H2V_TRY(write_rows(pk, pk->pa_L.as<fe>(), n, u, bf + 1, BL, ta));
-        H2V_TRY(write_rows(pk, pk->ps_L.as<fe>(), n, u, bf + 1, BL, ts));
-        std::vector<affine> ca, cs_;
+        H2V_TRY(write_rows(pk, pk->pa_L.as<fe>(), n, g.u, bf + 1, BL, ta));
+        H2V_TRY(write_rows(pk, pk->ps_L.as<fe>(), n, g.u, bf + 1, BL, ts));
+        std::vector<affine> ca, cs;
         H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->pa_L.as<fe>(), BL, ca));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->ps_L.as<fe>(), BL, cs_));
-        for (size_t p = 0; p < B; ++p) {
-            (void)P[p]->T.squeeze_challenge();      // theta
-            for (uint32_t l = 0; l < L; ++l)
-                if (!P[p]->T.write_point(ca[p * L + l]) || !P[p]->T.write_point(cs_[p * L + l])) {
-                    bad = p;
-                    return failf(H2V_EINVAL, "create_proof: Cannot write points at infinity to the transcript");
-                }
+        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->ps_L.as<fe>(), BL, cs));
+        for (size_t c = 0; c < BL; ++c) {
+            written[2 * c] = ca[c];
+            written[2 * c + 1] = cs[c];
         }
-    } else {
-        for (auto &s : P) (void)s->T.squeeze_challenge();     // theta
     }
-    lap();   // phase 1: lookup permutations
-    // ---- 6. beta, gamma; permutation grand products                          (permutation/prover.rs commit)
-    std::vector<Fr64> beta_gamma(2 * B);
-    for (size_t p = 0; p < B; ++p) {
-        P[p]->beta = beta_gamma[2 * p] = P[p]->T.squeeze_challenge();
-        P[p]->gamma = beta_gamma[2 * p + 1] = P[p]->T.squeeze_challenge();
+    for (auto &s : g.P) (void)s->T.squeeze_challenge();      // theta
+    return write_commitments(g, written, 2 * L, false);
+}
+
+// ---- phase 2.  permutation/prover.rs Argument::commit (step 6): beta, gamma; the grand product of every permutation set
+int permutation_products(Group &g) {
+    h2v_pk *pk = g.pk;
+    const size_t B = g.B, n = g.n, BS = B * g.NS;
+    const uint32_t NP = g.NP, NS = g.NS, L = g.L, u = g.u;
+    for (auto &s : g.P) {
+        s->beta = s->T.squeeze_challenge();
+        s->gamma = s->T.squeeze_challenge();
     }
     H2V_TRY(pk->z_L.ensure(std::max<size_t>(1, BS) * n * sizeof(fe)));
     H2V_TRY(pk->num.ensure(std::max<size_t>(1, B * std::max(NS, L)) * n * sizeof(fe)));
     H2V_TRY(pk->den.ensure(std::max<size_t>(1, B * std::max(NS, L)) * n * sizeof(fe)));
-    H2V_TRY(pk->ptrs.ensure((size_t)(4 * (NP + G + L) * B + 4096) * sizeof(void *)));
-    H2V_TRY(pk->scal.ensure((size_t)(NS + A + F + NP + 3 * NS + 5 * L + 64) * B * sizeof(fe) + 4096));
-    if (NS) {
-        std::vector<const fe *> hp((B + 1) * NP);
-        for (size_t p = 0; p < B; ++p)
-            for (uint32_t c = 0; c < NP; ++c) hp[p * NP + c] = col_L(p, pk->perm_kind[c], pk->perm_index[c]);
-        for (uint32_t c = 0; c < NP; ++c) hp[B * NP + c] = pk->sigma_L.as<fe>() + (size_t)c * n;
-        H2V_TRY(put(pk, pk->ptrs, hp));
-        std::vector<Fr64> sc(NS);                       // delta^(s * chunk), then beta, gamma of every proof
-        const Fr64 dchunk = frh::pow_u64(pk->delta, pk->chunk);
-        Fr64 cur = frh::ONE;
+    H2V_TRY(pk->ptrs.ensure((size_t)(4 * (NP + g.G + L) * B + 4096) * sizeof(void *)));
+    H2V_TRY(pk->scal.ensure((size_t)(NS + g.A + g.F + NP + 3 * NS + 5 * L + 64) * B * sizeof(fe) + 4096));
+    if (!NS) return H2V_OK;
+    std::vector<const fe *> hp((B + 1) * NP);
+    for (size_t p = 0; p < B; ++p)
+        for (uint32_t c = 0; c < NP; ++c) hp[p * NP + c] = g.col(LAGRANGE, p, pk->perm_kind[c], pk->perm_index[c]);
+    for (uint32_t c = 0; c < NP; ++c) hp[B * NP + c] = pk->sigma_L.as<fe>() + (size_t)c * n;
+    H2V_TRY(put(pk, pk->ptrs, hp));
+    std::vector<Fr64> sc(NS);                       // delta^(s * chunk), then beta, gamma of every proof
+    const Fr64 dchunk = frh::pow_u64(pk->delta, pk->chunk);
+    Fr64 cur = frh::ONE;
+    for (uint32_t s = 0; s < NS; ++s) {
+        sc[s] = cur;
+        cur = frh::mul(cur, dchunk);
+    }
+    for (const Fr64 &v : g.beta_gamma()) sc.push_back(v);
+    H2V_TRY(put(pk, pk->scal, sc));
+    PermArgs pa;
+    pa.cols = (const fe *const *)pk->ptrs.p;
+    pa.sigma = pa.cols + B * NP;
+    pa.omega_pows = pk->omega_pows.as<fe>();
+    pa.delta_start = pk->scal.as<fe>();
+    pa.beta_gamma = pk->scal.as<fe>() + NS;
+    pa.delta = frh::to_fe(pk->delta);
+    pa.n_cols = NP; pa.chunk = pk->chunk; pa.n = (uint32_t)n;
+    perm_numden_kernel<<<dim3(g.gn, NS, (unsigned)B), 256, 0, pk->st>>>(pa, pk->num.as<fe>(), pk->den.as<fe>());
+    H2V_LAUNCHED();
+    H2V_TRY(sync(pk));
+    // z_s with z_s[0] = 1; then chain: z_s *= z_{s-1}[u] (upstream carries `last_z` from set to set)
+    H2V_TRY(h2v_grand_product_dev(pk->num.p, pk->den.p, n, BS, pk->z_L.p));
+    std::vector<Fr64> last(BS), scale(BS);
+    H2V_CU(cudaMemcpy2D(last.data(), sizeof(fe), pk->z_L.as<fe>() + u, n * sizeof(fe), sizeof(fe), BS, cudaMemcpyDeviceToHost));
+    for (size_t p = 0; p < B; ++p) {
+        cur = frh::ONE;
         for (uint32_t s = 0; s < NS; ++s) {
-            sc[s] = cur;
-            cur = frh::mul(cur, dchunk);
-        }
-        sc.insert(sc.end(), beta_gamma.begin(), beta_gamma.end());
-        H2V_TRY(put(pk, pk->scal, sc));
-        PermArgs pa;
-        pa.cols = (const fe *const *)pk->ptrs.p;
-        pa.sigma = pa.cols + B * NP;
-        pa.omega_pows = pk->omega_pows.as<fe>();
-        pa.delta_start = pk->scal.as<fe>();
-        pa.beta_gamma = pk->scal.as<fe>() + NS;
-        pa.delta = frh::to_fe(pk->delta);
-        pa.n_cols = NP; pa.chunk = pk->chunk; pa.n = (uint32_t)n;
-        perm_numden_kernel<<<dim3(gn, NS, (unsigned)B), 256, 0, st>>>(pa, pk->num.as<fe>(), pk->den.as<fe>());
-        H2V_LAUNCHED();
-        H2V_TRY(sync(pk));
-        // z_s with z_s[0] = 1; then chain: z_s *= z_{s-1}[u] (upstream carries `last_z` from set to set)
-        H2V_TRY(h2v_grand_product_dev(pk->num.p, pk->den.p, n, BS, pk->z_L.p));
-        std::vector<Fr64> last(BS), scale(BS);
-        H2V_CU(cudaMemcpy2D(last.data(), sizeof(fe), pk->z_L.as<fe>() + u, n * sizeof(fe), sizeof(fe), BS, cudaMemcpyDeviceToHost));
-        for (size_t p = 0; p < B; ++p) {
-            cur = frh::ONE;
-            for (uint32_t s = 0; s < NS; ++s) {
-                scale[p * NS + s] = cur;
-                cur = frh::mul(cur, last[p * NS + s]);
-            }
-        }
-        H2V_TRY(put(pk, pk->scal, scale));
-        scale_cols_kernel<<<dim3(gn, (unsigned)BS), 256, 0, st>>>(pk->z_L.as<fe>(), (uint32_t)n, pk->scal.as<fe>());
-        H2V_LAUNCHED();
-        std::vector<Fr64> zt(BS * bf);
-        for (size_t p = 0; p < B; ++p)
-            for (uint32_t s = 0; s < NS; ++s) {
-                for (uint32_t i = 0; i < bf; ++i) zt[(p * NS + s) * bf + i] = P[p]->rng.fr_random();     // rows n - bf .. n - 1
-                (void)P[p]->rng.fr_random();                                                           // product blind
-            }
-        H2V_TRY(write_rows(pk, pk->z_L.as<fe>(), n, n - bf, bf, BS, zt));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->z_L.as<fe>(), BS, pts));
-        for (size_t p = 0; p < B; ++p) {
-            if (int rc = write_points(P[p]->T, pts.data() + p * NS, NS)) {
-                bad = p;
-                return rc;
-            }
-            P[p]->T.absorb_async();      // hashed while the lookup products are built and committed
+            scale[p * NS + s] = cur;
+            cur = frh::mul(cur, last[p * NS + s]);
         }
     }
-    // ---- 7. lookup grand products                                             (lookup/prover.rs commit_product)
+    H2V_TRY(put(pk, pk->scal, scale));
+    scale_cols_kernel<<<dim3(g.gn, (unsigned)BS), 256, 0, pk->st>>>(pk->z_L.as<fe>(), (uint32_t)n, pk->scal.as<fe>());
+    H2V_LAUNCHED();
+    return commit_products(g, pk->z_L, NS);      // hashed while the lookup products are built and committed
+}
+
+//      lookup/prover.rs Permuted::commit_product (step 7): the grand product of every lookup
+int lookup_products(Group &g) {
+    h2v_pk *pk = g.pk;
+    const size_t B = g.B, n = g.n, L = g.L, BL = B * L;
     H2V_TRY(pk->zl_L.ensure(std::max<size_t>(1, BL) * n * sizeof(fe)));
-    if (L) {
-        std::vector<const fe *> hp(BL + L);
-        for (size_t p = 0; p < B; ++p)
-            for (uint32_t l = 0; l < L; ++l) hp[p * L + l] = col_L(p, 0, pk->lookup_input[l]);
-        for (uint32_t l = 0; l < L; ++l) hp[BL + l] = col_L(0, 1, pk->lookup_table[l]);
-        H2V_TRY(put(pk, pk->ptrs, hp));
-        H2V_TRY(put(pk, pk->scal, beta_gamma));
-        lookup_numden_kernel<<<dim3(gn, L, (unsigned)B), 256, 0, st>>>((const fe *const *)pk->ptrs.p, (const fe *const *)pk->ptrs.p + BL,
-                                                                      pk->pa_L.as<fe>(), pk->ps_L.as<fe>(), pk->scal.as<fe>(), (uint32_t)n,
-                                                                      pk->num.as<fe>(), pk->den.as<fe>());
-        H2V_LAUNCHED();
-        H2V_TRY(sync(pk));
-        H2V_TRY(h2v_grand_product_dev(pk->num.p, pk->den.p, n, BL, pk->zl_L.p));
-        std::vector<Fr64> lt(BL * bf);
-        for (size_t p = 0; p < B; ++p)
-            for (uint32_t l = 0; l < L; ++l) {
-                for (uint32_t i = 0; i < bf; ++i) lt[(p * L + l) * bf + i] = P[p]->rng.fr_random();
-                (void)P[p]->rng.fr_random();
-            }
-        H2V_TRY(write_rows(pk, pk->zl_L.as<fe>(), n, n - bf, bf, BL, lt));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->zl_L.as<fe>(), BL, pts));
-        for (size_t p = 0; p < B; ++p) {
-            if (int rc = write_points(P[p]->T, pts.data() + p * L, L)) {
-                bad = p;
-                return rc;
-            }
-            P[p]->T.absorb_async();
-        }
+    if (!L) return H2V_OK;
+    std::vector<const fe *> hp(BL + L);
+    for (size_t p = 0; p < B; ++p)
+        for (uint32_t l = 0; l < L; ++l) hp[p * L + l] = g.col(LAGRANGE, p, 0, pk->lookup_input[l]);
+    for (uint32_t l = 0; l < L; ++l) hp[BL + l] = g.col(LAGRANGE, 0, 1, pk->lookup_table[l]);
+    H2V_TRY(put(pk, pk->ptrs, hp));
+    H2V_TRY(put(pk, pk->scal, g.beta_gamma()));
+    lookup_numden_kernel<<<dim3(g.gn, (unsigned)L, (unsigned)B), 256, 0, pk->st>>>((const fe *const *)pk->ptrs.p, (const fe *const *)pk->ptrs.p + BL,
+                                                                                 pk->pa_L.as<fe>(), pk->ps_L.as<fe>(), pk->scal.as<fe>(), (uint32_t)n,
+                                                                                 pk->num.as<fe>(), pk->den.as<fe>());
+    H2V_LAUNCHED();
+    H2V_TRY(sync(pk));
+    H2V_TRY(h2v_grand_product_dev(pk->num.p, pk->den.p, n, BL, pk->zl_L.p));
+    return commit_products(g, pk->zl_L, L);
+}
+
+// ---- phase 3.  vanishing/prover.rs Argument::commit (step 8): the random polynomial, n consecutive Fr::random draws =
+//      n consecutive key-stream blocks, produced on the device, every proof's in one launch
+int random_polynomial(Group &g) {
+    h2v_pk *pk = g.pk;
+    H2V_TRY(pk->rnd_C.ensure(g.B * g.n * sizeof(fe)));
+    std::vector<ChaChaStream> cs(g.B);
+    for (size_t p = 0; p < g.B; ++p) {
+        ChaCha20Rng &rng = g.P[p]->rng;
+        memcpy(cs[p].key.k, rng.key, 32);
+        cs[p].counter0 = rng.next_block();
+        rng.skip_fr(g.n);
+        (void)rng.fr_random();      // random_blind
     }
-    lap();   // phase 2: grand products
-    // ---- 8. vanishing argument: random polynomial                             (vanishing/prover.rs commit)
-    H2V_TRY(pk->rnd_C.ensure(B * n * sizeof(fe)));
-    {
-        // n consecutive Fr::random draws = n consecutive key-stream blocks: produced on the device, every proof's in one launch
-        std::vector<ChaChaStream> cs(B);
-        for (size_t p = 0; p < B; ++p) {
-            ChaCha20Rng &rng = P[p]->rng;
-            memcpy(cs[p].key.k, rng.key, 32);
-            cs[p].counter0 = rng.next_block();
-            rng.skip_fr(n);
-            (void)rng.fr_random();      // random_blind
-        }
-        H2V_TRY(put(pk, pk->streams, cs));
-        chacha_fr_kernel<<<dim3(gn, (unsigned)B), 256, 0, st>>>(pk->streams.as<ChaChaStream>(), (uint32_t)n, pk->rnd_C.as<fe>());
-        H2V_LAUNCHED();
-        H2V_TRY(sync(pk));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, pk->rnd_C.as<fe>(), B, pts));
-        for (size_t p = 0; p < B; ++p) {
-            if (int rc = write_points(P[p]->T, pts.data() + p, 1)) {
-                bad = p;
-                return rc;
-            }
-            P[p]->T.absorb_async();
-        }
-    }
-    // ---- 9-11. coefficient and extended forms (no challenge involved: they run while the commitments above are hashed);
-    //            then y, evaluate_h, quotient pieces
+    H2V_TRY(put(pk, pk->streams, cs));
+    chacha_fr_kernel<<<dim3(g.gn, (unsigned)g.B), 256, 0, pk->st>>>(pk->streams.as<ChaChaStream>(), (uint32_t)g.n, pk->rnd_C.as<fe>());
+    H2V_LAUNCHED();
+    H2V_TRY(sync(pk));
+    H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, pk->rnd_C.as<fe>(), g.B, g.pts));
+    return write_commitments(g, g.pts, 1, true);
+}
+
+//      plonk/prover.rs create_proof, the polynomials of steps 9-11: coefficient and extended forms of the proof's columns
+//      (no challenge involved: they run while the commitments above are hashed).  A streamed key keeps no extended
+//      advice columns: evaluate_h_streamed rebuilds them slice by slice.
+int transform_columns(Group &g) {
+    h2v_pk *pk = g.pk;
+    const size_t n = g.n, ne = g.ne, BA = g.B * g.A, BI = g.B * g.I, BL = g.B * g.L, BS = g.B * g.NS;
     const int L2C = H2V_OP_LAGRANGE_TO_COEFF, C2E = H2V_OP_COEFF_TO_EXTENDED;
     const bool stream = pk->stream_ext;      // (a streamed key proves in groups of one)
     // (the per-proof buffers are kept between proofs, also in streamed mode: with peer access enabled, freeing and
@@ -834,7 +861,7 @@ int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector
     if (!stream) H2V_TRY(pk->adv_E.ensure(BA * ne * sizeof(fe)));
     H2V_TRY(h2v_domain_transform_dev(pk->dom, L2C, pk->adv_L.p, n, pk->adv_C.p, n, BA));
     if (!stream) H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, pk->adv_C.p, n, pk->adv_E.p, ne, BA));
-    if (I) H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, pk->inst_C.p, n, pk->inst_E.p, ne, BI));
+    if (g.I) H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, pk->inst_C.p, n, pk->inst_E.p, ne, BI));
     struct Tr { DevBuf *Lb, *Cb, *Eb; size_t cnt; } trs[4] = {{&pk->pa_L, &pk->pa_C, &pk->pa_E, BL}, {&pk->ps_L, &pk->ps_C, &pk->ps_E, BL},
                                                             {&pk->z_L, &pk->z_C, &pk->z_E, BS}, {&pk->zl_L, &pk->zl_C, &pk->zl_E, BL}};
     for (auto &t : trs) {
@@ -844,167 +871,172 @@ int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector
         H2V_TRY(h2v_domain_transform_dev(pk->dom, L2C, t.Lb->p, n, t.Cb->p, n, t.cnt));
         H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, t.Cb->p, n, t.Eb->p, ne, t.cnt));
     }
-    for (auto &s : P) s->y = s->T.squeeze_challenge();
-    lap();   // phase 3: random poly + transforms
-    // h_ext of proof p at hq + p ne, its quotient after the division at hq + (B + p) ne
-    H2V_TRY(pk->hq.ensure(2 * B * ne * sizeof(fe)));
-    fe *h_ext0 = pk->hq.as<fe>(), *h_out0 = pk->hq.as<fe>() + B * ne;
-    H2V_CU(cudaMemsetAsync(h_ext0, 0, B * ne * sizeof(fe), st));
-    H2V_TRY(sync(pk));
+    return H2V_OK;
+}
+
+// ---- phase 4.  plonk/evaluation.rs Evaluator::evaluate_h over resident extended columns: the gate, permutation and
+//      lookup folds of every proof into h (proof p's at h + p ne), three launches through one pointer table
+int evaluate_h_resident(Group &g, fe *h) {
+    h2v_pk *pk = g.pk;
+    const size_t B = g.B, ne = g.ne;
+    const uint32_t G = g.G, NP = g.NP, L = g.L;
+    const size_t per = 2 * (size_t)G + 2 * (size_t)NP;
+    std::vector<const fe *> hp(B * per);
+    for (size_t p = 0; p < B; ++p) {
+        const fe **t = hp.data() + p * per;
+        for (uint32_t j = 0; j < G; ++j) {
+            t[j] = g.col(EXTENDED, p, 1, pk->gate_selector[j]);
+            t[G + j] = g.col(EXTENDED, p, 0, pk->gate_advice[j]);
+        }
+        for (uint32_t c = 0; c < NP; ++c) {
+            t[2 * G + c] = g.col(EXTENDED, p, pk->perm_kind[c], pk->perm_index[c]);
+            t[2 * G + NP + c] = pk->sigma_E.as<fe>() + (size_t)c * ne;
+        }
+    }
+    // the lookups' five columns per lookup after the gate and permutation tables; every proof's y, beta, gamma
+    for (size_t p = 0; p < B; ++p)
+        for (uint32_t l = 0; l < L; ++l) {
+            const size_t col = p * L + l;
+            const fe *five[5] = {g.col(EXTENDED, p, 0, pk->lookup_input[l]), g.col(EXTENDED, p, 1, pk->lookup_table[l]), pk->pa_E.as<fe>() + col * ne,
+                                 pk->ps_E.as<fe>() + col * ne, pk->zl_E.as<fe>() + col * ne};
+            hp.insert(hp.end(), five, five + 5);
+        }
+    H2V_TRY(put(pk, pk->ptrs, hp));
+    std::vector<Fr64> ybg;
+    for (auto &s : g.P) ybg.insert(ybg.end(), {s->y, s->beta, s->gamma});
+    H2V_TRY(put(pk, pk->scal, ybg));
+    const void *const *tab = (const void *const *)pk->ptrs.p;
+    const fe *l0 = pk->lrows_E.as<fe>();
+    QuotientBatch qb;
+    qb.h = h; qb.h_stride = ne; qb.scal = pk->scal.p; qb.n_proofs = B;
+    qb.n_gates = G; qb.gate_tab = tab; qb.gate_pstride = per;
+    qb.n_perm = NP; qb.chunk = pk->chunk; qb.perm_tab = tab + 2 * G; qb.perm_pstride = per;
+    qb.z = pk->z_E.p; qb.z_stride = ne; qb.z_pstride = (size_t)g.NS * ne; qb.blinding_factors = g.bf;
+    qb.n_lookups = L; qb.lookup_tab = tab + B * per; qb.lookup_pstride = 5 * (size_t)L;
+    qb.l0 = l0; qb.l_last = l0 + ne; qb.l_active = l0 + 2 * ne;
+    return quotient_batch_dev(pk->dom, qb);
+}
+
+// Once per streamed key: what is left of the device's memory after the first proof's buffers exist keeps the extended forms
+// of the first sigma polynomials (H2V_EXT_CACHE_COLS of them if set, else as many as leave 8 GB free)
+int fill_sigma_cache(Group &g) {
+    h2v_pk *pk = g.pk;
+    if (pk->cache_tried) return H2V_OK;
+    pk->cache_tried = true;
+    size_t free_b = 0, total_b = 0;
+    cudaMemGetInfo(&free_b, &total_b);
+    const char *e = getenv("H2V_EXT_CACHE_COLS");
+    const size_t margin = (size_t)8 << 30;
+    size_t want = e ? (size_t)atoi(e) : (free_b > margin ? (free_b - margin) / (g.ne * sizeof(fe)) : 0);
+    want = std::min<size_t>(want, g.NP);
+    if (want >= (e ? 1u : 8u) && pk->ext_cache.ensure(want * g.ne * sizeof(fe)) == H2V_OK) {
+        H2V_TRY(h2v_domain_transform_dev(pk->dom, H2V_OP_COEFF_TO_EXTENDED, pk->sigma_C.p, g.n, pk->ext_cache.p, g.ne, want));
+        pk->cached_sigma = want;
+    }
+    return H2V_OK;
+}
+
+//      plonk/evaluation.rs Evaluator::evaluate_h for a streamed key (one proof): the same folds, in upstream's order, over
+//      slices of columns whose extended forms are rebuilt into `scr_E` from the resident coefficient forms (every term
+//      reads columns of its own gate / set / lookup only).  hp_acc: ne elements free until the division.
+int evaluate_h_streamed(Group &g, fe *h_ext, fe *hp_acc) {
+    h2v_pk *pk = g.pk;
+    const size_t n = g.n, ne = g.ne, SC = pk->scr_cols;
+    const uint32_t A = g.A, G = g.G, NP = g.NP, NS = g.NS, L = g.L, bf = g.bf;
+    const int C2E = H2V_OP_COEFF_TO_EXTENDED;
+    const Fr64 &y = g.P[0]->y, &beta = g.P[0]->beta, &gamma = g.P[0]->gamma;
     const fe *l0 = pk->lrows_E.as<fe>(), *ll = l0 + ne, *la = l0 + 2 * ne;
-    if (!stream) {
-        const size_t per = 2 * (size_t)G + 2 * (size_t)NP;
-        std::vector<const fe *> hp(B * per);
-        for (size_t p = 0; p < B; ++p) {
-            const fe **t = hp.data() + p * per;
-            for (uint32_t j = 0; j < G; ++j) {
-                t[j] = col_E(p, 1, pk->gate_selector[j]);
-                t[G + j] = col_E(p, 0, pk->gate_advice[j]);
-            }
-            for (uint32_t c = 0; c < NP; ++c) {
-                t[2 * G + c] = col_E(p, pk->perm_kind[c], pk->perm_index[c]);
-                t[2 * G + NP + c] = pk->sigma_E.as<fe>() + (size_t)c * ne;
-            }
+    H2V_TRY(pk->scr_E.ensure(SC * ne * sizeof(fe)));
+    fe *scr = pk->scr_E.as<fe>();
+    // coeff_to_extended of a list of coefficient columns into consecutive scratch slots; neighbours share one launch
+    const bool timing = getenv("H2V_PROVE_TIMING") != nullptr;
+    double t_ext = 0, t_fold = 0, t_mark = now_ms();
+    auto mark = [&](double &acc) {
+        if (!timing) return;
+        cudaDeviceSynchronize();
+        const double t = now_ms();
+        acc += t - t_mark;
+        t_mark = t;
+    };
+    auto extend = [&](const std::vector<const fe *> &src, fe *dst) -> int {
+        for (size_t i = 0; i < src.size();) {
+            size_t j = i + 1;
+            while (j < src.size() && src[j] == src[j - 1] + n) ++j;
+            H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, src[i], n, dst + i * ne, ne, j - i));
+            i = j;
         }
-        // the lookups' five columns per lookup after the gate and permutation tables; every proof's y, beta, gamma
-        const size_t lper = 5 * (size_t)L;
-        for (size_t p = 0; p < B; ++p)
-            for (uint32_t l = 0; l < L; ++l) {
-                const size_t col = p * L + l;
-                const fe *five[5] = {col_E(p, 0, pk->lookup_input[l]), col_E(p, 1, pk->lookup_table[l]), pk->pa_E.as<fe>() + col * ne,
-                                     pk->ps_E.as<fe>() + col * ne, pk->zl_E.as<fe>() + col * ne};
-                hp.insert(hp.end(), five, five + 5);
+        return H2V_OK;
+    };
+    const void *const *tab = (const void *const *)pk->ptrs.p;
+    std::vector<const fe *> src, hp;
+    // Gate j reads one advice column, and (in halo2-base's constraint system) every gate column is also a permutation
+    // column: when the gates meet their columns in gate order along the permutation, one pass over the permutation
+    // slices serves both folds -- the gates into h, the permutation into a second accumulator hp_acc, joined as
+    // h <- h y^(permutation terms) + hp_acc.  Each advice column is then extended once instead of twice.  Any other
+    // constraint system takes the two separate loops below.
+    std::vector<int32_t> gate_of_adv(A, -1);
+    for (uint32_t j = 0; j < G; ++j) gate_of_adv[pk->gate_advice[j]] = gate_of_adv[pk->gate_advice[j]] == -1 ? (int32_t)j : -2;
+    bool fused = NP > 0 && G > 0;
+    {
+        uint32_t next_gate = 0;
+        for (uint32_t c = 0; c < NP && fused; ++c)
+            if (pk->perm_kind[c] == 0 && gate_of_adv[pk->perm_index[c]] != -1) fused = gate_of_adv[pk->perm_index[c]] == (int32_t)next_gate++;
+        fused = fused && next_gate == G;
+    }
+    if (fused) {
+        H2V_CU(cudaMemsetAsync(hp_acc, 0, ne * sizeof(fe), pk->st));
+        H2V_TRY(sync(pk));
+        H2V_TRY(fill_sigma_cache(g));
+        const size_t BS = std::max<size_t>(1, SC / (3 * (size_t)pk->chunk));
+        std::vector<const fe *> pc, sg, gq, ga;
+        for (size_t s0 = 0; s0 < NS; s0 += BS) {
+            const size_t s1 = std::min<size_t>(NS, s0 + BS), c0 = s0 * pk->chunk, c1 = std::min<size_t>(NP, s1 * pk->chunk), cnt = c1 - c0;
+            src.clear(); pc.clear(); sg.clear(); gq.clear(); ga.clear();
+            size_t slot = 0;
+            for (size_t c = c0; c < c1; ++c) {
+                src.push_back(g.col(COEFF, 0, pk->perm_kind[c], pk->perm_index[c]));
+                pc.push_back(scr + slot++ * ne);
             }
-        H2V_TRY(put(pk, pk->ptrs, hp));
-        std::vector<Fr64> ybg(3 * B);
-        for (size_t p = 0; p < B; ++p) {
-            ybg[3 * p] = P[p]->y;
-            ybg[3 * p + 1] = P[p]->beta;
-            ybg[3 * p + 2] = P[p]->gamma;
-        }
-        H2V_TRY(put(pk, pk->scal, ybg));
-        const void *const *tab = (const void *const *)pk->ptrs.p;
-        QuotientBatch qb;
-        qb.h = h_ext0; qb.h_stride = ne; qb.scal = pk->scal.p; qb.n_proofs = B;
-        qb.n_gates = G; qb.gate_tab = tab; qb.gate_pstride = per;
-        qb.n_perm = NP; qb.chunk = pk->chunk; qb.perm_tab = tab + 2 * G; qb.perm_pstride = per;
-        qb.z = pk->z_E.p; qb.z_stride = ne; qb.z_pstride = (size_t)NS * ne; qb.blinding_factors = bf;
-        qb.n_lookups = L; qb.lookup_tab = tab + B * per; qb.lookup_pstride = lper;
-        qb.l0 = l0; qb.l_last = ll; qb.l_active = la;
-        H2V_TRY(quotient_batch_dev(pk->dom, qb));
-    } else {
-        // the same folds, in upstream's order, over slices of columns whose extended forms are rebuilt into `scr_E` from
-        // the resident coefficient forms (every term reads columns of its own gate / set / lookup only); one proof
-        fe *h_ext = h_ext0, *h_out = h_out0;
-        const Fr64 &y = P[0]->y, &beta = P[0]->beta, &gamma = P[0]->gamma;
-        const size_t SC = pk->scr_cols;
-        H2V_TRY(pk->scr_E.ensure(SC * ne * sizeof(fe)));
-        fe *scr = pk->scr_E.as<fe>();
-        auto col_C = [&](uint8_t kind, uint32_t idx) -> const fe * {
-            return kind == 0 ? pk->adv_C.as<fe>() + (size_t)idx * n : kind == 1 ? pk->fixed_C.as<fe>() + (size_t)idx * n : pk->inst_C.as<fe>() + (size_t)idx * n;
-        };
-        // coeff_to_extended of a list of coefficient columns into consecutive scratch slots; neighbours share one launch
-        const bool timing = getenv("H2V_PROVE_TIMING") != nullptr;
-        double t_ext = 0, t_fold = 0, t_mark = PhaseClock::now();
-        auto mark = [&](double &acc) {
-            if (!timing) return;
-            cudaDeviceSynchronize();
-            const double t = PhaseClock::now();
-            acc += t - t_mark;
-            t_mark = t;
-        };
-        auto extend = [&](const std::vector<const fe *> &src, fe *dst) -> int {
-            for (size_t i = 0; i < src.size();) {
-                size_t j = i + 1;
-                while (j < src.size() && src[j] == src[j - 1] + n) ++j;
-                H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, src[i], n, dst + i * ne, ne, j - i));
-                i = j;
-            }
-            return H2V_OK;
-        };
-        const void *const *tab = (const void *const *)pk->ptrs.p;
-        std::vector<const fe *> src, hp;
-        // Gate j reads one advice column, and (in halo2-base's constraint system) every gate column is also a permutation
-        // column: when the gates meet their columns in gate order along the permutation, one pass over the permutation
-        // slices serves both folds -- the gates into h, the permutation into a second accumulator hp (the memory of the
-        // quotient's output, free until the division), joined as h <- h y^(permutation terms) + hp.  Each advice column is
-        // then extended once instead of twice.  Any other constraint system takes the two separate loops below.
-        std::vector<int32_t> gate_of_adv(A, -1);
-        for (uint32_t j = 0; j < G; ++j) gate_of_adv[pk->gate_advice[j]] = gate_of_adv[pk->gate_advice[j]] == -1 ? (int32_t)j : -2;
-        bool fused = NP > 0 && G > 0;
-        {
-            uint32_t next_gate = 0;
-            for (uint32_t c = 0; c < NP && fused; ++c)
-                if (pk->perm_kind[c] == 0 && gate_of_adv[pk->perm_index[c]] != -1) fused = gate_of_adv[pk->perm_index[c]] == (int32_t)next_gate++;
-            fused = fused && next_gate == G;
-        }
-        if (fused) {
-            fe *hp_acc = h_out;
-            H2V_CU(cudaMemsetAsync(hp_acc, 0, ne * sizeof(fe), st));
-            H2V_TRY(sync(pk));
-            if (!pk->cache_tried) {
-                pk->cache_tried = true;
-                size_t free_b = 0, total_b = 0;
-                cudaMemGetInfo(&free_b, &total_b);
-                const char *e = getenv("H2V_EXT_CACHE_COLS");
-                const size_t margin = (size_t)8 << 30;
-                size_t want = e ? (size_t)atoi(e) : (free_b > margin ? (free_b - margin) / (ne * sizeof(fe)) : 0);
-                want = std::min<size_t>(want, NP);
-                if (want >= (e ? 1u : 8u) && pk->ext_cache.ensure(want * ne * sizeof(fe)) == H2V_OK) {
-                    H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, pk->sigma_C.p, n, pk->ext_cache.p, ne, want));
-                    pk->cached_sigma = want;
+            for (size_t c = c0; c < c1; ++c) {
+                if (c < pk->cached_sigma) {
+                    sg.push_back(pk->ext_cache.as<fe>() + c * ne);
+                } else {
+                    src.push_back(pk->sigma_C.as<fe>() + c * n);
+                    sg.push_back(scr + slot++ * ne);
                 }
             }
-            const size_t BS = std::max<size_t>(1, SC / (3 * (size_t)pk->chunk));
-            std::vector<const fe *> pc, sg, gq, ga;
-            for (size_t s0 = 0; s0 < NS; s0 += BS) {
-                const size_t s1 = std::min<size_t>(NS, s0 + BS), c0 = s0 * pk->chunk, c1 = std::min<size_t>(NP, s1 * pk->chunk), cnt = c1 - c0;
-                src.clear(); pc.clear(); sg.clear(); gq.clear(); ga.clear();
-                size_t slot = 0;
-                for (size_t c = c0; c < c1; ++c) {
-                    src.push_back(col_C(pk->perm_kind[c], pk->perm_index[c]));
-                    pc.push_back(scr + slot++ * ne);
-                }
-                for (size_t c = c0; c < c1; ++c) {
-                    if (c < pk->cached_sigma) {
-                        sg.push_back(pk->ext_cache.as<fe>() + c * ne);
-                    } else {
-                        src.push_back(pk->sigma_C.as<fe>() + c * n);
-                        sg.push_back(scr + slot++ * ne);
-                    }
-                }
-                // this slice's gates: selector extended behind the slice, advice already in it
-                for (size_t c = c0; c < c1; ++c) {
-                    if (pk->perm_kind[c] != 0 || gate_of_adv[pk->perm_index[c]] < 0) continue;
-                    src.push_back(col_C(1, pk->gate_selector[gate_of_adv[pk->perm_index[c]]]));
-                    gq.push_back(scr + slot++ * ne);
-                    ga.push_back(pc[c - c0]);
-                }
-                H2V_TRY(extend(src, scr));
-                mark(t_ext);
-                hp.clear();
-                hp.insert(hp.end(), pc.begin(), pc.end());
-                hp.insert(hp.end(), sg.begin(), sg.end());
-                hp.insert(hp.end(), gq.begin(), gq.end());
-                hp.insert(hp.end(), ga.begin(), ga.end());
-                H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), hp.size() * sizeof(void *)));
-                H2V_TRY(h2v_quotient_permutation_range_ptrs_dev(pk->dom, hp_acc, u64(y), u64(beta), u64(gamma), NP, pk->chunk, s0, s1, s0 == 0,
-                                                                tab, tab + cnt, pk->z_E.p, ne, l0, ll, la, bf));
-                if (!gq.empty()) H2V_TRY(h2v_quotient_gates_ptrs_dev(pk->dom, h_ext, u64(y), gq.size(), tab + 2 * cnt, tab + 2 * cnt + gq.size()));
-                mark(t_fold);
+            // this slice's gates: selector extended behind the slice, advice already in it
+            for (size_t c = c0; c < c1; ++c) {
+                if (pk->perm_kind[c] != 0 || gate_of_adv[pk->perm_index[c]] < 0) continue;
+                src.push_back(g.col(COEFF, 0, 1, pk->gate_selector[gate_of_adv[pk->perm_index[c]]]));
+                gq.push_back(scr + slot++ * ne);
+                ga.push_back(pc[c - c0]);
             }
-            // h <- h y^T + hp, T = the permutation argument's terms: 2 + (NS - 1) + NS
-            H2V_TRY(lincomb(pk, {h_ext, hp_acc}, {frh::pow_u64(y, 2ull * NS + 1), frh::ONE}, {0, 2}, h_ext, ne, ne));
-            H2V_TRY(sync(pk));
+            H2V_TRY(extend(src, scr));
+            mark(t_ext);
+            hp.clear();
+            hp.insert(hp.end(), pc.begin(), pc.end());
+            hp.insert(hp.end(), sg.begin(), sg.end());
+            hp.insert(hp.end(), gq.begin(), gq.end());
+            hp.insert(hp.end(), ga.begin(), ga.end());
+            H2V_TRY(upload(pk, pk->ptrs, 0, hp.data(), hp.size() * sizeof(void *)));
+            H2V_TRY(h2v_quotient_permutation_range_ptrs_dev(pk->dom, hp_acc, u64(y), u64(beta), u64(gamma), NP, pk->chunk, s0, s1, s0 == 0,
+                                                            tab, tab + cnt, pk->z_E.p, ne, l0, ll, la, bf));
+            if (!gq.empty()) H2V_TRY(h2v_quotient_gates_ptrs_dev(pk->dom, h_ext, u64(y), gq.size(), tab + 2 * cnt, tab + 2 * cnt + gq.size()));
             mark(t_fold);
-        } else {
+        }
+        // h <- h y^T + hp_acc, T = the permutation argument's terms: 2 + (NS - 1) + NS
+        H2V_TRY(lincomb(pk, {h_ext, hp_acc}, {frh::pow_u64(y, 2ull * NS + 1), frh::ONE}, {0, 2}, h_ext, ne, ne));
+        H2V_TRY(sync(pk));
+        mark(t_fold);
+    } else {
         const size_t BG = SC / 2;
         for (size_t g0 = 0; g0 < G; g0 += BG) {
             const size_t b = std::min<size_t>(BG, G - g0);
             src.clear();
             hp.assign(2 * b, nullptr);
-            for (size_t j = 0; j < b; ++j) src.push_back(col_C(1, pk->gate_selector[g0 + j]));
-            for (size_t j = 0; j < b; ++j) src.push_back(col_C(0, pk->gate_advice[g0 + j]));
+            for (size_t j = 0; j < b; ++j) src.push_back(g.col(COEFF, 0, 1, pk->gate_selector[g0 + j]));
+            for (size_t j = 0; j < b; ++j) src.push_back(g.col(COEFF, 0, 0, pk->gate_advice[g0 + j]));
             H2V_TRY(extend(src, scr));
             mark(t_ext);
             for (size_t j = 0; j < 2 * b; ++j) hp[j] = scr + j * ne;
@@ -1017,7 +1049,7 @@ int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector
             const size_t s1 = std::min<size_t>(NS, s0 + BS), c0 = s0 * pk->chunk, c1 = std::min<size_t>(NP, s1 * pk->chunk), cnt = c1 - c0;
             src.clear();
             hp.assign(2 * cnt, nullptr);
-            for (size_t c = c0; c < c1; ++c) src.push_back(col_C(pk->perm_kind[c], pk->perm_index[c]));
+            for (size_t c = c0; c < c1; ++c) src.push_back(g.col(COEFF, 0, pk->perm_kind[c], pk->perm_index[c]));
             for (size_t c = c0; c < c1; ++c) src.push_back(pk->sigma_C.as<fe>() + c * n);
             H2V_TRY(extend(src, scr));
             mark(t_ext);
@@ -1027,50 +1059,76 @@ int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector
                                                             tab, tab + cnt, pk->z_E.p, ne, l0, ll, la, bf));
             mark(t_fold);
         }
-        }
-        // lookups: the table's extended form in slot 0 (one table for all of halo2-base's range lookups), the inputs of up
-        // to SC - 1 lookups extended together (a single 2^22-point column transforms four times slower per column than a batch)
-        uint32_t table_in_slot = UINT32_MAX;
-        for (uint32_t l0_ = 0; l0_ < L;) {
-            if (pk->lookup_table[l0_] != table_in_slot) {
-                H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, col_C(1, pk->lookup_table[l0_]), n, scr, ne, 1));
-                table_in_slot = pk->lookup_table[l0_];
-            }
-            uint32_t l1_ = l0_;
-            src.clear();
-            while (l1_ < L && pk->lookup_table[l1_] == table_in_slot && src.size() + 1 < SC) src.push_back(col_C(0, pk->lookup_input[l1_++]));
-            H2V_TRY(extend(src, scr + ne));
-            mark(t_ext);
-            for (uint32_t l = l0_; l < l1_; ++l)
-                H2V_TRY(h2v_quotient_lookup_dev(pk->dom, h_ext, u64(y), u64(beta), u64(gamma), scr + (size_t)(1 + l - l0_) * ne, scr,
-                                                pk->pa_E.as<fe>() + (size_t)l * ne, pk->ps_E.as<fe>() + (size_t)l * ne, pk->zl_E.as<fe>() + (size_t)l * ne, l0, ll, la));
-            mark(t_fold);
-            l0_ = l1_;
-        }
-        if (timing) fprintf(stderr, "evaluate_h (streamed): coeff_to_extended of the slices %.1f ms, folds %.1f ms\n", t_ext, t_fold);
     }
-    H2V_TRY(h2v_domain_transform_dev(pk->dom, H2V_OP_DIVIDE_BY_VANISHING, h_ext0, ne, h_out0, ne, B));
-    const uint32_t NH = pk->degree - 1;          // quotient pieces of n coefficients each
-    for (auto &s : P)
-        for (uint32_t i = 0; i < NH; ++i) (void)s->rng.fr_random();     // h_blinds
+    // lookups: the table's extended form in slot 0 (one table for all of halo2-base's range lookups), the inputs of up
+    // to SC - 1 lookups extended together (a single 2^22-point column transforms four times slower per column than a batch)
+    uint32_t table_in_slot = UINT32_MAX;
+    for (uint32_t l0_ = 0; l0_ < L;) {
+        if (pk->lookup_table[l0_] != table_in_slot) {
+            H2V_TRY(h2v_domain_transform_dev(pk->dom, C2E, g.col(COEFF, 0, 1, pk->lookup_table[l0_]), n, scr, ne, 1));
+            table_in_slot = pk->lookup_table[l0_];
+        }
+        uint32_t l1_ = l0_;
+        src.clear();
+        while (l1_ < L && pk->lookup_table[l1_] == table_in_slot && src.size() + 1 < SC) src.push_back(g.col(COEFF, 0, 0, pk->lookup_input[l1_++]));
+        H2V_TRY(extend(src, scr + ne));
+        mark(t_ext);
+        for (uint32_t l = l0_; l < l1_; ++l)
+            H2V_TRY(h2v_quotient_lookup_dev(pk->dom, h_ext, u64(y), u64(beta), u64(gamma), scr + (size_t)(1 + l - l0_) * ne, scr,
+                                            pk->pa_E.as<fe>() + (size_t)l * ne, pk->ps_E.as<fe>() + (size_t)l * ne, pk->zl_E.as<fe>() + (size_t)l * ne, l0, ll, la));
+        mark(t_fold);
+        l0_ = l1_;
+    }
+    if (timing) fprintf(stderr, "evaluate_h (streamed): coeff_to_extended of the slices %.1f ms, folds %.1f ms\n", t_ext, t_fold);
+    return H2V_OK;
+}
+
+//      steps 9-11: h_ext of proof p at hq + p ne, zeroed, then evaluate_h; its quotient after the division at hq + (B + p) ne
+int evaluate_h(Group &g) {
+    h2v_pk *pk = g.pk;
+    H2V_TRY(pk->hq.ensure(2 * g.B * g.ne * sizeof(fe)));
+    fe *h_ext = pk->hq.as<fe>(), *h_out = h_ext + g.B * g.ne;
+    H2V_CU(cudaMemsetAsync(h_ext, 0, g.B * g.ne * sizeof(fe), pk->st));
+    H2V_TRY(sync(pk));
+    return pk->stream_ext ? evaluate_h_streamed(g, h_ext, h_out) : evaluate_h_resident(g, h_ext);
+}
+
+//      vanishing/prover.rs Committed::construct: h divided by the vanishing polynomial (back in coefficients), one blind
+//      per piece, the NH pieces of n coefficients committed and written
+int commit_quotient(Group &g) {
+    h2v_pk *pk = g.pk;
+    const size_t B = g.B, n = g.n, ne = g.ne, NH = g.NH;
+    fe *h_ext = pk->hq.as<fe>(), *h_out = h_ext + B * ne;
+    H2V_TRY(h2v_domain_transform_dev(pk->dom, H2V_OP_DIVIDE_BY_VANISHING, h_ext, ne, h_out, ne, B));
+    for (auto &s : g.P)
+        for (size_t i = 0; i < NH; ++i) (void)s->rng.fr_random();     // h_blinds
     // the B x NH pieces as contiguous columns of n (they already are when NH n = ne, and for one proof)
-    fe *pieces = h_out0;
+    g.pieces = h_out;
     if (B > 1 && NH * n != ne) {
         H2V_TRY(pk->hx_pieces.ensure(B * NH * n * sizeof(fe)));
-        pieces = pk->hx_pieces.as<fe>();
-        H2V_CU(cudaMemcpy2DAsync(pieces, NH * n * sizeof(fe), h_out0, ne * sizeof(fe), NH * n * sizeof(fe), B, cudaMemcpyDeviceToDevice, st));
+        g.pieces = pk->hx_pieces.as<fe>();
+        H2V_CU(cudaMemcpy2DAsync(g.pieces, NH * n * sizeof(fe), h_out, ne * sizeof(fe), NH * n * sizeof(fe), B, cudaMemcpyDeviceToDevice, pk->st));
         H2V_TRY(sync(pk));
     }
-    H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, pieces, B * NH, pts));
-    for (size_t p = 0; p < B; ++p) {
-        if (int rc = write_points(P[p]->T, pts.data() + p * NH, NH)) {
-            bad = p;
-            return rc;
-        }
-    }
-    lap();   // phase 4: evaluate_h + quotient commitments
-    // ---- 12. x; evaluations
-    for (auto &s : P) {
+    H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, g.pieces, B * NH, g.pts));
+    return write_commitments(g, g.pts, NH, false);
+}
+
+// ---- phase 5.  plonk/prover.rs create_proof step 12: x, h(X) = sum_i xn^i h_i(X) (vanishing/prover.rs
+//      Constructed::evaluate), and every (polynomial, point) pair that is evaluated.  The list is the same for every
+//      proof, over its own columns: in transcript order first, then the two the transcript skips.
+struct Evaluations {
+    std::vector<EvalPair> pairs;     // NE per proof; .point indexes the proof's NPT distinct points x w^rot
+    std::vector<Fr64> evals;         // of the pairs
+    std::vector<Fr64> points;        // proof p's at p NPT
+    size_t NE = 0, NPT = 0;
+    std::vector<uint32_t> queries;   // the pairs (of one proof) in the order upstream's prover queries them
+};
+int evaluations(Group &g, Evaluations &ev) {
+    h2v_pk *pk = g.pk;
+    const size_t B = g.B, n = g.n;
+    const uint32_t L = g.L, NP = g.NP, NS = g.NS;
+    for (auto &s : g.P) {
         s->x = s->T.squeeze_challenge();
         s->xn = s->x;
         for (uint32_t i = 0; i < pk->k; ++i) s->xn = frh::sqr(s->xn);
@@ -1083,37 +1141,20 @@ int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector
         rots.push_back(rot);
         return (uint32_t)(rots.size() - 1);
     };
-    const uint32_t p_cur = point_of(0), p_next = point_of(1), p_prev = point_of(-1), p_last = point_of(-(int32_t)(bf + 1));
-    // h(X) = sum_i xn^i h_i(X); proof p's at sh_h + p n
+    const uint32_t p_cur = point_of(0), p_next = point_of(1), p_prev = point_of(-1), p_last = point_of(-(int32_t)(g.bf + 1));
+    // h(X) of proof p at sh_h + p n
     H2V_TRY(pk->sh_h.ensure(2 * B * n * sizeof(fe)));
-    fe *h_poly0 = pk->sh_h.as<fe>(), *hx0 = pk->sh_h.as<fe>() + B * n;
-    {
-        std::vector<const fe *> hp(B * NH);
-        std::vector<Fr64> cf(B * NH);
-        std::vector<uint32_t> off(B + 1);
-        for (size_t p = 0; p < B; ++p) {
-            Fr64 cur = frh::ONE;
-            off[p] = (uint32_t)(p * NH);
-            for (uint32_t i = 0; i < NH; ++i) {
-                hp[p * NH + i] = pieces + (p * NH + i) * n;
-                cf[p * NH + i] = cur;
-                cur = frh::mul(cur, P[p]->xn);
-            }
-        }
-        off[B] = (uint32_t)(B * NH);
-        H2V_TRY(lincomb(pk, hp, cf, off, h_poly0, n, n));
-    }
-    // every (polynomial, point) pair that is evaluated, in transcript order first, then the two the transcript skips; the
-    // same list for every proof, over its own columns
-    std::vector<EvalPair> pairs;
+    fe *h_poly0 = pk->sh_h.as<fe>();
+    H2V_TRY(sum_powers(g, g.pieces, g.NH, &ProofState::xn, h_poly0));
+    std::vector<EvalPair> &pairs = ev.pairs;
     uint32_t e_random = 0, e_perm = 0, e_lookup = 0, n_written = 0, e_h = 0;
     for (size_t p = 0; p < B; ++p) {
         const size_t base = pairs.size();
         auto push = [&](const fe *poly, uint32_t pt) { pairs.push_back(EvalPair{poly, pt}); return (uint32_t)(pairs.size() - 1 - base); };
-        const fe *adv_C = pk->adv_C.as<fe>() + p * A * n, *z_C = pk->z_C.as<fe>() + p * NS * n, *zl_C = pk->zl_C.as<fe>() + p * L * n,
-                 *pa_C = pk->pa_C.as<fe>() + p * L * n, *ps_C = pk->ps_C.as<fe>() + p * L * n;
-        for (size_t q = 0; q < pk->aq_col.size(); ++q) push(adv_C + (size_t)pk->aq_col[q] * n, point_of(pk->aq_rot[q]));
-        for (size_t q = 0; q < pk->fq_col.size(); ++q) push(pk->fixed_C.as<fe>() + (size_t)pk->fq_col[q] * n, point_of(pk->fq_rot[q]));
+        const fe *z_C = pk->z_C.as<fe>() + p * NS * n, *zl_C = pk->zl_C.as<fe>() + p * L * n, *pa_C = pk->pa_C.as<fe>() + p * L * n,
+                 *ps_C = pk->ps_C.as<fe>() + p * L * n;
+        for (size_t q = 0; q < pk->aq_col.size(); ++q) push(g.col(COEFF, p, 0, pk->aq_col[q]), point_of(pk->aq_rot[q]));
+        for (size_t q = 0; q < pk->fq_col.size(); ++q) push(g.col(COEFF, p, 1, pk->fq_col[q]), point_of(pk->fq_rot[q]));
         e_random = push(pk->rnd_C.as<fe>() + p * n, p_cur);
         for (uint32_t c = 0; c < NP; ++c) push(pk->sigma_C.as<fe>() + (size_t)c * n, p_cur);
         e_perm = e_random + 1 + NP;
@@ -1133,154 +1174,137 @@ int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector
         n_written = e_lookup + 5 * L;
         e_h = push(h_poly0 + p * n, p_cur);       // h(x): opened by the multi-open argument, not written
     }
-    const size_t NE = e_h + 1, NPT = rots.size();        // pairs and distinct points per proof
-    std::vector<Fr64> points(B * NPT);                   // proof p's points at p NPT
+    ev.NE = e_h + 1;
+    ev.NPT = rots.size();
+    // the queries of the multi-open argument in upstream's order: advice; permutation products
+    // (permutation::prover::Evaluated::open: (x, z_s), (wx, z_s) for every set, then (w^last x, z_s) for all but the last
+    // set taken in reverse order); lookups (lookup::prover::Evaluated::open: (x, z), (x, a'), (x, s'), (w^-1 x, a'),
+    // (wx, z)); fixed; sigma; vanishing (h, then the random polynomial)
+    std::vector<uint32_t> &q = ev.queries;
+    for (uint32_t e = 0; e < pk->aq_col.size(); ++e) q.push_back(e);
+    for (uint32_t s = 0; s < NS; ++s) q.insert(q.end(), {e_perm + 3 * s, e_perm + 3 * s + 1});
+    for (uint32_t s = NS; s-- > 0;)
+        if (s + 1 < NS) q.push_back(e_perm + 3 * s + 2);
+    for (uint32_t l = 0; l < L; ++l) {
+        const uint32_t b = e_lookup + 5 * l;
+        q.insert(q.end(), {b, b + 2, b + 4, b + 3, b + 1});
+    }
+    for (uint32_t e = 0; e < pk->fq_col.size(); ++e) q.push_back((uint32_t)pk->aq_col.size() + e);
+    for (uint32_t c = 0; c < NP; ++c) q.push_back(e_random + 1 + c);
+    q.insert(q.end(), {e_h, e_random});
+    const size_t NE = ev.NE, NPT = ev.NPT;
+    ev.points.resize(B * NPT);
     for (size_t p = 0; p < B; ++p)
-        for (size_t i = 0; i < NPT; ++i) points[p * NPT + i] = frh::rotate(P[p]->x, pk->omega, pk->omega_inv, rots[i]);
+        for (size_t i = 0; i < NPT; ++i) ev.points[p * NPT + i] = frh::rotate(g.P[p]->x, pk->omega, pk->omega_inv, rots[i]);
     std::vector<EvalPair> dev_pairs(pairs);
     for (size_t e = 0; e < dev_pairs.size(); ++e) dev_pairs[e].point += (uint32_t)((e / NE) * NPT);
-    std::vector<Fr64> evals(pairs.size());
-    {
-        H2V_TRY(put(pk, pk->pairs, dev_pairs));
-        H2V_TRY(put(pk, pk->pts, points));
-        H2V_TRY(pk->evals.ensure(pairs.size() * sizeof(fe)));
-        eval_pairs_kernel<<<(unsigned)pairs.size(), 256, 0, st>>>((const EvalPair *)pk->pairs.p, pk->pts.as<fe>(), (uint32_t)n, pk->evals.as<fe>());
-        H2V_LAUNCHED();
-        H2V_CU(cudaMemcpyAsync(evals.data(), pk->evals.p, pairs.size() * sizeof(fe), cudaMemcpyDeviceToHost, st));
-        H2V_TRY(sync(pk));
-    }
+    ev.evals.resize(pairs.size());
+    H2V_TRY(put(pk, pk->pairs, dev_pairs));
+    H2V_TRY(put(pk, pk->pts, ev.points));
+    H2V_TRY(pk->evals.ensure(pairs.size() * sizeof(fe)));
+    eval_pairs_kernel<<<(unsigned)pairs.size(), 256, 0, pk->st>>>((const EvalPair *)pk->pairs.p, pk->pts.as<fe>(), (uint32_t)n, pk->evals.as<fe>());
+    H2V_LAUNCHED();
+    H2V_CU(cudaMemcpyAsync(ev.evals.data(), pk->evals.p, pairs.size() * sizeof(fe), cudaMemcpyDeviceToHost, pk->st));
+    H2V_TRY(sync(pk));
     for (size_t p = 0; p < B; ++p)
-        for (uint32_t i = 0; i < n_written; ++i) P[p]->T.write_scalar(evals[p * NE + i]);
-    lap();   // phase 5: evaluations
-    // ---- 13. multi-open argument (SHPLONK)
-    // Host side per proof, on B threads: the queries, construct_intermediate_sets, y / v, the Lagrange bases and the
-    // interpolated R_ij.  Every proof has the same rotation sets (commitments grouped by the rotations they are opened
-    // at, in order of first appearance); only the numeric order of the points inside a set differs.
-    struct RSet { uint64_t mask; std::vector<const fe *> polys; };
-    struct MultiOpen {
-        std::vector<RSet> rsets;
-        std::vector<Fr64> sorted_pts;
-        uint64_t super_mask = 0;
-        std::vector<std::vector<Fr64>> r_comb;                 // sum_j y^j R_ij(X), low degree
-        std::vector<std::vector<std::vector<Fr64>>> r_ij;
-        std::vector<std::vector<Fr64>> set_pts;                // the points of set i, numeric order
-        std::vector<std::vector<Fr64>> ypow;
-        std::vector<Fr64> pts_of(uint64_t mask) const {
-            std::vector<Fr64> v;
-            for (size_t r = 0; r < sorted_pts.size(); ++r)
-                if ((mask >> r) & 1) v.push_back(sorted_pts[r]);
-            return v;
+        for (uint32_t i = 0; i < n_written; ++i) g.P[p]->T.write_scalar(ev.evals[p * NE + i]);
+    return H2V_OK;
+}
+
+// ---- phase 6.  The multi-open argument, poly/kzg/multiopen/shplonk/prover.rs ProverSHPLONK::create_proof.  Every proof
+//      has the same rotation sets (commitments grouped by the rotations they are opened at, in order of first
+//      appearance); only the numeric order of the points inside a set differs.
+struct RSet { uint64_t mask; std::vector<const fe *> polys; };
+struct MultiOpen {
+    std::vector<RSet> rsets;
+    std::vector<Fr64> sorted_pts;
+    uint64_t super_mask = 0;
+    std::vector<std::vector<Fr64>> r_comb;                 // sum_j y^j R_ij(X), low degree
+    std::vector<std::vector<std::vector<Fr64>>> r_ij;
+    std::vector<std::vector<Fr64>> set_pts;                // the points of set i, numeric order
+    std::vector<std::vector<Fr64>> ypow;
+    std::vector<Fr64> pts_of(uint64_t mask) const {
+        std::vector<Fr64> v;
+        for (size_t r = 0; r < sorted_pts.size(); ++r)
+            if ((mask >> r) & 1) v.push_back(sorted_pts[r]);
+        return v;
+    }
+};
+
+//      The host side for proof p (one host thread per proof): shplonk.rs construct_intermediate_sets, y / v, the Lagrange
+//      bases and the interpolated R_ij
+MultiOpen multi_open_sets(Group &g, const Evaluations &ev, size_t p) {
+    const size_t NPT = ev.NPT;
+    MultiOpen mo;
+    const EvalPair *pr = ev.pairs.data() + p * ev.NE;
+    const Fr64 *val = ev.evals.data() + p * ev.NE, *pt = ev.points.data() + p * NPT;
+    // construct_intermediate_sets: point sets are ordered sets of field elements (BTreeSet<Fr>: numeric order of the
+    // canonical values); commitments and rotation sets keep their order of first appearance
+    std::vector<uint32_t> rank(NPT), ord(NPT);      // rank[i] = position of point i in the numeric order
+    for (size_t i = 0; i < NPT; ++i) ord[i] = (uint32_t)i;
+    std::sort(ord.begin(), ord.end(), [&](uint32_t a, uint32_t b) { return frh::less_canonical(pt[a], pt[b]); });
+    for (size_t i = 0; i < NPT; ++i) rank[ord[i]] = (uint32_t)i;
+    // a polynomial is identified by its device address, as upstream's PolynomialPointer
+    struct Com { const fe *poly; uint64_t mask; };       // mask over ranks
+    std::vector<Com> coms;
+    std::map<const fe *, size_t> com_of;
+    std::map<std::pair<const fe *, uint32_t>, Fr64> eval_of;
+    for (uint32_t e : ev.queries) {
+        const uint64_t bit = (uint64_t)1 << rank[pr[e].point];
+        mo.super_mask |= bit;
+        auto it = com_of.find(pr[e].poly);
+        if (it == com_of.end()) {
+            com_of[pr[e].poly] = coms.size();
+            coms.push_back(Com{pr[e].poly, bit});
+        } else {
+            coms[it->second].mask |= bit;
         }
-    };
-    std::vector<MultiOpen> MO(B);
-    H2V_TRY(par_proofs(B, [&](size_t p) -> int {
-        MultiOpen &mo = MO[p];
-        const EvalPair *pr = pairs.data() + p * NE;
-        const Fr64 *ev = evals.data() + p * NE, *pt = points.data() + p * NPT;
-        // the prover's queries, in upstream's order: advice, permutation products, lookups, fixed, sigma, vanishing
-        std::vector<Query> queries;
-        {
-            size_t e = 0;
-            std::vector<Query> adv_q, fix_q, sig_q;
-            for (size_t q = 0; q < pk->aq_col.size(); ++q, ++e) adv_q.push_back(Query{pr[e].poly, pr[e].point, ev[e]});
-            for (size_t q = 0; q < pk->fq_col.size(); ++q, ++e) fix_q.push_back(Query{pr[e].poly, pr[e].point, ev[e]});
-            ++e;   // random_eval
-            for (uint32_t c = 0; c < NP; ++c, ++e) sig_q.push_back(Query{pr[e].poly, pr[e].point, ev[e]});
-            queries = adv_q;
-            // permutation::prover::Evaluated::open: (x, z_s), (wx, z_s) for every set, then (w^last x, z_s) for all but the
-            // last set taken in reverse order
-            {
-                std::vector<uint32_t> at(NS);
-                uint32_t pos = e_perm;
-                for (uint32_t s = 0; s < NS; ++s) {
-                    at[s] = pos;
-                    queries.push_back(Query{pr[pos].poly, p_cur, ev[pos]});
-                    queries.push_back(Query{pr[pos + 1].poly, p_next, ev[pos + 1]});
-                    pos += (s + 1 < NS) ? 3 : 2;
-                }
-                for (uint32_t s = NS; s-- > 0;) {
-                    if (s + 1 == NS) continue;
-                    queries.push_back(Query{pr[at[s] + 2].poly, p_last, ev[at[s] + 2]});
-                }
-            }
-            // lookup::prover::Evaluated::open: (x, z), (x, a'), (x, s'), (w^-1 x, a'), (wx, z)
-            for (uint32_t l = 0; l < L; ++l) {
-                const uint32_t b = e_lookup + 5 * l;
-                queries.push_back(Query{pr[b].poly, p_cur, ev[b]});
-                queries.push_back(Query{pr[b + 2].poly, p_cur, ev[b + 2]});
-                queries.push_back(Query{pr[b + 4].poly, p_cur, ev[b + 4]});
-                queries.push_back(Query{pr[b + 3].poly, p_prev, ev[b + 3]});
-                queries.push_back(Query{pr[b + 1].poly, p_next, ev[b + 1]});
-            }
-            queries.insert(queries.end(), fix_q.begin(), fix_q.end());
-            queries.insert(queries.end(), sig_q.begin(), sig_q.end());
-            queries.push_back(Query{pr[e_h].poly, p_cur, ev[e_h]});
-            queries.push_back(Query{pr[e_random].poly, p_cur, ev[e_random]});
+        eval_of[{pr[e].poly, rank[pr[e].point]}] = val[e];
+    }
+    for (const Com &c : coms) {
+        size_t i = 0;
+        for (; i < mo.rsets.size(); ++i)
+            if (mo.rsets[i].mask == c.mask) break;
+        if (i == mo.rsets.size()) mo.rsets.push_back(RSet{c.mask, {}});
+        mo.rsets[i].polys.push_back(c.poly);
+    }
+    mo.sorted_pts.resize(NPT);
+    for (size_t i = 0; i < NPT; ++i) mo.sorted_pts[rank[i]] = pt[i];
+    ProofState &S = *g.P[p];
+    S.ys = S.T.squeeze_challenge();
+    S.vs = S.T.squeeze_challenge();
+    const size_t NR = mo.rsets.size();
+    mo.r_comb.resize(NR);
+    mo.r_ij.resize(NR);
+    mo.set_pts.resize(NR);
+    mo.ypow.resize(NR);
+    for (size_t i = 0; i < NR; ++i) {
+        const std::vector<Fr64> ps = mo.pts_of(mo.rsets[i].mask);
+        const size_t m = ps.size(), nc = mo.rsets[i].polys.size();
+        const std::vector<std::vector<Fr64>> basis = lagrange_basis(ps);
+        Fr64 cur = frh::ONE;
+        mo.r_comb[i].assign(m, frh::zero());
+        mo.r_ij[i].resize(nc);
+        mo.ypow[i].resize(nc);
+        for (size_t j = 0; j < nc; ++j) {
+            mo.ypow[i][j] = cur;
+            std::vector<Fr64> evj;
+            for (size_t r = 0; r < NPT; ++r)
+                if ((mo.rsets[i].mask >> r) & 1) evj.push_back(eval_of[{mo.rsets[i].polys[j], (uint32_t)r}]);
+            mo.r_ij[i][j] = lagrange_interpolate(basis, evj);
+            for (size_t t = 0; t < m; ++t) mo.r_comb[i][t] = frh::add(mo.r_comb[i][t], frh::mul(mo.r_ij[i][j][t], cur));
+            cur = frh::mul(cur, S.ys);
         }
-        // construct_intermediate_sets: point sets are ordered sets of field elements (BTreeSet<Fr>: numeric order of the
-        // canonical values); commitments and rotation sets keep their order of first appearance
-        std::vector<uint32_t> rank(NPT);      // rank[i] = position of point i in the numeric order
-        {
-            std::vector<uint32_t> ord(NPT);
-            for (size_t i = 0; i < NPT; ++i) ord[i] = (uint32_t)i;
-            std::sort(ord.begin(), ord.end(), [&](uint32_t a, uint32_t b) { return frh::less_canonical(pt[a], pt[b]); });
-            for (size_t i = 0; i < NPT; ++i) rank[ord[i]] = (uint32_t)i;
-        }
-        struct Com { const fe *poly; uint64_t mask; };       // mask over ranks
-        std::vector<Com> coms;
-        std::map<const fe *, size_t> com_of;
-        std::map<std::pair<const fe *, uint32_t>, Fr64> eval_of;
-        for (const Query &q : queries) {
-            const uint64_t bit = (uint64_t)1 << rank[q.pt];
-            mo.super_mask |= bit;
-            auto it = com_of.find(q.poly);
-            if (it == com_of.end()) {
-                com_of[q.poly] = coms.size();
-                coms.push_back(Com{q.poly, bit});
-            } else {
-                coms[it->second].mask |= bit;
-            }
-            eval_of[{q.poly, rank[q.pt]}] = q.eval;
-        }
-        for (const Com &c : coms) {
-            size_t i = 0;
-            for (; i < mo.rsets.size(); ++i)
-                if (mo.rsets[i].mask == c.mask) break;
-            if (i == mo.rsets.size()) mo.rsets.push_back(RSet{c.mask, {}});
-            mo.rsets[i].polys.push_back(c.poly);
-        }
-        mo.sorted_pts.resize(NPT);
-        for (size_t i = 0; i < NPT; ++i) mo.sorted_pts[rank[i]] = pt[i];
-        ProofState &S = *P[p];
-        S.ys = S.T.squeeze_challenge();
-        S.vs = S.T.squeeze_challenge();
-        const size_t NR = mo.rsets.size();
-        mo.r_comb.resize(NR);
-        mo.r_ij.resize(NR);
-        mo.set_pts.resize(NR);
-        mo.ypow.resize(NR);
-        for (size_t i = 0; i < NR; ++i) {
-            const std::vector<Fr64> ps = mo.pts_of(mo.rsets[i].mask);
-            const size_t m = ps.size(), nc = mo.rsets[i].polys.size();
-            const std::vector<std::vector<Fr64>> basis = lagrange_basis(ps);
-            Fr64 cur = frh::ONE;
-            mo.r_comb[i].assign(m, frh::zero());
-            mo.r_ij[i].resize(nc);
-            mo.ypow[i].resize(nc);
-            for (size_t j = 0; j < nc; ++j) {
-                mo.ypow[i][j] = cur;
-                std::vector<Fr64> evj;
-                for (size_t r = 0; r < NPT; ++r)
-                    if ((mo.rsets[i].mask >> r) & 1) evj.push_back(eval_of[{mo.rsets[i].polys[j], (uint32_t)r}]);
-                mo.r_ij[i][j] = lagrange_interpolate(basis, evj);
-                for (size_t t = 0; t < m; ++t) mo.r_comb[i][t] = frh::add(mo.r_comb[i][t], frh::mul(mo.r_ij[i][j][t], cur));
-                cur = frh::mul(cur, S.ys);
-            }
-            mo.set_pts[i] = ps;
-        }
-        return H2V_OK;
-    }));
-    const size_t NR = MO[0].rsets.size();
+        mo.set_pts[i] = ps;
+    }
+    return mo;
+}
+
+//      The device side for the group: S_i = sum_j y^j P_ij, Q_i = (S_i - sum_j y^j R_ij) / prod (X - p), h = sum_i v^i Q_i
+//      (committed), u, then L(X) and W = L / (X - u) / z_0 (committed)
+int shplonk(Group &g, const std::vector<MultiOpen> &MO) {
+    h2v_pk *pk = g.pk;
+    const size_t B = g.B, n = g.n, NR = MO[0].rsets.size();
     for (const MultiOpen &mo : MO)
         if (mo.rsets.size() != NR) return failf(H2V_EINVAL, "create_proof: rotation sets differ between the proofs of a group");
     size_t max_m = 1;
@@ -1289,6 +1313,7 @@ int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector
     H2V_TRY(pk->sh_A.ensure((B * n + 8) * sizeof(fe)));
     H2V_TRY(pk->sh_B.ensure(std::max<size_t>(B * NR, B) * n * sizeof(fe)));
     fe *S0 = pk->sh_S.as<fe>(), *Q = pk->sh_B.as<fe>();       // S_i and the quotient contributions Q_i of proof p: (p NR + i) n
+    fe *hx0 = pk->sh_h.as<fe>() + B * n;                      // proof p's h(X) at hx0 + p n
     {
         // S_i(X) = sum_j y^j P_ij(X) for every proof and set in one launch; N_i = S_i - sum_j y^j R_ij
         std::vector<const fe *> hp;
@@ -1303,135 +1328,126 @@ int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector
             }
         off.push_back((uint32_t)hp.size());
         H2V_TRY(lincomb(pk, hp, cf, off, S0, n, n));
-        H2V_CU(cudaMemcpyAsync(Q, S0, B * NR * n * sizeof(fe), cudaMemcpyDeviceToDevice, st));
+        H2V_CU(cudaMemcpyAsync(Q, S0, B * NR * n * sizeof(fe), cudaMemcpyDeviceToDevice, pk->st));
         H2V_TRY(sub_low(pk, Q, n, low, B * NR));
         H2V_TRY(sync(pk));
     }
     // Q_i = N_i / prod (X - p): one division per point of the set, every (proof, set) with a t-th point in one batched
     // pass; each column ping-pongs between its home in Q and its own slot in sh_T
     H2V_TRY(pk->sh_T.ensure(B * NR * n * sizeof(fe)));
-    {
-        std::vector<KateJob> jobs;
-        for (size_t t = 0; t < max_m; ++t) {
-            jobs.clear();
-            for (size_t p = 0; p < B; ++p)
-                for (size_t i = 0; i < NR; ++i) {
-                    const std::vector<Fr64> &ps = MO[p].set_pts[i];
-                    if (t >= ps.size()) continue;
-                    fe *home = Q + (p * NR + i) * n, *slot = pk->sh_T.as<fe>() + (p * NR + i) * n;
-                    KateJob j{t % 2 ? slot : home, t % 2 ? home : slot, n - t, {}};
-                    memcpy(j.b, u64(ps[t]), sizeof j.b);
-                    jobs.push_back(j);
-                }
-            H2V_TRY(kate_division_batch_dev(jobs.data(), jobs.size()));
-        }
+    std::vector<KateJob> jobs;
+    for (size_t t = 0; t < max_m; ++t) {
+        jobs.clear();
         for (size_t p = 0; p < B; ++p)
             for (size_t i = 0; i < NR; ++i) {
-                const size_t m = MO[p].set_pts[i].size(), len = n - m;
-                fe *home = Q + (p * NR + i) * n;
-                if (m % 2) H2V_CU(cudaMemcpyAsync(home, pk->sh_T.as<fe>() + (p * NR + i) * n, len * sizeof(fe), cudaMemcpyDeviceToDevice, st));
-                H2V_CU(cudaMemsetAsync(home + len, 0, m * sizeof(fe), st));
+                const std::vector<Fr64> &ps = MO[p].set_pts[i];
+                if (t >= ps.size()) continue;
+                fe *home = Q + (p * NR + i) * n, *slot = pk->sh_T.as<fe>() + (p * NR + i) * n;
+                KateJob j{t % 2 ? slot : home, t % 2 ? home : slot, n - t, {}};
+                memcpy(j.b, u64(ps[t]), sizeof j.b);
+                jobs.push_back(j);
             }
+        H2V_TRY(kate_division_batch_dev(jobs.data(), jobs.size()));
     }
-    // h(X) = sum_i v^i Q_i(X)
-    {
-        std::vector<const fe *> hp(B * NR);
-        std::vector<Fr64> cf(B * NR);
-        std::vector<uint32_t> off(B + 1);
-        for (size_t p = 0; p < B; ++p) {
-            Fr64 cur = frh::ONE;
-            off[p] = (uint32_t)(p * NR);
-            for (size_t i = 0; i < NR; ++i) {
-                hp[p * NR + i] = Q + (p * NR + i) * n;
-                cf[p * NR + i] = cur;
-                cur = frh::mul(cur, P[p]->vs);
-            }
+    for (size_t p = 0; p < B; ++p)
+        for (size_t i = 0; i < NR; ++i) {
+            const size_t m = MO[p].set_pts[i].size(), len = n - m;
+            fe *home = Q + (p * NR + i) * n;
+            if (m % 2) H2V_CU(cudaMemcpyAsync(home, pk->sh_T.as<fe>() + (p * NR + i) * n, len * sizeof(fe), cudaMemcpyDeviceToDevice, pk->st));
+            H2V_CU(cudaMemsetAsync(home + len, 0, m * sizeof(fe), pk->st));
         }
-        off[B] = (uint32_t)(B * NR);
-        H2V_TRY(lincomb(pk, hp, cf, off, hx0, n, n));
-        H2V_TRY(sync(pk));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, hx0, B, pts));
-        for (size_t p = 0; p < B; ++p) {
-            if (int rc = write_points(P[p]->T, pts.data() + p, 1)) {
-                bad = p;
-                return rc;
+    H2V_TRY(sum_powers(g, Q, NR, &ProofState::vs, hx0));      // h(X) = sum_i v^i Q_i(X)
+    H2V_TRY(sync(pk));
+    H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, hx0, B, g.pts));
+    H2V_TRY(write_commitments(g, g.pts, 1, false));
+    for (auto &s : g.P) s->uc = s->T.squeeze_challenge();
+    // L(X) = sum_i v^i z_i (S_i(X) - sum_j y^j R_ij(u)) - Z_T(u) h(X);  second opening proof = L / (X - u) / z_0
+    std::vector<const fe *> hp(B * (NR + 1));
+    std::vector<Fr64> cf(B * (NR + 1)), konst(B), z0inv(B);
+    std::vector<uint32_t> off(B + 1);
+    H2V_TRY(par_proofs(B, [&](size_t p) -> int {
+        const MultiOpen &mo = MO[p];
+        const Fr64 &uc = g.P[p]->uc;
+        Fr64 vp = frh::ONE, z0 = frh::ONE;
+        konst[p] = frh::zero();
+        for (size_t i = 0; i < NR; ++i) {
+            Fr64 zi = frh::ONE;
+            for (size_t r = 0; r < mo.sorted_pts.size(); ++r)
+                if (((mo.super_mask & ~mo.rsets[i].mask) >> r) & 1) zi = frh::mul(zi, frh::sub(uc, mo.sorted_pts[r]));
+            if (i == 0) z0 = zi;
+            Fr64 ri = frh::zero(), yp = frh::ONE;
+            for (size_t j = 0; j < mo.rsets[i].polys.size(); ++j) {
+                ri = frh::add(ri, frh::mul(yp, eval_small(mo.r_ij[i][j], uc)));
+                yp = frh::mul(yp, g.P[p]->ys);
             }
+            hp[p * (NR + 1) + i] = S0 + (p * NR + i) * n;
+            cf[p * (NR + 1) + i] = frh::mul(vp, zi);
+            konst[p] = frh::add(konst[p], frh::mul(cf[p * (NR + 1) + i], ri));
+            vp = frh::mul(vp, g.P[p]->vs);
         }
+        Fr64 zt = frh::ONE;
+        for (const Fr64 &x : mo.pts_of(mo.super_mask)) zt = frh::mul(zt, frh::sub(uc, x));
+        hp[p * (NR + 1) + NR] = hx0 + p * n;
+        cf[p * (NR + 1) + NR] = frh::neg(zt);
+        off[p] = (uint32_t)(p * (NR + 1));
+        z0inv[p] = frh::inv(z0);
+        return H2V_OK;
+    }));
+    off[B] = (uint32_t)(B * (NR + 1));
+    fe *Lx = pk->sh_A.as<fe>();           // proof p's L at Lx + p n
+    H2V_TRY(lincomb(pk, hp, cf, off, Lx, n, n));
+    H2V_TRY(sub_low(pk, Lx, n, konst, B));
+    H2V_TRY(sync(pk));
+    fe *W = Q;        // the quotient contributions are no longer needed; proof p's W at W + p n
+    jobs.resize(B);
+    for (size_t p = 0; p < B; ++p) {
+        jobs[p] = KateJob{Lx + p * n, W + p * n, n, {}};
+        memcpy(jobs[p].b, u64(g.P[p]->uc), sizeof jobs[p].b);
     }
-    for (auto &s : P) s->uc = s->T.squeeze_challenge();
-    {
-        // L(X) = sum_i v^i z_i (S_i(X) - sum_j y^j R_ij(u)) - Z_T(u) h(X);  second opening proof = L / (X - u) / z_0
-        std::vector<const fe *> hp(B * (NR + 1));
-        std::vector<Fr64> cf(B * (NR + 1)), konst(B), z0inv(B);
-        std::vector<uint32_t> off(B + 1);
-        H2V_TRY(par_proofs(B, [&](size_t p) -> int {
-            const MultiOpen &mo = MO[p];
-            const Fr64 &uc = P[p]->uc;
-            Fr64 vp = frh::ONE, z0 = frh::ONE;
-            konst[p] = frh::zero();
-            for (size_t i = 0; i < NR; ++i) {
-                Fr64 zi = frh::ONE;
-                for (size_t r = 0; r < NPT; ++r)
-                    if (((mo.super_mask & ~mo.rsets[i].mask) >> r) & 1) zi = frh::mul(zi, frh::sub(uc, mo.sorted_pts[r]));
-                if (i == 0) z0 = zi;
-                Fr64 ri = frh::zero(), yp = frh::ONE;
-                for (size_t j = 0; j < mo.rsets[i].polys.size(); ++j) {
-                    ri = frh::add(ri, frh::mul(yp, eval_small(mo.r_ij[i][j], uc)));
-                    yp = frh::mul(yp, P[p]->ys);
-                }
-                hp[p * (NR + 1) + i] = S0 + (p * NR + i) * n;
-                cf[p * (NR + 1) + i] = frh::mul(vp, zi);
-                konst[p] = frh::add(konst[p], frh::mul(cf[p * (NR + 1) + i], ri));
-                vp = frh::mul(vp, P[p]->vs);
-            }
-            Fr64 zt = frh::ONE;
-            for (const Fr64 &x : mo.pts_of(mo.super_mask)) zt = frh::mul(zt, frh::sub(uc, x));
-            hp[p * (NR + 1) + NR] = hx0 + p * n;
-            cf[p * (NR + 1) + NR] = frh::neg(zt);
-            off[p] = (uint32_t)(p * (NR + 1));
-            z0inv[p] = frh::inv(z0);
-            return H2V_OK;
-        }));
-        off[B] = (uint32_t)(B * (NR + 1));
-        fe *Lx = pk->sh_A.as<fe>();           // proof p's L at Lx + p n
-        H2V_TRY(lincomb(pk, hp, cf, off, Lx, n, n));
-        H2V_TRY(sub_low(pk, Lx, n, konst, B));
-        H2V_TRY(sync(pk));
-        fe *W = Q;        // the quotient contributions are no longer needed; proof p's W at W + p n
-        std::vector<KateJob> jobs(B);
-        for (size_t p = 0; p < B; ++p) {
-            jobs[p] = KateJob{Lx + p * n, W + p * n, n, {}};
-            memcpy(jobs[p].b, u64(P[p]->uc), sizeof jobs[p].b);
-        }
-        H2V_TRY(kate_division_batch_dev(jobs.data(), B));
-        for (size_t p = 0; p < B; ++p) H2V_CU(cudaMemsetAsync(W + p * n + (n - 1), 0, sizeof(fe), st));
-        H2V_TRY(put(pk, pk->scal, z0inv));
-        scale_cols_kernel<<<dim3(gn, (unsigned)B), 256, 0, st>>>(W, (uint32_t)n, pk->scal.as<fe>());
-        H2V_LAUNCHED();
-        H2V_TRY(sync(pk));
-        H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, W, B, pts));
-        for (size_t p = 0; p < B; ++p) {
-            if (int rc = write_points(P[p]->T, pts.data() + p, 1)) {
-                bad = p;
-                return rc;
-            }
-        }
-    }
-    lap();   // phase 6: multi-open argument
+    H2V_TRY(kate_division_batch_dev(jobs.data(), B));
+    for (size_t p = 0; p < B; ++p) H2V_CU(cudaMemsetAsync(W + p * n + (n - 1), 0, sizeof(fe), pk->st));
+    H2V_TRY(put(pk, pk->scal, z0inv));
+    scale_cols_kernel<<<dim3(g.gn, (unsigned)B), 256, 0, pk->st>>>(W, (uint32_t)n, pk->scal.as<fe>());
+    H2V_LAUNCHED();
+    H2V_TRY(sync(pk));
+    H2V_TRY(commit_dev(pk, H2V_BASIS_MONOMIAL, W, B, g.pts));
+    return write_commitments(g, g.pts, 1, false);
+}
+
+// The prover: a group of B proofs phase by phase, each phase ended by lap() (h2v_pk_last_phase_ms).  The caller holds
+// pk->mu and has checked the inputs; on a failure traced to one proof, `bad` is that proof (else it stays SIZE_MAX).
+int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector<uint8_t>> &proofs, size_t &bad) {
+    Group g(pk, B, in, bad);
+    H2V_TRY(instances_and_advice(g));
+    g.lap();   // phase 0: upload + advice commitments
+    H2V_TRY(permuted_lookups(g));
+    g.lap();   // phase 1: lookup permutations
+    H2V_TRY(permutation_products(g));
+    H2V_TRY(lookup_products(g));
+    g.lap();   // phase 2: grand products
+    H2V_TRY(random_polynomial(g));
+    H2V_TRY(transform_columns(g));
+    for (auto &s : g.P) s->y = s->T.squeeze_challenge();
+    g.lap();   // phase 3: random poly + transforms
+    H2V_TRY(evaluate_h(g));
+    H2V_TRY(commit_quotient(g));
+    g.lap();   // phase 4: evaluate_h + quotient commitments
+    Evaluations ev;
+    H2V_TRY(evaluations(g, ev));
+    g.lap();   // phase 5: evaluations
+    std::vector<MultiOpen> mo(B);
+    H2V_TRY(par_proofs(B, [&](size_t p) -> int {
+        mo[p] = multi_open_sets(g, ev, p);
+        return H2V_OK;
+    }));
+    H2V_TRY(shplonk(g, mo));
+    g.lap();   // phase 6: multi-open argument
     proofs.resize(B);
-    for (size_t p = 0; p < B; ++p) proofs[p].swap(P[p]->T.out);
+    for (size_t p = 0; p < B; ++p) proofs[p].swap(g.P[p]->T.out);
     return H2V_OK;
 }
 
 // ---------------------------------------------------------------- groups
-// The per-proof workspace; a group of B proofs holds B times the buffers of one.
-DevBuf *workspace(h2v_pk *pk, size_t i) {
-    DevBuf *all[] = {&pk->adv_L, &pk->adv_C, &pk->adv_E, &pk->inst_L, &pk->inst_C, &pk->inst_E, &pk->pa_L, &pk->ps_L, &pk->pa_C, &pk->ps_C,
-                     &pk->pa_E, &pk->ps_E, &pk->z_L, &pk->z_C, &pk->z_E, &pk->zl_L, &pk->zl_C, &pk->zl_E, &pk->num, &pk->den,
-                     &pk->tails, &pk->ptrs, &pk->scal, &pk->offs, &pk->streams, &pk->pts, &pk->rnd_C, &pk->hq, &pk->hx_pieces,
-                     &pk->evals, &pk->pairs, &pk->sh_S, &pk->sh_A, &pk->sh_B, &pk->sh_T, &pk->sh_h, &pk->commits};
-    return i < sizeof all / sizeof all[0] ? all[i] : nullptr;
-}
 // device bytes one proof of a group adds (the rotation sets of the multi-open argument are counted as 8)
 size_t proof_bytes(const h2v_pk *pk) {
     const size_t n = pk->n, ne = pk->ne, L = pk->lookup_input.size(), NS = pk->n_sets;
@@ -1478,6 +1494,8 @@ int check_inputs(const h2v_pk *pk, const ProofIn &in, const std::string &who) {
 // n_proofs proofs in groups; emit(i, bytes) receives proof i.  A group that runs out of device memory is halved and run
 // again (a group of one needs what one proof always needed).  `batch`: prefix error texts with the proof they concern.
 template <class Emit> int run_proofs(h2v_pk *pk, size_t n_proofs, const ProofIn *in, bool batch, Emit emit) {
+    H2V_TRY(set_device(pk->dev, batch ? "create_proofs" : "create_proof"));
+    std::lock_guard<std::mutex> lk(pk->mu);
     for (double &v : pk->last_ms) v = 0;
     size_t G = group_size(pk, n_proofs);
     for (size_t p0 = 0; p0 < n_proofs;) {
@@ -1524,11 +1542,6 @@ int h2v_create_proof(h2v_pk_t pk, const uint64_t *const *advice, const uint64_t 
     if (!pk || !rng_seed || !proof_len) return failf(H2V_EINVAL, "create_proof: NULL argument");
     const ProofIn in{advice, instances, instance_len, rng_seed};
     H2V_TRY(check_inputs(pk, in, "create_proof"));
-    if (cudaSetDevice(pk->dev) != cudaSuccess) {
-        cudaGetLastError();
-        return failf(H2V_ECUDA, "create_proof: no CUDA device (libh2v has no CPU fallback)");
-    }
-    std::lock_guard<std::mutex> lk(pk->mu);
     return run_proofs(pk, 1, &in, false, [&](size_t, const std::vector<uint8_t> &proof) -> int {
         *proof_len = proof.size();
         if (proof.size() > proof_cap || !proof_out)
@@ -1553,11 +1566,6 @@ int h2v_create_proofs(h2v_pk_t pk, size_t n_proofs, const uint64_t *const *const
         snprintf(who, sizeof who, "create_proofs: proof %zu", p);
         H2V_TRY(check_inputs(pk, in[p], who));
     }
-    if (cudaSetDevice(pk->dev) != cudaSuccess) {
-        cudaGetLastError();
-        return failf(H2V_ECUDA, "create_proofs: no CUDA device (libh2v has no CPU fallback)");
-    }
-    std::lock_guard<std::mutex> lk(pk->mu);
     return run_proofs(pk, n_proofs, in.data(), true, [&](size_t p, const std::vector<uint8_t> &proof) -> int {
         if (proof.size() != size) return failf(H2V_EINVAL, "create_proofs: proof %zu has %zu bytes, expected %zu", p, proof.size(), size);
         memcpy(proofs_out + p * proof_stride, proof.data(), size);
