@@ -115,6 +115,8 @@ extern "C" {
     pub fn h2v_mock_prover(cs: *const H2vCircuit, fixed: *const *const u64, sigma: *const *const u64, advice: *const *const u64,
                            instances: *const *const u64, instance_len: *const u32, failures_out: *mut H2vMockFailure, cap: usize,
                            n_failures: *mut u64) -> c_int;
+    pub fn h2v_pk_mock_prover(pk: *mut H2vPk, n_witnesses: usize, advice: *const *const *const u64, instances: *const *const *const u64,
+                              instance_len: *const *const u32, failures_out: *mut H2vMockFailure, cap: usize, n_failures: *mut u64) -> c_int;
     pub fn h2v_quotient_gates_dev(dom: *mut H2vDomain, d_h: *mut c_void, y: *const u64, n_gates: usize, d_q: *const c_void,
                                   q_stride: usize, d_a: *const c_void, a_stride: usize) -> c_int;
     pub fn h2v_quotient_permutation_dev(dom: *mut H2vDomain, d_h: *mut c_void, y: *const u64, beta: *const u64, gamma: *const u64,
@@ -366,6 +368,25 @@ impl DeviceProvingKey {
             ok(unsafe { h2v_create_proofs(self.0, b, ap.as_ptr(), ip.as_ptr(), lp.as_ptr(), seeds.as_ptr(), out.as_mut_ptr(), size) });
         }
         out.chunks(size.max(1)).take(b).map(|c| c.to_vec()).collect()
+    }
+    /// result w = `mock_prover(cs, fixed, sigma, advice[w], instances[w], max_failures)` with this key's circuit and
+    /// columns; one device call for the batch, the key-only work done once per key
+    pub fn mock_prover(&self, n: usize, advice: &[&[&[Fr]]], instances: &[&[&[Fr]]], max_failures: usize) -> Vec<(Vec<H2vMockFailure>, u64)> {
+        let b = advice.len();
+        assert!(instances.len() == b);
+        assert!(advice.iter().all(|a| a.iter().all(|c| c.len() == n)));
+        let a: Vec<Vec<*const u64>> = advice.iter().map(|a| a.iter().map(|c| c.as_ptr() as *const u64).collect()).collect();
+        let i: Vec<Vec<*const u64>> = instances.iter().map(|a| a.iter().map(|c| c.as_ptr() as *const u64).collect()).collect();
+        let il: Vec<Vec<u32>> = instances.iter().map(|a| a.iter().map(|c| c.len() as u32).collect()).collect();
+        let ap: Vec<*const *const u64> = a.iter().map(|v| v.as_ptr()).collect();
+        let ip: Vec<*const *const u64> = i.iter().map(|v| v.as_ptr()).collect();
+        let lp: Vec<*const u32> = il.iter().map(|v| v.as_ptr()).collect();
+        let mut out = vec![H2vMockFailure::default(); b * max_failures];
+        let mut totals = vec![0u64; b];
+        if b > 0 {
+            ok(unsafe { h2v_pk_mock_prover(self.0, b, ap.as_ptr(), ip.as_ptr(), lp.as_ptr(), out.as_mut_ptr(), max_failures, totals.as_mut_ptr()) });
+        }
+        (0..b).map(|w| (out[w * max_failures..w * max_failures + (totals[w] as usize).min(max_failures)].to_vec(), totals[w])).collect()
     }
 }
 impl Drop for DeviceProvingKey {

@@ -38,7 +38,7 @@ ABI_SYMBOLS = [
     "h2v_domain_rotate_omega", "h2v_domain_rotate_extended", "h2v_domain_l_i_range", "h2v_domain_fill", "h2v_kate_division_dev",
     "h2v_quotient_gates_ptrs_dev", "h2v_quotient_permutation_ptrs_dev", "h2v_quotient_permutation_range_ptrs_dev", "h2v_commit_batch_resident",
     "h2v_pk_load", "h2v_pk_free", "h2v_create_proof", "h2v_create_proofs", "h2v_proof_size", "h2v_pk_last_phase_ms",
-    "h2v_mock_prover", "h2v_mock_last_ms",
+    "h2v_mock_prover", "h2v_pk_mock_prover", "h2v_mock_last_ms",
     "h2v_transcript_new", "h2v_transcript_free", "h2v_transcript_common_point", "h2v_transcript_common_scalar",
     "h2v_transcript_write_point", "h2v_transcript_write_scalar", "h2v_transcript_squeeze_challenge", "h2v_transcript_bytes",
     "h2v_poseidon_permutation", "h2v_poseidon_permutation_variant", "h2v_chacha20_fr_random", "h2v_chacha20_block",
@@ -155,6 +155,7 @@ def lib():
         L.h2v_proof_size.restype = C.c_size_t
         L.h2v_pk_last_phase_ms.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
         L.h2v_mock_prover.argtypes = [C.c_void_p] * 7 + [C.c_size_t, C.POINTER(C.c_uint64)]
+        L.h2v_pk_mock_prover.argtypes = [C.c_void_p, C.c_size_t] + [C.c_void_p] * 4 + [C.c_size_t, C.c_void_p]
         L.h2v_mock_last_ms.argtypes = [C.POINTER(C.c_double)]
         L.h2v_transcript_new.argtypes = [C.POINTER(C.c_void_p)]
         L.h2v_transcript_free.argtypes = [C.c_void_p]
@@ -916,6 +917,42 @@ class ProvingKey:
         arr = lambda xs: (C.c_void_p * B)(*xs)
         _check(lib().h2v_create_proofs(self._h, B, arr(adv_ptrs), arr(inst_ptrs), arr(len_ptrs), seeds, _ptr(out), size))
         return [bytes(out[p * size:(p + 1) * size]) for p in range(B)]
+
+    def mock_prover(self, advice_list, instances_list, max_failures=64):
+        """MockProver.run on this key's circuit for every witness of a batch, in one call (h2v_pk_mock_prover): result w
+        equals MockProver.run(cs, fixed, sigma, advice_list[w], instances_list[w], max_failures) with the key's cs, fixed
+        and sigma.  Only the witnesses are uploaded; the key-only work is done by the first call -> list of MockProver"""
+        B = len(advice_list)
+        if len(instances_list) != B:
+            raise ValueError("mock_prover: advice_list and instances_list differ in length")
+        if not B:
+            return []
+        n = 1 << self.cs["k"]
+        keep, adv_ptrs, inst_ptrs, len_ptrs = [], [], [], []
+        for w, (advice, instances) in enumerate(zip(advice_list, instances_list)):
+            adv = [_fr(c, n) for c in advice]
+            if len(adv) != self.cs["n_advice"] or len(instances) != self.cs["n_instance"]:
+                raise ValueError(f"mock_prover: witness {w}: advice / instance column count does not match the constraint system")
+            inst = [_fr(np.asarray(c, dtype=np.uint64).reshape(-1, 4)) for c in instances]
+            aa = (C.c_void_p * max(1, len(adv)))(*[c.ctypes.data for c in adv])
+            ia = (C.c_void_p * max(1, len(inst)))(*[c.ctypes.data for c in inst])
+            il = np.ascontiguousarray([c.shape[0] for c in inst] or [0], dtype=np.uint32)
+            keep += [adv, inst, aa, ia, il]
+            adv_ptrs.append(C.cast(aa, C.c_void_p))
+            inst_ptrs.append(C.cast(ia, C.c_void_p))
+            len_ptrs.append(il.ctypes.data)
+        out = (_MockFailureT * max(1, B * max_failures))()
+        totals = np.zeros(B, dtype=np.uint64)
+        arr = lambda xs: (C.c_void_p * B)(*xs)
+        _check(lib().h2v_pk_mock_prover(self._h, B, arr(adv_ptrs), arr(inst_ptrs), arr(len_ptrs), out, max_failures, _ptr(totals)))
+        ms = (C.c_double * 2)()
+        _check(lib().h2v_mock_last_ms(ms))
+        res = []
+        for w in range(B):
+            got = min(max_failures, int(totals[w]))
+            fails = [MockFailure(*(getattr(out[w * max_failures + i], f) for f in MockFailure._fields)) for i in range(got)]
+            res.append(MockProver(fails, int(totals[w]), ms[0], ms[1]))
+        return res
 
     def last_phase_ms(self):
         buf = (C.c_double * 8)()

@@ -91,6 +91,26 @@ struct fe;
 int sort_canonical_dev(cudaStream_t st, const fe *const *d_srcs, uint32_t slices, uint32_t u, uint32_t n_pad, fe *keys);
 // offs = exclusive prefix sums of cnt[0 .. len), *total = their sum (device); tiles: ceil(len / 2048) words, scratch: len words
 int scan_u32_dev(cudaStream_t st, const uint32_t *cnt, uint32_t len, uint32_t *offs, uint32_t *tiles, uint32_t *scratch, uint32_t *total);
+
+// The mock prover's checks (mock.cu).  MockKey: what they need from the key alone (each permutation cell's image, the
+// permutation's key-only flags, the sorted lookup tables), built once per key from its fixed and sigma columns on the
+// device (Lagrange form, n rows each, contiguous).  The fixed columns must stay in place while the MockKey is used.
+struct MockKey;
+int mock_key_build(cudaStream_t st, const h2v_circuit_t *cs, const fe *fixed, const fe *sigma, MockKey **out);   // synchronous
+void mock_key_free(MockKey *key);
+size_t mock_witness_bytes(const MockKey &key);     // device bytes one witness of a check needs
+size_t mock_max_batch(const MockKey &key);         // the most witnesses one mock_check takes
+// B witnesses: witness w's advice columns are uploaded to adv + w A n and its instance columns, zero-padded, to inst + w I n
+// (prove_group's layout; adv and inst grow to fit), then checked: failures_out + w cap and n_failures[w] as h2v_mock_prover
+// writes them.  ms[0] += the upload, ms[1] += the checks.  Synchronous.
+int mock_check(cudaStream_t st, const MockKey &key, size_t B, const uint64_t *const *const *advice, const uint64_t *const *const *instances,
+               const uint32_t *const *instance_len, DevBuf &adv, DevBuf &inst, h2v_mock_failure_t *failures_out, size_t cap,
+               uint64_t *n_failures, double ms[2]);
+void mock_set_last_ms(const double ms[2]);         // h2v_mock_last_ms
+// the argument checks of h2v_mock_prover and h2v_pk_mock_prover; errors start with `who`
+int mock_check_advice(const h2v_circuit_t *cs, const uint64_t *const *advice, const char *who);
+int mock_check_instances(const h2v_circuit_t *cs, const uint64_t *const *instances, const uint32_t *instance_len, const char *who);
+int mock_check_limits(const h2v_circuit_t *cs, const char *who);
 }  // namespace h2v
 
 #define H2V_CU(x)                                                                                                  \

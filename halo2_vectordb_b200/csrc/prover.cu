@@ -290,6 +290,7 @@ struct h2v_pk {
     DevBuf ext_cache;
     size_t cached_sigma = 0;
     bool cache_tried = false;
+    h2v::MockKey *mock = nullptr;   // the mock prover's key tables, built by the first h2v_pk_mock_prover call
     cudaStream_t st = nullptr;
     int dev = 0;                 // the proof runs on the primary device (columns and key resident there)
     std::mutex mu;
@@ -375,6 +376,7 @@ void h2v_pk_free(h2v_pk_t pk) {
     for (DevBuf *b : {&pk->fixed_L, &pk->fixed_C, &pk->fixed_E, &pk->sigma_L, &pk->sigma_C, &pk->sigma_E, &pk->lrows_E, &pk->omega_pows, &pk->scr_E,
                       &pk->ext_cache}) b->release();
     for (size_t i = 0; DevBuf *b = workspace(pk, i); ++i) b->release();
+    mock_key_free(pk->mock);
     if (pk->dom) h2v_domain_free(pk->dom);
     if (pk->st) cudaStreamDestroy(pk->st);
     delete pk;
@@ -1455,14 +1457,11 @@ size_t proof_bytes(const h2v_pk *pk) {
     const size_t ncols = 2 * std::max(NS, L) + 1 + (pk->degree - 1) + 2 + 2 * 8 + 1;   // num / den, random, pieces, h, S / Q, L
     return sizeof(fe) * (cols * (2 * n + (pk->stream_ext ? 0 : ne)) + 2 * ne + ncols * n) + 4096;
 }
-// The group size for n_proofs proofs: H2V_PROOF_GROUP if set, else as many as fit in the device memory left after the
-// key, with 8 GB kept free as the extended-sigma cache keeps it; capped so that every grid dimension and batch call
-// stays within its limits.  Streamed keys prove one at a time.
-size_t group_size(h2v_pk *pk, size_t n_proofs) {
-    if (pk->stream_ext || n_proofs <= 1) return 1;
-    const size_t cmax = std::max<size_t>({pk->n_sets, pk->lookup_input.size(), 16});
-    size_t cap = std::min<size_t>(65535 / cmax, (((size_t)1 << 31) - 1) / (pk->n * cmax));
-    cap = std::max<size_t>(1, std::min(cap, n_proofs));
+// The group size for n_items items (proofs, or witnesses to check) of item_bytes device bytes each: H2V_PROOF_GROUP if
+// set, else as many as fit in the device memory left after the key, with 8 GB kept free as the extended-sigma cache
+// keeps it; at most `cap`, the largest group every grid dimension and batch call allows.
+size_t group_size(h2v_pk *pk, size_t n_items, size_t item_bytes, size_t cap) {
+    cap = std::max<size_t>(1, std::min(cap, n_items));
     if (const char *e = getenv("H2V_PROOF_GROUP")) {
         const long g = atol(e);
         if (g > 0) return std::min<size_t>((size_t)g, cap);
@@ -1472,8 +1471,14 @@ size_t group_size(h2v_pk *pk, size_t n_proofs) {
     size_t held = 0;
     for (size_t i = 0; DevBuf *b = workspace(pk, i); ++i) held += b->cap;
     const size_t margin = (size_t)8 << 30, avail = free_b + held;
-    const size_t fit = avail > margin ? (avail - margin) / proof_bytes(pk) : 1;
+    const size_t fit = avail > margin ? (avail - margin) / item_bytes : 1;
     return std::max<size_t>(1, std::min(fit, cap));
+}
+// ... for n_proofs proofs.  Streamed keys prove one at a time.
+size_t proof_group_size(h2v_pk *pk, size_t n_proofs) {
+    if (pk->stream_ext || n_proofs <= 1) return 1;
+    const size_t cmax = std::max<size_t>({pk->n_sets, pk->lookup_input.size(), 16});
+    return group_size(pk, n_proofs, proof_bytes(pk), std::min<size_t>(65535 / cmax, (((size_t)1 << 31) - 1) / (pk->n * cmax)));
 }
 
 // Inputs of proof `idx` (who: the prefix of the error text)
@@ -1491,26 +1496,29 @@ int check_inputs(const h2v_pk *pk, const ProofIn &in, const std::string &who) {
     return H2V_OK;
 }
 
+// The key's opportunistic cache of extended sigma columns (streamed mode) took memory something else now needs: give it
+// back for good, if it holds any, so that the caller runs its step again
+bool release_sigma_cache(h2v_pk *pk) {
+    if (!pk->cached_sigma) return false;
+    cudaStreamSynchronize(pk->st);
+    pk->ext_cache.release();
+    pk->cached_sigma = 0;
+    return true;
+}
+
 // n_proofs proofs in groups; emit(i, bytes) receives proof i.  A group that runs out of device memory is halved and run
 // again (a group of one needs what one proof always needed).  `batch`: prefix error texts with the proof they concern.
 template <class Emit> int run_proofs(h2v_pk *pk, size_t n_proofs, const ProofIn *in, bool batch, Emit emit) {
     H2V_TRY(set_device(pk->dev, batch ? "create_proofs" : "create_proof"));
     std::lock_guard<std::mutex> lk(pk->mu);
     for (double &v : pk->last_ms) v = 0;
-    size_t G = group_size(pk, n_proofs);
+    size_t G = proof_group_size(pk, n_proofs);
     for (size_t p0 = 0; p0 < n_proofs;) {
         const size_t b = std::min(G, n_proofs - p0);
         std::vector<std::vector<uint8_t>> out;
         size_t bad = SIZE_MAX;
         int rc = prove_group(pk, b, in + p0, out, bad);
-        if (rc == H2V_ENOMEM && pk->cached_sigma) {
-            // the key's opportunistic cache of extended sigma columns (streamed mode) took memory something else now needs:
-            // give it back for good and run the group again
-            cudaStreamSynchronize(pk->st);
-            pk->ext_cache.release();
-            pk->cached_sigma = 0;
-            continue;
-        }
+        if (rc == H2V_ENOMEM && release_sigma_cache(pk)) continue;
         if (rc == H2V_ENOMEM && b > 1) {
             cudaStreamSynchronize(pk->st);
             for (size_t i = 0; DevBuf *w = workspace(pk, i); ++i) w->release();
@@ -1531,6 +1539,33 @@ template <class Emit> int run_proofs(h2v_pk *pk, size_t n_proofs, const ProofIn 
         p0 += b;
     }
     return H2V_OK;
+}
+
+// the key's constraint system, as h2v_pk_load received it
+h2v_circuit_t circuit_of(const h2v_pk *pk) {
+    h2v_circuit_t cs{};
+    cs.k = pk->k;
+    cs.degree = pk->degree;
+    cs.blinding_factors = pk->bf;
+    cs.n_advice = pk->n_advice;
+    cs.n_fixed = pk->n_fixed;
+    cs.n_instance = pk->n_instance;
+    cs.n_gates = (uint32_t)pk->gate_advice.size();
+    cs.gate_advice = pk->gate_advice.data();
+    cs.gate_selector = pk->gate_selector.data();
+    cs.n_lookups = (uint32_t)pk->lookup_input.size();
+    cs.lookup_input = pk->lookup_input.data();
+    cs.lookup_table = pk->lookup_table.data();
+    cs.n_perm = (uint32_t)pk->perm_kind.size();
+    cs.perm_kind = pk->perm_kind.data();
+    cs.perm_index = pk->perm_index.data();
+    cs.n_advice_queries = (uint32_t)pk->aq_col.size();
+    cs.advice_query_col = pk->aq_col.data();
+    cs.advice_query_rot = pk->aq_rot.data();
+    cs.n_fixed_queries = (uint32_t)pk->fq_col.size();
+    cs.fixed_query_col = pk->fq_col.data();
+    cs.fixed_query_rot = pk->fq_rot.data();
+    return cs;
 }
 
 }  // namespace
@@ -1571,6 +1606,59 @@ int h2v_create_proofs(h2v_pk_t pk, size_t n_proofs, const uint64_t *const *const
         memcpy(proofs_out + p * proof_stride, proof.data(), size);
         return H2V_OK;
     });
+}
+int h2v_pk_mock_prover(h2v_pk_t pk, size_t n_witnesses, const uint64_t *const *const *advice, const uint64_t *const *const *instances,
+                       const uint32_t *const *instance_len, h2v_mock_failure_t *failures_out, size_t cap, uint64_t *n_failures) {
+    if (!pk) return failf(H2V_EINVAL, "pk_mock_prover: NULL key");
+    if (!n_witnesses) return H2V_OK;
+    if (!n_failures || (cap && !failures_out) || (pk->n_advice && !advice) || (pk->n_instance && (!instances || !instance_len)))
+        return failf(H2V_EINVAL, "pk_mock_prover: NULL argument");
+    const h2v_circuit_t cs = circuit_of(pk);
+    for (size_t w = 0; w < n_witnesses; ++w) {
+        char who[64];
+        snprintf(who, sizeof who, "pk_mock_prover: witness %zu", w);
+        if ((pk->n_advice && !advice[w]) || (pk->n_instance && (!instances[w] || !instance_len[w])))
+            return failf(H2V_EINVAL, "%s: NULL column list", who);
+        if (pk->n_advice) H2V_TRY(mock_check_advice(&cs, advice[w], who));
+        if (pk->n_instance) H2V_TRY(mock_check_instances(&cs, instances[w], instance_len[w], who));
+    }
+    H2V_TRY(mock_check_limits(&cs, "pk_mock_prover"));
+    H2V_TRY(set_device(pk->dev, "pk_mock_prover"));
+    std::lock_guard<std::mutex> lk(pk->mu);
+    double ms[2] = {0, 0};
+    while (!pk->mock) {      // the key tables, on the first call
+        const double t = now_ms();
+        const int rc = mock_key_build(pk->st, &cs, pk->fixed_L.as<fe>(), pk->sigma_L.as<fe>(), &pk->mock);
+        ms[1] += now_ms() - t;
+        if (rc == H2V_ENOMEM && release_sigma_cache(pk)) continue;
+        if (rc) {
+            cudaStreamSynchronize(pk->st);
+            return rc;
+        }
+    }
+    // the witnesses in groups, as run_proofs runs proofs; they are staged in the key's adv_L / inst_L workspace
+    size_t G = group_size(pk, n_witnesses, mock_witness_bytes(*pk->mock), mock_max_batch(*pk->mock));
+    for (size_t w0 = 0; w0 < n_witnesses;) {
+        const size_t b = std::min(G, n_witnesses - w0);
+        const int rc = mock_check(pk->st, *pk->mock, b, advice ? advice + w0 : nullptr, instances ? instances + w0 : nullptr,
+                                  instance_len ? instance_len + w0 : nullptr, pk->adv_L, pk->inst_L, cap ? failures_out + w0 * cap : nullptr,
+                                  cap, n_failures + w0, ms);
+        if (rc == H2V_ENOMEM && release_sigma_cache(pk)) continue;
+        if (rc == H2V_ENOMEM && b > 1) {
+            cudaStreamSynchronize(pk->st);
+            for (size_t i = 0; DevBuf *w = workspace(pk, i); ++i) w->release();
+            G = b / 2;
+            continue;
+        }
+        if (rc) {
+            cudaStreamSynchronize(pk->st);
+            const std::string msg = h2v_last_error();
+            return failf(rc, "pk_mock_prover: witnesses %zu .. %zu: %s", w0, w0 + b - 1, msg.c_str());
+        }
+        w0 += b;
+    }
+    mock_set_last_ms(ms);
+    return H2V_OK;
 }
 size_t h2v_proof_size(h2v_pk_t pk) {
     if (!pk) return 0;

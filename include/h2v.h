@@ -304,9 +304,10 @@ int h2v_pk_last_phase_ms(h2v_pk_t pk, double out[8]);
  * COPY_UNUSABLE, COPY.  *n_failures = the exact total.  The same inputs always give the same output.
  * Every argument is checked before any device work (H2V_EINVAL: NULL pointers, the column indices of cs as h2v_pk_load
  * checks them, instance_len[c] > 2^k, more than 65535 gates / lookups / permutation columns, more than 2^32 flags).
- * Device memory: the columns (32 bytes per cell of every advice, fixed, sigma and instance column), 4 bytes per
- * permutation cell, one bit per gate row, lookup row and 4 per permutation cell, and the table of the 2^k values w^r
- * (40 bytes per row): about 29.8 GB for the SIFT-shaped k = 20 circuit (28.3 GB of columns, 290 permutation columns). */
+ * Device memory: the columns (32 bytes per cell of every advice, fixed, sigma and instance column), 8 bytes per
+ * permutation cell, one bit per gate row, lookup row and 8 per permutation cell, the table of the 2^k values w^r (40 bytes
+ * per row) and the sorted lookup tables (32 bytes per row and distinct table): about 31 GB for the SIFT-shaped k = 20
+ * circuit (28.3 GB of columns, 290 permutation columns). */
 typedef struct {
     uint32_t kind, column, row, other_column, other_row;
 } h2v_mock_failure_t;
@@ -317,8 +318,22 @@ enum {
 int h2v_mock_prover(const h2v_circuit_t *cs, const uint64_t *const *fixed, const uint64_t *const *sigma, const uint64_t *const *advice,
                     const uint64_t *const *instances, const uint32_t *instance_len, h2v_mock_failure_t *failures_out, size_t cap,
                     uint64_t *n_failures);
-/* wall-clock milliseconds of the calling thread's last h2v_mock_prover call: out[0] the upload of the columns, out[1] the
- * checks (every kernel, the compaction and the download of the failures) */
+/* The mock prover on a loaded key, for n_witnesses witnesses in one call: with cs, fixed and sigma what h2v_pk_load
+ * received, failures_out + w * cap receives what h2v_mock_prover(cs, fixed, sigma, advice[w], instances[w],
+ * instance_len[w], ., cap, .) writes, and n_failures[w] that call's exact total (same order, same fields, same cap).
+ * Only the witnesses are uploaded, into the key's proof workspace.  What depends on the key alone (each sigma cell
+ * decoded into its image, the permutation's key-only failures, the sorted lookup tables: about 4.5 bytes per permutation
+ * cell and 32 bytes per row and distinct table) is built by the first call and kept with the key until h2v_pk_free.
+ * The witnesses run in groups, as h2v_create_proofs runs proofs (H2V_PROOF_GROUP if set, else as many as fit with 8 GB
+ * kept free; a group that runs out of memory is halved).  Every argument is checked before any device work, as
+ * h2v_mock_prover checks it; an error text names the witness it concerns ("pk_mock_prover: witness 2: ...") and the key
+ * stays usable.  The call writes none of the key's columns: proofs made after it are unchanged.  n_witnesses = 0 does
+ * nothing.  Calls on one key serialise with its proofs. */
+int h2v_pk_mock_prover(h2v_pk_t pk, size_t n_witnesses, const uint64_t *const *const *advice, const uint64_t *const *const *instances,
+                       const uint32_t *const *instance_len, h2v_mock_failure_t *failures_out, size_t cap, uint64_t *n_failures);
+/* wall-clock milliseconds of the calling thread's last h2v_mock_prover or h2v_pk_mock_prover call: out[0] the upload of
+ * the columns (h2v_pk_mock_prover: the witnesses' columns), out[1] the checks (building the key tables -- for
+ * h2v_pk_mock_prover on the key's first call only --, every kernel, the compaction and the download of the failures) */
 int h2v_mock_last_ms(double out[2]);
 
 /* ---- circuit builder ("next": SURVEY.md 8(f) row 4; host-side, no device needed) -----------------------------------

@@ -236,6 +236,42 @@ class PoseidonTranscript {
     h2v_transcript_t h_ = nullptr;
 };
 
+// halo2 MockProver::run(k, circuit, instances) on the device (h2v_mock_prover): the first max_failures failures in the order
+// gates, lookups, permutation, and how many there are in all
+struct MockProver {
+    std::vector<h2v_mock_failure_t> failures;
+    uint64_t n_failures = 0;
+
+    static MockProver run(const h2v_circuit_t &cs, const std::vector<const Fr *> &fixed, const std::vector<const Fr *> &sigma,
+                          const std::vector<const Fr *> &advice, const std::vector<std::vector<Fr>> &instances, size_t max_failures = 64) {
+        if (fixed.size() != cs.n_fixed || sigma.size() != cs.n_perm || advice.size() != cs.n_advice || instances.size() != cs.n_instance)
+            throw std::invalid_argument("MockProver: column count does not match the constraint system");
+        std::vector<const uint64_t *> ip;
+        std::vector<uint32_t> il;
+        for (const auto &c : instances) {
+            ip.push_back(reinterpret_cast<const uint64_t *>(c.data()));
+            il.push_back((uint32_t)c.size());
+        }
+        MockProver m;
+        m.failures.resize(max_failures);
+        check(h2v_mock_prover(&cs, reinterpret_cast<const uint64_t *const *>(fixed.data()), reinterpret_cast<const uint64_t *const *>(sigma.data()),
+                              reinterpret_cast<const uint64_t *const *>(advice.data()), ip.data(), il.data(), m.failures.data(), max_failures,
+                              &m.n_failures));
+        m.failures.resize((size_t)std::min<uint64_t>(max_failures, m.n_failures));
+        return m;
+    }
+    // MockProver::assert_satisfied: throws std::logic_error naming the first failures
+    void assert_satisfied() const {
+        if (!n_failures) return;
+        static const char *kinds[] = {"?", "gate", "gate_unusable", "lookup", "sigma_not_delta_omega", "sigma_not_permutation", "copy_unusable", "copy"};
+        std::string msg = std::to_string(n_failures) + " constraint(s) not satisfied";
+        for (const auto &f : failures)
+            msg += "\n  " + std::string(kinds[f.kind < 8 ? f.kind : 0]) + ": column " + std::to_string(f.column) + " row " + std::to_string(f.row) +
+                   " (other: column " + std::to_string(f.other_column) + " row " + std::to_string(f.other_row) + ")";
+        throw std::logic_error(msg);
+    }
+};
+
 // halo2 ProvingKey for a halo2-base-shaped constraint system + create_proof (plonk/prover.rs), resident on the device
 class ProvingKey {
   public:
@@ -291,45 +327,38 @@ class ProvingKey {
         for (size_t p = 0; p < B; ++p) out[p].assign(flat.begin() + p * size, flat.begin() + (p + 1) * size);
         return out;
     }
+    // MockProver::run on this key's circuit for each witness: result w = MockProver::run(cs, fixed, sigma, advice[w],
+    // instances[w], max_failures) with the key's cs, fixed and sigma; one call for the whole batch (h2v_pk_mock_prover)
+    std::vector<MockProver> mock_prover(const std::vector<std::vector<const Fr *>> &advice, const std::vector<std::vector<std::vector<Fr>>> &instances,
+                                        size_t max_failures = 64) const {
+        const size_t B = advice.size();
+        if (instances.size() != B) throw std::invalid_argument("mock_prover: list lengths differ");
+        std::vector<std::vector<const uint64_t *>> ip(B);
+        std::vector<std::vector<uint32_t>> il(B);
+        std::vector<const uint64_t *const *> ap(B), ipp(B);
+        std::vector<const uint32_t *> ilp(B);
+        for (size_t w = 0; w < B; ++w) {
+            for (const auto &c : instances[w]) {
+                ip[w].push_back(reinterpret_cast<const uint64_t *>(c.data()));
+                il[w].push_back((uint32_t)c.size());
+            }
+            ap[w] = reinterpret_cast<const uint64_t *const *>(advice[w].data());
+            ipp[w] = ip[w].data();
+            ilp[w] = il[w].data();
+        }
+        std::vector<h2v_mock_failure_t> flat(B * max_failures);
+        std::vector<uint64_t> totals(B);
+        check(h2v_pk_mock_prover(h_, B, ap.data(), ipp.data(), ilp.data(), flat.data(), max_failures, totals.data()));
+        std::vector<MockProver> out(B);
+        for (size_t w = 0; w < B; ++w) {
+            out[w].n_failures = totals[w];
+            out[w].failures.assign(flat.begin() + w * max_failures, flat.begin() + w * max_failures + (size_t)std::min<uint64_t>(max_failures, totals[w]));
+        }
+        return out;
+    }
 
   private:
     h2v_pk_t h_ = nullptr;
-};
-
-// halo2 MockProver::run(k, circuit, instances) on the device (h2v_mock_prover): the first max_failures failures in the order
-// gates, lookups, permutation, and how many there are in all
-struct MockProver {
-    std::vector<h2v_mock_failure_t> failures;
-    uint64_t n_failures = 0;
-
-    static MockProver run(const h2v_circuit_t &cs, const std::vector<const Fr *> &fixed, const std::vector<const Fr *> &sigma,
-                          const std::vector<const Fr *> &advice, const std::vector<std::vector<Fr>> &instances, size_t max_failures = 64) {
-        if (fixed.size() != cs.n_fixed || sigma.size() != cs.n_perm || advice.size() != cs.n_advice || instances.size() != cs.n_instance)
-            throw std::invalid_argument("MockProver: column count does not match the constraint system");
-        std::vector<const uint64_t *> ip;
-        std::vector<uint32_t> il;
-        for (const auto &c : instances) {
-            ip.push_back(reinterpret_cast<const uint64_t *>(c.data()));
-            il.push_back((uint32_t)c.size());
-        }
-        MockProver m;
-        m.failures.resize(max_failures);
-        check(h2v_mock_prover(&cs, reinterpret_cast<const uint64_t *const *>(fixed.data()), reinterpret_cast<const uint64_t *const *>(sigma.data()),
-                              reinterpret_cast<const uint64_t *const *>(advice.data()), ip.data(), il.data(), m.failures.data(), max_failures,
-                              &m.n_failures));
-        m.failures.resize((size_t)std::min<uint64_t>(max_failures, m.n_failures));
-        return m;
-    }
-    // MockProver::assert_satisfied: throws std::logic_error naming the first failures
-    void assert_satisfied() const {
-        if (!n_failures) return;
-        static const char *kinds[] = {"?", "gate", "gate_unusable", "lookup", "sigma_not_delta_omega", "sigma_not_permutation", "copy_unusable", "copy"};
-        std::string msg = std::to_string(n_failures) + " constraint(s) not satisfied";
-        for (const auto &f : failures)
-            msg += "\n  " + std::string(kinds[f.kind < 8 ? f.kind : 0]) + ": column " + std::to_string(f.column) + " row " + std::to_string(f.row) +
-                   " (other: column " + std::to_string(f.other_column) + " row " + std::to_string(f.other_row) + ")";
-        throw std::logic_error(msg);
-    }
 };
 
 }  // namespace h2v_host

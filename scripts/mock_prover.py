@@ -1,12 +1,15 @@
-"""Wall-clock time of h2v_mock_prover (MockProver::run on the device) on the three reference examples (distances and query
-at k = 13, kmeans at k = 16) and, with --sift, on the SIFT-shaped k = 20 circuit of scripts/sift_k20_proof.py.
+"""Wall-clock time of h2v_mock_prover (MockProver::run on the device) and of h2v_pk_mock_prover (the same checks on a loaded
+proving key, for a batch of witnesses) on the three reference examples (distances and query at k = 13, kmeans at k = 16)
+and, with --sift, on the SIFT-shaped k = 20 circuit of scripts/sift_k20_proof.py.
 
-    python scripts/mock_prover.py [--names distances query kmeans] [--reps 3] [--sift] [--out profiles/mock_prover_b200.json]
+    python scripts/mock_prover.py [--names distances query kmeans] [--reps 3] [--sift] [--out profiles/pk_mock_prover_b200.json]
 
 The columns come from the restated builder and layouter (host numpy arrays, pageable).  Each circuit is checked once as a
 warm-up, then `reps` times; the library reports each call's upload of the columns and its checks separately
 (h2v_mock_last_ms).  query runs on data/query.in as it is, whose repeated vectors leave 12 gates unsatisfied, so its
-number includes the compaction of real failures.  Writes one JSON object (also printed) with the GPU's name and power
+number includes the compaction of real failures.  Then the circuit's proving key is loaded and checked with the key path:
+its first call (which builds the key tables), then `reps` later calls with B = 1 and with B = 8 copies of the witness;
+each witness's total must equal h2v_mock_prover's.  Writes one JSON object (also printed) with the GPU's name and power
 limit read in the same run."""
 import argparse
 import json
@@ -15,6 +18,8 @@ import random
 import subprocess
 import sys
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -48,12 +53,41 @@ def measure(h, rc, reps):
             "call_ms": [round(x, 2) for x in walls], "upload_gb_per_s": round(col_bytes / 1e6 / min(ups), 2)}
 
 
+def measure_key(h, rc, reps, n_failures):
+    """h2v_pk_mock_prover on the circuit's proving key: the first call, then later calls at B = 1 and B = 8"""
+    srs = h.ParamsKZG.gen_srs(rc.k)
+    t0 = time.perf_counter()
+    pk = h.ProvingKey(srs, rc.cs, rc.fixed, rc.sigma, np.array([rc.k, 0, 0, 0], dtype=np.uint64))
+    load_ms = (time.perf_counter() - t0) * 1e3
+
+    def call(B):
+        t0 = time.perf_counter()
+        mps = pk.mock_prover([rc.advice] * B, [rc.instances] * B)
+        wall = (time.perf_counter() - t0) * 1e3
+        assert [m.n_failures for m in mps] == [n_failures] * B, [m.n_failures for m in mps]
+        return {"upload_ms": round(mps[0].upload_ms, 2), "check_ms": round(mps[0].check_ms, 2), "call_ms": round(wall, 2)}
+
+    out = {"pk_load_ms": round(load_ms, 1), "first_call_b1": call(1)}
+    for B in (1, 8):
+        runs = [call(B) for _ in range(reps)]
+        out[f"later_b{B}"] = {key: [r[key] for r in runs] for key in runs[0]}
+    pk.close()
+    srs.close()
+    return out
+
+
+def measure_both(h, rc, reps):
+    res = measure(h, rc, reps)
+    res["pk_mock_prover"] = measure_key(h, rc, reps, res["n_failures"])
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--names", nargs="+", default=["distances", "query", "kmeans"])
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--sift", action="store_true", help="also the k = 20 circuit of scripts/sift_k20_proof.py (1024 x 128)")
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "mock_prover_b200.json"))
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "pk_mock_prover_b200.json"))
     args = ap.parse_args()
 
     import halo2_vectordb_b200 as h
@@ -62,11 +96,13 @@ def main():
     if h.device_count() < 1:
         raise SystemExit("mock_prover.py measures on a GPU; none is visible")
     h.init(0)
-    res = {"what": "h2v_mock_prover wall-clock: upload of the columns and the checks, ms per call", **gpu_info(), "circuits": {}}
+    res = {"what": "h2v_mock_prover wall-clock: upload of the columns and the checks, ms per call; pk_mock_prover: the same for "
+                   "h2v_pk_mock_prover on the loaded key (first call with the key tables, later calls at B = 1 and 8 witnesses)",
+           **gpu_info(), "circuits": {}}
     for name in args.names:
         k, bits = Z.EXAMPLE_PARAMS[name]
         rc, _ = Z.create_circuit(Z.EXAMPLES[name], Z.example_input(name), k, bits)
-        res["circuits"][f"{name}_k{k}"] = measure(h, rc, args.reps)
+        res["circuits"][f"{name}_k{k}"] = measure_both(h, rc, args.reps)
         print(f"# {name}: {res['circuits'][f'{name}_k{k}']}", file=sys.stderr, flush=True)
         rc.close()
     if args.sift:
@@ -81,7 +117,7 @@ def main():
         Z.exhaustive_merkle(builder.main(0), inp, public)
         builder.make_public(public)
         rc = Z.RangeCircuit(builder, k)
-        res["circuits"][f"sift_k{k}"] = measure(h, rc, min(args.reps, 2))
+        res["circuits"][f"sift_k{k}"] = measure_both(h, rc, min(args.reps, 2))
         print(f"# sift: {res['circuits'][f'sift_k{k}']}", file=sys.stderr, flush=True)
         rc.close()
         builder.close()
