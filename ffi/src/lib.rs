@@ -19,6 +19,8 @@ pub struct H2vSrs(c_void);
 pub struct H2vDomain(c_void);
 
 #[repr(C)] pub struct H2vPk { _private: [u8; 0] }
+#[repr(C)] pub struct H2vBuilder { _private: [u8; 0] }
+#[repr(C)] pub struct H2vWitnessProgram { _private: [u8; 0] }
 /// `h2v_circuit_t`: the constraint-system description `h2v_pk_load` takes (include/h2v.h)
 #[repr(C)]
 pub struct H2vCircuit {
@@ -117,6 +119,16 @@ extern "C" {
                            n_failures: *mut u64) -> c_int;
     pub fn h2v_pk_mock_prover(pk: *mut H2vPk, n_witnesses: usize, advice: *const *const *const u64, instances: *const *const *const u64,
                               instance_len: *const *const u32, failures_out: *mut H2vMockFailure, cap: usize, n_failures: *mut u64) -> c_int;
+    // witness generation on the device for many inputs of one recorded circuit (halo2-base `witness_gen_only`)
+    pub fn h2v_builder_new_recording(precision_bits: u32, lookup_bits: u32, out: *mut *mut H2vBuilder) -> c_int;
+    pub fn h2v_builder_free(b: *mut H2vBuilder);
+    pub fn h2v_witness_program_new(b: *mut H2vBuilder, k: u32, minimum_rows: u32, out: *mut *mut H2vWitnessProgram) -> c_int;
+    pub fn h2v_witness_program_free(p: *mut H2vWitnessProgram);
+    pub fn h2v_witness_program_info(p: *mut H2vWitnessProgram, out: *mut u64) -> c_int;
+    pub fn h2v_witness_program_inputs(p: *mut H2vWitnessProgram, out: *mut u64) -> c_int;
+    pub fn h2v_witness_generate(p: *mut H2vWitnessProgram, n_witnesses: usize, n_inputs: usize, inputs: *const u64, advice_out: *mut u64,
+                                instances_out: *mut u64) -> c_int;
+    pub fn h2v_witness_last_ms(out: *mut f64) -> c_int;
     pub fn h2v_quotient_gates_dev(dom: *mut H2vDomain, d_h: *mut c_void, y: *const u64, n_gates: usize, d_q: *const c_void,
                                   q_stride: usize, d_a: *const c_void, a_stride: usize) -> c_int;
     pub fn h2v_quotient_permutation_dev(dom: *mut H2vDomain, d_h: *mut c_void, y: *const u64, beta: *const u64, gamma: *const u64,
@@ -318,6 +330,37 @@ impl DeviceDomain {
 }
 impl Drop for DeviceDomain {
     fn drop(&mut self) { unsafe { h2v_domain_free(self.h) } }
+}
+
+/// A circuit recorded by a builder from `h2v_builder_new_recording`, replayed for batches of inputs on the device
+/// (`witness_gen_only` for many inputs): `generate` gives each input's advice columns and instances, byte for byte what
+/// the host builder and layouter give.  Inputs are the values the circuit passed to `assign_witnesses`, in order.
+pub struct WitnessProgram { h: *mut H2vWitnessProgram, info: [u64; 8] }
+unsafe impl Send for WitnessProgram {}
+impl WitnessProgram {
+    /// `recording` may be freed (`h2v_builder_free`) once this returns
+    pub fn new(recording: *mut H2vBuilder, k: u32, minimum_rows: u32) -> Self {
+        let mut h = std::ptr::null_mut();
+        ok(unsafe { h2v_witness_program_new(recording, k, minimum_rows, &mut h) });
+        let mut info = [0u64; 8];
+        ok(unsafe { h2v_witness_program_info(h, info.as_mut_ptr()) });
+        WitnessProgram { h, info }
+    }
+    pub fn n_inputs(&self) -> usize { self.info[0] as usize }
+    /// inputs: one slice of n_inputs values per witness -> (advice columns, instances) per witness
+    pub fn generate(&self, inputs: &[&[Fr]]) -> Vec<(Vec<Vec<Fr>>, Vec<Fr>)> {
+        let (b, ni, na, nin, n) = (inputs.len(), self.n_inputs(), self.info[4] as usize, self.info[5] as usize, 1usize << self.info[6]);
+        assert!(inputs.iter().all(|x| x.len() == ni));
+        let flat: Vec<Fr> = inputs.iter().flat_map(|x| x.iter().copied()).collect();
+        let mut adv = vec![Fr::zero(); b * na * n];
+        let mut inst = vec![Fr::zero(); b * nin];
+        ok(unsafe { h2v_witness_generate(self.h, b, ni, flat.as_ptr() as *const u64, adv.as_mut_ptr() as *mut u64, inst.as_mut_ptr() as *mut u64) });
+        (0..b).map(|w| ((0..na).map(|c| adv[(w * na + c) * n..(w * na + c + 1) * n].to_vec()).collect(), inst[w * nin..(w + 1) * nin].to_vec()))
+            .collect()
+    }
+}
+impl Drop for WitnessProgram {
+    fn drop(&mut self) { unsafe { h2v_witness_program_free(self.h) } }
 }
 
 /// A halo2 `ProvingKey` (fixed columns, permutation polynomials, constraint-system shape) resident on the device;

@@ -39,6 +39,9 @@ ABI_SYMBOLS = [
     "h2v_quotient_gates_ptrs_dev", "h2v_quotient_permutation_ptrs_dev", "h2v_quotient_permutation_range_ptrs_dev", "h2v_commit_batch_resident",
     "h2v_pk_load", "h2v_pk_free", "h2v_create_proof", "h2v_create_proofs", "h2v_proof_size", "h2v_pk_last_phase_ms",
     "h2v_mock_prover", "h2v_pk_mock_prover", "h2v_mock_last_ms",
+    "h2v_witness_program_new", "h2v_witness_program_free", "h2v_witness_program_info", "h2v_witness_program_inputs",
+    "h2v_witness_program_rule_counts",
+    "h2v_witness_generate", "h2v_witness_last_ms",
     "h2v_transcript_new", "h2v_transcript_free", "h2v_transcript_common_point", "h2v_transcript_common_scalar",
     "h2v_transcript_write_point", "h2v_transcript_write_scalar", "h2v_transcript_squeeze_challenge", "h2v_transcript_bytes",
     "h2v_poseidon_permutation", "h2v_poseidon_permutation_variant", "h2v_chacha20_fr_random", "h2v_chacha20_block",
@@ -51,6 +54,7 @@ BUILDER_SYMBOLS = [      # the circuit builder (halo2_vectordb_b200.circuit)
     "h2v_builder_nearest_vector", "h2v_builder_kmeans", "h2v_builder_poseidon_new", "h2v_builder_poseidon_hash",
     "h2v_builder_merkle_commitment", "h2v_builder_stats", "h2v_builder_config", "h2v_builder_trace", "h2v_builder_layout",
     "h2v_layout_free", "h2v_layout_info", "h2v_layout_columns", "h2v_layout_instance", "h2v_layout_break_points",
+    "h2v_builder_new_recording",
 ]
 ABI_SYMBOLS += BUILDER_SYMBOLS
 

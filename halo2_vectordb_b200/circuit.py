@@ -12,7 +12,8 @@ Same names, argument meaning and failure behaviour as the reference, so that tes
     d = dist.euclidean_distance(ctx, a, b);  fp.dequantization(d.value())
 
 All the work happens in libh2v.so (csrc/zk_builder.hpp, zk_chips.hpp, circuit.cu); this file only marshals cell indices.
-`RangeCircuit` lays the trace out into the columns `ProvingKey` / `create_proof` take.
+`RangeCircuit` lays the trace out into the columns `ProvingKey` / `create_proof` take.  `WitnessProgram` replays a recorded
+circuit for many new inputs on the GPU and gives the same advice columns and instances without the host builder.
 """
 import ctypes as C
 
@@ -61,6 +62,15 @@ def _L():
         L.h2v_layout_columns.argtypes = [C.c_void_p, C.c_int, C.POINTER(_u64pp), C.POINTER(C.c_size_t)]
         L.h2v_layout_instance.argtypes = [C.c_void_p, C.POINTER(C.POINTER(C.c_uint64)), C.POINTER(C.c_size_t)]
         L.h2v_layout_break_points.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
+        L.h2v_builder_new_recording.argtypes = [C.c_uint32, C.c_uint32, C.POINTER(C.c_void_p)]
+        L.h2v_witness_program_new.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32, C.POINTER(C.c_void_p)]
+        L.h2v_witness_program_free.argtypes = [C.c_void_p]
+        L.h2v_witness_program_free.restype = None
+        L.h2v_witness_program_info.argtypes = [C.c_void_p, C.c_void_p]
+        L.h2v_witness_program_inputs.argtypes = [C.c_void_p, C.c_void_p]
+        L.h2v_witness_program_rule_counts.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
+        L.h2v_witness_generate.argtypes = [C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.h2v_witness_last_ms.argtypes = [C.POINTER(C.c_double)]
         _typed = True
     return L
 
@@ -107,12 +117,14 @@ class Context:
 
 class GateThreadBuilder:
     """halo2-base `GateThreadBuilder<Fr>` together with the `LOOKUP_BITS` the scaffold reads from the environment
-    (mod.rs:361-372) and the PRECISION_BITS of the chips built over it (48 in every example)."""
+    (mod.rs:361-372) and the PRECISION_BITS of the chips built over it (48 in every example).  record=True also keeps
+    the rule of every cell, so that `WitnessProgram` can replay the circuit for other inputs."""
 
-    def __init__(self, lookup_bits, precision_bits=48):
-        self.lookup_bits, self.precision_bits = lookup_bits, precision_bits
+    def __init__(self, lookup_bits, precision_bits=48, record=False):
+        self.lookup_bits, self.precision_bits, self.record = lookup_bits, precision_bits, record
         self._h = C.c_void_p()
-        _check(_L().h2v_builder_new(precision_bits, lookup_bits, C.byref(self._h)))
+        new = _L().h2v_builder_new_recording if record else _L().h2v_builder_new
+        _check(new(precision_bits, lookup_bits, C.byref(self._h)))
         self._ctx = Context(self)
         self.assigned_instances = []
 
@@ -385,6 +397,70 @@ class RangeCircuit:
             pass
 
 
+class WitnessProgram:
+    """A recorded circuit compiled for replay on the GPU (h2v_witness_program_new): `generate(inputs_list)` gives, for
+    each list of inputs (the values the recording passed to `assign_witnesses`, in that order, Montgomery limbs), the
+    advice columns and instances `RangeCircuit(builder, k, minimum_rows)` would give for a builder run on those inputs.
+    The recording's fixed and sigma columns serve them all.  The builder may be closed afterwards."""
+
+    INFO = ("inputs", "cells", "computed_cells", "levels", "advice_columns", "instances", "k", "bytes_per_witness")
+
+    def __init__(self, builder, k, minimum_rows=9):
+        self._h = C.c_void_p()
+        _check(_L().h2v_witness_program_new(builder._h, k, minimum_rows, C.byref(self._h)))
+        out = np.zeros(8, dtype=np.uint64)
+        _check(_L().h2v_witness_program_info(self._h, _ptr(out)))
+        self.info = {name: int(v) for name, v in zip(self.INFO, out)}
+        self.n_inputs, self.k = self.info["inputs"], self.info["k"]
+
+    def inputs(self):
+        """the recording's own inputs, (n_inputs, 4) Montgomery limbs"""
+        out = np.zeros((self.n_inputs, 4), dtype=np.uint64)
+        _check(_L().h2v_witness_program_inputs(self._h, _ptr(out)))
+        return out
+
+    def rule_counts(self):
+        """computed cells per rule kind (zk_builder.hpp's RuleKind order)"""
+        n = C.c_size_t()
+        _check(_L().h2v_witness_program_rule_counts(self._h, None, 0, C.byref(n)))
+        out = np.zeros(n.value, dtype=np.uint64)
+        _check(_L().h2v_witness_program_rule_counts(self._h, _ptr(out), n.value, C.byref(n)))
+        return [int(x) for x in out]
+
+    def generate(self, inputs_list):
+        """-> [(advice, instances)] per witness, shaped like `RangeCircuit.advice` / `.instances`"""
+        B = len(inputs_list)
+        inp = np.zeros((B, self.n_inputs, 4), dtype=np.uint64)
+        for w, x in enumerate(inputs_list):
+            x = np.asarray(x, dtype=np.uint64).reshape(-1, 4)
+            if x.shape[0] != self.n_inputs:
+                raise ValueError(f"witness_generate: witness {w}: {x.shape[0]} inputs, the program has {self.n_inputs}")
+            inp[w] = x
+        n, A, I = 1 << self.k, self.info["advice_columns"], self.info["instances"]
+        adv = np.zeros((B, A, n, 4), dtype=np.uint64)
+        inst = np.zeros((B, I, 4), dtype=np.uint64)
+        _check(_L().h2v_witness_generate(self._h, B, self.n_inputs, _ptr(inp), _ptr(adv), _ptr(inst)))
+        return [([adv[w, c] for c in range(A)], [inst[w]]) for w in range(B)]
+
+    @staticmethod
+    def last_ms():
+        """(upload, evaluation + gather, download) of the last generate, ms"""
+        ms = (C.c_double * 3)()
+        _check(_L().h2v_witness_last_ms(ms))
+        return tuple(ms)
+
+    def close(self):
+        if getattr(self, "_h", None) and self._h.value:
+            _L().h2v_witness_program_free(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 # ---------------------------------------------------------------------------------------------- the example circuits
 def distance_functions(ctx, inp, make_public, fp=None):
     """/root/reference/examples/distances.rs:24-63"""
@@ -437,12 +513,13 @@ def kmeans(ctx, inp, make_public, K=4, I=10, distance=DISTANCE_COSINE, fp=None):
 EXAMPLES = dict(distances=distance_functions, query=exhaustive_merkle, kmeans=kmeans)
 
 
-def create_circuit(f, inp, k, lookup_bits, minimum_rows=9, **kw):
+def create_circuit(f, inp, k, lookup_bits, minimum_rows=9, record=False, **kw):
     """the scaffold's `create_circuit` (mod.rs:347-402): run the circuit function on `builder.main(0)`, expose the public
-    values, lay the trace out.  Returns (RangeCircuit, whatever f returned)."""
+    values, lay the trace out.  Returns (RangeCircuit, whatever f returned); the circuit's `.builder` is a recording
+    builder when record=True."""
     if not lookup_bits < k:
         raise ValueError("LOOKUP_BITS needs to be less than DEGREE")      # mod.rs:367
-    builder = GateThreadBuilder(lookup_bits)
+    builder = GateThreadBuilder(lookup_bits, record=record)
     public = []
     out = f(builder.main(0), inp, public, **kw)
     builder.make_public(public)
@@ -466,3 +543,21 @@ def example_input(name):
 
 # BASELINE.json configs[0..2]: (k, LOOKUP_BITS) of the README's commands
 EXAMPLE_PARAMS = dict(distances=(13, 12), query=(13, 12), kmeans=(16, 15))
+
+
+def example_witness_inputs(name, inp, precision_bits=48):
+    """the inputs the example circuit `name` assigns for `inp`, in assignment order: the `WitnessProgram` inputs of a
+    recording of that example -> (n, 4) Montgomery limbs"""
+    if name == "distances":
+        leaves = list(inp["a"]) + list(inp["b"])
+    elif name == "query":
+        leaves = list(inp["query"]) + [x for v in inp["database"] for x in v]
+    elif name == "kmeans":
+        leaves = [x for v in inp["vectors"] for x in v]
+    else:
+        raise ValueError(name)
+    b = GateThreadBuilder(EXAMPLE_PARAMS[name][1], precision_bits)
+    try:
+        return FixedPointChip.default(b).quantize_vector(leaves)
+    finally:
+        b.close()

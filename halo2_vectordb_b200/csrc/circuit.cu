@@ -27,6 +27,7 @@ struct h2v_builder {
     VectorDBChip vdb;
     std::unique_ptr<PoseidonChip3> poseidon;
     std::vector<int64_t> instances;      // `make_public`
+    uint32_t n_inputs = 0;               // values passed to h2v_builder_assign_witnesses
     h2v_builder(unsigned p, unsigned lb) : fp(p, lb), dist(fp), vdb(fp) {
         // the trace of a real circuit has 10^7 - 10^8 cells: reserve address space once (untouched pages cost nothing) instead
         // of re-copying gigabytes at every doubling of the vectors; H2V_TRACE_RESERVE = cells (0 = let them grow)
@@ -140,6 +141,55 @@ struct Cycles {
     }
 };
 
+// Where assign_all puts each trace cell: the gate columns with their break points, and the lookup-advice columns
+struct Placement {
+    size_t n, max_rows, num_advice, num_lookup;
+    std::vector<uint32_t> pos_col, pos_row;
+    struct Break {
+        size_t cell;
+        uint32_t col, row;
+    };
+    std::vector<Break> breaks;      // the cell closing column col at row `row` is repeated on row 0 of column col + 1
+    std::vector<uint32_t> break_points;
+    // the j-th lookup cell: (advice column, row)
+    std::pair<size_t, size_t> lookup_pos(size_t j) const { return {num_advice + j / max_rows, j % max_rows}; }
+};
+void place(const h2v_builder *b, uint32_t k, uint32_t minimum_rows, Placement &P) {
+    const Context &ctx = b->ctx;
+    if (k < 3 || k > 26) throw std::runtime_error("k out of range");
+    const size_t n = (size_t)1 << k;
+    if (minimum_rows >= n) throw std::runtime_error("minimum_rows >= 2^k");
+    if (b->fp.lookup_bits >= k) throw std::runtime_error("LOOKUP_BITS needs to be less than DEGREE");      // mod.rs:367
+    const size_t max_rows = n - minimum_rows;
+    // ---- config(): column counts
+    const size_t total_advice = ctx.advice.size(), total_lookup = ctx.cells_to_lookup.size();
+    const size_t num_advice = (total_advice + max_rows - 1) / max_rows;
+    P.n = n;
+    P.max_rows = max_rows;
+    P.num_advice = num_advice;
+    P.num_lookup = (total_lookup + max_rows - 1) / max_rows;
+    // ---- assign_all, first loop: positions and break points of the trace down the gate columns
+    P.pos_col.resize(total_advice);
+    P.pos_row.resize(total_advice);
+    size_t gate_index = 0, row = 0;
+    for (size_t i = 0; i < total_advice; ++i) {
+        if (gate_index >= num_advice) throw std::runtime_error("NOT ENOUGH ADVICE COLUMNS IN PHASE 0. Perhaps blinding factors were not taken into account.");
+        P.pos_col[i] = (uint32_t)gate_index;
+        P.pos_row[i] = (uint32_t)row;
+        const bool q = ctx.selector[i] != 0;
+        if ((q && row + 4 > max_rows) || row >= max_rows - 1) {
+            // the cell closes this column; it is repeated on row 0 of the next one (where its gate, if any, lives)
+            // and tied to the original, which stays the cell's position for the equality constraints
+            P.break_points.push_back((uint32_t)row);
+            P.breaks.push_back(Placement::Break{i, (uint32_t)gate_index, (uint32_t)row});
+            row = 0;
+            ++gate_index;
+            if (gate_index >= num_advice) throw std::runtime_error("NOT ENOUGH ADVICE COLUMNS IN PHASE 0. Perhaps blinding factors were not taken into account.");
+        }
+        ++row;
+    }
+}
+
 int do_layout(const h2v_builder *b, uint32_t k, uint32_t minimum_rows, h2v_layout *L) {
     const Context &ctx = b->ctx;
     const bool timing = getenv("H2V_LAYOUT_TIMING") != nullptr;
@@ -150,18 +200,13 @@ int do_layout(const h2v_builder *b, uint32_t k, uint32_t minimum_rows, h2v_layou
         fprintf(stderr, "layout: %-28s %8.1f ms\n", what, std::chrono::duration<double, std::milli>(t - t_last).count());
         t_last = t;
     };
-    if (k < 3 || k > 26) throw std::runtime_error("k out of range");
-    const size_t n = (size_t)1 << k;
-    if (minimum_rows >= n) throw std::runtime_error("minimum_rows >= 2^k");
-    if (b->fp.lookup_bits >= k) throw std::runtime_error("LOOKUP_BITS needs to be less than DEGREE");      // mod.rs:367
-    const size_t max_rows = n - minimum_rows;
+    Placement pl;
+    place(b, k, minimum_rows, pl);
+    const size_t n = pl.n, max_rows = pl.max_rows, total_advice = ctx.advice.size();
+    const size_t num_advice = pl.num_advice, num_lookup = pl.num_lookup;
     L->k = k;
     L->minimum_rows = minimum_rows;
     L->lookup_bits = b->fp.lookup_bits;
-    // ---- config(): column counts
-    const size_t total_advice = ctx.advice.size(), total_lookup = ctx.cells_to_lookup.size();
-    const size_t num_advice = (total_advice + max_rows - 1) / max_rows;
-    const size_t num_lookup = (total_lookup + max_rows - 1) / max_rows;
     std::unordered_map<U256, std::pair<uint32_t, uint32_t>, U256Hash> assigned_constants;
     std::vector<U256> const_order;
     for (const auto &ce : ctx.constant_eq)
@@ -186,28 +231,10 @@ int do_layout(const h2v_builder *b, uint32_t k, uint32_t minimum_rows, h2v_layou
     Cycles cyc(P, n);
     tick("cycles init");
     // ---- assign_all, first loop: the trace down the gate columns
-    std::vector<uint32_t> pos_col(total_advice), pos_row(total_advice);
+    const std::vector<uint32_t> &pos_col = pl.pos_col, &pos_row = pl.pos_row;
+    L->break_points = pl.break_points;
     {
-        // positions and break points first (serial, selectors only), then the values and selector cells by all cores
-        struct Break { size_t cell; uint32_t col, row; };
-        std::vector<Break> breaks;
-        size_t gate_index = 0, row = 0;
-        for (size_t i = 0; i < total_advice; ++i) {
-            if (gate_index >= num_advice) throw std::runtime_error("NOT ENOUGH ADVICE COLUMNS IN PHASE 0. Perhaps blinding factors were not taken into account.");
-            pos_col[i] = (uint32_t)gate_index;
-            pos_row[i] = (uint32_t)row;
-            const bool q = ctx.selector[i] != 0;
-            if ((q && row + 4 > max_rows) || row >= max_rows - 1) {
-                // the cell closes this column; it is repeated on row 0 of the next one (where its gate, if any, lives)
-                // and tied to the original, which stays the cell's position for the equality constraints
-                L->break_points.push_back((uint32_t)row);
-                breaks.push_back(Break{i, (uint32_t)gate_index, (uint32_t)row});
-                row = 0;
-                ++gate_index;
-                if (gate_index >= num_advice) throw std::runtime_error("NOT ENOUGH ADVICE COLUMNS IN PHASE 0. Perhaps blinding factors were not taken into account.");
-            }
-            ++row;
-        }
+        // the values and selector cells by all cores
         const size_t parts = 64;
         parallel_for(parts, [&](size_t part) {
             const size_t i0 = total_advice * part / parts, i1 = total_advice * (part + 1) / parts;
@@ -216,7 +243,7 @@ int do_layout(const h2v_builder *b, uint32_t k, uint32_t minimum_rows, h2v_layou
                 if (ctx.selector[i]) put(fix[1 + num_fixed + pos_col[i]], pos_row[i], u_from(1));
             }
         });
-        for (const Break &bk : breaks) {
+        for (const Placement::Break &bk : pl.breaks) {
             put(adv[bk.col + 1], 0, ctx.advice[bk.cell]);
             if (ctx.selector[bk.cell]) {        // the gate starts on the repeated cell, not on the closing one
                 put(fix[1 + num_fixed + bk.col], bk.row, u_from(0));
@@ -248,17 +275,11 @@ int do_layout(const h2v_builder *b, uint32_t k, uint32_t minimum_rows, h2v_layou
         const auto fc = assigned_constants[e.first];
         cyc.copy(pc_const + fc.first, fc.second, pc_adv + pos_col[(size_t)e.second], pos_row[(size_t)e.second]);
     }
-    {
-        size_t lcol = 0, loff = 0;
-        for (int64_t off : ctx.cells_to_lookup) {
-            if (loff >= max_rows) {
-                loff = 0;
-                ++lcol;
-            }
-            put(adv[num_advice + lcol], loff, ctx.advice[(size_t)off]);
-            cyc.copy(pc_adv + pos_col[(size_t)off], pos_row[(size_t)off], pc_adv + num_advice + lcol, loff);
-            ++loff;
-        }
+    for (size_t j = 0; j < ctx.cells_to_lookup.size(); ++j) {
+        const size_t off = (size_t)ctx.cells_to_lookup[j];
+        const auto lp = pl.lookup_pos(j);
+        put(adv[lp.first], lp.second, ctx.advice[off]);
+        cyc.copy(pc_adv + pos_col[off], pos_row[off], pc_adv + lp.first, lp.second);
     }
     tick("constant + lookup copies");
     // lookup table 0 .. 2^lookup_bits - 1 (the remaining rows hold the default 0)
@@ -310,9 +331,163 @@ int do_layout(const h2v_builder *b, uint32_t k, uint32_t minimum_rows, h2v_layou
     return H2V_OK;
 }
 
+// The witness program of a recording: copies resolved to their roots, the cells no input reaches folded to their recorded
+// values, the others sorted by level; the gather map from the layout's advice positions and instances to them.
+void make_plan(const h2v_builder *b, uint32_t k, uint32_t minimum_rows, WitnessPlan &W) {
+    const Context &ctx = b->ctx;
+    if (!ctx.recording) throw std::runtime_error("witness_program: the builder is not a recording builder (h2v_builder_new_recording)");
+    Placement pl;
+    place(b, k, minimum_rows, pl);
+    if (b->instances.size() > pl.max_rows) throw std::runtime_error("too many public inputs");
+    const size_t N = ctx.advice.size();
+    if (N >= WREF_POOL) throw std::runtime_error("witness_program: too many cells");
+    const std::vector<Rule> &rules = ctx.rules;
+    auto nargs = [](uint8_t kind) {
+        switch (kind) {
+            case OP_ADD: case OP_SUB: case OP_MUL: case OP_OR: case OP_DIV_Q: case OP_DIV_R: return 2;
+            case OP_MUL_ADD: case OP_SELECT_IND: return 3;
+            default: return 1;
+        }
+    };
+    std::vector<uint32_t> root(N);
+    for (size_t i = 0; i < N; ++i) {
+        const Rule &r = rules[i];
+        if (r.kind == RULE_NONE || r.kind >= RULE_KINDS) throw std::runtime_error("witness_program: cell " + std::to_string(i) + " has no rule");
+        if (r.kind == RULE_COPY) {
+            if (r.a < 0 || (size_t)r.a >= i) throw std::runtime_error("witness_program: cell " + std::to_string(i) + " copies a later cell");
+            root[i] = root[(size_t)r.a];
+        } else {
+            root[i] = (uint32_t)i;
+        }
+        const int64_t ops[3] = {r.a, r.b, r.c};
+        if (r.kind >= OP_ADD)
+            for (int j = 0; j < nargs(r.kind); ++j)
+                if (ops[j] < 0 || (size_t)ops[j] >= N || (size_t)ops[j] == i) throw std::runtime_error("witness_program: cell " + std::to_string(i) + " has a bad operand");
+    }
+    // level of each root: -1 folded (no input reaches it), 0 input, else 1 + the deepest computed operand
+    const int32_t UNSEEN = -2, VISITING = -3;
+    std::vector<int32_t> level(N, UNSEEN);
+    auto operands = [&](size_t i, uint32_t *o) {      // the operands' roots (unused operands are cell 0, never read)
+        const int na = nargs(rules[i].kind);
+        o[0] = root[(size_t)rules[i].a];
+        o[1] = na > 1 ? root[(size_t)rules[i].b] : 0;
+        o[2] = na > 2 ? root[(size_t)rules[i].c] : 0;
+    };
+    std::vector<uint32_t> stack;
+    uint32_t n_levels = 0;
+    for (size_t i0 = 0; i0 < N; ++i0) {
+        if (root[i0] != i0 || level[i0] != UNSEEN) continue;
+        stack.push_back((uint32_t)i0);
+        while (!stack.empty()) {
+            const uint32_t i = stack.back();
+            const Rule &r = rules[i];
+            if (level[i] >= -1) {      // pushed twice
+                stack.pop_back();
+                continue;
+            }
+            if (r.kind == RULE_INPUT || r.kind == RULE_CONST) {
+                level[i] = r.kind == RULE_INPUT ? 0 : -1;
+                stack.pop_back();
+                continue;
+            }
+            uint32_t o[3];
+            operands(i, o);
+            const int na = nargs(r.kind);
+            bool ready = true;
+            for (int j = 0; j < na; ++j)
+                if (level[o[j]] == UNSEEN) {
+                    if (ready) level[i] = VISITING;
+                    ready = false;
+                    stack.push_back(o[j]);
+                } else if (level[o[j]] == VISITING) {
+                    throw std::runtime_error("witness_program: cell " + std::to_string(i) + " depends on itself");
+                }
+            if (!ready) continue;
+            int32_t lv = -1;
+            for (int j = 0; j < na; ++j) lv = std::max(lv, level[o[j]]);
+            level[i] = lv < 0 ? -1 : lv + 1;
+            n_levels = std::max(n_levels, (uint32_t)std::max(level[i], 0));
+            stack.pop_back();
+        }
+    }
+    // slots: inputs by their index, then the computed cells level by level (trace order within a level)
+    W.k = k;
+    W.n_cells = N;
+    W.n_inputs = b->n_inputs;
+    W.n_levels = n_levels;
+    W.level_start.assign((size_t)n_levels + 2, 0);
+    for (size_t i = 0; i < N; ++i)
+        if (root[i] == i && level[i] > 0) ++W.level_start[(size_t)level[i] + 1];
+    for (size_t l = 1; l < W.level_start.size(); ++l) W.level_start[l] += W.level_start[l - 1];
+    W.level_start.erase(W.level_start.begin());      // level l (1-based) occupies [level_start[l - 1], level_start[l])
+    const size_t n_computed = W.level_start.back();
+    std::vector<uint32_t> slot(N, WREF_ZERO), fill(W.level_start.begin(), W.level_start.end() - 1);
+    W.inputs.assign(W.n_inputs * 4, 0);
+    for (size_t i = 0; i < N; ++i) {
+        if (root[i] != i) continue;
+        if (level[i] == 0) {
+            slot[i] = rules[i].imm;
+            to_abi(&W.inputs[4 * (size_t)rules[i].imm], ctx.advice[i]);
+        } else if (level[i] > 0) {
+            slot[i] = (uint32_t)(W.n_inputs + fill[(size_t)level[i] - 1]++);
+        }
+    }
+    if (W.n_inputs + n_computed >= WREF_POOL) throw std::runtime_error("witness_program: too many cells");
+    std::unordered_map<uint32_t, uint32_t> pool_of;
+    auto ref = [&](uint32_t c) -> uint32_t {      // c: a root cell
+        if (slot[c] != WREF_ZERO) return slot[c];
+        if (u_is_zero(ctx.advice[c])) return WREF_ZERO;
+        auto it = pool_of.emplace(c, (uint32_t)(W.pool.size() / 4));
+        if (it.second) W.pool.insert(W.pool.end(), ctx.advice[c].l, ctx.advice[c].l + 4);
+        return WREF_POOL | it.first->second;
+    };
+    W.kind_counts.assign(RULE_KINDS, 0);
+    W.rules.resize(n_computed);
+    W.cell_of.resize(n_computed);
+    for (size_t i = 0; i < N; ++i) {
+        if (root[i] != i || level[i] <= 0) continue;
+        const Rule &r = rules[i];
+        if (r.imm >= (1u << 24)) throw std::runtime_error("witness_program: immediate out of range");
+        uint32_t o[3], rr[3] = {WREF_ZERO, WREF_ZERO, WREF_ZERO};
+        operands(i, o);
+        for (int j = 0; j < nargs(r.kind); ++j) rr[j] = ref(o[j]);
+        const size_t s_ = slot[i] - W.n_inputs;
+        W.rules[s_] = WitnessRule{rr[0], rr[1], rr[2], (uint32_t)r.kind | r.imm << 8};
+        W.cell_of[s_] = i;
+        ++W.kind_counts[r.kind];
+    }
+    // gather map: the layout's advice columns (gate columns with the break repeats, lookup columns), then the instances
+    const size_t n = pl.n, A = pl.num_advice + pl.num_lookup;
+    W.n_adv_cols = A;
+    W.n_instances = b->instances.size();
+    W.map.assign(A * n + W.n_instances, WREF_ZERO);
+    for (size_t i = 0; i < N; ++i) W.map[(size_t)pl.pos_col[i] * n + pl.pos_row[i]] = ref(root[i]);
+    for (const Placement::Break &bk : pl.breaks) W.map[(size_t)(bk.col + 1) * n] = ref(root[bk.cell]);
+    for (size_t j = 0; j < ctx.cells_to_lookup.size(); ++j) {
+        const auto lp = pl.lookup_pos(j);
+        W.map[lp.first * n + lp.second] = ref(root[(size_t)ctx.cells_to_lookup[j]]);
+    }
+    for (size_t i = 0; i < W.n_instances; ++i) W.map[A * n + i] = ref(root[(size_t)b->instances[i]]);
+}
+
 }  // namespace
 
 extern "C" {
+
+int h2v_builder_new_recording(uint32_t precision_bits, uint32_t lookup_bits, h2v_builder_t *out) {
+    H2V_TRY(h2v_builder_new(precision_bits, lookup_bits, out));
+    (*out)->ctx.recording = true;
+    return H2V_OK;
+}
+int h2v_witness_program_new(h2v_builder_t b, uint32_t k, uint32_t minimum_rows, h2v_witness_program_t *out) {
+    if (!b || !out) return failf(H2V_EINVAL, "witness_program_new: NULL argument");
+    WitnessPlan plan;
+    H2V_TRY(guarded([&]() {
+        make_plan(b, k, minimum_rows, plan);
+        return (int)H2V_OK;
+    }));
+    return witness_program_make(std::move(plan), out);
+}
 
 int h2v_builder_new(uint32_t precision_bits, uint32_t lookup_bits, h2v_builder_t *out) {
     if (!out) return failf(H2V_EINVAL, "builder_new: out is NULL");
@@ -335,7 +510,7 @@ int h2v_builder_dequantize(h2v_builder_t b, const uint64_t *x, size_t n, double 
 }
 int h2v_builder_assign_witnesses(h2v_builder_t b, const uint64_t *values, size_t n, int64_t *cells_out) {
     if (!b || (n && (!values || !cells_out))) return failf(H2V_EINVAL, "assign_witnesses: NULL argument");
-    for (size_t i = 0; i < n; ++i) cells_out[i] = b->ctx.load_witness(from_abi(values + 4 * i)).off;
+    for (size_t i = 0; i < n; ++i) cells_out[i] = b->ctx.load_witness(Witness(from_abi(values + 4 * i), RULE_INPUT, 0, 0, 0, b->n_inputs++)).off;
     return H2V_OK;
 }
 int h2v_builder_load_constant(h2v_builder_t b, const uint64_t value[4], int64_t *cell_out) {

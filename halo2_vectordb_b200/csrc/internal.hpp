@@ -5,6 +5,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <vector>
+
 #include "h2v.h"
 
 namespace h2v {
@@ -111,6 +113,31 @@ void mock_set_last_ms(const double ms[2]);         // h2v_mock_last_ms
 int mock_check_advice(const h2v_circuit_t *cs, const uint64_t *const *advice, const char *who);
 int mock_check_instances(const h2v_circuit_t *cs, const uint64_t *const *instances, const uint32_t *instance_len, const char *who);
 int mock_check_limits(const h2v_circuit_t *cs, const char *who);
+
+// The group size for n_items items of item_bytes device bytes each when `held` bytes of device buffers can be reused:
+// H2V_PROOF_GROUP if set, else as many as fit with 8 GB kept free; at most `cap` (prover.cu)
+size_t group_size_free(size_t n_items, size_t item_bytes, size_t cap, size_t held);
+
+// A witness program (circuit.cu builds it from a recording builder, witness.cu runs it).  Values are canonical.  An operand
+// or gather reference is a slot (inputs first, then the computed cells in level order), WREF_POOL | i for constant i of the
+// pool, or WREF_ZERO.
+enum : uint32_t { WREF_POOL = 0x80000000u, WREF_ZERO = 0xffffffffu };
+struct WitnessRule {
+    uint32_t a, b, c;
+    uint32_t op;      // zk::RuleKind | imm << 8
+};
+struct WitnessPlan {
+    uint32_t k = 0, n_levels = 0;
+    uint64_t n_inputs = 0, n_cells = 0, n_adv_cols = 0, n_instances = 0;
+    std::vector<WitnessRule> rules;        // the computed cells, level by level
+    std::vector<uint32_t> level_start;     // n_levels + 1 offsets into rules
+    std::vector<uint64_t> cell_of;         // trace cell of each computed cell (error texts)
+    std::vector<uint64_t> pool;            // 4 limbs per constant
+    std::vector<uint32_t> map;             // 2^k rows of each advice column, then the instances
+    std::vector<uint64_t> inputs;          // the recording's own inputs, Montgomery form
+    std::vector<uint64_t> kind_counts;     // computed cells per zk::RuleKind
+};
+int witness_program_make(WitnessPlan &&plan, h2v_witness_program **out);      // witness.cu; takes the plan
 }  // namespace h2v
 
 #define H2V_CU(x)                                                                                                  \

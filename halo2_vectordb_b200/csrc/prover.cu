@@ -366,6 +366,18 @@ int check_circuit(const h2v_circuit_t *cs, bool have_column_lists, const char *w
         if (cs->fixed_query_col[j] >= cs->n_fixed) return failf(H2V_EINVAL, "%s: fixed query %u out of range", who, j);
     return H2V_OK;
 }
+size_t group_size_free(size_t n_items, size_t item_bytes, size_t cap, size_t held) {
+    cap = std::max<size_t>(1, std::min(cap, n_items));
+    if (const char *e = getenv("H2V_PROOF_GROUP")) {
+        const long g = atol(e);
+        if (g > 0) return std::min<size_t>((size_t)g, cap);
+    }
+    size_t free_b = 0, total_b = 0;
+    cudaMemGetInfo(&free_b, &total_b);
+    const size_t margin = (size_t)8 << 30, avail = free_b + held;
+    const size_t fit = avail > margin ? (avail - margin) / item_bytes : 1;
+    return std::max<size_t>(1, std::min(fit, cap));
+}
 }  // namespace h2v
 
 extern "C" {
@@ -1461,18 +1473,9 @@ size_t proof_bytes(const h2v_pk *pk) {
 // set, else as many as fit in the device memory left after the key, with 8 GB kept free as the extended-sigma cache
 // keeps it; at most `cap`, the largest group every grid dimension and batch call allows.
 size_t group_size(h2v_pk *pk, size_t n_items, size_t item_bytes, size_t cap) {
-    cap = std::max<size_t>(1, std::min(cap, n_items));
-    if (const char *e = getenv("H2V_PROOF_GROUP")) {
-        const long g = atol(e);
-        if (g > 0) return std::min<size_t>((size_t)g, cap);
-    }
-    size_t free_b = 0, total_b = 0;
-    cudaMemGetInfo(&free_b, &total_b);
     size_t held = 0;
     for (size_t i = 0; DevBuf *b = workspace(pk, i); ++i) held += b->cap;
-    const size_t margin = (size_t)8 << 30, avail = free_b + held;
-    const size_t fit = avail > margin ? (avail - margin) / item_bytes : 1;
-    return std::max<size_t>(1, std::min(fit, cap));
+    return group_size_free(n_items, item_bytes, cap, held);
 }
 // ... for n_proofs proofs.  Streamed keys prove one at a time.
 size_t proof_group_size(h2v_pk *pk, size_t n_proofs) {

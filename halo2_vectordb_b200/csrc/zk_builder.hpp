@@ -10,9 +10,11 @@
 //   * the reference's own chips, which ARE in /root/reference and are followed call by call:
 //     FixedPointChip (src/gadget/fixed_point.rs), DistanceChip (src/gadget/distance.rs), VectorDBChip
 //     (src/gadget/vectordb.rs).
-// Like upstream this is serial host code (a Context is single-threaded); it is not a kernel and never will be.
+// Like upstream this is serial host code (a Context is single-threaded).  A recording Context also keeps one `Rule` per
+// cell -- how the cell's value follows from the inputs and earlier cells -- so that witness.cu can replay the trace for
+// many inputs on the GPU (halo2-base's `witness_gen_only` idea); a normal Context records nothing.
 // Values are kept as canonical 256-bit integers (most of the work is bit / limb decomposition and integer division);
-// the layouter (circuit.cpp) converts to the Montgomery form of the C ABI.
+// the layouter (circuit.cu) converts to the Montgomery form of the C ABI.
 #pragma once
 #include <math.h>
 #include <stdint.h>
@@ -137,6 +139,34 @@ inline U256 f_from_u(const U256 &a) {      // biguint_to_fe: reduce mod r (input
 }
 
 // ------------------------------------------------------------------------------------------- Context
+// How a cell's value is computed (recording builders only).  Operands a, b, c are trace offsets; a negative operand
+// -1 - i names cell i of the region being assigned (it may come later in the trace than the cell it feeds).
+enum RuleKind : uint8_t {
+    RULE_NONE,                     // no rule: a recording with such a cell cannot become a program
+    RULE_INPUT,                    // imm-th value passed to h2v_builder_assign_witnesses
+    RULE_CONST,                    // the recorded value (constants, fixed witnesses)
+    RULE_COPY,                     // the value of cell a
+    OP_ADD, OP_SUB, OP_NEG, OP_MUL,
+    OP_MUL_ADD,                    // a b + c
+    OP_OR,                         // a + b - a b
+    OP_IS_ZERO, OP_INV_OR_ONE,     // a == 0; a^-1, or 1 when a == 0
+    OP_BITS,                       // (a >> (imm & 255)) mod 2^(imm >> 8), on the canonical integer
+    OP_DIV_Q, OP_DIV_R,            // floor(a / b), a mod b (b == 0: "attempt to divide by zero")
+    OP_SDS_Q, OP_SDS_R,            // signed_div_scale's q and r for the scale 2^imm
+    OP_IND, OP_IND_VAL,            // idx_to_indicator: low32(a) == imm ? 1 : 0, and ? a : 0
+    OP_SELECT_IND,                 // b != 0 ? a : c
+    OP_MSB,                        // qlog2: index of the highest set bit of a (1 when a == 0)
+    OP_POW2_MSB, OP_POW2_LOW32,    // 2^msb(a), 2^low32(a) (>= 254: "index out of bounds: pow_of_two")
+    OP_QCOUNT,                     // quantization((double)low128(a)) at precision imm
+    RULE_KINDS
+};
+struct Rule {
+    int64_t a, b, c;
+    uint32_t imm;
+    uint8_t kind;
+};
+inline constexpr int64_t R(int i) { return -1 - (int64_t)i; }      // operand: cell i of the current region
+
 // halo2-base `AssignedValue`: a value and the position of its cell in the execution trace
 struct Assigned {
     U256 v;
@@ -147,11 +177,16 @@ struct QCell {
     enum Kind : uint8_t { W, C, E } kind;
     U256 v;
     int64_t off;
+    Rule rule;      // of a W cell; kept by recording builders only
 };
-inline QCell Witness(const U256 &v) { return QCell{QCell::W, v, -1}; }
-inline QCell Constant(const U256 &v) { return QCell{QCell::C, v, -1}; }
-inline QCell Constant(uint64_t v) { return QCell{QCell::C, u_from(v), -1}; }
-inline QCell Existing(const Assigned &a) { return QCell{QCell::E, a.v, a.off}; }
+inline QCell Witness(const U256 &v) { return QCell{QCell::W, v, -1, Rule{0, 0, 0, 0, RULE_NONE}}; }
+// a witness cell and its rule (every Witness site of the chips)
+inline QCell Witness(const U256 &v, RuleKind k, int64_t a, int64_t b = 0, int64_t c = 0, uint32_t imm = 0) {
+    return QCell{QCell::W, v, -1, Rule{a, b, c, imm, k}};
+}
+inline QCell Constant(const U256 &v) { return QCell{QCell::C, v, -1, Rule{}}; }
+inline QCell Constant(uint64_t v) { return QCell{QCell::C, u_from(v), -1, Rule{}}; }
+inline QCell Existing(const Assigned &a) { return QCell{QCell::E, a.v, a.off, Rule{}}; }
 
 // halo2-base `Context<F>` (src/lib.rs of that crate): the trace of one thread.  witness_gen_only = false, i.e. the
 // keygen / mock form that also records selectors and copy constraints (CircuitBuilderStage::{Mock, Keygen});
@@ -164,6 +199,8 @@ struct Context {
     std::vector<std::pair<U256, int64_t>> constant_eq;          // constant_equality_constraints
     bool has_zero = false;
     Assigned zero_cell{};
+    bool recording = false;
+    std::vector<Rule> rules;      // one per cell when recording
 
     Assigned get(int64_t i) const {      // negative offsets count from the end, as upstream's `ctx.get`
         const int64_t o = i < 0 ? (int64_t)advice.size() + i : i;
@@ -171,21 +208,33 @@ struct Context {
         return Assigned{advice[(size_t)o], o};
     }
     Assigned last() const { return get(-1); }
-    void assign_cell(const QCell &q) {
+    // row: the first cell of the region q belongs to (operands R(i) of its rule are relative to it)
+    void assign_cell(const QCell &q, int64_t row = -1) {
         advice.push_back(q.v);
         const int64_t here = (int64_t)advice.size() - 1;
         if (q.kind == QCell::C) constant_eq.emplace_back(q.v, here);
         else if (q.kind == QCell::E) advice_eq.emplace_back(here, q.off);
+        if (recording) record(q, row < 0 ? here : row);
+    }
+    void record(const QCell &q, int64_t row) {
+        Rule r{0, 0, 0, 0, RULE_CONST};
+        if (q.kind == QCell::E) r = Rule{q.off, 0, 0, 0, RULE_COPY};
+        else if (q.kind == QCell::W) {
+            r = q.rule;
+            for (int64_t *o : {&r.a, &r.b, &r.c})
+                if (*o < 0) *o = row - 1 - *o;
+        }
+        rules.push_back(r);
     }
     void assign_region(std::initializer_list<QCell> cells, std::initializer_list<int> gates) {
         const size_t row = advice.size();
-        for (const QCell &q : cells) assign_cell(q);
+        for (const QCell &q : cells) assign_cell(q, (int64_t)row);
         selector.resize(advice.size(), 0);
         for (int g : gates) selector[row + (size_t)g] = 1;
     }
     void assign_region(const std::vector<QCell> &cells, const std::vector<int> &gates) {
         const size_t row = advice.size();
-        for (const QCell &q : cells) assign_cell(q);
+        for (const QCell &q : cells) assign_cell(q, (int64_t)row);
         selector.resize(advice.size(), 0);
         for (int g : gates) selector[row + (size_t)g] = 1;
     }
@@ -197,8 +246,8 @@ struct Context {
         for (auto &e : eqs) advice_eq.emplace_back(row + e.first, row + e.second);
     }
     void constrain_equal(const Assigned &a, const Assigned &b) { advice_eq.emplace_back(a.off, b.off); }
-    Assigned load_witness(const U256 &v) {
-        assign_cell(Witness(v));
+    Assigned load_witness(const QCell &w) {
+        assign_cell(w);
         selector.resize(advice.size(), 0);
         return last();
     }
@@ -214,12 +263,6 @@ struct Context {
         }
         return zero_cell;
     }
-    std::vector<Assigned> assign_witnesses(const std::vector<U256> &vs) {
-        std::vector<Assigned> out;
-        out.reserve(vs.size());
-        for (const U256 &v : vs) out.push_back(load_witness(v));
-        return out;
-    }
 };
 
 // ------------------------------------------------------------------------------------------- GateChip
@@ -232,27 +275,27 @@ struct GateChip {
     }
     // | a | b | 1 | a + b |
     Assigned add(Context &ctx, const QCell &a, const QCell &b) const {
-        ctx.assign_region({a, b, Constant(1), Witness(f_add(a.v, b.v))}, {0});
+        ctx.assign_region({a, b, Constant(1), Witness(f_add(a.v, b.v), OP_ADD, R(0), R(1))}, {0});
         return ctx.last();
     }
     // | a - b | b | 1 | a |
     Assigned sub(Context &ctx, const QCell &a, const QCell &b) const {
-        ctx.assign_region({Witness(f_sub(a.v, b.v)), b, Constant(1), a}, {0});
+        ctx.assign_region({Witness(f_sub(a.v, b.v), OP_SUB, R(3), R(1)), b, Constant(1), a}, {0});
         return ctx.get(-4);
     }
     // | a | -a | 1 | 0 |
     Assigned neg(Context &ctx, const QCell &a) const {
-        ctx.assign_region({a, Witness(f_neg(a.v)), Constant(1), Constant(0)}, {0});
+        ctx.assign_region({a, Witness(f_neg(a.v), OP_NEG, R(0)), Constant(1), Constant(0)}, {0});
         return ctx.get(-3);
     }
     // | 0 | a | b | a b |
     Assigned mul(Context &ctx, const QCell &a, const QCell &b) const {
-        ctx.assign_region({Constant(0), a, b, Witness(f_mul(a.v, b.v))}, {0});
+        ctx.assign_region({Constant(0), a, b, Witness(f_mul(a.v, b.v), OP_MUL, R(1), R(2))}, {0});
         return ctx.last();
     }
     // | c | a | b | a b + c |
     Assigned mul_add(Context &ctx, const QCell &a, const QCell &b, const QCell &c) const {
-        ctx.assign_region({c, a, b, Witness(f_add(f_mul(a.v, b.v), c.v))}, {0});
+        ctx.assign_region({c, a, b, Witness(f_add(f_mul(a.v, b.v), c.v), OP_MUL_ADD, R(1), R(2), R(0))}, {0});
         return ctx.last();
     }
     // | 0 | x | x | x |
@@ -266,21 +309,26 @@ struct GateChip {
     Assigned or_(Context &ctx, const QCell &a, const QCell &b) const {
         const U256 not_b = f_sub(u_from(1), b.v);
         const U256 out = f_sub(f_add(a.v, b.v), f_mul(a.v, b.v));
-        ctx.assign_region_smart({Witness(not_b), Constant(1), b, Constant(1), b, a, Witness(not_b), Witness(out)}, {0, 4}, {{0, 6}, {2, 4}});
+        ctx.assign_region_smart({Witness(not_b, OP_SUB, R(1), R(2)), Constant(1), b, Constant(1), b, a, Witness(not_b, OP_SUB, R(1), R(2)),
+                                 Witness(out, OP_OR, R(5), R(2))},
+                                {0, 4}, {{0, 6}, {2, 4}});
         return ctx.last();
     }
     // | a - b | 1 | b | a | b | sel | a - b | out |
     Assigned select(Context &ctx, const QCell &a, const QCell &b, const QCell &sel) const {
         const U256 diff = f_sub(a.v, b.v);
         const U256 out = f_add(f_mul(diff, sel.v), b.v);
-        ctx.assign_region_smart({Witness(diff), Constant(1), b, a, b, sel, Witness(diff), Witness(out)}, {0, 4}, {{0, 6}, {2, 4}});
+        ctx.assign_region_smart({Witness(diff, OP_SUB, R(3), R(2)), Constant(1), b, a, b, sel, Witness(diff, OP_SUB, R(3), R(2)),
+                                 Witness(out, OP_MUL_ADD, R(0), R(5), R(2))},
+                                {0, 4}, {{0, 6}, {2, 4}});
         return ctx.last();
     }
     // | is_zero | a | inv | 1 | 0 | a | is_zero | 0 |
     Assigned is_zero(Context &ctx, const Assigned &a) const {
         const bool z = u_is_zero(a.v);
         const U256 isz = u_from(z ? 1 : 0), inv = z ? u_from(1) : f_inv(a.v);
-        ctx.assign_region_smart({Witness(isz), Existing(a), Witness(inv), Constant(1), Constant(0), Existing(a), Witness(isz), Constant(0)},
+        ctx.assign_region_smart({Witness(isz, OP_IS_ZERO, R(1)), Existing(a), Witness(inv, OP_INV_OR_ONE, R(1)), Constant(1), Constant(0),
+                                 Existing(a), Witness(isz, OP_IS_ZERO, R(1)), Constant(0)},
                                 {0, 4}, {{0, 6}, {1, 5}});
         return ctx.get(-2);
     }
@@ -304,7 +352,7 @@ struct GateChip {
             s = f_add(s, a[i].v);
             cells.push_back(a[i]);
             cells.push_back(Constant(1));
-            cells.push_back(Witness(s));
+            cells.push_back(Witness(s, OP_ADD, R((int)(3 * i - 3)), R((int)(3 * i - 2))));
             gates.push_back((int)(3 * (i - 1)));
         }
         ctx.assign_region(cells, gates);
@@ -329,10 +377,11 @@ struct GateChip {
         }
         for (size_t i = first; i < a.size(); ++i) {
             s = f_add(s, f_mul(a[i].v, b[i].v));
-            gates.push_back((int)cells.size() - 1);
+            const int prev = (int)cells.size() - 1;
+            gates.push_back(prev);
             cells.push_back(a[i]);
             cells.push_back(b[i]);
-            cells.push_back(Witness(s));
+            cells.push_back(Witness(s, OP_MUL_ADD, R(prev + 1), R(prev + 2), R(prev)));
         }
         ctx.assign_region(cells, gates);
         return ctx.last();
@@ -341,7 +390,7 @@ struct GateChip {
     std::vector<Assigned> num_to_bits(Context &ctx, const Assigned &a, unsigned range_bits) const {
         std::vector<QCell> bits, pows;
         for (unsigned i = 0; i < range_bits; ++i) {
-            bits.push_back(Witness(u_from(u_bit(a.v, i) ? 1 : 0)));
+            bits.push_back(Witness(u_from(u_bit(a.v, i) ? 1 : 0), OP_BITS, a.off, 0, 0, i | 1u << 8));
             pows.push_back(Constant(pow_of_two[i]));
         }
         const int64_t row = (int64_t)ctx.advice.size();
@@ -361,7 +410,8 @@ struct GateChip {
         for (size_t i = 0; i < len; ++i) {
             const bool hit = idx_val == i;
             const U256 ind_val = u_from(hit ? 1 : 0), val = hit ? idx.v : u_zero();
-            ctx.assign_region_smart({Constant(0), Witness(ind_val), idx, Witness(val), Constant(f_neg(u_from(i))), Witness(ind_val), Constant(0)},
+            ctx.assign_region_smart({Constant(0), Witness(ind_val, OP_IND, R(2), 0, 0, (uint32_t)i), idx, Witness(val, OP_IND_VAL, R(2), 0, 0, (uint32_t)i),
+                                     Constant(f_neg(u_from(i))), Witness(ind_val, OP_IND, R(2), 0, 0, (uint32_t)i), Constant(0)},
                                     {0, 3}, {{1, 5}});
             if (i == 0) idx = Existing(ctx.get(-5));
             const Assigned cell = ctx.get(-2);
@@ -383,7 +433,7 @@ struct GateChip {
             gates.push_back((int)(3 * i));
             cells.push_back(a[i]);
             cells.push_back(Existing(ind[i]));
-            cells.push_back(Witness(s));
+            cells.push_back(Witness(s, OP_SELECT_IND, R((int)(3 * i + 1)), R((int)(3 * i + 2)), R((int)(3 * i))));
         }
         ctx.assign_region(cells, gates);
         return ctx.last();
@@ -412,7 +462,7 @@ struct RangeChip {
         } else {
             std::vector<QCell> limbs, bases;
             for (unsigned i = 0; i < k; ++i) {      // decompose_fe_to_u64_limbs
-                limbs.push_back(Witness(u_low_bits(u_shr(a.v, i * lookup_bits), lookup_bits)));
+                limbs.push_back(Witness(u_low_bits(u_shr(a.v, i * lookup_bits), lookup_bits), OP_BITS, a.off, 0, 0, i * lookup_bits | lookup_bits << 8));
                 bases.push_back(Constant(limb_bases[i]));
             }
             const int64_t row = (int64_t)ctx.advice.size();
@@ -431,7 +481,9 @@ struct RangeChip {
     // | a + 2^bits - b | b | 1 | a + 2^bits | -2^bits | 1 | a |, then the first cell is range-checked
     void check_less_than(Context &ctx, const QCell &a, const QCell &b, unsigned num_bits) const {
         const U256 pow = gate.pow_of_two[num_bits], shift_a = f_add(pow, a.v);
-        ctx.assign_region({Witness(f_sub(shift_a, b.v)), b, Constant(1), Witness(shift_a), Constant(f_neg(pow)), Constant(1), a}, {0, 3});
+        ctx.assign_region({Witness(f_sub(shift_a, b.v), OP_SUB, R(3), R(1)), b, Constant(1), Witness(shift_a, OP_SUB, R(6), R(4)), Constant(f_neg(pow)),
+                           Constant(1), a},
+                          {0, 3});
         range_check(ctx, ctx.get(-7), num_bits);
     }
     void check_big_less_than_safe(Context &ctx, const Assigned &a, const U256 &b) const {
@@ -442,7 +494,9 @@ struct RangeChip {
     Assigned is_less_than(Context &ctx, const QCell &a, const QCell &b, unsigned num_bits) const {
         const unsigned k = (num_bits + lookup_bits - 1) / lookup_bits, padded_bits = k * lookup_bits;
         const U256 pow = gate.pow_of_two[padded_bits], shift_a = f_add(pow, a.v);
-        ctx.assign_region({Witness(f_sub(shift_a, b.v)), b, Constant(1), Witness(shift_a), Constant(f_neg(pow)), Constant(1), a}, {0, 3});
+        ctx.assign_region({Witness(f_sub(shift_a, b.v), OP_SUB, R(3), R(1)), b, Constant(1), Witness(shift_a, OP_SUB, R(6), R(4)), Constant(f_neg(pow)),
+                           Constant(1), a},
+                          {0, 3});
         range_check(ctx, ctx.get(-7), padded_bits + lookup_bits);
         return gate.is_zero(ctx, ctx.get(ctx.cells_to_lookup.back()));      // the top limb is zero iff a < b
     }
@@ -450,7 +504,12 @@ struct RangeChip {
     std::pair<Assigned, Assigned> div_mod(Context &ctx, const QCell &a, const U256 &b, unsigned a_num_bits) const {
         U256 q, r;
         u_divmod(a.v, b, q, r);
-        ctx.assign_region({Witness(r), Constant(f_from_u(b)), Witness(q), a}, {0});
+        unsigned e = 0;      // the recorder replays division by a power of two only (the only divisors these chips use)
+        if (ctx.recording) {
+            e = (unsigned)u_bits(b) - 1;
+            if (u_is_zero(b) || u_pow2(e) != b) throw std::runtime_error("recording: div_mod by a constant that is not a power of two");
+        }
+        ctx.assign_region({Witness(r, OP_BITS, R(3), 0, 0, e << 8), Constant(f_from_u(b)), Witness(q, OP_BITS, R(3), 0, 0, e | 256u << 8), a}, {0});
         const Assigned rem = ctx.get(-4), div = ctx.get(-2);
         U256 bound, unused;
         u_divmod(u_pow2(a_num_bits), b, bound, unused);
@@ -463,7 +522,7 @@ struct RangeChip {
     std::pair<Assigned, Assigned> div_mod_var(Context &ctx, const QCell &a, const QCell &b, unsigned a_num_bits, unsigned b_num_bits) const {
         U256 q, r;
         u_divmod(a.v, b.v, q, r);
-        ctx.assign_region({Witness(r), b, Witness(q), a}, {0});
+        ctx.assign_region({Witness(r, OP_DIV_R, R(3), R(1)), b, Witness(q, OP_DIV_Q, R(3), R(1)), a}, {0});
         const Assigned rem = ctx.get(-4), div = ctx.get(-2);
         range_check(ctx, div, a_num_bits);
         range_check(ctx, rem, b_num_bits);

@@ -144,7 +144,9 @@ struct FixedPointChip {
         } else {
             u_divmod(a.v, b, q, r);
         }
-        ctx.assign_region({Witness(f_from_u(r)), Constant(f_from_u(b)), Witness(f_from_u(q)), a}, {0});
+        ctx.assign_region({Witness(f_from_u(r), OP_SDS_R, R(3), 0, 0, precision_bits), Constant(f_from_u(b)),
+                           Witness(f_from_u(q), OP_SDS_Q, R(3), 0, 0, precision_bits), a},
+                          {0});
         const Assigned rem = ctx.get(-4), div = ctx.get(-2);
         range.check_big_less_than_safe(ctx, rem, b);
         const Assigned div_abs = qabs(ctx, Existing(div));
@@ -243,8 +245,8 @@ struct FixedPointChip {
             if (u_bit(a_assigned.v, i)) num_digits = i;
         if (num_digits >= gate().pow_of_two.size()) throw std::runtime_error("index out of bounds: pow_of_two");
         const U256 pow1 = gate().pow_of_two[num_digits];
-        const Assigned pow1_witness = gate().add(ctx, Witness(pow1), Constant(0));
-        const Assigned exp1 = gate().add(ctx, Witness(u_from(num_digits)), Constant(0));
+        const Assigned pow1_witness = gate().add(ctx, Witness(pow1, OP_POW2_MSB, a_assigned.off), Constant(0));
+        const Assigned exp1 = gate().add(ctx, Witness(u_from(num_digits), OP_MSB, a_assigned.off), Constant(0));
         check_power_of_two(ctx, pow1_witness, exp1);
         const Assigned pow2_witness = gate().mul(ctx, Existing(pow1_witness), Constant(2));
         const Assigned exp2 = gate().add(ctx, Existing(exp1), Constant(1));
@@ -261,7 +263,7 @@ struct FixedPointChip {
         const Assigned shift_abs = qabs(ctx, Existing(shift));
         const uint64_t sidx = shift_abs.v.l[0] & 0xffffffffull;
         if (sidx >= gate().pow_of_two.size()) throw std::runtime_error("index out of bounds: pow_of_two");
-        const Assigned shift_pow2_witness = gate().add(ctx, Witness(gate().pow_of_two[sidx]), Constant(0));
+        const Assigned shift_pow2_witness = gate().add(ctx, Witness(gate().pow_of_two[sidx], OP_POW2_LOW32, shift_abs.off), Constant(0));
         check_power_of_two(ctx, shift_pow2_witness, shift_abs);
         const Assigned a_ls = gate().mul(ctx, a, Existing(shift_pow2_witness));
         const auto dm = range.div_mod_var(ctx, a, Existing(shift_pow2_witness), num_bits, precision_bits + 1);
@@ -400,9 +402,9 @@ struct DistanceChip {
         std::vector<Assigned> ab;
         for (size_t i = 0; i < a.size(); ++i) ab.push_back(fp.gate().is_equal(ctx, Existing(a[i]), Existing(b[i])));
         const Assigned ab_sum = fp.gate().sum(ctx, existing(ab));
-        const Assigned len = ctx.load_witness(fp.quantization((double)a.size()));
+        const Assigned len = ctx.load_witness(Witness(fp.quantization((double)a.size()), RULE_CONST, 0));
         const u128 lo = ((u128)ab_sum.v.l[1] << 64) | ab_sum.v.l[0];
-        const Assigned ab_sum_q = ctx.load_witness(fp.quantization((double)lo));
+        const Assigned ab_sum_q = ctx.load_witness(Witness(fp.quantization((double)lo), OP_QCOUNT, ab_sum.off, 0, 0, fp.precision_bits));
         const Assigned sim = fp.qdiv(ctx, Existing(ab_sum_q), Existing(len));
         const Assigned one = ctx.load_constant(fp.quantization(1.0));
         return fp.qsub(ctx, Existing(one), Existing(sim));

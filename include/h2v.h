@@ -399,6 +399,38 @@ int h2v_layout_instance(h2v_layout_t l, const uint64_t **out, size_t *n);
 /* the pinned break points (configs/<name>.json, mod.rs:272, 285-287) */
 int h2v_layout_break_points(h2v_layout_t l, uint32_t *out, size_t cap, size_t *n);
 
+/* ---- witness generation on the GPU (halo2-base's `witness_gen_only`) ---------------------------------------------
+ * A recording builder behaves like h2v_builder_new's and also keeps, for every cell, the rule that computes its value:
+ * the i-th value passed through h2v_builder_assign_witnesses, a constant, a copy of an earlier cell, or one chip
+ * operation on other cells.  h2v_witness_program_new compiles a recording into a program (the builder may be freed
+ * afterwards); h2v_witness_generate runs it for a batch of new inputs on the primary device and writes what
+ * h2v_builder_layout + h2v_layout_columns(kind 0) / h2v_layout_instance give for each input, ready for
+ * h2v_create_proofs / h2v_pk_mock_prover.  The program relies on the circuit's cells not depending on the inputs'
+ * values: inputs are exactly the values passed to h2v_builder_assign_witnesses, and constants (h2v_builder_load_constant)
+ * belong to the circuit.  The fixed and sigma columns of the recording's layout serve every input. */
+typedef struct h2v_witness_program *h2v_witness_program_t;
+int h2v_builder_new_recording(uint32_t precision_bits, uint32_t lookup_bits, h2v_builder_t *out);
+/* k, minimum_rows as h2v_builder_layout; H2V_EINVAL if b is not a recording builder or a cell has no rule */
+int h2v_witness_program_new(h2v_builder_t b, uint32_t k, uint32_t minimum_rows, h2v_witness_program_t *out);
+void h2v_witness_program_free(h2v_witness_program_t p);
+/* out: inputs, cells, computed cells (those an input reaches; every other cell is folded to its recorded value), levels
+ * (longest dependency path from the inputs), advice columns, instances, k, device bytes per witness */
+int h2v_witness_program_info(h2v_witness_program_t p, uint64_t out[8]);
+/* out[k] = computed cells of rule kind k for k < *n_kinds (cap >= *n_kinds; out may be NULL to query *n_kinds).  Kinds:
+ * 0 none, 1 input, 2 constant, 3 copy (these three are never computed), then the chip operations of zk_builder.hpp */
+int h2v_witness_program_rule_counts(h2v_witness_program_t p, uint64_t *out, size_t cap, size_t *n_kinds);
+/* the recording's own inputs, Montgomery form, inputs x 4 limbs */
+int h2v_witness_program_inputs(h2v_witness_program_t p, uint64_t *out);
+/* inputs: n_witnesses x n_inputs x 4 limbs (Montgomery, reduced).  advice_out: n_witnesses x advice columns x 2^k x 4
+ * limbs; instances_out: n_witnesses x instances x 4 limbs (pinned host memory recommended).  Every argument is checked
+ * before any device work.  A witness whose values make the recorded circuit panic ("attempt to divide by zero",
+ * "index out of bounds: pow_of_two") gives H2V_EINVAL naming the lowest such witness; the outputs are then unspecified
+ * and the program stays usable.  Witnesses run in groups as h2v_create_proofs' do (H2V_PROOF_GROUP, else what fits). */
+int h2v_witness_generate(h2v_witness_program_t p, size_t n_witnesses, size_t n_inputs, const uint64_t *inputs, uint64_t *advice_out,
+                         uint64_t *instances_out);
+/* the calling process's last h2v_witness_generate, ms: upload, evaluation + gather, download */
+int h2v_witness_last_ms(double out[3]);
+
 /* ---- Fiat-Shamir transcript, RNG ("next": SURVEY.md 8(f) row 3; host-side, no device needed) ---------------------
  * snark-verifier PoseidonTranscript<G1Affine, NativeLoader, Vec<u8>, T = 5, RATE = 4, R_F = 8, R_P = 60>::new::<0>
  * (scaffold mod.rs:309-310): points are absorbed as (x mod r, y mod r), scalars as themselves; write_* also append the

@@ -361,4 +361,32 @@ class ProvingKey {
     h2v_pk_t h_ = nullptr;
 };
 
+// A recorded circuit replayed for many inputs on the GPU (h2v_witness_program_new / h2v_witness_generate).  The builder
+// must come from h2v_builder_new_recording; it may be freed once the program exists.
+class WitnessProgram {
+  public:
+    WitnessProgram(h2v_builder_t recording, uint32_t k, uint32_t minimum_rows = 9) {
+        check(h2v_witness_program_new(recording, k, minimum_rows, &h_));
+        check(h2v_witness_program_info(h_, info_));
+    }
+    ~WitnessProgram() { h2v_witness_program_free(h_); }
+    WitnessProgram(const WitnessProgram &) = delete;
+    WitnessProgram &operator=(const WitnessProgram &) = delete;
+    size_t n_inputs() const { return (size_t)info_[0]; }
+    size_t n_advice() const { return (size_t)info_[4]; }
+    size_t n_instances() const { return (size_t)info_[5]; }
+    // inputs: n_witnesses x n_inputs values -> advice (n_witnesses x n_advice x 2^k) and instances (n_witnesses x n_instances)
+    void generate(size_t n_witnesses, const std::vector<Fr> &inputs, std::vector<Fr> &advice, std::vector<Fr> &instances) const {
+        if (inputs.size() != n_witnesses * n_inputs()) throw std::invalid_argument("witness_generate: inputs.size() != n_witnesses * n_inputs");
+        advice.resize(n_witnesses * n_advice() * ((size_t)1 << info_[6]));
+        instances.resize(n_witnesses * n_instances());
+        check(h2v_witness_generate(h_, n_witnesses, n_inputs(), inputs.empty() ? nullptr : &inputs[0].l[0], &advice[0].l[0],
+                                   instances.empty() ? nullptr : &instances[0].l[0]));
+    }
+
+  private:
+    h2v_witness_program_t h_ = nullptr;
+    uint64_t info_[8] = {};
+};
+
 }  // namespace h2v_host
