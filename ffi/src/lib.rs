@@ -129,6 +129,10 @@ extern "C" {
     pub fn h2v_witness_generate(p: *mut H2vWitnessProgram, n_witnesses: usize, n_inputs: usize, inputs: *const u64, advice_out: *mut u64,
                                 instances_out: *mut u64) -> c_int;
     pub fn h2v_witness_last_ms(out: *mut f64) -> c_int;
+    pub fn h2v_create_proofs_from_inputs(pk: *mut H2vPk, prog: *mut H2vWitnessProgram, n_proofs: usize, n_inputs: usize, inputs: *const u64,
+                                         rng_seeds: *const u8, proofs_out: *mut u8, proof_stride: usize, instances_out: *mut u64) -> c_int;
+    pub fn h2v_pk_mock_prover_from_inputs(pk: *mut H2vPk, prog: *mut H2vWitnessProgram, n_witnesses: usize, n_inputs: usize, inputs: *const u64,
+                                          failures_out: *mut H2vMockFailure, cap: usize, n_failures: *mut u64) -> c_int;
     pub fn h2v_quotient_gates_dev(dom: *mut H2vDomain, d_h: *mut c_void, y: *const u64, n_gates: usize, d_q: *const c_void,
                                   q_stride: usize, d_a: *const c_void, a_stride: usize) -> c_int;
     pub fn h2v_quotient_permutation_dev(dom: *mut H2vDomain, d_h: *mut c_void, y: *const u64, beta: *const u64, gamma: *const u64,
@@ -428,6 +432,35 @@ impl DeviceProvingKey {
         let mut totals = vec![0u64; b];
         if b > 0 {
             ok(unsafe { h2v_pk_mock_prover(self.0, b, ap.as_ptr(), ip.as_ptr(), lp.as_ptr(), out.as_mut_ptr(), max_failures, totals.as_mut_ptr()) });
+        }
+        (0..b).map(|w| (out[w * max_failures..w * max_failures + (totals[w] as usize).min(max_failures)].to_vec(), totals[w])).collect()
+    }
+    /// `create_proofs` on the columns `program.generate(inputs)` gives, generated in this key's workspace on the device
+    /// without crossing to the host -> (proof, instances) per input
+    pub fn create_proofs_from_inputs(&self, program: &WitnessProgram, inputs: &[&[Fr]], rng_seeds: &[[u8; 32]]) -> Vec<(Vec<u8>, Vec<Fr>)> {
+        let (b, ni, nin) = (inputs.len(), program.n_inputs(), program.info[5] as usize);
+        assert!(rng_seeds.len() == b && inputs.iter().all(|x| x.len() == ni));
+        let flat: Vec<Fr> = inputs.iter().flat_map(|x| x.iter().copied()).collect();
+        let seeds: Vec<u8> = rng_seeds.iter().flatten().copied().collect();
+        let size = unsafe { h2v_proof_size(self.0) };
+        let mut out = vec![0u8; b * size];
+        let mut inst = vec![Fr::zero(); b * nin];
+        if b > 0 {
+            ok(unsafe { h2v_create_proofs_from_inputs(self.0, program.h, b, ni, flat.as_ptr() as *const u64, seeds.as_ptr(), out.as_mut_ptr(), size,
+                                                      inst.as_mut_ptr() as *mut u64) });
+        }
+        (0..b).map(|p| (out[p * size..(p + 1) * size].to_vec(), inst[p * nin..(p + 1) * nin].to_vec())).collect()
+    }
+    /// `mock_prover` on the same generated columns, one device call for the batch
+    pub fn mock_prover_from_inputs(&self, program: &WitnessProgram, inputs: &[&[Fr]], max_failures: usize) -> Vec<(Vec<H2vMockFailure>, u64)> {
+        let (b, ni) = (inputs.len(), program.n_inputs());
+        assert!(inputs.iter().all(|x| x.len() == ni));
+        let flat: Vec<Fr> = inputs.iter().flat_map(|x| x.iter().copied()).collect();
+        let mut out = vec![H2vMockFailure::default(); b * max_failures];
+        let mut totals = vec![0u64; b];
+        if b > 0 {
+            ok(unsafe { h2v_pk_mock_prover_from_inputs(self.0, program.h, b, ni, flat.as_ptr() as *const u64, out.as_mut_ptr(), max_failures,
+                                                       totals.as_mut_ptr()) });
         }
         (0..b).map(|w| (out[w * max_failures..w * max_failures + (totals[w] as usize).min(max_failures)].to_vec(), totals[w])).collect()
     }

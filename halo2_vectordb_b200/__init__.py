@@ -41,7 +41,7 @@ ABI_SYMBOLS = [
     "h2v_mock_prover", "h2v_pk_mock_prover", "h2v_mock_last_ms",
     "h2v_witness_program_new", "h2v_witness_program_free", "h2v_witness_program_info", "h2v_witness_program_inputs",
     "h2v_witness_program_rule_counts",
-    "h2v_witness_generate", "h2v_witness_last_ms",
+    "h2v_witness_generate", "h2v_witness_last_ms", "h2v_create_proofs_from_inputs", "h2v_pk_mock_prover_from_inputs",
     "h2v_transcript_new", "h2v_transcript_free", "h2v_transcript_common_point", "h2v_transcript_common_scalar",
     "h2v_transcript_write_point", "h2v_transcript_write_scalar", "h2v_transcript_squeeze_challenge", "h2v_transcript_bytes",
     "h2v_poseidon_permutation", "h2v_poseidon_permutation_variant", "h2v_chacha20_fr_random", "h2v_chacha20_block",
@@ -161,6 +161,10 @@ def lib():
         L.h2v_mock_prover.argtypes = [C.c_void_p] * 7 + [C.c_size_t, C.POINTER(C.c_uint64)]
         L.h2v_pk_mock_prover.argtypes = [C.c_void_p, C.c_size_t] + [C.c_void_p] * 4 + [C.c_size_t, C.c_void_p]
         L.h2v_mock_last_ms.argtypes = [C.POINTER(C.c_double)]
+        L.h2v_create_proofs_from_inputs.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p, C.c_char_p, C.c_void_p,
+                                                    C.c_size_t, C.c_void_p]
+        L.h2v_pk_mock_prover_from_inputs.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p, C.c_void_p, C.c_size_t,
+                                                     C.c_void_p]
         L.h2v_transcript_new.argtypes = [C.POINTER(C.c_void_p)]
         L.h2v_transcript_free.argtypes = [C.c_void_p]
         L.h2v_transcript_free.restype = None
@@ -949,14 +953,38 @@ class ProvingKey:
         totals = np.zeros(B, dtype=np.uint64)
         arr = lambda xs: (C.c_void_p * B)(*xs)
         _check(lib().h2v_pk_mock_prover(self._h, B, arr(adv_ptrs), arr(inst_ptrs), arr(len_ptrs), out, max_failures, _ptr(totals)))
-        ms = (C.c_double * 2)()
-        _check(lib().h2v_mock_last_ms(ms))
-        res = []
-        for w in range(B):
-            got = min(max_failures, int(totals[w]))
-            fails = [MockFailure(*(getattr(out[w * max_failures + i], f) for f in MockFailure._fields)) for i in range(got)]
-            res.append(MockProver(fails, int(totals[w]), ms[0], ms[1]))
-        return res
+        return _mock_results(B, out, totals, max_failures)
+
+    def create_proofs_from_inputs(self, program, inputs_list, rng_seeds):
+        """create_proofs on the columns program.generate(inputs_list) gives, byte for byte with the same seeds; the columns
+        are generated in this key's device workspace and never reach the host (h2v_create_proofs_from_inputs).  The key
+        must come from the recording's layout -> (proofs, instances), instances[p] as program.generate gives them"""
+        B = len(inputs_list)
+        if len(rng_seeds) != B:
+            raise ValueError("create_proofs_from_inputs: inputs_list and rng_seeds differ in length")
+        if not B:
+            return [], []
+        inp = program.pack_inputs(inputs_list, "create_proofs_from_inputs")
+        if any(len(bytes(s_)) != 32 for s_ in rng_seeds):
+            raise ValueError("create_proofs_from_inputs: an rng seed is not 32 bytes")
+        seeds = b"".join(bytes(s_) for s_ in rng_seeds)
+        size = self.proof_size()
+        out = np.zeros(B * size, dtype=np.uint8)
+        inst = np.zeros((B, program.info["instances"], 4), dtype=np.uint64)
+        _check(lib().h2v_create_proofs_from_inputs(self._h, program._h, B, program.n_inputs, _ptr(inp), seeds, _ptr(out), size, _ptr(inst)))
+        return [bytes(out[p * size:(p + 1) * size]) for p in range(B)], [[inst[p]] if self.cs["n_instance"] else [] for p in range(B)]
+
+    def mock_prover_from_inputs(self, program, inputs_list, max_failures=64):
+        """mock_prover on the columns program.generate(inputs_list) gives, generated in this key's device workspace
+        (h2v_pk_mock_prover_from_inputs) -> list of MockProver (upload_ms: the generation)"""
+        B = len(inputs_list)
+        if not B:
+            return []
+        inp = program.pack_inputs(inputs_list, "mock_prover_from_inputs")
+        out = (_MockFailureT * max(1, B * max_failures))()
+        totals = np.zeros(B, dtype=np.uint64)
+        _check(lib().h2v_pk_mock_prover_from_inputs(self._h, program._h, B, program.n_inputs, _ptr(inp), out, max_failures, _ptr(totals)))
+        return _mock_results(B, out, totals, max_failures)
 
     def last_phase_ms(self):
         buf = (C.c_double * 8)()
@@ -975,6 +1003,18 @@ MockFailure = namedtuple("MockFailure", "kind column row other_column other_row"
 
 class _MockFailureT(C.Structure):
     _fields_ = [(f, C.c_uint32) for f in MockFailure._fields]
+
+
+def _mock_results(B, out, totals, max_failures):
+    """the MockProver of each witness of the last h2v_pk_mock_prover* call"""
+    ms = (C.c_double * 2)()
+    _check(lib().h2v_mock_last_ms(ms))
+    res = []
+    for w in range(B):
+        got = min(max_failures, int(totals[w]))
+        fails = [MockFailure(*(getattr(out[w * max_failures + i], f) for f in MockFailure._fields)) for i in range(got)]
+        res.append(MockProver(fails, int(totals[w]), ms[0], ms[1]))
+    return res
 
 
 class MockProver:

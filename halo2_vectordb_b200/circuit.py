@@ -427,15 +427,20 @@ class WitnessProgram:
         _check(_L().h2v_witness_program_rule_counts(self._h, _ptr(out), n.value, C.byref(n)))
         return [int(x) for x in out]
 
-    def generate(self, inputs_list):
-        """-> [(advice, instances)] per witness, shaped like `RangeCircuit.advice` / `.instances`"""
-        B = len(inputs_list)
-        inp = np.zeros((B, self.n_inputs, 4), dtype=np.uint64)
+    def pack_inputs(self, inputs_list, who):
+        """inputs_list as one (B, n_inputs, 4) array; errors start with `who`"""
+        inp = np.zeros((len(inputs_list), self.n_inputs, 4), dtype=np.uint64)
         for w, x in enumerate(inputs_list):
             x = np.asarray(x, dtype=np.uint64).reshape(-1, 4)
             if x.shape[0] != self.n_inputs:
-                raise ValueError(f"witness_generate: witness {w}: {x.shape[0]} inputs, the program has {self.n_inputs}")
+                raise ValueError(f"{who}: witness {w}: {x.shape[0]} inputs, the program has {self.n_inputs}")
             inp[w] = x
+        return inp
+
+    def generate(self, inputs_list):
+        """-> [(advice, instances)] per witness, shaped like `RangeCircuit.advice` / `.instances`"""
+        B = len(inputs_list)
+        inp = self.pack_inputs(inputs_list, "witness_generate")
         n, A, I = 1 << self.k, self.info["advice_columns"], self.info["instances"]
         adv = np.zeros((B, A, n, 4), dtype=np.uint64)
         inst = np.zeros((B, I, 4), dtype=np.uint64)

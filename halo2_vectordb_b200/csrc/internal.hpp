@@ -5,6 +5,7 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <mutex>
 #include <vector>
 
 #include "h2v.h"
@@ -102,11 +103,13 @@ int mock_key_build(cudaStream_t st, const h2v_circuit_t *cs, const fe *fixed, co
 void mock_key_free(MockKey *key);
 size_t mock_witness_bytes(const MockKey &key);     // device bytes one witness of a check needs
 size_t mock_max_batch(const MockKey &key);         // the most witnesses one mock_check takes
-// B witnesses: witness w's advice columns are uploaded to adv + w A n and its instance columns, zero-padded, to inst + w I n
-// (prove_group's layout; adv and inst grow to fit), then checked: failures_out + w cap and n_failures[w] as h2v_mock_prover
-// writes them.  ms[0] += the upload, ms[1] += the checks.  Synchronous.
-int mock_check(cudaStream_t st, const MockKey &key, size_t B, const uint64_t *const *const *advice, const uint64_t *const *const *instances,
-               const uint32_t *const *instance_len, DevBuf &adv, DevBuf &inst, h2v_mock_failure_t *failures_out, size_t cap,
+// B witnesses' host columns staged: witness w's advice columns uploaded to adv + w A n and its instance columns,
+// zero-padded, to inst + w I n (prove_group's layout; adv and inst grow to fit).  ms[0] += the upload.  Synchronous.
+int mock_stage(cudaStream_t st, const MockKey &key, size_t B, const uint64_t *const *const *advice, const uint64_t *const *const *instances,
+               const uint32_t *const *instance_len, DevBuf &adv, DevBuf &inst, double ms[2]);
+// B witnesses whose columns are resident in that layout checked: failures_out + w cap and n_failures[w] as
+// h2v_mock_prover writes them.  ms[1] += the checks.  Synchronous.
+int mock_check(cudaStream_t st, const MockKey &key, size_t B, const fe *adv, const fe *inst, h2v_mock_failure_t *failures_out, size_t cap,
                uint64_t *n_failures, double ms[2]);
 void mock_set_last_ms(const double ms[2]);         // h2v_mock_last_ms
 // the argument checks of h2v_mock_prover and h2v_pk_mock_prover; errors start with `who`
@@ -138,6 +141,20 @@ struct WitnessPlan {
     std::vector<uint64_t> kind_counts;     // computed cells per zk::RuleKind
 };
 int witness_program_make(WitnessPlan &&plan, h2v_witness_program **out);      // witness.cu; takes the plan
+bool fr_reduced(const uint64_t *x);      // 4 limbs below r
+// A program run into a proving key's workspace (witness.cu).  The caller holds the program's mutex (after the key's).
+std::mutex &witness_program_mutex(h2v_witness_program *p);
+// The program on device dev, uploaded there in copies on st on first use (H2V_EINVAL naming `who` if it is resident on
+// another device); the buffers of generated columns h2v_witness_generate grew are released and h2v_witness_last_ms starts
+// from zero.  *held: the device bytes of the evaluation buffers the groups will reuse.
+int witness_program_bind(h2v_witness_program *p, int dev, cudaStream_t st, const char *who, size_t *held);
+size_t witness_eval_bytes(const h2v_witness_program *p);      // device bytes one witness's evaluation needs
+// B witnesses (inputs: B x n_inputs x 4 limbs) evaluated and gathered on st: witness w's advice columns to adv + w A n,
+// its instances to inst + w inst_stride, zero-padded to inst_stride rows, and to inst_host + w n_instances 4 unless
+// inst_host is NULL; h2v_witness_last_ms accumulates.  A witness that panics: H2V_EINVAL with the panic text, *bad_w =
+// the first such witness of the group (else B).  Synchronous.
+int witness_generate_dev(h2v_witness_program *p, cudaStream_t st, size_t B, const uint64_t *inputs, fe *adv, fe *inst, size_t inst_stride,
+                         uint64_t *inst_host, size_t *bad_w);
 }  // namespace h2v
 
 #define H2V_CU(x)                                                                                                  \

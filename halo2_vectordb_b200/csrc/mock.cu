@@ -415,11 +415,9 @@ size_t mock_max_batch(const MockKey &K) {
     return std::max<size_t>(1, std::min<size_t>(65535, (((uint64_t)1 << 32) - 1) / std::max<uint64_t>(K.wbits, 1)));
 }
 
-int mock_check(cudaStream_t st, const MockKey &K, size_t B, const uint64_t *const *const *advice, const uint64_t *const *const *instances,
-               const uint32_t *const *instance_len, DevBuf &adv, DevBuf &inst, h2v_mock_failure_t *failures_out, size_t cap,
-               uint64_t *n_failures, double ms[2]) {
+int mock_stage(cudaStream_t st, const MockKey &K, size_t B, const uint64_t *const *const *advice, const uint64_t *const *const *instances,
+               const uint32_t *const *instance_len, DevBuf &adv, DevBuf &inst, double ms[2]) {
     const uint32_t n = K.n, A = K.A, I = K.I;
-    // the witnesses' columns, in prove_group's layout
     const double t0 = now_ms();
     H2V_TRY(adv.ensure(B * A * n * sizeof(fe)));
     H2V_TRY(inst.ensure(std::max<size_t>(1, B * I) * n * sizeof(fe)));
@@ -433,6 +431,13 @@ int mock_check(cudaStream_t st, const MockKey &K, size_t B, const uint64_t *cons
             if (instance_len[w][c])
                 H2V_CU(cudaMemcpyAsync(inst_d + (w * I + c) * n, instances[w][c], instance_len[w][c] * sizeof(fe), cudaMemcpyHostToDevice, st));
     H2V_CU(cudaStreamSynchronize(st));
+    ms[0] += now_ms() - t0;
+    return H2V_OK;
+}
+
+int mock_check(cudaStream_t st, const MockKey &K, size_t B, const fe *adv_d, const fe *inst_d, h2v_mock_failure_t *failures_out, size_t cap,
+               uint64_t *n_failures, double ms[2]) {
+    const uint32_t n = K.n, A = K.A, I = K.I;
     const double t1 = now_ms();
 
     // flags: every witness's section zeroed, the key's permutation flags copied in
@@ -492,7 +497,6 @@ int mock_check(cudaStream_t st, const MockKey &K, size_t B, const uint64_t *cons
         H2V_CU(cudaStreamSynchronize(st));
     }
     for (size_t w = 0; w < B; ++w) n_failures[w] = firsts[w + 1] - firsts[w];
-    ms[0] += t1 - t0;
     ms[1] += now_ms() - t1;
     return H2V_OK;
 }
@@ -555,7 +559,8 @@ int mock_run(const h2v_circuit_t *cs, const uint64_t *const *fixed, const uint64
     const double t1 = now_ms();
     H2V_TRY(mock_key_build(m.st, cs, fix_d, sig_d, &m.key));
     double ms[2] = {t1 - t0, now_ms() - t1};
-    H2V_TRY(mock_check(m.st, *m.key, 1, &advice, &instances, &instance_len, m.adv, m.inst, failures_out, cap, n_failures, ms));
+    H2V_TRY(mock_stage(m.st, *m.key, 1, &advice, &instances, &instance_len, m.adv, m.inst, ms));
+    H2V_TRY(mock_check(m.st, *m.key, 1, m.adv.as<fe>(), m.inst.as<fe>(), failures_out, cap, n_failures, ms));
     mock_set_last_ms(ms);
     return H2V_OK;
 }

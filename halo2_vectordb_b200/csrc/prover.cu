@@ -522,6 +522,16 @@ struct ProofIn {
     const uint32_t *instance_len;
     const uint8_t *seed;
 };
+// The advice and instances of a group's proofs generated on the device by a witness program
+// (h2v_create_proofs_from_inputs): proof p of the group has the inputs at inputs + p n_inputs 4, and its instances are
+// downloaded to instances + p n_instances 4, where the proof's ProofIn.instances points
+struct Generated {
+    h2v_witness_program *prog;
+    size_t n_inputs, n_instances;
+    const uint64_t *inputs;
+    uint64_t *instances;
+    Generated at(size_t p) const { return {prog, n_inputs, n_instances, inputs + p * n_inputs * 4, instances + p * n_instances * 4}; }
+};
 // what one proof of a group carries from phase to phase: its own RNG, transcript and challenges
 struct ProofState {
     PoseidonTranscript T;
@@ -539,6 +549,7 @@ struct Group {
     h2v_pk *pk;
     size_t B;
     const ProofIn *in;
+    const Generated *gen;                           // NULL: in[p].advice and in[p].instances are host columns
     std::vector<std::unique_ptr<ProofState>> P;
     size_t n, ne;
     uint32_t A, F, I, L, G, NP, NS, NH, bf, u;      // NH: quotient pieces of n coefficients each
@@ -549,8 +560,8 @@ struct Group {
     double t_phase = now_ms();
     int phase = 0;
 
-    Group(h2v_pk *pk_, size_t B_, const ProofIn *in_, size_t &bad_)
-        : pk(pk_), B(B_), in(in_), n(pk_->n), ne(pk_->ne), A(pk_->n_advice), F(pk_->n_fixed), I(pk_->n_instance),
+    Group(h2v_pk *pk_, size_t B_, const ProofIn *in_, const Generated *gen_, size_t &bad_)
+        : pk(pk_), B(B_), in(in_), gen(gen_), n(pk_->n), ne(pk_->ne), A(pk_->n_advice), F(pk_->n_fixed), I(pk_->n_instance),
           L((uint32_t)pk_->lookup_input.size()), G((uint32_t)pk_->gate_advice.size()), NP((uint32_t)pk_->perm_kind.size()),
           NS(pk_->n_sets), NH(pk_->degree - 1), bf(pk_->bf), u(pk_->u), gn((unsigned)((pk_->n + 255) / 256)), bad(bad_) {
         bad = SIZE_MAX;
@@ -667,7 +678,7 @@ int commit_products(Group &g, DevBuf &z, size_t cols_per_proof) {
 }
 
 // ---- phase 0.  plonk/prover.rs create_proof steps 1-4: vk and instances into the transcripts (hash_into, common_scalar);
-//      the advice columns uploaded, blinded in their last bf + 1 rows and committed
+//      the advice columns uploaded (or generated in place), blinded in their last bf + 1 rows and committed
 int instances_and_advice(Group &g) {
     h2v_pk *pk = g.pk;
     const size_t B = g.B, n = g.n, BA = B * g.A, BI = B * g.I;
@@ -676,34 +687,46 @@ int instances_and_advice(Group &g) {
     H2V_TRY(pk->inst_L.ensure(std::max<size_t>(1, BI) * n * sizeof(fe)));
     H2V_TRY(pk->inst_C.ensure(std::max<size_t>(1, BI) * n * sizeof(fe)));
     H2V_TRY(pk->inst_E.ensure(std::max<size_t>(1, BI) * g.ne * sizeof(fe)));
+    H2V_TRY(pk->adv_L.ensure(BA * n * sizeof(fe)));
+    H2V_TRY(pk->adv_C.ensure(BA * n * sizeof(fe)));
+    if (g.gen) {      // the columns straight into adv_L / inst_L; the instances also to the host, for the transcripts
+        size_t bad_w = B;
+        const int rc = witness_generate_dev(g.gen->prog, pk->st, B, g.gen->inputs, pk->adv_L.as<fe>(), pk->inst_L.as<fe>(), g.I ? n : 0,
+                                            g.gen->instances, &bad_w);
+        if (bad_w < B) g.bad = bad_w;
+        H2V_TRY(rc);
+    }
     if (g.I) {
-        std::vector<Fr64> inst(BI * n, frh::zero());
+        std::vector<Fr64> inst(g.gen ? 0 : BI * n, frh::zero());
         for (size_t p = 0; p < B; ++p)
             for (uint32_t c = 0; c < g.I; ++c)
                 for (uint32_t i = 0; i < g.in[p].instance_len[c]; ++i) {
-                    Fr64 &v = inst[(p * g.I + c) * n + i];
-                    v = frh::load(g.in[p].instances[c] + 4 * i);
+                    const Fr64 v = frh::load(g.in[p].instances[c] + 4 * i);
                     g.P[p]->T.common_scalar(v);
+                    if (!g.gen) inst[(p * g.I + c) * n + i] = v;
                 }
-        H2V_TRY(upload(pk, pk->inst_L, 0, inst.data(), BI * n * sizeof(fe)));
+        if (!g.gen) H2V_TRY(upload(pk, pk->inst_L, 0, inst.data(), BI * n * sizeof(fe)));
         H2V_TRY(h2v_domain_transform_dev(pk->dom, H2V_OP_LAGRANGE_TO_COEFF, pk->inst_L.p, n, pk->inst_C.p, n, BI));
     }
-    H2V_TRY(pk->adv_L.ensure(BA * n * sizeof(fe)));
-    H2V_TRY(pk->adv_C.ensure(BA * n * sizeof(fe)));
-    // h2v_commit_batch_resident: each device uploads its block of the B x A columns in sub-batches (the next one crosses
-    // while the previous one is committed), writes the tails, commits the block and leaves it in adv_L
     std::vector<Fr64> tails(BA * (bf + 1));
-    std::vector<const uint64_t *> adv(BA);
+    std::vector<const uint64_t *> adv(g.gen ? 0 : BA);
     for (size_t p = 0; p < B; ++p) {
         ChaCha20Rng &rng = g.P[p]->rng;
         for (size_t t = 0; t < (size_t)A * (bf + 1); ++t) tails[p * A * (bf + 1) + t] = rng.fr_random();   // column by column, rows u .. n-1
         for (uint32_t c = 0; c < A; ++c) (void)rng.fr_random();          // one Blind per column (unused by KZG, but drawn)
-        for (uint32_t c = 0; c < A; ++c) adv[p * A + c] = g.in[p].advice[c];
+        if (!g.gen)
+            for (uint32_t c = 0; c < A; ++c) adv[p * A + c] = g.in[p].advice[c];
     }
-    g.pts.resize(BA);
-    H2V_TRY(h2v_commit_batch_resident(pk->srs, H2V_BASIS_LAGRANGE, adv.data(), BA, n, (const uint64_t *)tails.data(), g.u, bf + 1, pk->adv_L.p, n,
-                                      (uint64_t *)g.pts.data()));
-    H2V_CU(cudaSetDevice(pk->dev));
+    if (g.gen) {      // rows u .. n-1 of the resident columns <- the tails; h2v_commit_batch_dev spreads the commits over the devices
+        H2V_TRY(write_rows(pk, pk->adv_L.as<fe>(), n, g.u, bf + 1, BA, tails));
+        H2V_TRY(commit_dev(pk, H2V_BASIS_LAGRANGE, pk->adv_L.as<fe>(), BA, g.pts));
+    } else {      // each device uploads its block of the B x A columns in sub-batches (the next one crosses while the previous
+                  // one is committed), writes the tails, commits the block and leaves it in adv_L
+        g.pts.resize(BA);
+        H2V_TRY(h2v_commit_batch_resident(pk->srs, H2V_BASIS_LAGRANGE, adv.data(), BA, n, (const uint64_t *)tails.data(), g.u, bf + 1, pk->adv_L.p,
+                                          n, (uint64_t *)g.pts.data()));
+        H2V_CU(cudaSetDevice(pk->dev));
+    }
     return write_commitments(g, g.pts, A, true);      // hashed while the lookup permutations run
 }
 
@@ -1430,10 +1453,10 @@ int shplonk(Group &g, const std::vector<MultiOpen> &MO) {
 
 // The prover: a group of B proofs phase by phase, each phase ended by lap() (h2v_pk_last_phase_ms).  The caller holds
 // pk->mu and has checked the inputs; on a failure traced to one proof, `bad` is that proof (else it stays SIZE_MAX).
-int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, std::vector<std::vector<uint8_t>> &proofs, size_t &bad) {
-    Group g(pk, B, in, bad);
+int prove_group(h2v_pk *pk, size_t B, const ProofIn *in, const Generated *gen, std::vector<std::vector<uint8_t>> &proofs, size_t &bad) {
+    Group g(pk, B, in, gen, bad);
     H2V_TRY(instances_and_advice(g));
-    g.lap();   // phase 0: upload + advice commitments
+    g.lap();   // phase 0: upload (or generation) + advice commitments
     H2V_TRY(permuted_lookups(g));
     g.lap();   // phase 1: lookup permutations
     H2V_TRY(permutation_products(g));
@@ -1471,17 +1494,19 @@ size_t proof_bytes(const h2v_pk *pk) {
 }
 // The group size for n_items items (proofs, or witnesses to check) of item_bytes device bytes each: H2V_PROOF_GROUP if
 // set, else as many as fit in the device memory left after the key, with 8 GB kept free as the extended-sigma cache
-// keeps it; at most `cap`, the largest group every grid dimension and batch call allows.
-size_t group_size(h2v_pk *pk, size_t n_items, size_t item_bytes, size_t cap) {
-    size_t held = 0;
+// keeps it; at most `cap`, the largest group every grid dimension and batch call allows.  extra_held: device bytes
+// outside the key's workspace that the groups reuse.
+size_t group_size(h2v_pk *pk, size_t n_items, size_t item_bytes, size_t cap, size_t extra_held = 0) {
+    size_t held = extra_held;
     for (size_t i = 0; DevBuf *b = workspace(pk, i); ++i) held += b->cap;
     return group_size_free(n_items, item_bytes, cap, held);
 }
-// ... for n_proofs proofs.  Streamed keys prove one at a time.
-size_t proof_group_size(h2v_pk *pk, size_t n_proofs) {
+// ... for n_proofs proofs, each also needing extra_bytes (a witness program's evaluation).  Streamed keys prove one at a time.
+size_t proof_group_size(h2v_pk *pk, size_t n_proofs, size_t extra_bytes = 0, size_t extra_held = 0) {
     if (pk->stream_ext || n_proofs <= 1) return 1;
     const size_t cmax = std::max<size_t>({pk->n_sets, pk->lookup_input.size(), 16});
-    return group_size(pk, n_proofs, proof_bytes(pk), std::min<size_t>(65535 / cmax, (((size_t)1 << 31) - 1) / (pk->n * cmax)));
+    return group_size(pk, n_proofs, proof_bytes(pk) + extra_bytes, std::min<size_t>(65535 / cmax, (((size_t)1 << 31) - 1) / (pk->n * cmax)),
+                      extra_held);
 }
 
 // Inputs of proof `idx` (who: the prefix of the error text)
@@ -1510,17 +1535,27 @@ bool release_sigma_cache(h2v_pk *pk) {
 }
 
 // n_proofs proofs in groups; emit(i, bytes) receives proof i.  A group that runs out of device memory is halved and run
-// again (a group of one needs what one proof always needed).  `batch`: prefix error texts with the proof they concern.
-template <class Emit> int run_proofs(h2v_pk *pk, size_t n_proofs, const ProofIn *in, bool batch, Emit emit) {
-    H2V_TRY(set_device(pk->dev, batch ? "create_proofs" : "create_proof"));
+// again (a group of one needs what one proof always needed).  `who` (NULL for h2v_create_proof): prefix error texts
+// with the call and the proof they concern.  gen: the columns come from a witness program, bound to the key's device
+// here, under its mutex (taken after the key's).
+template <class Emit> int run_proofs(h2v_pk *pk, size_t n_proofs, const ProofIn *in, const char *who, const Generated *gen, Emit emit) {
+    H2V_TRY(set_device(pk->dev, who ? who : "create_proof"));
     std::lock_guard<std::mutex> lk(pk->mu);
+    std::unique_lock<std::mutex> lk_prog;
+    size_t gen_bytes = 0, gen_held = 0;
+    if (gen) {
+        lk_prog = std::unique_lock<std::mutex>(witness_program_mutex(gen->prog));
+        H2V_TRY(witness_program_bind(gen->prog, pk->dev, pk->st, who, &gen_held));
+        gen_bytes = witness_eval_bytes(gen->prog);
+    }
     for (double &v : pk->last_ms) v = 0;
-    size_t G = proof_group_size(pk, n_proofs);
+    size_t G = proof_group_size(pk, n_proofs, gen_bytes, gen_held);
     for (size_t p0 = 0; p0 < n_proofs;) {
         const size_t b = std::min(G, n_proofs - p0);
         std::vector<std::vector<uint8_t>> out;
         size_t bad = SIZE_MAX;
-        int rc = prove_group(pk, b, in + p0, out, bad);
+        const Generated gen_b = gen ? gen->at(p0) : Generated{};
+        int rc = prove_group(pk, b, in + p0, gen ? &gen_b : nullptr, out, bad);
         if (rc == H2V_ENOMEM && release_sigma_cache(pk)) continue;
         if (rc == H2V_ENOMEM && b > 1) {
             cudaStreamSynchronize(pk->st);
@@ -1530,10 +1565,10 @@ template <class Emit> int run_proofs(h2v_pk *pk, size_t n_proofs, const ProofIn 
         }
         if (rc) {
             cudaStreamSynchronize(pk->st);
-            if (batch) {
+            if (who) {
                 const std::string msg = h2v_last_error();
-                if (bad != SIZE_MAX) return failf(rc, "create_proofs: proof %zu: %s", p0 + bad, msg.c_str());
-                return failf(rc, "create_proofs: group of proofs %zu .. %zu: %s", p0, p0 + b - 1, msg.c_str());
+                if (bad != SIZE_MAX) return failf(rc, "%s: %s %zu: %s", who, gen ? "witness" : "proof", p0 + bad, msg.c_str());
+                return failf(rc, "%s: group of proofs %zu .. %zu: %s", who, p0, p0 + b - 1, msg.c_str());
             }
             return rc;
         }
@@ -1571,6 +1606,82 @@ h2v_circuit_t circuit_of(const h2v_pk *pk) {
     return cs;
 }
 
+// run_proofs' emit for proofs written to out + p stride
+auto proofs_to(uint8_t *out, size_t stride, size_t size, const char *who) {
+    return [=](size_t p, const std::vector<uint8_t> &proof) -> int {
+        if (proof.size() != size) return failf(H2V_EINVAL, "%s: proof %zu has %zu bytes, expected %zu", who, p, proof.size(), size);
+        memcpy(out + p * stride, proof.data(), size);
+        return H2V_OK;
+    };
+}
+
+// n_witnesses witnesses checked in groups against the key's tables, as run_proofs runs proofs: stage(w0, b, ms, bad)
+// puts witnesses w0 .. w0 + b - 1 into adv_L / inst_L (ms[0] += its time; bad: the witness of the group a failure is
+// traced to).  Each witness also needs extra_bytes of device memory, and extra_held bytes outside the key's workspace
+// are reused by the groups.  The caller holds pk->mu and has checked the arguments.
+template <class Stage>
+int run_mock(h2v_pk *pk, size_t n_witnesses, const char *who, size_t extra_bytes, size_t extra_held, h2v_mock_failure_t *failures_out,
+             size_t cap, uint64_t *n_failures, Stage stage) {
+    const h2v_circuit_t cs = circuit_of(pk);
+    double ms[2] = {0, 0};
+    while (!pk->mock) {      // the key tables, on the first call
+        const double t = now_ms();
+        const int rc = mock_key_build(pk->st, &cs, pk->fixed_L.as<fe>(), pk->sigma_L.as<fe>(), &pk->mock);
+        ms[1] += now_ms() - t;
+        if (rc == H2V_ENOMEM && release_sigma_cache(pk)) continue;
+        if (rc) {
+            cudaStreamSynchronize(pk->st);
+            return rc;
+        }
+    }
+    // the witnesses in groups, as run_proofs runs proofs; they are staged in the key's adv_L / inst_L workspace
+    size_t G = group_size(pk, n_witnesses, mock_witness_bytes(*pk->mock) + extra_bytes, mock_max_batch(*pk->mock), extra_held);
+    for (size_t w0 = 0; w0 < n_witnesses;) {
+        const size_t b = std::min(G, n_witnesses - w0);
+        size_t bad = SIZE_MAX;
+        int rc = stage(w0, b, ms, bad);
+        if (!rc)
+            rc = mock_check(pk->st, *pk->mock, b, pk->adv_L.as<fe>(), pk->inst_L.as<fe>(), cap ? failures_out + w0 * cap : nullptr, cap,
+                            n_failures + w0, ms);
+        if (rc == H2V_ENOMEM && release_sigma_cache(pk)) continue;
+        if (rc == H2V_ENOMEM && b > 1) {
+            cudaStreamSynchronize(pk->st);
+            for (size_t i = 0; DevBuf *w = workspace(pk, i); ++i) w->release();
+            G = b / 2;
+            continue;
+        }
+        if (rc) {
+            cudaStreamSynchronize(pk->st);
+            const std::string msg = h2v_last_error();
+            if (bad != SIZE_MAX) return failf(rc, "%s: witness %zu: %s", who, w0 + bad, msg.c_str());
+            return failf(rc, "%s: witnesses %zu .. %zu: %s", who, w0, w0 + b - 1, msg.c_str());
+        }
+        w0 += b;
+    }
+    mock_set_last_ms(ms);
+    return H2V_OK;
+}
+
+// The argument checks of the _from_inputs calls that concern the program, in the order h2v.h states them; info: the
+// program's h2v_witness_program_info
+int check_program(const h2v_pk *pk, h2v_witness_program_t prog, size_t n_witnesses, size_t n_inputs, const uint64_t *inputs, const char *who,
+                  uint64_t info[8]) {
+    H2V_TRY(h2v_witness_program_info(prog, info));
+    if (n_inputs != info[0])
+        return failf(H2V_EINVAL, "%s: %zu inputs per witness, the program has %llu", who, n_inputs, (unsigned long long)info[0]);
+    for (size_t w = 0; w < n_witnesses; ++w)
+        for (size_t i = 0; i < n_inputs; ++i)
+            if (!fr_reduced(inputs + 4 * (w * n_inputs + i)))
+                return failf(H2V_EINVAL, "%s: witness %zu: input %zu is not a reduced Montgomery value", who, w, i);
+    if (info[6] != pk->k) return failf(H2V_EINVAL, "%s: the program has k = %llu, the key k = %u", who, (unsigned long long)info[6], pk->k);
+    if (info[4] != pk->n_advice)
+        return failf(H2V_EINVAL, "%s: the program has %llu advice columns, the key %u", who, (unsigned long long)info[4], pk->n_advice);
+    if (pk->n_instance > 1 || (pk->n_instance == 1 && info[5] > pk->u) || (pk->n_instance == 0 && info[5]))
+        return failf(H2V_EINVAL, "%s: the program's %llu instances do not fit the key's %u instance columns of %u usable rows", who,
+                     (unsigned long long)info[5], pk->n_instance, pk->u);
+    return H2V_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1580,7 +1691,7 @@ int h2v_create_proof(h2v_pk_t pk, const uint64_t *const *advice, const uint64_t 
     if (!pk || !rng_seed || !proof_len) return failf(H2V_EINVAL, "create_proof: NULL argument");
     const ProofIn in{advice, instances, instance_len, rng_seed};
     H2V_TRY(check_inputs(pk, in, "create_proof"));
-    return run_proofs(pk, 1, &in, false, [&](size_t, const std::vector<uint8_t> &proof) -> int {
+    return run_proofs(pk, 1, &in, nullptr, nullptr, [&](size_t, const std::vector<uint8_t> &proof) -> int {
         *proof_len = proof.size();
         if (proof.size() > proof_cap || !proof_out)
             return failf(H2V_EINVAL, "create_proof: proof needs %zu bytes, buffer has %zu", proof.size(), proof_cap);
@@ -1604,11 +1715,31 @@ int h2v_create_proofs(h2v_pk_t pk, size_t n_proofs, const uint64_t *const *const
         snprintf(who, sizeof who, "create_proofs: proof %zu", p);
         H2V_TRY(check_inputs(pk, in[p], who));
     }
-    return run_proofs(pk, n_proofs, in.data(), true, [&](size_t p, const std::vector<uint8_t> &proof) -> int {
-        if (proof.size() != size) return failf(H2V_EINVAL, "create_proofs: proof %zu has %zu bytes, expected %zu", p, proof.size(), size);
-        memcpy(proofs_out + p * proof_stride, proof.data(), size);
-        return H2V_OK;
-    });
+    return run_proofs(pk, n_proofs, in.data(), "create_proofs", nullptr, proofs_to(proofs_out, proof_stride, size, "create_proofs"));
+}
+int h2v_create_proofs_from_inputs(h2v_pk_t pk, h2v_witness_program_t prog, size_t n_proofs, size_t n_inputs, const uint64_t *inputs,
+                                  const uint8_t *rng_seeds, uint8_t *proofs_out, size_t proof_stride, uint64_t *instances_out) {
+    const char *who = "create_proofs_from_inputs";
+    if (!pk || !prog) return failf(H2V_EINVAL, "%s: NULL key or program", who);
+    if (!n_proofs) return H2V_OK;
+    if ((n_inputs && !inputs) || !rng_seeds || !proofs_out) return failf(H2V_EINVAL, "%s: NULL argument", who);
+    uint64_t info[8];
+    H2V_TRY(check_program(pk, prog, n_proofs, n_inputs, inputs, who, info));
+    const size_t size = h2v_proof_size(pk);
+    if (proof_stride < size) return failf(H2V_EINVAL, "%s: proof_stride %zu is shorter than a proof (%zu bytes)", who, proof_stride, size);
+    // the instances come back to the host for the transcripts: into instances_out, or a buffer of the call
+    const size_t n_inst = info[5];
+    std::vector<uint64_t> inst_own(instances_out ? 0 : n_proofs * n_inst * 4);
+    uint64_t *inst = instances_out ? instances_out : inst_own.data();
+    const uint32_t inst_len = (uint32_t)n_inst;
+    std::vector<const uint64_t *> inst_col(n_proofs);
+    std::vector<ProofIn> in(n_proofs);
+    for (size_t p = 0; p < n_proofs; ++p) {
+        inst_col[p] = inst + p * n_inst * 4;
+        in[p] = ProofIn{nullptr, pk->n_instance ? &inst_col[p] : nullptr, pk->n_instance ? &inst_len : nullptr, rng_seeds + 32 * p};
+    }
+    const Generated gen{prog, n_inputs, n_inst, inputs, inst};
+    return run_proofs(pk, n_proofs, in.data(), who, &gen, proofs_to(proofs_out, proof_stride, size, who));
 }
 int h2v_pk_mock_prover(h2v_pk_t pk, size_t n_witnesses, const uint64_t *const *const *advice, const uint64_t *const *const *instances,
                        const uint32_t *const *instance_len, h2v_mock_failure_t *failures_out, size_t cap, uint64_t *n_failures) {
@@ -1628,40 +1759,39 @@ int h2v_pk_mock_prover(h2v_pk_t pk, size_t n_witnesses, const uint64_t *const *c
     H2V_TRY(mock_check_limits(&cs, "pk_mock_prover"));
     H2V_TRY(set_device(pk->dev, "pk_mock_prover"));
     std::lock_guard<std::mutex> lk(pk->mu);
-    double ms[2] = {0, 0};
-    while (!pk->mock) {      // the key tables, on the first call
-        const double t = now_ms();
-        const int rc = mock_key_build(pk->st, &cs, pk->fixed_L.as<fe>(), pk->sigma_L.as<fe>(), &pk->mock);
-        ms[1] += now_ms() - t;
-        if (rc == H2V_ENOMEM && release_sigma_cache(pk)) continue;
-        if (rc) {
-            cudaStreamSynchronize(pk->st);
-            return rc;
-        }
-    }
-    // the witnesses in groups, as run_proofs runs proofs; they are staged in the key's adv_L / inst_L workspace
-    size_t G = group_size(pk, n_witnesses, mock_witness_bytes(*pk->mock), mock_max_batch(*pk->mock));
-    for (size_t w0 = 0; w0 < n_witnesses;) {
-        const size_t b = std::min(G, n_witnesses - w0);
-        const int rc = mock_check(pk->st, *pk->mock, b, advice ? advice + w0 : nullptr, instances ? instances + w0 : nullptr,
-                                  instance_len ? instance_len + w0 : nullptr, pk->adv_L, pk->inst_L, cap ? failures_out + w0 * cap : nullptr,
-                                  cap, n_failures + w0, ms);
-        if (rc == H2V_ENOMEM && release_sigma_cache(pk)) continue;
-        if (rc == H2V_ENOMEM && b > 1) {
-            cudaStreamSynchronize(pk->st);
-            for (size_t i = 0; DevBuf *w = workspace(pk, i); ++i) w->release();
-            G = b / 2;
-            continue;
-        }
-        if (rc) {
-            cudaStreamSynchronize(pk->st);
-            const std::string msg = h2v_last_error();
-            return failf(rc, "pk_mock_prover: witnesses %zu .. %zu: %s", w0, w0 + b - 1, msg.c_str());
-        }
-        w0 += b;
-    }
-    mock_set_last_ms(ms);
-    return H2V_OK;
+    return run_mock(pk, n_witnesses, "pk_mock_prover", 0, 0, failures_out, cap, n_failures, [&](size_t w0, size_t b, double ms[2], size_t &) {
+        return mock_stage(pk->st, *pk->mock, b, advice ? advice + w0 : nullptr, instances ? instances + w0 : nullptr,
+                          instance_len ? instance_len + w0 : nullptr, pk->adv_L, pk->inst_L, ms);
+    });
+}
+int h2v_pk_mock_prover_from_inputs(h2v_pk_t pk, h2v_witness_program_t prog, size_t n_witnesses, size_t n_inputs, const uint64_t *inputs,
+                                   h2v_mock_failure_t *failures_out, size_t cap, uint64_t *n_failures) {
+    const char *who = "pk_mock_prover_from_inputs";
+    if (!pk || !prog) return failf(H2V_EINVAL, "%s: NULL key or program", who);
+    if (!n_witnesses) return H2V_OK;
+    if ((n_inputs && !inputs) || !n_failures || (cap && !failures_out)) return failf(H2V_EINVAL, "%s: NULL argument", who);
+    uint64_t info[8];
+    H2V_TRY(check_program(pk, prog, n_witnesses, n_inputs, inputs, who, info));
+    const h2v_circuit_t cs = circuit_of(pk);
+    H2V_TRY(mock_check_limits(&cs, who));
+    H2V_TRY(set_device(pk->dev, who));
+    std::lock_guard<std::mutex> lk(pk->mu);
+    std::lock_guard<std::mutex> lk_prog(witness_program_mutex(prog));      // after the key's
+    size_t held = 0;
+    H2V_TRY(witness_program_bind(prog, pk->dev, pk->st, who, &held));
+    const size_t n = pk->n, A = pk->n_advice, I = pk->n_instance;
+    return run_mock(pk, n_witnesses, who, witness_eval_bytes(prog), held, failures_out, cap, n_failures,
+                    [&](size_t w0, size_t b, double ms[2], size_t &bad) -> int {
+                        const double t = now_ms();
+                        H2V_TRY(pk->adv_L.ensure(b * A * n * sizeof(fe)));
+                        H2V_TRY(pk->inst_L.ensure(std::max<size_t>(1, b * I) * n * sizeof(fe)));
+                        size_t bad_w = b;
+                        const int rc = witness_generate_dev(prog, pk->st, b, inputs + w0 * n_inputs * 4, pk->adv_L.as<fe>(), pk->inst_L.as<fe>(),
+                                                            I ? n : 0, nullptr, &bad_w);
+                        ms[0] += now_ms() - t;
+                        if (bad_w < b) bad = bad_w;
+                        return rc;
+                    });
 }
 size_t h2v_proof_size(h2v_pk_t pk) {
     if (!pk) return 0;

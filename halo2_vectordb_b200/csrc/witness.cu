@@ -246,17 +246,18 @@ __global__ void __launch_bounds__(WG_THREADS) witness_eval(const WitnessRule *__
     }
 }
 
-// out: B witnesses x (A n advice cells), inst: B x n_inst, Montgomery form
+// adv: B witnesses x (A n advice cells); inst: B x inst_stride, witness w's n_inst instances then zeros (inst_stride >=
+// n_inst); Montgomery form
 __global__ void __launch_bounds__(WG_THREADS) witness_gather(const uint32_t *__restrict__ map, uint64_t n_adv, uint64_t n_inst,
-                                                             const fe *__restrict__ pool, const fe *__restrict__ vals, uint64_t S, uint32_t B,
-                                                             fe *adv, fe *inst) {
-    const uint64_t P = n_adv + n_inst, stride = (uint64_t)gridDim.x * blockDim.x;
+                                                             uint64_t inst_stride, const fe *__restrict__ pool, const fe *__restrict__ vals,
+                                                             uint64_t S, uint32_t B, fe *adv, fe *inst) {
+    const uint64_t P = n_adv + inst_stride, stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; t < (uint64_t)B * P; t += stride) {
         const uint64_t w = t / P, pos = t - w * P;
-        const uint32_t ref = map[pos];
+        const uint32_t ref = pos < n_adv + n_inst ? map[pos] : WREF_ZERO;
         const fe v = ref == WREF_ZERO ? fe_zero() : fe_to_mont<FrP>(load(ref, vals + w * S, pool));
         if (pos < n_adv) adv[w * n_adv + pos] = v;
-        else inst[w * n_inst + (pos - n_adv)] = v;
+        else inst[w * inst_stride + (pos - n_adv)] = v;
     }
 }
 
@@ -267,7 +268,8 @@ double ms_since(std::chrono::steady_clock::time_point &t) {
     return ms;
 }
 
-int upload(h2v_witness_program *p) {
+// the program to the current device, in copies on st
+int upload(h2v_witness_program *p, cudaStream_t st) {
     WitnessPlan &P = p->plan;
     p->n_computed = P.rules.size();
     p->n_pool = P.pool.size() / 4;
@@ -278,11 +280,12 @@ int upload(h2v_witness_program *p) {
     H2V_TRY(p->pool.ensure(std::max<size_t>(1, p->n_pool) * sizeof(fe)));
     H2V_TRY(p->map.ensure(std::max<size_t>(1, P.map.size()) * sizeof(uint32_t)));
     std::vector<uint32_t> cell32(P.cell_of.begin(), P.cell_of.end());
-    H2V_CU(cudaMemcpy(p->rules.p, P.rules.data(), P.rules.size() * sizeof(WitnessRule), cudaMemcpyHostToDevice));
-    H2V_CU(cudaMemcpy(p->cell_of.p, cell32.data(), cell32.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    H2V_CU(cudaMemcpy(p->level_start.p, P.level_start.data(), P.level_start.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    H2V_CU(cudaMemcpy(p->pool.p, P.pool.data(), P.pool.size() * sizeof(uint64_t), cudaMemcpyHostToDevice));
-    H2V_CU(cudaMemcpy(p->map.p, P.map.data(), P.map.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    H2V_CU(cudaMemcpyAsync(p->rules.p, P.rules.data(), P.rules.size() * sizeof(WitnessRule), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(p->cell_of.p, cell32.data(), cell32.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(p->level_start.p, P.level_start.data(), P.level_start.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(p->pool.p, P.pool.data(), P.pool.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(p->map.p, P.map.data(), P.map.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaStreamSynchronize(st));      // the host vectors are released below
     int blocks = 0, sms = 0;
     H2V_CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, witness_eval, WG_THREADS, 0));
     H2V_CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, p->dev));
@@ -295,15 +298,17 @@ int upload(h2v_witness_program *p) {
     return H2V_OK;
 }
 
-// witnesses [w0, w0 + B) of one call; *bad = the first failing witness of the group, or B when none
-int run_group(h2v_witness_program *p, size_t w0, size_t B, const uint64_t *inputs, uint64_t *advice_out, uint64_t *instances_out,
-              size_t *bad_w, uint64_t *bad_code, double ms[3]) {
+// B witnesses (inputs: B x n_inputs x 4 limbs) evaluated and gathered on st: witness w's advice columns to adv + w A n, its
+// instances to inst + w inst_stride, zero-padded.  Then downloaded: the advice to advice_out (unless NULL), the instances
+// to instances_out + w n_instances 4 (unless NULL).  *bad_w = the first failing witness of the group, or B when none
+int run_group(h2v_witness_program *p, cudaStream_t st, size_t B, const uint64_t *inputs, fe *adv, fe *inst, size_t inst_stride,
+              uint64_t *advice_out, uint64_t *instances_out, size_t *bad_w, uint64_t *bad_code, double ms[3]) {
     const WitnessPlan &P = p->plan;
     const size_t n = (size_t)1 << P.k, n_adv = P.n_adv_cols * n, n_in = P.n_inputs, S = n_in + p->n_computed;
     auto t = std::chrono::steady_clock::now();
-    if (B * n_in) H2V_CU(cudaMemcpyAsync(p->in.p, inputs + w0 * n_in * 4, B * n_in * sizeof(fe), cudaMemcpyHostToDevice, 0));
-    H2V_CU(cudaMemsetAsync(p->err.p, 0xff, B * sizeof(uint64_t), 0));
-    H2V_CU(cudaStreamSynchronize(0));
+    if (B * n_in) H2V_CU(cudaMemcpyAsync(p->in.p, inputs, B * n_in * sizeof(fe), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemsetAsync(p->err.p, 0xff, B * sizeof(uint64_t), st));
+    H2V_CU(cudaStreamSynchronize(st));
     ms[0] += ms_since(t);
     const WitnessRule *rules = p->rules.as<WitnessRule>();
     const uint32_t *cell_of = p->cell_of.as<uint32_t>(), *level_start = p->level_start.as<uint32_t>();
@@ -313,21 +318,22 @@ int run_group(h2v_witness_program *p, size_t w0, size_t B, const uint64_t *input
     uint64_t S64 = S;
     unsigned long long *err = p->err.as<unsigned long long>();
     void *args[] = {&rules, &cell_of, &level_start, &n_levels, &pool, &in, &vals, &S64, &n_inputs, &Bu, &err};
-    H2V_CU(cudaLaunchCooperativeKernel((const void *)witness_eval, dim3(p->grid), dim3(WG_THREADS), args, 0, 0));
+    H2V_CU(cudaLaunchCooperativeKernel((const void *)witness_eval, dim3(p->grid), dim3(WG_THREADS), args, 0, st));
     H2V_LAUNCHED();
-    const uint64_t total = (uint64_t)B * (n_adv + P.n_instances);
+    const uint64_t total = (uint64_t)B * (n_adv + inst_stride);
     const unsigned gblocks = (unsigned)std::min<uint64_t>((total + WG_THREADS - 1) / WG_THREADS, (uint64_t)p->grid * 8);
-    witness_gather<<<std::max(1u, gblocks), WG_THREADS>>>(p->map.as<uint32_t>(), n_adv, P.n_instances, pool, vals, S, Bu, p->adv.as<fe>(),
-                                                         p->inst.as<fe>());
+    witness_gather<<<std::max(1u, gblocks), WG_THREADS, 0, st>>>(p->map.as<uint32_t>(), n_adv, P.n_instances, inst_stride, pool, vals, S, Bu,
+                                                                 adv, inst);
     H2V_LAUNCHED();
-    H2V_CU(cudaStreamSynchronize(0));
+    H2V_CU(cudaStreamSynchronize(st));
     ms[1] += ms_since(t);
     std::vector<uint64_t> err_h(B);
-    H2V_CU(cudaMemcpyAsync(err_h.data(), p->err.p, B * sizeof(uint64_t), cudaMemcpyDeviceToHost, 0));
-    H2V_CU(cudaMemcpyAsync(advice_out + w0 * n_adv * 4, p->adv.p, B * n_adv * sizeof(fe), cudaMemcpyDeviceToHost, 0));
-    if (P.n_instances)
-        H2V_CU(cudaMemcpyAsync(instances_out + w0 * P.n_instances * 4, p->inst.p, B * P.n_instances * sizeof(fe), cudaMemcpyDeviceToHost, 0));
-    H2V_CU(cudaStreamSynchronize(0));
+    H2V_CU(cudaMemcpyAsync(err_h.data(), p->err.p, B * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (advice_out) H2V_CU(cudaMemcpyAsync(advice_out, adv, B * n_adv * sizeof(fe), cudaMemcpyDeviceToHost, st));
+    if (P.n_instances && instances_out)
+        H2V_CU(cudaMemcpy2DAsync(instances_out, P.n_instances * sizeof(fe), inst, inst_stride * sizeof(fe), P.n_instances * sizeof(fe), B,
+                                 cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaStreamSynchronize(st));
     ms[2] += ms_since(t);
     *bad_w = B;
     for (size_t w = 0; w < B; ++w)
@@ -339,20 +345,26 @@ int run_group(h2v_witness_program *p, size_t w0, size_t B, const uint64_t *input
     return H2V_OK;
 }
 
+// the evaluation buffers of a group of B witnesses
+int ensure_eval(h2v_witness_program *p, size_t B) {
+    const size_t S = p->plan.n_inputs + p->n_computed;
+    H2V_TRY(p->in.ensure(std::max<size_t>(1, B * p->plan.n_inputs) * sizeof(fe)));
+    H2V_TRY(p->vals.ensure(std::max<size_t>(1, B * S) * sizeof(fe)));
+    return p->err.ensure(B * sizeof(uint64_t));
+}
+
 int generate(h2v_witness_program *p, size_t n_witnesses, const uint64_t *inputs, uint64_t *advice_out, uint64_t *instances_out) {
-    if (!p->uploaded) H2V_TRY(upload(p));
+    if (!p->uploaded) H2V_TRY(upload(p, 0));
     const WitnessPlan &P = p->plan;
-    const size_t n = (size_t)1 << P.k, n_adv = P.n_adv_cols * n, S = P.n_inputs + p->n_computed;
+    const size_t n = (size_t)1 << P.k, n_adv = P.n_adv_cols * n;
     const size_t held = p->in.cap + p->vals.cap + p->adv.cap + p->inst.cap + p->err.cap;
     size_t G = group_size_free(n_witnesses, p->witness_bytes(), 65535, held);
     double ms[3] = {0, 0, 0};
     for (size_t w0 = 0; w0 < n_witnesses;) {
         const size_t B = std::min(G, n_witnesses - w0);
-        int rc = p->in.ensure(std::max<size_t>(1, B * P.n_inputs) * sizeof(fe));
-        if (!rc) rc = p->vals.ensure(std::max<size_t>(1, B * S) * sizeof(fe));
+        int rc = ensure_eval(p, B);
         if (!rc) rc = p->adv.ensure(std::max<size_t>(1, B * n_adv) * sizeof(fe));
         if (!rc) rc = p->inst.ensure(std::max<size_t>(1, B * P.n_instances) * sizeof(fe));
-        if (!rc) rc = p->err.ensure(B * sizeof(uint64_t));
         if (rc == H2V_ENOMEM && G > 1) {      // halve the group and try again
             for (DevBuf *b : {&p->in, &p->vals, &p->adv, &p->inst, &p->err}) b->release();
             G = std::max<size_t>(1, G / 2);
@@ -361,7 +373,8 @@ int generate(h2v_witness_program *p, size_t n_witnesses, const uint64_t *inputs,
         H2V_TRY(rc);
         size_t bad = B;
         uint64_t code = 0;
-        H2V_TRY(run_group(p, w0, B, inputs, advice_out, instances_out, &bad, &code, ms));
+        H2V_TRY(run_group(p, 0, B, inputs + w0 * P.n_inputs * 4, p->adv.as<fe>(), p->inst.as<fe>(), P.n_instances, advice_out + w0 * n_adv * 4,
+                          P.n_instances ? instances_out + w0 * P.n_instances * 4 : nullptr, &bad, &code, ms));
         if (bad < B) {
             std::copy(ms, ms + 3, t_last_ms);
             return failf(H2V_EINVAL, "witness_generate: witness %zu: %s (cell %llu)", w0 + bad, werr_text((uint32_t)(code & 255)),
@@ -373,16 +386,39 @@ int generate(h2v_witness_program *p, size_t n_witnesses, const uint64_t *inputs,
     return H2V_OK;
 }
 
-bool reduced(const uint64_t *x) {
+}  // namespace
+
+namespace h2v {
+bool fr_reduced(const uint64_t *x) {
     static const uint64_t M[4] = {0x43e1f593f0000001ull, 0x2833e84879b97091ull, 0xb85045b68181585dull, 0x30644e72e131a029ull};
     for (int i = 3; i >= 0; --i)
         if (x[i] != M[i]) return x[i] < M[i];
     return false;
 }
-
-}  // namespace
-
-namespace h2v {
+std::mutex &witness_program_mutex(h2v_witness_program *p) { return p->mu; }
+int witness_program_bind(h2v_witness_program *p, int dev, cudaStream_t st, const char *who, size_t *held) {
+    if (p->uploaded && p->dev != dev)
+        return failf(H2V_EINVAL, "%s: the program is resident on device %d, the key on device %d", who, p->dev, dev);
+    if (!p->uploaded) {
+        p->dev = dev;
+        H2V_TRY(upload(p, st));
+    }
+    p->adv.release();
+    p->inst.release();
+    std::fill(t_last_ms, t_last_ms + 3, 0.0);
+    *held = p->in.cap + p->vals.cap + p->err.cap;
+    return H2V_OK;
+}
+size_t witness_eval_bytes(const h2v_witness_program *p) { return sizeof(fe) * (p->plan.n_inputs * 2 + p->n_computed) + 8; }
+int witness_generate_dev(h2v_witness_program *p, cudaStream_t st, size_t B, const uint64_t *inputs, fe *adv, fe *inst, size_t inst_stride,
+                         uint64_t *inst_host, size_t *bad_w) {
+    *bad_w = B;
+    H2V_TRY(ensure_eval(p, B));
+    uint64_t code = 0;
+    H2V_TRY(run_group(p, st, B, inputs, adv, inst, inst_stride, nullptr, inst_host, bad_w, &code, t_last_ms));
+    if (*bad_w < B) return failf(H2V_EINVAL, "%s (cell %llu)", werr_text((uint32_t)(code & 255)), (unsigned long long)(code >> 8));
+    return H2V_OK;
+}
 int witness_program_make(WitnessPlan &&plan, h2v_witness_program **out) {
     h2v_witness_program *p = new (std::nothrow) h2v_witness_program();
     if (!p) return failf(H2V_ENOMEM, "witness_program_new: out of host memory");
@@ -436,7 +472,7 @@ int h2v_witness_generate(h2v_witness_program_t p, size_t n_witnesses, size_t n_i
     if ((n_inputs && !inputs) || !advice_out || (p->plan.n_instances && !instances_out)) return failf(H2V_EINVAL, "witness_generate: NULL argument");
     for (size_t w = 0; w < n_witnesses; ++w)
         for (size_t i = 0; i < n_inputs; ++i)
-            if (!reduced(inputs + 4 * (w * n_inputs + i)))
+            if (!fr_reduced(inputs + 4 * (w * n_inputs + i)))
                 return failf(H2V_EINVAL, "witness_generate: witness %zu: input %zu is not a reduced Montgomery value", w, i);
     std::lock_guard<std::mutex> lock(p->mu);
     const int dev = p->uploaded ? p->dev : current_device();

@@ -428,8 +428,36 @@ int h2v_witness_program_inputs(h2v_witness_program_t p, uint64_t *out);
  * and the program stays usable.  Witnesses run in groups as h2v_create_proofs' do (H2V_PROOF_GROUP, else what fits). */
 int h2v_witness_generate(h2v_witness_program_t p, size_t n_witnesses, size_t n_inputs, const uint64_t *inputs, uint64_t *advice_out,
                          uint64_t *instances_out);
-/* the calling process's last h2v_witness_generate, ms: upload, evaluation + gather, download */
+/* the calling process's last h2v_witness_generate, ms: upload, evaluation + gather, download.  After
+ * h2v_create_proofs_from_inputs / h2v_pk_mock_prover_from_inputs: the inputs' upload, evaluation + gather, and the
+ * download of the instances, summed over the call's groups */
 int h2v_witness_last_ms(double out[3]);
+
+/* Proofs and mock checks straight from inputs: the program's columns are generated in the key's workspace on the key's
+ * device and never cross to the host; only the inputs, the instances and the results do.
+ *   Equal bytes: proof p (at proofs_out + p * proof_stride) is byte for byte what h2v_create_proofs gives on the columns
+ *   h2v_witness_generate(prog, ...) gives for inputs + p * n_inputs * 4, with rng_seeds + 32 p; instances_out (may be
+ *   NULL) receives h2v_witness_generate's instances, n_proofs x instances x 4 limbs, the public inputs the verifier needs.
+ *   The mock call's failures_out + w * cap and n_failures[w] are what h2v_pk_mock_prover gives on those columns.
+ *   Argument checks, all before any device work (H2V_EINVAL, the text starts with the call's name): NULL key, program or
+ *   buffers; n_inputs differs from the program's; an input is not a reduced Montgomery value; the program's k or advice
+ *   column count differs from the key's; the instances do not fit (the key must have one instance column with at least
+ *   as many usable rows as the program has instances, or no instance column and a program without instances);
+ *   proof_stride < h2v_proof_size(pk); the program is already resident on a device other than the key's.
+ *   A witness whose values make the recorded circuit panic fails the call with h2v_witness_generate's text naming the
+ *   lowest such witness ("create_proofs_from_inputs: witness 2: attempt to divide by zero (cell N)"); proofs_out is then
+ *   unspecified, and the key and the program stay usable.
+ *   The caller's responsibility: the key is loaded from the recording's layout (its fixed and sigma columns).  This is
+ *   not checked: a mismatched key gives proofs that do not verify, as wrong advice does; the mock call finds it.
+ *   The program is uploaded to the key's device on first use and runs on the key's stream; the buffers of generated
+ *   columns h2v_witness_generate keeps are released.  Groups as h2v_create_proofs / h2v_pk_mock_prover form them, each
+ *   witness also counting the program's evaluation (inputs, computed values, error word).  h2v_pk_last_phase_ms phase 0
+ *   covers generation, blinding rows and advice commitments; h2v_mock_last_ms out[0] the generation.  n = 0 does nothing.
+ *   Calls on one key serialise; lock order: the key, then the program. */
+int h2v_create_proofs_from_inputs(h2v_pk_t pk, h2v_witness_program_t prog, size_t n_proofs, size_t n_inputs, const uint64_t *inputs,
+                                  const uint8_t *rng_seeds, uint8_t *proofs_out, size_t proof_stride, uint64_t *instances_out);
+int h2v_pk_mock_prover_from_inputs(h2v_pk_t pk, h2v_witness_program_t prog, size_t n_witnesses, size_t n_inputs, const uint64_t *inputs,
+                                   h2v_mock_failure_t *failures_out, size_t cap, uint64_t *n_failures);
 
 /* ---- Fiat-Shamir transcript, RNG ("next": SURVEY.md 8(f) row 3; host-side, no device needed) ---------------------
  * snark-verifier PoseidonTranscript<G1Affine, NativeLoader, Vec<u8>, T = 5, RATE = 4, R_F = 8, R_P = 60>::new::<0>

@@ -272,6 +272,8 @@ struct MockProver {
     }
 };
 
+class WitnessProgram;
+
 // halo2 ProvingKey for a halo2-base-shaped constraint system + create_proof (plonk/prover.rs), resident on the device
 class ProvingKey {
   public:
@@ -356,6 +358,13 @@ class ProvingKey {
         }
         return out;
     }
+    // create_proofs on the columns program.generate gives for inputs (n_proofs x n_inputs values), generated in this key's
+    // workspace without crossing to the host (h2v_create_proofs_from_inputs); instances: n_proofs x program.n_instances()
+    std::vector<std::vector<uint8_t>> create_proofs_from_inputs(const WitnessProgram &program, size_t n_proofs, const std::vector<Fr> &inputs,
+                                                                const std::vector<std::array<uint8_t, 32>> &rng_seeds, std::vector<Fr> &instances) const;
+    // mock_prover on the same generated columns (h2v_pk_mock_prover_from_inputs)
+    std::vector<MockProver> mock_prover_from_inputs(const WitnessProgram &program, size_t n_witnesses, const std::vector<Fr> &inputs,
+                                                    size_t max_failures = 64) const;
 
   private:
     h2v_pk_t h_ = nullptr;
@@ -375,6 +384,7 @@ class WitnessProgram {
     size_t n_inputs() const { return (size_t)info_[0]; }
     size_t n_advice() const { return (size_t)info_[4]; }
     size_t n_instances() const { return (size_t)info_[5]; }
+    h2v_witness_program_t handle() const { return h_; }
     // inputs: n_witnesses x n_inputs values -> advice (n_witnesses x n_advice x 2^k) and instances (n_witnesses x n_instances)
     void generate(size_t n_witnesses, const std::vector<Fr> &inputs, std::vector<Fr> &advice, std::vector<Fr> &instances) const {
         if (inputs.size() != n_witnesses * n_inputs()) throw std::invalid_argument("witness_generate: inputs.size() != n_witnesses * n_inputs");
@@ -388,5 +398,37 @@ class WitnessProgram {
     h2v_witness_program_t h_ = nullptr;
     uint64_t info_[8] = {};
 };
+
+inline std::vector<std::vector<uint8_t>> ProvingKey::create_proofs_from_inputs(const WitnessProgram &program, size_t n_proofs,
+                                                                               const std::vector<Fr> &inputs,
+                                                                               const std::vector<std::array<uint8_t, 32>> &rng_seeds,
+                                                                               std::vector<Fr> &instances) const {
+    if (inputs.size() != n_proofs * program.n_inputs() || rng_seeds.size() != n_proofs)
+        throw std::invalid_argument("create_proofs_from_inputs: inputs.size() != n_proofs * n_inputs or rng_seeds.size() != n_proofs");
+    std::vector<uint8_t> seeds(32 * n_proofs);
+    for (size_t p = 0; p < n_proofs; ++p) std::copy(rng_seeds[p].begin(), rng_seeds[p].end(), seeds.begin() + 32 * p);
+    instances.resize(n_proofs * program.n_instances());
+    const size_t size = h2v_proof_size(h_);
+    std::vector<uint8_t> flat(n_proofs * size);
+    check(h2v_create_proofs_from_inputs(h_, program.handle(), n_proofs, program.n_inputs(), inputs.empty() ? nullptr : &inputs[0].l[0],
+                                        seeds.data(), flat.data(), size, instances.empty() ? nullptr : &instances[0].l[0]));
+    std::vector<std::vector<uint8_t>> out(n_proofs);
+    for (size_t p = 0; p < n_proofs; ++p) out[p].assign(flat.begin() + p * size, flat.begin() + (p + 1) * size);
+    return out;
+}
+inline std::vector<MockProver> ProvingKey::mock_prover_from_inputs(const WitnessProgram &program, size_t n_witnesses, const std::vector<Fr> &inputs,
+                                                                   size_t max_failures) const {
+    if (inputs.size() != n_witnesses * program.n_inputs()) throw std::invalid_argument("mock_prover_from_inputs: inputs.size() != n_witnesses * n_inputs");
+    std::vector<h2v_mock_failure_t> flat(n_witnesses * max_failures);
+    std::vector<uint64_t> totals(n_witnesses);
+    check(h2v_pk_mock_prover_from_inputs(h_, program.handle(), n_witnesses, program.n_inputs(), inputs.empty() ? nullptr : &inputs[0].l[0],
+                                         flat.data(), max_failures, totals.data()));
+    std::vector<MockProver> out(n_witnesses);
+    for (size_t w = 0; w < n_witnesses; ++w) {
+        out[w].n_failures = totals[w];
+        out[w].failures.assign(flat.begin() + w * max_failures, flat.begin() + w * max_failures + (size_t)std::min<uint64_t>(max_failures, totals[w]));
+    }
+    return out;
+}
 
 }  // namespace h2v_host

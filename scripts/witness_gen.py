@@ -6,10 +6,13 @@ on the reference examples (distances and query at k = 13, kmeans at k = 16) and,
 
 For every example: one recording, one program; then for every B, B distinct inputs (the recording's, shifted by w / 64)
 are generated in one call (after a warm-up call) and built on the host one by one, and every generated witness is
-checked byte for byte against the host's.  Then inputs -> proofs both ways: host builder + layout per witness then
-create_proofs, against generate then create_proofs, in chunks of 8 witnesses.  Prints one JSON line: per example and B the host and GPU seconds per
-witness, the program's levels, cells and folded share, generate's upload / evaluate / download ms, proofs per second of
-both flows, and the GPU's name and power limit read in the same run."""
+checked byte for byte against the host's.  Then inputs -> proofs three ways, each over all B witnesses in chunks of 8
+with the same seeds: host builder + layout per witness then create_proofs; generate then create_proofs; and
+create_proofs_from_inputs, which generates the columns in the key's workspace (no columns on the host).  The proofs of
+the three flows must be equal.  Prints one JSON line: per example and B the host and GPU seconds per witness, the
+program's levels, cells and folded share, generate's upload / evaluate / download ms, proofs per second of the three
+flows, the new flow's phase-0 and generation ms, and the GPU's name and power limit read in the same run.  --out PATH
+also rewrites that JSON to PATH after every line, so that a run that ends early keeps what it measured."""
 import argparse
 import json
 import os
@@ -41,6 +44,7 @@ def main():
     ap.add_argument("--batches", nargs="+", type=int, default=[1, 8, 32])
     ap.add_argument("--sift", action="store_true")
     ap.add_argument("--no-proofs", action="store_true")
+    ap.add_argument("--out", default=None)
     args = ap.parse_args()
 
     import random
@@ -53,7 +57,9 @@ def main():
     if h.lib().h2v_device_count() < 1:
         raise SystemExit("witness_gen.py measures on a GPU; none is visible")
     h.init(0)
-    res = {"what": "witness generation: host builder + RangeCircuit vs WitnessProgram.generate", **gpu_info(), "examples": {}}
+    res = {"what": "witness generation: host builder + RangeCircuit vs WitnessProgram.generate; inputs -> proofs three ways",
+           "command": f"scripts/witness_gen.py --names {' '.join(args.names)} --batches {' '.join(map(str, args.batches))}"
+                      + (" --sift" if args.sift else "") + (" --no-proofs" if args.no_proofs else ""), **gpu_info(), "examples": {}}
     cases = [(name, Z.EXAMPLES[name], Z.example_input(name), *Z.EXAMPLE_PARAMS[name]) for name in args.names]
     if args.sift:
         rnd = random.Random(20)
@@ -102,25 +108,39 @@ def main():
             row = {"host_s_per_witness": round(t_host / B, 5), "generate_s_per_witness": round(t_gen / B, 5),
                    "generate_ms": {"upload": round(ms[0], 3), "evaluate_gather": round(ms[1], 3), "download": round(ms[2], 3)},
                    "bytes_equal": same}
-            if pk is not None:      # inputs -> proofs, in chunks of at most 8 witnesses both ways (host memory)
+            if pk is not None:      # inputs -> proofs, each flow in chunks of at most 8 witnesses (host memory)
                 seeds = [bytes([w % 256]) * 32 for w in range(B)]
-                p_host, p_gen, t_host_e2e, t_gen_e2e = [], [], 0.0, 0.0
-                for c0 in range(0, B, 8):
-                    chunk, sd = ins[c0:c0 + 8], seeds[c0:c0 + 8]
+                chunks = [(ins[c0:c0 + 8], seeds[c0:c0 + 8]) for c0 in range(0, B, 8)]
+                p_host, p_gen, p_dev, t_host_e2e, t_gen_e2e, t_dev_e2e, phase0, wms = [], [], [], 0.0, 0.0, 0.0, 0.0, [0.0] * 3
+                for chunk, sd in chunks:
                     t0 = time.perf_counter()
                     hs = [Z.create_circuit(f, v, k, bits)[0] for v in chunk]
                     p_host += pk.create_proofs([rc.advice for rc in hs], [rc.instances for rc in hs], sd)
                     t_host_e2e += time.perf_counter() - t0
                     del hs
+                for chunk, sd in chunks:
                     t0 = time.perf_counter()
                     g = prog.generate([leaves(v) for v in chunk])
                     p_gen += pk.create_proofs([a for a, _ in g], [i for _, i in g], sd)
                     t_gen_e2e += time.perf_counter() - t0
                     del g
+                for chunk, sd in chunks:
+                    t0 = time.perf_counter()
+                    p_dev += pk.create_proofs_from_inputs(prog, [leaves(v) for v in chunk], sd)[0]
+                    t_dev_e2e += time.perf_counter() - t0
+                    phase0 += pk.last_phase_ms()["advice_commit"]
+                    wms = [a + b for a, b in zip(wms, prog.last_ms())]
                 row.update(proofs_per_s_host=round(B / t_host_e2e, 3), proofs_per_s_generate=round(B / t_gen_e2e, 3),
-                           proofs_equal=p_host == p_gen)
+                           proofs_per_s_from_inputs=round(B / t_dev_e2e, 3), from_inputs_phase0_ms=round(phase0, 3),
+                           from_inputs_generate_ms={"upload": round(wms[0], 3), "evaluate_gather": round(wms[1], 3),
+                                                    "instances_download": round(wms[2], 3)},
+                           proofs_equal=p_host == p_gen == p_dev)
             ex["batches"][str(B)] = row
+            res["examples"][name] = ex
             print(json.dumps({name: {str(B): row}}), file=sys.stderr, flush=True)
+            if args.out:
+                with open(args.out, "w") as fo:
+                    json.dump(res, fo, indent=1)
         if pk is not None:
             pk.close()
             srs.close()
