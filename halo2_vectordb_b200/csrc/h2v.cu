@@ -31,12 +31,10 @@ namespace {
 
 thread_local std::string g_err;
 // The devices this process drives (h2v_init): handles hold one replica per device, `_dev` entry points run on the device
-// that owns their buffers, host-facing batch entry points split their columns across all of them.  t_dev is the device
-// the calling thread's current entry point runs on (-1: the primary device, g_devs[0]).
+// that owns their buffers, host-facing batch entry points split their columns across all of them.  Every entry point
+// picks its device once and passes it down; g_devs[0] is the primary device.
 #define H2V_MAX_DEV 16
 std::vector<int> g_devs = {0};
-thread_local int t_dev = -1;
-int cur_dev() { return t_dev >= 0 ? t_dev : g_devs[0]; }
 // the device a device pointer lives on (the primary one for anything the runtime does not know)
 int device_of(const void *p) {
     cudaPointerAttributes at;
@@ -64,9 +62,47 @@ void count_launches(uint64_t n) { g_launches.fetch_add(n, std::memory_order_rela
 int current_device() { return g_devs[0]; }
 }  // namespace h2v
 namespace {
-int use_device() {
-    cudaError_t e = cudaSetDevice(cur_dev());
-    if (e != cudaSuccess) return failf(H2V_ECUDA, "cudaSetDevice(%d): %s (libh2v has no CPU fallback)", cur_dev(), cudaGetErrorString(e));
+struct MsmWorkspace {
+    DevBuf buf;
+};
+// The polynomial primitives' stream and buffers on one device (their calls serialise on mu)
+struct PolyCtx {
+    std::mutex mu;
+    cudaStream_t st = nullptr;
+    DevBuf a, b, c, d, e, tree;
+};
+// What the calls without a handle keep on one device: the polynomial primitives, the MSM over caller-supplied bases
+// (h2v_best_multiexp, h2v_g1_sum), h2v_best_fft, and the kernel attributes set once per device
+struct DevCtx {
+    PolyCtx poly;
+    struct {
+        std::mutex mu;
+        MsmWorkspace ws;
+        DevBuf sc, pts, outb;
+        cudaStream_t st = nullptr;
+    } raw;
+    struct {
+        std::mutex mu;
+        DevBuf A, B, TW;
+        cudaStream_t st = nullptr;
+        fe cached_omega;
+        int cached_L = -1;
+    } fft;
+    std::once_flag ntt_attr, tree_attr;
+};
+// One DevCtx per visible device: a `_dev` call runs on the device that owns its buffers, listed in h2v_init or not.
+// NULL (error recorded) for an ordinal outside the table.
+DevCtx *dev_ctx(int dev) {
+    static std::vector<DevCtx> table(std::max(0, h2v_device_count()));
+    if (dev >= 0 && dev < (int)table.size()) return &table[dev];
+    failf(H2V_EINVAL, "device %d is not a visible CUDA device", dev);
+    return nullptr;
+}
+// make `dev` the calling thread's device; *cx <- its DevCtx when asked for
+int use_device(int dev, DevCtx **cx = nullptr) {
+    cudaError_t e = cudaSetDevice(dev);
+    if (e != cudaSuccess) return failf(H2V_ECUDA, "cudaSetDevice(%d): %s (libh2v has no CPU fallback)", dev, cudaGetErrorString(e));
+    if (cx && !(*cx = dev_ctx(dev))) return H2V_EINVAL;
     return H2V_OK;
 }
 
@@ -152,7 +188,6 @@ template <class Rep> typename Rep::Lane *lock_lane(Rep *r) {
 
 // ================================================================== NTT host side
 const size_t NTT_SMEM_BYTES = (2 * 2048 + H2V_NTT_PLANE_PAD) * 16;
-std::once_flag g_ntt_attr_once[H2V_MAX_DEV];      // function attributes are per device
 
 struct NttPlan {
     int P;
@@ -167,13 +202,15 @@ NttPlan ntt_plan(int L) {
     return pl;
 }
 
-// dst != src.  Columns are independent; pass 0 goes src -> dst, later passes run in place on dst.
-int run_ntt(cudaStream_t st, const fe *src, size_t src_stride, fe *dst, size_t dst_stride, int L, const fe *tw,
+// dst != src, both on device `dev`.  Columns are independent; pass 0 goes src -> dst, later passes run in place on dst.
+int run_ntt(int dev, cudaStream_t st, const fe *src, size_t src_stride, fe *dst, size_t dst_stride, int L, const fe *tw,
             const fe *pre, uint32_t pre_mod, uint32_t n_in, const fe *post, uint32_t post_mod, uint32_t n_out,
             size_t n_cols, uint32_t post_shift = 0) {
     if (n_cols == 0) return H2V_OK;
     if ((const void *)src == (const void *)dst) return failf(H2V_EINVAL, "run_ntt: in-place transform needs distinct buffers");
-    std::call_once(g_ntt_attr_once[cur_dev()], [] {
+    DevCtx *cx = dev_ctx(dev);
+    if (!cx) return H2V_EINVAL;
+    std::call_once(cx->ntt_attr, [] {      // function attributes are per device
         cudaFuncSetAttribute(ntt_pass_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NTT_SMEM_BYTES);
         cudaFuncSetAttribute(ntt_pass_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NTT_SMEM_BYTES);
     });
@@ -305,8 +342,8 @@ DomRep *dom_on(h2v_domain *h, int dev) {
         if (r->dev == dev) return r;
     return nullptr;
 }
-// the replica a call on `h` runs on, made the calling thread's device: the one on the device that holds `ptr`, the primary
-// one for host columns (ptr = NULL).  NULL (error recorded) when there is none.
+// the replica a call on `h` runs on: the one on the device that holds `ptr`, the primary one for host columns
+// (ptr = NULL).  NULL (error recorded) when there is none.
 DomRep *dom_rep(h2v_domain *h, const void *ptr) {
     if (!h) {
         failf(H2V_EINVAL, "NULL domain");
@@ -314,7 +351,6 @@ DomRep *dom_rep(h2v_domain *h, const void *ptr) {
     }
     DomRep *r = ptr ? dom_on(h, device_of(ptr)) : h->rep[0];
     if (!r) failf(H2V_EINVAL, "the columns live on device %d, which is not in the h2v_init list", device_of(ptr));
-    else t_dev = r->dev;
     return r;
 }
 
@@ -341,19 +377,19 @@ int domain_op_dev(DomRep *d, cudaStream_t st, int op, const fe *in, size_t in_st
     switch (op) {
     case H2V_OP_LAGRANGE_TO_COEFF:
         if ((rc = domain_twiddles(d, 1, &tw))) return rc;
-        return run_ntt(st, in, in_stride, out, out_stride, d->k, tw, nullptr, 1, n, dc + 3, 1, n, n_cols, (uint32_t)d->k);      // 1/n = 2^-k
+        return run_ntt(d->dev, st, in, in_stride, out, out_stride, d->k, tw, nullptr, 1, n, dc + 3, 1, n, n_cols, (uint32_t)d->k);      // 1/n = 2^-k
     case H2V_OP_COEFF_TO_LAGRANGE:
         if ((rc = domain_twiddles(d, 0, &tw))) return rc;
-        return run_ntt(st, in, in_stride, out, out_stride, d->k, tw, nullptr, 1, n, nullptr, 1, n, n_cols);
+        return run_ntt(d->dev, st, in, in_stride, out, out_stride, d->k, tw, nullptr, 1, n, nullptr, 1, n, n_cols);
     case H2V_OP_COEFF_TO_EXTENDED:
         if ((rc = domain_twiddles(d, 2, &tw))) return rc;
-        return run_ntt(st, in, in_stride, out, out_stride, d->ek, tw, dc, 3, n, nullptr, 1, en, n_cols);
+        return run_ntt(d->dev, st, in, in_stride, out, out_stride, d->ek, tw, dc, 3, n, nullptr, 1, en, n_cols);
     case H2V_OP_EXTENDED_TO_COEFF:
         if ((rc = domain_twiddles(d, 3, &tw))) return rc;
-        return run_ntt(st, in, in_stride, out, out_stride, d->ek, tw, nullptr, 1, en, dc + 4, 3, n * (d->j - 1), n_cols);
+        return run_ntt(d->dev, st, in, in_stride, out, out_stride, d->ek, tw, nullptr, 1, en, dc + 4, 3, n * (d->j - 1), n_cols);
     case H2V_OP_DIVIDE_BY_VANISHING:
         if ((rc = domain_twiddles(d, 3, &tw))) return rc;
-        return run_ntt(st, in, in_stride, out, out_stride, d->ek, tw, dc + 8, d->nt, en, dc + 4, 3, n * (d->j - 1), n_cols);
+        return run_ntt(d->dev, st, in, in_stride, out, out_stride, d->ek, tw, dc + 8, d->nt, en, dc + 4, 3, n * (d->j - 1), n_cols);
     default:
         return failf(H2V_EINVAL, "unknown domain op %d", op);
     }
@@ -416,9 +452,6 @@ void fill_kadd(MsmShape &sh) {
     for (int i = 0; i < 9; ++i) sh.kadd[i] = k[i];
 }
 
-struct MsmWorkspace {
-    DevBuf buf;
-};
 struct Carver {
     char *base;
     size_t off = 0;
@@ -494,7 +527,6 @@ MsmLayout msm_layout(void *base, const MsmShape &sh, uint32_t cols) {
 }
 
 const size_t MSM_WS_BUDGET = (size_t)16 << 30;   // per handle; columns per launch are sized to fit
-std::once_flag g_tree_attr_once[H2V_MAX_DEV];
 
 // the two passes over the scalars are instantiated per window size (compile-time limb indices and shifts)
 template <int C> struct WindowDispatch {
@@ -539,10 +571,10 @@ MsmShape make_shape(size_t len, const MsmCfg &cfg, size_t pstride) {
     return sh;
 }
 
-// d_scalars: n_cols columns of `len` Fr (Montgomery), col_stride apart.  points: bases (raw) or
+// d_scalars: n_cols columns of `len` Fr (Montgomery), col_stride apart, on device `dev`.  points: bases (raw) or
 // window tables (precomputed, level stride `pstride`).  Results: affine and/or Jacobian per column.
 // `density` in (0, 1]: expected share of non-zero digits (sizes the accumulate chunks; 1 = uniform scalars).
-int run_msm(cudaStream_t st, MsmWorkspace &ws, const fe *d_scalars, size_t col_stride, size_t n_cols, size_t len,
+int run_msm(int dev, cudaStream_t st, MsmWorkspace &ws, const fe *d_scalars, size_t col_stride, size_t n_cols, size_t len,
             const affine *points, MsmCfg cfg, size_t pstride, affine *d_out_aff, jacobian *d_out_jac, Timer *tm, double density = 1.0) {
     if (n_cols == 0) return H2V_OK;
     if (len == 0) {   // empty sum = identity: affine (0, 0); Jacobian (0, 1, 0) as halo2curves `G1::identity()`
@@ -577,7 +609,9 @@ int run_msm(cudaStream_t st, MsmWorkspace &ws, const fe *d_scalars, size_t col_s
         int rc = ws.buf.ensure(probe.bytes);
         if (rc) return rc;
     }
-    std::call_once(g_tree_attr_once[cur_dev()], [] {
+    DevCtx *cx = dev_ctx(dev);
+    if (!cx) return H2V_EINVAL;
+    std::call_once(cx->tree_attr, [] {
         cudaFuncSetAttribute(msm_reduce_tree_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * H2V_TREE_MAX * sizeof(xyzz)));
     });
     for (size_t c0 = 0; c0 < n_cols; c0 += max_cols) {
@@ -699,7 +733,7 @@ struct SrsRep {
     MsmCfg cfg[2];
     MsmWorkspace ws, ws2;
     DevBuf stage, out;
-    DevBuf peer_stage, peer_out;      // columns of another device's batch pulled over NVLink (h2v_commit_batch_dev with several devices)
+    DevBuf peer_in, peer_out;      // columns of another device's batch and their commitments (several devices)
     std::mutex peer_mu;               // held from the pull to the write-back
     cudaStream_t stream = nullptr, stream2 = nullptr, copy_stream = nullptr, up_stream = nullptr;
     cudaEvent_t copied[2] = {nullptr, nullptr}, computed[2] = {nullptr, nullptr};
@@ -763,7 +797,7 @@ int msm_srs(SrsRep *s, cudaStream_t st, MsmWorkspace &ws, int basis, const fe *d
         }
     }
     s->last_variant = variant;
-    return run_msm(st, ws, d_scalars, col_stride, n_cols, len, s->table[basis][variant].as<affine>(), s->cfg[variant], s->n, d_out, nullptr, tm,
+    return run_msm(s->dev, st, ws, d_scalars, col_stride, n_cols, len, s->table[basis][variant].as<affine>(), s->cfg[variant], s->n, d_out, nullptr, tm,
                    density);
 }
 }  // namespace
@@ -816,7 +850,6 @@ int h2v_init(const int *devices, int n_dev) {
             }
         }
     g_devs = devs;
-    t_dev = -1;
     H2V_CU(cudaSetDevice(g_devs[0]));
     return H2V_OK;
 }
@@ -853,9 +886,7 @@ int h2v_fr_to_repr(const uint64_t *fr_mont, size_t n, uint8_t *out) {
     return H2V_OK;
 }
 int h2v_dev_alloc(size_t bytes, void **d_out) {
-    t_dev = -1;
-    int rc = use_device();
-    if (rc) return rc;
+    H2V_TRY(use_device(g_devs[0]));
     if (!d_out || !bytes) return failf(H2V_EINVAL, "dev_alloc: bad argument");
     cudaError_t e = cudaMalloc(d_out, bytes);
     if (e != cudaSuccess) {
@@ -865,40 +896,30 @@ int h2v_dev_alloc(size_t bytes, void **d_out) {
     return H2V_OK;
 }
 int h2v_dev_free(void *d_ptr) {
-    t_dev = device_of(d_ptr);
-    int rc = use_device();
-    if (rc) return rc;
+    H2V_TRY(use_device(device_of(d_ptr)));
     if (d_ptr) H2V_CU(cudaFree(d_ptr));
     return H2V_OK;
 }
 int h2v_dev_upload(void *d_dst, const void *src, size_t bytes) {
-    t_dev = device_of(d_dst);
-    int rc = use_device();
-    if (rc) return rc;
+    H2V_TRY(use_device(device_of(d_dst)));
     if (bytes && (!d_dst || !src)) return failf(H2V_EINVAL, "dev_upload: NULL buffer");
     H2V_CU(cudaMemcpy(d_dst, src, bytes, cudaMemcpyHostToDevice));
     return H2V_OK;
 }
 int h2v_dev_download(void *dst, const void *d_src, size_t bytes) {
-    t_dev = device_of(d_src);
-    int rc = use_device();
-    if (rc) return rc;
+    H2V_TRY(use_device(device_of(d_src)));
     if (bytes && (!dst || !d_src)) return failf(H2V_EINVAL, "dev_download: NULL buffer");
     H2V_CU(cudaMemcpy(dst, d_src, bytes, cudaMemcpyDeviceToHost));
     return H2V_OK;
 }
 int h2v_host_register(void *ptr, size_t bytes) {
-    t_dev = -1;
-    int rc = use_device();
-    if (rc) return rc;
+    H2V_TRY(use_device(g_devs[0]));
     if (!ptr || !bytes) return failf(H2V_EINVAL, "host_register: bad argument");
     H2V_CU(cudaHostRegister(ptr, bytes, cudaHostRegisterDefault));
     return H2V_OK;
 }
 int h2v_host_unregister(void *ptr) {
-    t_dev = -1;
-    int rc = use_device();
-    if (rc) return rc;
+    H2V_TRY(use_device(g_devs[0]));
     H2V_CU(cudaHostUnregister(ptr));
     return H2V_OK;
 }
@@ -916,14 +937,13 @@ int h2v_last_kernel_ms(float out[8]) {
 
 // ---------------------------------------------------------------- SRS / commit
 static void rep_srs_free(SrsRep *s);
-static int rep_srs_load(uint32_t k, const uint64_t *g, const uint64_t *g_lagrange, SrsRep **out) {
-    if (!out) return failf(H2V_EINVAL, "h2v_srs_load: out is NULL");
-    *out = nullptr;
+// the replica on device `dev` built from the host bases: the window tables are computed there
+static int rep_srs_load(int dev, uint32_t k, const uint64_t *g, const uint64_t *g_lagrange, SrsRep **out) {
     if (k > 26) return failf(H2V_EINVAL, "h2v_srs_load: k = %u unsupported", k);
-    int rc = use_device();
+    int rc = use_device(dev);
     if (rc) return rc;
     SrsRep *s = new SrsRep();
-    s->dev = cur_dev();
+    s->dev = dev;
     s->k = k;
     s->n = (size_t)1 << k;
     s->cfg[0] = choose_cfg(s->n, true);
@@ -981,7 +1001,7 @@ int h2v_srs_info(h2v_srs_t h, uint32_t *window_bits, uint32_t *windows) {
 }
 static void rep_srs_free(SrsRep *s) {
     if (!s) return;
-    cudaSetDevice(cur_dev());
+    cudaSetDevice(s->dev);
     for (auto &tb : s->table)
         for (auto &t : tb) t.release();
     s->ws.buf.release();
@@ -994,7 +1014,7 @@ static void rep_srs_free(SrsRep *s) {
     }
     s->stage.release();
     s->out.release();
-    s->peer_stage.release();
+    s->peer_in.release();
     s->peer_out.release();
     if (s->stream) cudaStreamDestroy(s->stream);
     if (s->up_stream) cudaStreamDestroy(s->up_stream);
@@ -1016,7 +1036,7 @@ static int rep_commit_batch_dev(SrsRep *s, int basis, const void *d_polys, size_
     if (!s->have[basis]) return failf(H2V_EINVAL, "commit: basis %d was not loaded", basis);
     if (len > s->n) return failf(H2V_EINVAL, "commit: poly length %zu exceeds n = %zu", len, s->n);
     if (n_polys && (!d_polys || !d_out_affine)) return failf(H2V_EINVAL, "commit: NULL buffer");
-    H2V_TRY(use_device());
+    H2V_TRY(use_device(s->dev));
     t_entry_launches = 0;
     int rc = sync_call(s->mu, s->stream, -1, "commit", [&](Timer &tm) {
         return msm_srs(s, s->stream, s->ws, basis, (const fe *)d_polys, col_stride, n_polys, len, (affine *)d_out_affine, &tm);
@@ -1033,7 +1053,7 @@ static int rep_commit_batch(SrsRep *s, int basis, const uint64_t *const *polys, 
     if (len > s->n) return failf(H2V_EINVAL, "commit: poly length %zu exceeds n = %zu", len, s->n);
     if (n_polys == 0) return H2V_OK;
     if (!polys || !out_affine) return failf(H2V_EINVAL, "commit: NULL buffer");
-    int rc = use_device();
+    int rc = use_device(s->dev);
     if (rc) return rc;
     const size_t stride_small = std::max<size_t>(len, 1);
     if (n_polys * stride_small * sizeof(fe) <= ((size_t)48 << 20)) {
@@ -1122,22 +1142,14 @@ static int rep_commit_batch(SrsRep *s, int basis, const uint64_t *const *polys, 
 
 // one MSM over caller-supplied bases (no handle, no tables): Jacobian and / or affine result
 static int multiexp_raw(const uint64_t *coeffs, const uint64_t *bases, size_t n, uint64_t *out_jacobian, uint64_t *out_affine) {
-    t_dev = -1;
-    int rc = use_device();
+    const int dev = g_devs[0];
+    DevCtx *cx;
+    int rc = use_device(dev, &cx);
     if (rc) return rc;
-    struct RawCtx {
-        std::mutex mu;
-        MsmWorkspace ws;
-        DevBuf sc, pts, outb;
-        cudaStream_t st = nullptr;
-    };
-    static RawCtx ctxs[H2V_MAX_DEV];
-    RawCtx &cx = ctxs[cur_dev()];
-    std::mutex &mu = cx.mu;
-    MsmWorkspace &ws = cx.ws;
-    DevBuf &sc = cx.sc, &pts = cx.pts, &outb = cx.outb;
-    cudaStream_t &st = cx.st;
-    std::lock_guard<std::mutex> lk(mu);
+    MsmWorkspace &ws = cx->raw.ws;
+    DevBuf &sc = cx->raw.sc, &pts = cx->raw.pts, &outb = cx->raw.outb;
+    cudaStream_t &st = cx->raw.st;
+    std::lock_guard<std::mutex> lk(cx->raw.mu);
     if (!st) H2V_CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
     if ((rc = sc.ensure(n * sizeof(fe)))) return rc;
     if ((rc = pts.ensure(n * sizeof(affine)))) return rc;
@@ -1147,7 +1159,7 @@ static int multiexp_raw(const uint64_t *coeffs, const uint64_t *bases, size_t n,
     MsmCfg cfg = choose_cfg(n, false);
     jacobian *dj = outb.as<jacobian>();
     affine *da = reinterpret_cast<affine *>(dj + 1);
-    rc = run_msm(st, ws, sc.as<fe>(), n, 1, n, pts.as<affine>(), cfg, n, out_affine ? da : nullptr, out_jacobian ? dj : nullptr, nullptr);
+    rc = run_msm(dev, st, ws, sc.as<fe>(), n, 1, n, pts.as<affine>(), cfg, n, out_affine ? da : nullptr, out_jacobian ? dj : nullptr, nullptr);
     if (rc) { cudaStreamSynchronize(st); return rc; }
     if (out_jacobian) H2V_CU(cudaMemcpyAsync(out_jacobian, dj, sizeof(jacobian), cudaMemcpyDeviceToHost, st));
     if (out_affine) H2V_CU(cudaMemcpyAsync(out_affine, da, sizeof(affine), cudaMemcpyDeviceToHost, st));
@@ -1159,9 +1171,7 @@ int h2v_best_multiexp(const uint64_t *coeffs, const uint64_t *bases, size_t n, u
     if (n && (!coeffs || !bases)) return failf(H2V_EINVAL, "best_multiexp: NULL input");
     if (n >= ((size_t)1 << 27)) return failf(H2V_EINVAL, "best_multiexp: n = %zu unsupported", n);
     if (n == 0) {
-        t_dev = -1;
-        int rc = use_device();
-        if (rc) return rc;
+        H2V_TRY(use_device(g_devs[0]));
         jacobian id;      // halo2curves `G1::identity()` = (0, 1, 0)
         id.x = fe_zero(); id.y = fe_one<Fq>(); id.z = fe_zero();
         memcpy(out_jacobian, &id, 96);
@@ -1174,8 +1184,7 @@ int h2v_g1_sum(const uint64_t *affine_pts, size_t n, uint64_t out_affine[8]) {
     if (n && !affine_pts) return failf(H2V_EINVAL, "g1_sum: NULL input");
     if (n >= ((size_t)1 << 27)) return failf(H2V_EINVAL, "g1_sum: n = %zu unsupported", n);
     if (n == 0) {
-        int rc = use_device();
-        if (rc) return rc;
+        H2V_TRY(use_device(g_devs[0]));
         memset(out_affine, 0, 64);
         return H2V_OK;
     }
@@ -1187,24 +1196,15 @@ int h2v_g1_sum(const uint64_t *affine_pts, size_t n, uint64_t out_affine[8]) {
 int h2v_best_fft(uint64_t *a, const uint64_t omega[4], uint32_t log_n) {
     if (!a || !omega) return failf(H2V_EINVAL, "best_fft: NULL argument");
     if (log_n > 27) return failf(H2V_EINVAL, "best_fft: log_n = %u unsupported", log_n);
-    t_dev = -1;
-    int rc = use_device();
+    const int dev = g_devs[0];
+    DevCtx *cx;
+    int rc = use_device(dev, &cx);
     if (rc) return rc;
-    struct FftCtx {
-        std::mutex mu;
-        DevBuf A, B, TW;
-        cudaStream_t st = nullptr;
-        fe cached_omega;
-        int cached_L = -1;
-    };
-    static FftCtx ctxs[H2V_MAX_DEV];
-    FftCtx &cx = ctxs[cur_dev()];
-    std::mutex &mu = cx.mu;
-    DevBuf &A = cx.A, &B = cx.B, &TW = cx.TW;
-    cudaStream_t &st = cx.st;
-    fe &cached_omega = cx.cached_omega;
-    int &cached_L = cx.cached_L;
-    std::lock_guard<std::mutex> lk(mu);
+    DevBuf &A = cx->fft.A, &B = cx->fft.B, &TW = cx->fft.TW;
+    cudaStream_t &st = cx->fft.st;
+    fe &cached_omega = cx->fft.cached_omega;
+    int &cached_L = cx->fft.cached_L;
+    std::lock_guard<std::mutex> lk(cx->fft.mu);
     if (!st) H2V_CU(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
     size_t n = (size_t)1 << log_n;
     if ((rc = A.ensure(n * sizeof(fe)))) return rc;
@@ -1216,7 +1216,7 @@ int h2v_best_fft(uint64_t *a, const uint64_t omega[4], uint32_t log_n) {
         cached_omega = w;
     }
     H2V_CU(cudaMemcpyAsync(A.p, a, n * sizeof(fe), cudaMemcpyHostToDevice, st));
-    rc = run_ntt(st, A.as<fe>(), n, B.as<fe>(), n, (int)log_n, TW.as<fe>(), nullptr, 1, (uint32_t)n, nullptr, 1, (uint32_t)n, 1);
+    rc = run_ntt(dev, st, A.as<fe>(), n, B.as<fe>(), n, (int)log_n, TW.as<fe>(), nullptr, 1, (uint32_t)n, nullptr, 1, (uint32_t)n, 1);
     if (rc) { cudaStreamSynchronize(st); return rc; }
     H2V_CU(cudaMemcpyAsync(a, B.p, n * sizeof(fe), cudaMemcpyDeviceToHost, st));
     H2V_CU(cudaStreamSynchronize(st));
@@ -1224,17 +1224,15 @@ int h2v_best_fft(uint64_t *a, const uint64_t omega[4], uint32_t log_n) {
 }
 
 static void rep_domain_free(DomRep *d);
-static int rep_domain_new(uint32_t j, uint32_t k, DomRep **out) {
-    if (!out) return failf(H2V_EINVAL, "domain_new: out is NULL");
-    *out = nullptr;
+static int rep_domain_new(int dev, uint32_t j, uint32_t k, DomRep **out) {
     if (j < 2) return failf(H2V_EINVAL, "domain_new: j = %u (need j >= 2)", j);
     uint32_t ek = k;
     while (((uint64_t)1 << ek) < ((uint64_t)1 << k) * (j - 1)) ++ek;
     if (ek > 27 || ek - k > 6) return failf(H2V_EINVAL, "domain_new: extended_k = %u unsupported", ek);
-    int rc = use_device();
+    int rc = use_device(dev);
     if (rc) return rc;
     DomRep *d = new DomRep();
-    d->dev = cur_dev();
+    d->dev = dev;
     d->j = j;
     d->k = k;
     d->ek = ek;
@@ -1285,7 +1283,7 @@ static int rep_domain_new(uint32_t j, uint32_t k, DomRep **out) {
 }
 static void rep_domain_free(DomRep *d) {
     if (!d) return;
-    cudaSetDevice(cur_dev());
+    cudaSetDevice(d->dev);
     d->dconst.release();
     for (auto &t : d->tw) t.release();
     d->stage_a.release();
@@ -1409,7 +1407,7 @@ static int rep_domain_transform_dev(DomRep *d, int op, const void *d_in, size_t 
     if (in_stride < op_in_len(d, op) || out_stride < work_len)
         return failf(H2V_EINVAL, "transform: stride shorter than the column (out_stride must cover 2^%s)",
                     op >= H2V_OP_COEFF_TO_EXTENDED ? "extended_k" : "k");
-    H2V_TRY(use_device());
+    H2V_TRY(use_device(d->dev));
     return sync_call(d->mu, d->stream, 7, "transform", [&](Timer &) {
         return domain_op_dev(d, d->stream, op, (const fe *)d_in, in_stride, (fe *)d_out, out_stride, n_cols);
     });
@@ -1420,7 +1418,7 @@ static int rep_domain_transform_batch(DomRep *d, int op, const uint64_t *const *
     if (op < 0 || op > H2V_OP_DIVIDE_BY_VANISHING) return failf(H2V_EINVAL, "unknown domain op %d", op);
     if (n_cols == 0) return H2V_OK;
     if (!in || !out) return failf(H2V_EINVAL, "transform: NULL buffer");
-    int rc = use_device();
+    int rc = use_device(d->dev);
     if (rc) return rc;
     const size_t nin = op_in_len(d, op), nout = op_out_len(d, op);
     const size_t out_stride = std::max(nout, (size_t)1 << (op >= H2V_OP_COEFF_TO_EXTENDED ? d->ek : d->k));
@@ -1516,7 +1514,7 @@ int h2v_divide_by_vanishing_poly(h2v_domain_t h, uint64_t *a) {
     DomRep *d = dom_rep(h, nullptr);
     if (!d) return H2V_EINVAL;
     if (!a) return failf(H2V_EINVAL, "divide_by_vanishing_poly: NULL argument");
-    int rc = use_device();
+    int rc = use_device(d->dev);
     if (rc) return rc;
     std::lock_guard<std::mutex> lk(d->mu);
     size_t en = (size_t)1 << d->ek;
@@ -1534,15 +1532,15 @@ int h2v_divide_by_vanishing_poly(h2v_domain_t h, uint64_t *a) {
 
 // ================================================================== polynomial primitives ("next" row 2)
 namespace {
-struct PolyCtx {
-    std::mutex mu;
-    cudaStream_t st = nullptr;
-    DevBuf a, b, c, d, e, tree;
-};
-PolyCtx g_poly_all[H2V_MAX_DEV];
-#define g_poly (g_poly_all[cur_dev()])
-int poly_ctx_ready() {
-    if (!g_poly.st) H2V_CU(cudaStreamCreateWithFlags(&g_poly.st, cudaStreamNonBlocking));
+// the calling thread on device `dev`, *P <- the polynomial context there
+int poly_on(int dev, PolyCtx **P) {
+    DevCtx *cx;
+    H2V_TRY(use_device(dev, &cx));
+    *P = &cx->poly;
+    return H2V_OK;
+}
+int poly_ctx_ready(PolyCtx *P) {      // P->mu held
+    if (!P->st) H2V_CU(cudaStreamCreateWithFlags(&P->st, cudaStreamNonBlocking));
     return H2V_OK;
 }
 // I[i] = 1 / X[i] for n non-zero elements (one inversion in total); X and I are device arrays
@@ -1594,10 +1592,10 @@ int h2v_eval_polynomial_dev(const void *d_polys, size_t stride, size_t n_polys, 
     if (!n_polys || !n_points) return H2V_OK;
     if (!d_polys || !d_points || !d_out) return failf(H2V_EINVAL, "eval_polynomial: NULL buffer");
     if (n_polys > 65535 || n_points > (1u << 20) || len >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "eval_polynomial: batch too large");
-    t_dev = device_of(d_polys);
-    H2V_TRY(use_device());
-    return sync_call(g_poly.mu, g_poly.st, 7, "eval_polynomial", [&](Timer &) {
-        poly_eval_kernel<<<dim3((unsigned)n_points, (unsigned)n_polys), 256, 0, g_poly.st>>>((const fe *)d_polys, stride, (uint32_t)len,
+    PolyCtx *P;
+    H2V_TRY(poly_on(device_of(d_polys), &P));
+    return sync_call(P->mu, P->st, 7, "eval_polynomial", [&](Timer &) {
+        poly_eval_kernel<<<dim3((unsigned)n_points, (unsigned)n_polys), 256, 0, P->st>>>((const fe *)d_polys, stride, (uint32_t)len,
                                                                                            (const fe *)d_points, (uint32_t)n_points, (fe *)d_out);
         H2V_LAUNCHED();
         return H2V_OK;
@@ -1608,29 +1606,29 @@ int h2v_eval_polynomial_batch(const uint64_t *const *polys, size_t n_polys, size
     if (!n_polys || !n_points) return H2V_OK;
     if (!polys || !points || !out) return failf(H2V_EINVAL, "eval_polynomial: NULL buffer");
     if (n_points > (1u << 20) || len >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "eval_polynomial: batch too large");
-    t_dev = -1;
-    int rc = use_device();
+    PolyCtx *P;
+    int rc = poly_on(g_devs[0], &P);
     if (rc) return rc;
-    std::lock_guard<std::mutex> lk(g_poly.mu);
-    if ((rc = poly_ctx_ready())) return rc;
-    cudaStream_t st = g_poly.st;
+    std::lock_guard<std::mutex> lk(P->mu);
+    if ((rc = poly_ctx_ready(P))) return rc;
+    cudaStream_t st = P->st;
     const size_t stride = std::max<size_t>(len, 1);
     size_t per = std::max<size_t>(1, ((size_t)1 << 30) / (stride * sizeof(fe)));
     per = std::min<size_t>(std::min(per, n_polys), 65535);
-    if ((rc = g_poly.a.ensure(per * stride * sizeof(fe))) || (rc = g_poly.b.ensure(n_points * sizeof(fe))) ||
-        (rc = g_poly.c.ensure(per * n_points * sizeof(fe))))
+    if ((rc = P->a.ensure(per * stride * sizeof(fe))) || (rc = P->b.ensure(n_points * sizeof(fe))) ||
+        (rc = P->c.ensure(per * n_points * sizeof(fe))))
         return rc;
-    H2V_CU(cudaMemcpyAsync(g_poly.b.p, points, n_points * sizeof(fe), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(P->b.p, points, n_points * sizeof(fe), cudaMemcpyHostToDevice, st));
     for (size_t c0 = 0; c0 < n_polys; c0 += per) {
         size_t cols = std::min(per, n_polys - c0);
         for (size_t c = 0; c < cols; ++c) {
             if (!polys[c0 + c] && len) return failf(H2V_EINVAL, "eval_polynomial: polys[%zu] is NULL", c0 + c);
-            if (len) H2V_CU(cudaMemcpyAsync(g_poly.a.as<fe>() + c * stride, polys[c0 + c], len * sizeof(fe), cudaMemcpyHostToDevice, st));
+            if (len) H2V_CU(cudaMemcpyAsync(P->a.as<fe>() + c * stride, polys[c0 + c], len * sizeof(fe), cudaMemcpyHostToDevice, st));
         }
-        poly_eval_kernel<<<dim3((unsigned)n_points, (unsigned)cols), 256, 0, st>>>(g_poly.a.as<fe>(), stride, (uint32_t)len, g_poly.b.as<fe>(),
-                                                                                  (uint32_t)n_points, g_poly.c.as<fe>());
+        poly_eval_kernel<<<dim3((unsigned)n_points, (unsigned)cols), 256, 0, st>>>(P->a.as<fe>(), stride, (uint32_t)len, P->b.as<fe>(),
+                                                                                  (uint32_t)n_points, P->c.as<fe>());
         H2V_LAUNCHED();
-        H2V_CU(cudaMemcpyAsync(out + 4 * c0 * n_points, g_poly.c.p, cols * n_points * sizeof(fe), cudaMemcpyDeviceToHost, st));
+        H2V_CU(cudaMemcpyAsync(out + 4 * c0 * n_points, P->c.p, cols * n_points * sizeof(fe), cudaMemcpyDeviceToHost, st));
         H2V_CU(cudaStreamSynchronize(st));
     }
     return H2V_OK;
@@ -1639,46 +1637,47 @@ int h2v_batch_invert(uint64_t *a, size_t n) {
     if (!n) return H2V_OK;
     if (!a) return failf(H2V_EINVAL, "batch_invert: NULL buffer");
     if (n >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "batch_invert: n too large");
-    t_dev = -1;
-    int rc = use_device();
+    PolyCtx *P;
+    int rc = poly_on(g_devs[0], &P);
     if (rc) return rc;
-    std::lock_guard<std::mutex> lk(g_poly.mu);
-    if ((rc = poly_ctx_ready())) return rc;
-    cudaStream_t st = g_poly.st;
-    if ((rc = g_poly.a.ensure(n * sizeof(fe))) || (rc = g_poly.b.ensure(n * sizeof(fe))) || (rc = g_poly.c.ensure(n * sizeof(fe)))) return rc;
-    H2V_CU(cudaMemcpyAsync(g_poly.a.p, a, n * sizeof(fe), cudaMemcpyHostToDevice, st));
+    std::lock_guard<std::mutex> lk(P->mu);
+    if ((rc = poly_ctx_ready(P))) return rc;
+    cudaStream_t st = P->st;
+    if ((rc = P->a.ensure(n * sizeof(fe))) || (rc = P->b.ensure(n * sizeof(fe))) || (rc = P->c.ensure(n * sizeof(fe)))) return rc;
+    H2V_CU(cudaMemcpyAsync(P->a.p, a, n * sizeof(fe), cudaMemcpyHostToDevice, st));
     const unsigned gb = (unsigned)((n + 255) / 256);
-    fr_zero_to_one_kernel<<<gb, 256, 0, st>>>(g_poly.a.as<fe>(), g_poly.b.as<fe>(), (uint32_t)n);
+    fr_zero_to_one_kernel<<<gb, 256, 0, st>>>(P->a.as<fe>(), P->b.as<fe>(), (uint32_t)n);
     H2V_LAUNCHED();
-    if ((rc = run_batch_invert<FrP>(st, g_poly.b.as<fe>(), g_poly.c.as<fe>(), (uint32_t)n, g_poly.tree))) return rc;
-    fr_select_inverse_kernel<<<gb, 256, 0, st>>>(g_poly.a.as<fe>(), g_poly.c.as<fe>(), g_poly.b.as<fe>(), (uint32_t)n);
+    if ((rc = run_batch_invert<FrP>(st, P->b.as<fe>(), P->c.as<fe>(), (uint32_t)n, P->tree))) return rc;
+    fr_select_inverse_kernel<<<gb, 256, 0, st>>>(P->a.as<fe>(), P->c.as<fe>(), P->b.as<fe>(), (uint32_t)n);
     H2V_LAUNCHED();
-    H2V_CU(cudaMemcpyAsync(a, g_poly.b.p, n * sizeof(fe), cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaMemcpyAsync(a, P->b.p, n * sizeof(fe), cudaMemcpyDeviceToHost, st));
     H2V_CU(cudaStreamSynchronize(st));
     return H2V_OK;
 }
 // out[c][0] = 1, out[c][i+1] = out[c][i] * num[c][i] / den[c][i] for `cols` contiguous columns of n elements (device)
-static int run_grand_product(cudaStream_t st, const fe *num, const fe *den, uint32_t n, uint32_t cols, fe *out) {
+static int run_grand_product(PolyCtx *P, const fe *num, const fe *den, uint32_t n, uint32_t cols, fe *out) {
     int rc;
+    const cudaStream_t st = P->st;
     const uint32_t ntiles = (n + H2V_FR_TILE - 1) / H2V_FR_TILE;
     const size_t tot = (size_t)n * cols;
-    if ((rc = g_poly.c.ensure(tot * sizeof(fe))) || (rc = g_poly.e.ensure(tot * sizeof(fe))) ||
-        (rc = g_poly.d.ensure(((size_t)ntiles * cols + 1) * sizeof(fe))))
+    if ((rc = P->c.ensure(tot * sizeof(fe))) || (rc = P->e.ensure(tot * sizeof(fe))) ||
+        (rc = P->d.ensure(((size_t)ntiles * cols + 1) * sizeof(fe))))
         return rc;
     // One inversion for all columns, with the semantics of ff `BatchInvert::batch_invert` that upstream's permutation and
     // lookup provers call: a zero denominator is skipped (its "inverse" stays 0, the running product is 0 from there on)
     // and does not disturb any other element of the batch.
     const unsigned gt = (unsigned)((tot + 255) / 256);
-    fr_zero_to_one_kernel<<<gt, 256, 0, st>>>(den, g_poly.e.as<fe>(), (uint32_t)tot);
+    fr_zero_to_one_kernel<<<gt, 256, 0, st>>>(den, P->e.as<fe>(), (uint32_t)tot);
     H2V_LAUNCHED();
-    if ((rc = run_batch_invert<FrP>(st, g_poly.e.as<fe>(), g_poly.c.as<fe>(), (uint32_t)tot, g_poly.tree))) return rc;
-    fr_select_inverse_kernel<<<gt, 256, 0, st>>>(den, g_poly.c.as<fe>(), g_poly.e.as<fe>(), (uint32_t)tot);
+    if ((rc = run_batch_invert<FrP>(st, P->e.as<fe>(), P->c.as<fe>(), (uint32_t)tot, P->tree))) return rc;
+    fr_select_inverse_kernel<<<gt, 256, 0, st>>>(den, P->c.as<fe>(), P->e.as<fe>(), (uint32_t)tot);
     H2V_LAUNCHED();
-    fr_prod_tiles_kernel<<<dim3(ntiles, cols), 256, 0, st>>>(num, g_poly.e.as<fe>(), n, g_poly.d.as<fe>());
+    fr_prod_tiles_kernel<<<dim3(ntiles, cols), 256, 0, st>>>(num, P->e.as<fe>(), n, P->d.as<fe>());
     H2V_LAUNCHED();
-    fr_scan_top_kernel<OpMul><<<dim3(1, cols), 256, 0, st>>>(g_poly.d.as<fe>(), ntiles);
+    fr_scan_top_kernel<OpMul><<<dim3(1, cols), 256, 0, st>>>(P->d.as<fe>(), ntiles);
     H2V_LAUNCHED();
-    fr_prod_apply_kernel<<<dim3(ntiles, cols), 256, 0, st>>>(num, g_poly.e.as<fe>(), n, g_poly.d.as<fe>(), out);
+    fr_prod_apply_kernel<<<dim3(ntiles, cols), 256, 0, st>>>(num, P->e.as<fe>(), n, P->d.as<fe>(), out);
     H2V_LAUNCHED();
     return H2V_OK;
 }
@@ -1686,21 +1685,21 @@ int h2v_grand_product(const uint64_t *num, const uint64_t *den, size_t n, uint64
     if (!n) return H2V_OK;
     if (!num || !den || !out) return failf(H2V_EINVAL, "grand_product: NULL buffer");
     if (n >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "grand_product: n too large");
-    t_dev = -1;
-    int rc = use_device();
+    PolyCtx *P;
+    int rc = poly_on(g_devs[0], &P);
     if (rc) return rc;
-    std::lock_guard<std::mutex> lk(g_poly.mu);
-    if ((rc = poly_ctx_ready())) return rc;
-    cudaStream_t st = g_poly.st;
-    if ((rc = g_poly.a.ensure(n * sizeof(fe))) || (rc = g_poly.b.ensure(n * sizeof(fe)))) return rc;
-    H2V_CU(cudaMemcpyAsync(g_poly.a.p, num, n * sizeof(fe), cudaMemcpyHostToDevice, st));
-    H2V_CU(cudaMemcpyAsync(g_poly.b.p, den, n * sizeof(fe), cudaMemcpyHostToDevice, st));
+    std::lock_guard<std::mutex> lk(P->mu);
+    if ((rc = poly_ctx_ready(P))) return rc;
+    cudaStream_t st = P->st;
+    if ((rc = P->a.ensure(n * sizeof(fe))) || (rc = P->b.ensure(n * sizeof(fe)))) return rc;
+    H2V_CU(cudaMemcpyAsync(P->a.p, num, n * sizeof(fe), cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(P->b.p, den, n * sizeof(fe), cudaMemcpyHostToDevice, st));
     // the running product overwrites the staged denominators once their inverses exist
-    if ((rc = run_grand_product(st, g_poly.a.as<fe>(), g_poly.b.as<fe>(), (uint32_t)n, 1, g_poly.b.as<fe>()))) {
+    if ((rc = run_grand_product(P, P->a.as<fe>(), P->b.as<fe>(), (uint32_t)n, 1, P->b.as<fe>()))) {
         cudaStreamSynchronize(st);
         return rc;
     }
-    H2V_CU(cudaMemcpyAsync(out, g_poly.b.p, n * sizeof(fe), cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaMemcpyAsync(out, P->b.p, n * sizeof(fe), cudaMemcpyDeviceToHost, st));
     H2V_CU(cudaStreamSynchronize(st));
     return H2V_OK;
 }
@@ -1708,16 +1707,17 @@ int h2v_grand_product_dev(const void *d_num, const void *d_den, size_t n, size_t
     if (!n || !n_cols) return H2V_OK;
     if (!d_num || !d_den || !d_out) return failf(H2V_EINVAL, "grand_product: NULL buffer");
     if (n_cols > 65535 || n * n_cols >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "grand_product: batch too large");
-    t_dev = device_of(d_num);
-    H2V_TRY(use_device());
-    return sync_call(g_poly.mu, g_poly.st, 7, "grand_product", [&](Timer &) {
-        return run_grand_product(g_poly.st, (const fe *)d_num, (const fe *)d_den, (uint32_t)n, (uint32_t)n_cols, (fe *)d_out);
+    PolyCtx *P;
+    H2V_TRY(poly_on(device_of(d_num), &P));
+    return sync_call(P->mu, P->st, 7, "grand_product", [&](Timer &) {
+        return run_grand_product(P, (const fe *)d_num, (const fe *)d_den, (uint32_t)n, (uint32_t)n_cols, (fe *)d_out);
     });
 }
 // every job's division in one set of launches (poly.cuh KateCol); a, q device-resident (q: n - 1 coefficients, must not
-// overlap a); g_poly.mu held by the caller
-static int run_kate_division(cudaStream_t st, const KateJob *jobs, size_t n_jobs) {
+// overlap a); P->mu held by the caller
+static int run_kate_division(PolyCtx *P, const KateJob *jobs, size_t n_jobs) {
     int rc;
+    const cudaStream_t st = P->st;
     std::vector<KateCol> cols;
     uint32_t nmax = 0;
     for (size_t j = 0; j < n_jobs; ++j) {
@@ -1734,10 +1734,10 @@ static int run_kate_division(cudaStream_t st, const KateJob *jobs, size_t n_jobs
     if (cols.empty()) return H2V_OK;
     if (cols.size() > 65535) return failf(H2V_EINVAL, "kate_division: %zu columns in one call", cols.size());
     const uint32_t ntiles = (nmax + H2V_FR_TILE - 1) / H2V_FR_TILE;
-    if ((rc = g_poly.d.ensure((cols.size() * ntiles + 1) * sizeof(fe))) || (rc = g_poly.e.ensure(cols.size() * sizeof(KateCol)))) return rc;
-    H2V_CU(cudaMemcpyAsync(g_poly.e.p, cols.data(), cols.size() * sizeof(KateCol), cudaMemcpyHostToDevice, st));
-    const KateCol *d_cols = g_poly.e.as<KateCol>();
-    fe *tile = g_poly.d.as<fe>();
+    if ((rc = P->d.ensure((cols.size() * ntiles + 1) * sizeof(fe))) || (rc = P->e.ensure(cols.size() * sizeof(KateCol)))) return rc;
+    H2V_CU(cudaMemcpyAsync(P->e.p, cols.data(), cols.size() * sizeof(KateCol), cudaMemcpyHostToDevice, st));
+    const KateCol *d_cols = P->e.as<KateCol>();
+    fe *tile = P->d.as<fe>();
     const dim3 grid(ntiles, (unsigned)cols.size());
     kate_tiles_kernel<<<grid, 256, 0, st>>>(d_cols, tile, ntiles);
     H2V_LAUNCHED();
@@ -1757,13 +1757,13 @@ int kate_division_batch_dev(const KateJob *jobs, size_t n_jobs) {
         if (!jobs[j].a || !jobs[j].q) return failf(H2V_EINVAL, "kate_division: NULL buffer");
         if (jobs[j].n >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "kate_division: n too large");
     }
-    t_dev = device_of(jobs[0].a);
-    int rc = use_device();
+    PolyCtx *P;
+    int rc = poly_on(device_of(jobs[0].a), &P);
     if (rc) return rc;
-    std::lock_guard<std::mutex> lk(g_poly.mu);
-    if ((rc = poly_ctx_ready())) return rc;
-    rc = run_kate_division(g_poly.st, jobs, n_jobs);
-    cudaError_t e = cudaStreamSynchronize(g_poly.st);
+    std::lock_guard<std::mutex> lk(P->mu);
+    if ((rc = poly_ctx_ready(P))) return rc;
+    rc = run_kate_division(P, jobs, n_jobs);
+    cudaError_t e = cudaStreamSynchronize(P->st);
     if (rc) return rc;
     if (e != cudaSuccess) return failf(H2V_ECUDA, "kate_division: %s", cudaGetErrorString(e));
     return H2V_OK;
@@ -1780,20 +1780,20 @@ int h2v_kate_division(const uint64_t *a, size_t n, const uint64_t b[4], uint64_t
     if (n <= 1) return H2V_OK;
     if (!a || !b || !out) return failf(H2V_EINVAL, "kate_division: NULL buffer");
     if (n >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "kate_division: n too large");
-    t_dev = -1;
-    int rc = use_device();
+    PolyCtx *P;
+    int rc = poly_on(g_devs[0], &P);
     if (rc) return rc;
-    std::lock_guard<std::mutex> lk(g_poly.mu);
-    if ((rc = poly_ctx_ready())) return rc;
-    cudaStream_t st = g_poly.st;
-    if ((rc = g_poly.a.ensure(n * sizeof(fe))) || (rc = g_poly.b.ensure(n * sizeof(fe)))) return rc;
-    H2V_CU(cudaMemcpyAsync(g_poly.a.p, a, n * sizeof(fe), cudaMemcpyHostToDevice, st));
-    const KateJob job{g_poly.a.p, g_poly.b.p, n, {b[0], b[1], b[2], b[3]}};
-    if ((rc = run_kate_division(st, &job, 1))) {
+    std::lock_guard<std::mutex> lk(P->mu);
+    if ((rc = poly_ctx_ready(P))) return rc;
+    cudaStream_t st = P->st;
+    if ((rc = P->a.ensure(n * sizeof(fe))) || (rc = P->b.ensure(n * sizeof(fe)))) return rc;
+    H2V_CU(cudaMemcpyAsync(P->a.p, a, n * sizeof(fe), cudaMemcpyHostToDevice, st));
+    const KateJob job{P->a.p, P->b.p, n, {b[0], b[1], b[2], b[3]}};
+    if ((rc = run_kate_division(P, &job, 1))) {
         cudaStreamSynchronize(st);
         return rc;
     }
-    H2V_CU(cudaMemcpyAsync(out, g_poly.b.p, (n - 1) * sizeof(fe), cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaMemcpyAsync(out, P->b.p, (n - 1) * sizeof(fe), cudaMemcpyDeviceToHost, st));
     H2V_CU(cudaStreamSynchronize(st));
     return H2V_OK;
 }
@@ -1831,12 +1831,13 @@ int scan_u32_dev(cudaStream_t st, const uint32_t *cnt, uint32_t len, uint32_t *o
 }
 }  // namespace h2v
 namespace {
-// A', S' of `u` usable rows from device-resident input / table expressions (Montgomery); g_poly.mu held by the caller
+// A', S' of `u` usable rows from device-resident input / table expressions (Montgomery); P->mu held by the caller
 // All lookup arguments of one proof phase in one set of launches (lookup.cuh): inputs[l] / tables[l] are device columns,
 // the permuted columns land at out_a + l * a_stride / out_s + l * s_stride.  Identical table pointers are sorted once.
-int run_permute_batch(cudaStream_t st, const fe *const *inputs, const fe *const *tables, uint32_t L, uint32_t u, fe *d_out_a, size_t a_stride,
+int run_permute_batch(PolyCtx *P, const fe *const *inputs, const fe *const *tables, uint32_t L, uint32_t u, fe *d_out_a, size_t a_stride,
                       fe *d_out_s, size_t s_stride) {
     int rc;
+    const cudaStream_t st = P->st;
     uint32_t n_pad = 1;
     while (n_pad < u) n_pad <<= 1;
     std::vector<const fe *> srcs(inputs, inputs + L);
@@ -1853,11 +1854,11 @@ int run_permute_batch(cudaStream_t st, const fe *const *inputs, const fe *const 
     if (rows >= ((size_t)1 << 31)) return failf(H2V_EINVAL, "permute_expression_pair: batch too large");
     const uint32_t ntiles = (uint32_t)((rows + H2V_SCAN_TILE - 1) / H2V_SCAN_TILE);
     const size_t ptr_words = ((size_t)slices * sizeof(void *) + 3) / 4;
-    if ((rc = g_poly.a.ensure((size_t)slices * n_pad * sizeof(fe))) ||
-        (rc = g_poly.tree.ensure((6 * rows + 2 * ntiles + 16 + L + ptr_words + 8) * sizeof(uint32_t))))
+    if ((rc = P->a.ensure((size_t)slices * n_pad * sizeof(fe))) ||
+        (rc = P->tree.ensure((6 * rows + 2 * ntiles + 16 + L + ptr_words + 8) * sizeof(uint32_t))))
         return rc;
-    fe *keys = g_poly.a.as<fe>();
-    uint32_t *rep = g_poly.tree.as<uint32_t>(), *free_ = rep + rows, *rep_offs = free_ + rows, *free_offs = rep_offs + rows;
+    fe *keys = P->a.as<fe>();
+    uint32_t *rep = P->tree.as<uint32_t>(), *free_ = rep + rows, *rep_offs = free_ + rows, *free_offs = rep_offs + rows;
     uint32_t *scratch = free_offs + rows, *rep_rows = scratch + rows, *tiles = rep_rows + rows, *totals = tiles + 2 * ntiles;
     int *err = reinterpret_cast<int *>(totals + 2);
     uint32_t *d_tmap = totals + 4;
@@ -1887,8 +1888,8 @@ int run_permute_batch(cudaStream_t st, const fe *const *inputs, const fe *const 
     if (herr) return failf(H2V_ECUDA, "permute_expression_pair: leftover count mismatch");
     return H2V_OK;
 }
-int run_permute_pair(cudaStream_t st, const fe *d_in_a, const fe *d_in_t, uint32_t u, fe *d_out_a, fe *d_out_s) {
-    return run_permute_batch(st, &d_in_a, &d_in_t, 1, u, d_out_a, 0, d_out_s, 0);
+int run_permute_pair(PolyCtx *P, const fe *d_in_a, const fe *d_in_t, uint32_t u, fe *d_out_a, fe *d_out_s) {
+    return run_permute_batch(P, &d_in_a, &d_in_t, 1, u, d_out_a, 0, d_out_s, 0);
 }
 }  // namespace
 
@@ -1898,10 +1899,10 @@ int h2v_permute_expression_pair_dev(const void *d_input, const void *d_table, si
     if (!usable_rows) return H2V_OK;
     if (!d_input || !d_table || !d_permuted_input || !d_permuted_table) return failf(H2V_EINVAL, "permute_expression_pair: NULL buffer");
     if (usable_rows > ((size_t)1 << 28)) return failf(H2V_EINVAL, "permute_expression_pair: too many rows");
-    t_dev = device_of(d_input);
-    H2V_TRY(use_device());
-    return sync_call(g_poly.mu, g_poly.st, 7, "permute_expression_pair", [&](Timer &) {
-        return run_permute_pair(g_poly.st, (const fe *)d_input, (const fe *)d_table, (uint32_t)usable_rows, (fe *)d_permuted_input,
+    PolyCtx *P;
+    H2V_TRY(poly_on(device_of(d_input), &P));
+    return sync_call(P->mu, P->st, 7, "permute_expression_pair", [&](Timer &) {
+        return run_permute_pair(P, (const fe *)d_input, (const fe *)d_table, (uint32_t)usable_rows, (fe *)d_permuted_input,
                                 (fe *)d_permuted_table);
     });
 }
@@ -1914,10 +1915,10 @@ int h2v_permute_expression_pair_batch_dev(const void *const *d_inputs, const voi
         return failf(H2V_EINVAL, "permute_expression_pair: output stride shorter than the usable rows");
     for (size_t l = 0; l < n_lookups; ++l)
         if (!d_inputs[l] || !d_tables[l]) return failf(H2V_EINVAL, "permute_expression_pair: lookup %zu has a NULL column", l);
-    t_dev = device_of(d_inputs[0]);
-    H2V_TRY(use_device());
-    return sync_call(g_poly.mu, g_poly.st, 7, "permute_expression_pair", [&](Timer &) {
-        return run_permute_batch(g_poly.st, (const fe *const *)d_inputs, (const fe *const *)d_tables, (uint32_t)n_lookups, (uint32_t)usable_rows,
+    PolyCtx *P;
+    H2V_TRY(poly_on(device_of(d_inputs[0]), &P));
+    return sync_call(P->mu, P->st, 7, "permute_expression_pair", [&](Timer &) {
+        return run_permute_batch(P, (const fe *const *)d_inputs, (const fe *const *)d_tables, (uint32_t)n_lookups, (uint32_t)usable_rows,
                                  (fe *)d_permuted_inputs, input_stride, (fe *)d_permuted_tables, table_stride);
     });
 }
@@ -1926,23 +1927,23 @@ int h2v_permute_expression_pair(const uint64_t *input, const uint64_t *table, si
     if (!usable_rows) return H2V_OK;
     if (!input || !table || !permuted_input || !permuted_table) return failf(H2V_EINVAL, "permute_expression_pair: NULL buffer");
     if (usable_rows > ((size_t)1 << 28)) return failf(H2V_EINVAL, "permute_expression_pair: too many rows");
-    t_dev = -1;
-    int rc = use_device();
+    PolyCtx *P;
+    int rc = poly_on(g_devs[0], &P);
     if (rc) return rc;
-    std::lock_guard<std::mutex> lk(g_poly.mu);
-    if ((rc = poly_ctx_ready())) return rc;
-    cudaStream_t st = g_poly.st;
+    std::lock_guard<std::mutex> lk(P->mu);
+    if ((rc = poly_ctx_ready(P))) return rc;
+    cudaStream_t st = P->st;
     const size_t bytes = usable_rows * sizeof(fe);
-    if ((rc = g_poly.c.ensure(bytes)) || (rc = g_poly.d.ensure(bytes))) return rc;
-    H2V_CU(cudaMemcpyAsync(g_poly.c.p, input, bytes, cudaMemcpyHostToDevice, st));
-    H2V_CU(cudaMemcpyAsync(g_poly.d.p, table, bytes, cudaMemcpyHostToDevice, st));
+    if ((rc = P->c.ensure(bytes)) || (rc = P->d.ensure(bytes))) return rc;
+    H2V_CU(cudaMemcpyAsync(P->c.p, input, bytes, cudaMemcpyHostToDevice, st));
+    H2V_CU(cudaMemcpyAsync(P->d.p, table, bytes, cudaMemcpyHostToDevice, st));
     // the canonical copies are taken first, so the staging buffers double as the outputs
-    if ((rc = run_permute_pair(st, g_poly.c.as<fe>(), g_poly.d.as<fe>(), (uint32_t)usable_rows, g_poly.c.as<fe>(), g_poly.d.as<fe>()))) {
+    if ((rc = run_permute_pair(P, P->c.as<fe>(), P->d.as<fe>(), (uint32_t)usable_rows, P->c.as<fe>(), P->d.as<fe>()))) {
         cudaStreamSynchronize(st);
         return rc;
     }
-    H2V_CU(cudaMemcpyAsync(permuted_input, g_poly.c.p, bytes, cudaMemcpyDeviceToHost, st));
-    H2V_CU(cudaMemcpyAsync(permuted_table, g_poly.d.p, bytes, cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaMemcpyAsync(permuted_input, P->c.p, bytes, cudaMemcpyDeviceToHost, st));
+    H2V_CU(cudaMemcpyAsync(permuted_table, P->d.p, bytes, cudaMemcpyDeviceToHost, st));
     H2V_CU(cudaStreamSynchronize(st));
     return H2V_OK;
 }
@@ -1950,13 +1951,13 @@ int h2v_permute_expression_pair(const uint64_t *input, const uint64_t *table, si
 
 // ================================================================== quotient evaluation ("next" row 1)
 namespace {
-// the replica that holds d_h (made current) and the constants every quotient kernel takes
+// the replica that holds d_h (made the calling thread's device) and the constants every quotient kernel takes
 int quotient_common(h2v_domain_t h, const void *d_h, DomRep **d, QuotientCommon *c) {
     if (!(*d = dom_rep(h, d_h))) return H2V_EINVAL;
     if (!d_h) return failf(H2V_EINVAL, "quotient: NULL buffer");
     c->n_ext = 1u << (*d)->ek;
     c->rot = 1u << ((*d)->ek - (*d)->k);
-    return use_device();
+    return use_device((*d)->dev);
 }
 // one proof's y, beta, gamma (and `extra_bytes` behind them) into the replica's argument buffer, on its stream: the
 // public entry points are groups of one; d->mu held by the caller
@@ -2292,8 +2293,7 @@ __global__ void __launch_bounds__(256) imad_chain_probe_kernel(uint32_t *out, ui
 
 extern "C" {
 int h2v_selftest_field(int field, int op, const uint64_t *a, const uint64_t *b, size_t n, uint64_t *out) {
-    t_dev = -1;
-    int rc = use_device();
+    int rc = use_device(g_devs[0]);
     if (rc) return rc;
     if (!a || !out || n == 0) return failf(H2V_EINVAL, "selftest_field: bad argument");
     DevBuf A, B, O;
@@ -2310,8 +2310,7 @@ int h2v_selftest_field(int field, int op, const uint64_t *a, const uint64_t *b, 
     return H2V_OK;
 }
 int h2v_selftest_group(int mode, const uint64_t *p, const uint64_t *q, size_t n, uint64_t *out_affine) {
-    t_dev = -1;
-    int rc = use_device();
+    int rc = use_device(g_devs[0]);
     if (rc) return rc;
     if (!p || !q || !out_affine || n == 0) return failf(H2V_EINVAL, "selftest_group: bad argument");
     DevBuf A, B, O;
@@ -2326,8 +2325,7 @@ int h2v_selftest_group(int mode, const uint64_t *p, const uint64_t *q, size_t n,
     return H2V_OK;
 }
 int h2v_srs_setup(uint32_t k, const uint64_t s_mont[4], uint64_t *g_out, uint64_t *g_lagrange_out) {
-    t_dev = -1;
-    int rc = use_device();
+    int rc = use_device(g_devs[0]);
     if (rc) return rc;
     if (!s_mont || (!g_out && !g_lagrange_out)) return failf(H2V_EINVAL, "srs_setup: NULL argument");
     if (k > 26) return failf(H2V_EINVAL, "srs_setup: k = %u unsupported", k);
@@ -2357,8 +2355,7 @@ int h2v_srs_setup(uint32_t k, const uint64_t s_mont[4], uint64_t *g_out, uint64_
     return H2V_OK;
 }
 int h2v_synthetic_bases(uint64_t a, uint64_t b, size_t n, uint64_t *out_affine) {
-    t_dev = -1;
-    int rc = use_device();
+    int rc = use_device(g_devs[0]);
     if (rc) return rc;
     if (!out_affine || n == 0) return failf(H2V_EINVAL, "synthetic_bases: bad argument");
     if (a >> 62 || b >> 62 || n >> 32) return failf(H2V_EINVAL, "synthetic_bases: a, b < 2^62 and n < 2^32 required");
@@ -2374,14 +2371,13 @@ int h2v_synthetic_bases(uint64_t a, uint64_t b, size_t n, uint64_t *out_affine) 
 // which: 0 Fq mul, one dependent chain per thread; 1 Fq mul, two chains; 2 XYZZ mixed add chain.
 // Returns operations per second over the whole GPU.
 int h2v_selftest_op_rate(int which, double *out) {
-    t_dev = -1;
-    int rc = use_device();
+    int rc = use_device(g_devs[0]);
     if (rc) return rc;
     if (!out || which < 0 || which > 2) return failf(H2V_EINVAL, "selftest_op_rate: bad argument");
     DevBuf O;
     if ((rc = O.ensure(256))) return rc;
     cudaDeviceProp prop;
-    H2V_CU(cudaGetDeviceProperties(&prop, cur_dev()));
+    H2V_CU(cudaGetDeviceProperties(&prop, g_devs[0]));
     cudaEvent_t e0, e1;
     H2V_CU(cudaEventCreate(&e0));
     H2V_CU(cudaEventCreate(&e1));
@@ -2418,15 +2414,14 @@ int h2v_selftest_op_rate(int which, double *out) {
 int h2v_selftest_imad_peak(double *out);
 // which 0: the loop-variant stream of round 1 (one xorshift update per 8 multiply-adds); 1: the pure chain probe
 int h2v_selftest_imad_probe(int which, double *out) {
-    t_dev = -1;
-    int rc = use_device();
+    int rc = use_device(g_devs[0]);
     if (rc) return rc;
     if (!out || which < 0 || which > 1) return failf(H2V_EINVAL, "selftest_imad_probe: bad argument");
     if (which == 0) return h2v_selftest_imad_peak(out);
     DevBuf O;
     if ((rc = O.ensure(64))) return rc;
     cudaDeviceProp prop;
-    H2V_CU(cudaGetDeviceProperties(&prop, cur_dev()));
+    H2V_CU(cudaGetDeviceProperties(&prop, g_devs[0]));
     cudaEvent_t e0, e1;
     H2V_CU(cudaEventCreate(&e0));
     H2V_CU(cudaEventCreate(&e1));
@@ -2452,14 +2447,13 @@ int h2v_selftest_imad_probe(int which, double *out) {
     return H2V_OK;
 }
 int h2v_selftest_imad_peak(double *out) {
-    t_dev = -1;
-    int rc = use_device();
+    int rc = use_device(g_devs[0]);
     if (rc) return rc;
     if (!out) return failf(H2V_EINVAL, "selftest_imad_peak: NULL");
     DevBuf O;
     if ((rc = O.ensure(64))) return rc;
     cudaDeviceProp prop;
-    H2V_CU(cudaGetDeviceProperties(&prop, cur_dev()));
+    H2V_CU(cudaGetDeviceProperties(&prop, g_devs[0]));
     const unsigned blocks = prop.multiProcessorCount * 8, threads = 256, iters = 1 << 14;
     cudaEvent_t e0, e1;
     H2V_CU(cudaEventCreate(&e0));
@@ -2485,12 +2479,12 @@ int h2v_selftest_imad_peak(double *out) {
 }
 
 namespace {
-// a replica of `src` on the calling thread's current device: the window tables cross NVLink / PCIe once (peer copy)
-int rep_srs_clone(const SrsRep *src, SrsRep **out) {
-    int rc = use_device();
+// a replica of `src` on device `dev`: the window tables cross NVLink / PCIe once (peer copy)
+int rep_srs_clone(int dev, const SrsRep *src, SrsRep **out) {
+    int rc = use_device(dev);
     if (rc) return rc;
     SrsRep *s = new SrsRep();
-    s->dev = cur_dev();
+    s->dev = dev;
     s->k = src->k;
     s->n = src->n;
     s->cfg[0] = src->cfg[0];
@@ -2517,25 +2511,115 @@ int rep_srs_clone(const SrsRep *src, SrsRep **out) {
     *out = s;
     return H2V_OK;
 }
-// run fn(slot) on one host thread per device (each thread's entry points run on its device); first error wins
-template <class Fn> int fan_out(size_t n_slots, Fn fn) {
+// run fn(reps[i], i) for every replica, each on a host thread of its own (reps[0] on the calling thread, whose current
+// device is the same afterwards as before); first error wins
+template <class Rep, class Fn> int fan_out(const std::vector<Rep *> &reps, Fn fn) {
+    int home = 0;
+    cudaGetDevice(&home);
+    const size_t n_slots = reps.size();
     std::vector<int> rcs(n_slots, H2V_OK);
     std::vector<std::string> errs(n_slots);
     std::vector<std::thread> th;
     for (size_t i = 1; i < n_slots; ++i)
         th.emplace_back([&, i] {
-            rcs[i] = fn(i);
+            rcs[i] = fn(reps[i], i);
             if (rcs[i]) errs[i] = g_err;
         });
-    rcs[0] = fn(0);
+    rcs[0] = fn(reps[0], 0);
     if (rcs[0]) errs[0] = g_err;
     for (auto &t : th) t.join();
+    cudaSetDevice(home);
     for (size_t i = 0; i < n_slots; ++i)
         if (rcs[i]) {
             g_err = errs[i];
             return rcs[i];
         }
     return H2V_OK;
+}
+
+// The replicas of a handle: make(dev, &rep) builds one per h2v_init device, in list order; on an error the ones built so
+// far are freed, each on its own device.  Both leave the calling thread on the primary device.
+template <class Rep> void free_replicas(std::vector<Rep *> &reps, void (*free_rep)(Rep *)) {
+    for (Rep *r : reps) free_rep(r);
+    reps.clear();
+    cudaSetDevice(g_devs[0]);
+}
+template <class Rep, class Make> int make_replicas(std::vector<Rep *> &reps, void (*free_rep)(Rep *), Make make) {
+    for (int dev : g_devs) {
+        Rep *r = nullptr;
+        const int rc = make(dev, &r);
+        if (rc) {
+            free_replicas(reps, free_rep);
+            return rc;
+        }
+        reps.push_back(r);
+    }
+    cudaSetDevice(g_devs[0]);
+    return H2V_OK;
+}
+
+// cnt columns of `bytes` each from device src_dev to device dst_dev, on st: one copy when both sides hold them
+// contiguously, one per column otherwise
+cudaError_t peer_copy(void *dst, size_t dst_stride, int dst_dev, const void *src, size_t src_stride, int src_dev, size_t bytes, size_t cnt,
+                      cudaStream_t st) {
+    if (dst_stride == bytes && src_stride == bytes) return cudaMemcpyPeerAsync(dst, dst_dev, src, src_dev, cnt * bytes, st);
+    cudaError_t e = cudaSuccess;
+    for (size_t c = 0; c < cnt && e == cudaSuccess; ++c)
+        e = cudaMemcpyPeerAsync((char *)dst + c * dst_stride, dst_dev, (const char *)src + c * src_stride, src_dev, bytes, st);
+    return e;
+}
+
+bool peer_split_allowed() {
+    static const bool no_split = getenv("H2V_NO_PEER_SPLIT") != nullptr;      // keep resident batches on their owner (tuning)
+    return !no_split;
+}
+// Several devices, one resident batch on `owner`'s device (a phase of create_proof): the columns are independent, so the
+// batch is cut into one contiguous block per replica.  The owner runs its block in place; every other replica pulls its
+// block over NVLink, runs it and pushes the results back into the owner's output.  No collective; results in column
+// order.  A column is in_bytes of input, in_stride bytes apart, and out_bytes of result, out_stride bytes apart.
+// run(rep, in, in_stride, out, out_stride, count) runs `count` columns on `rep` (strides in bytes); a pulled block is
+// packed, and its results are out_stride apart.
+template <class Rep, class Run>
+int split_blocks(const std::vector<Rep *> &reps, Rep *owner, const char *what, const void *in, size_t in_bytes, size_t in_stride, void *out,
+                 size_t out_bytes, size_t out_stride, size_t n_cols, Run run) {
+    const size_t per = (n_cols + reps.size() - 1) / reps.size();
+    const char *src = (const char *)in;
+    char *dst = (char *)out;
+    return fan_out(reps, [&](Rep *rep, size_t d) -> int {
+        const size_t c0 = std::min(n_cols, d * per), cnt = std::min(n_cols, c0 + per) - c0;
+        if (!cnt) return H2V_OK;
+        if (rep == owner) return run(rep, src + c0 * in_stride, in_stride, dst + c0 * out_stride, out_stride, cnt);
+        H2V_TRY(use_device(rep->dev));
+        std::lock_guard<std::mutex> plk(rep->peer_mu);
+        {
+            std::lock_guard<std::mutex> lk(rep->mu);
+            H2V_TRY(rep->peer_in.ensure(cnt * in_bytes));
+            H2V_TRY(rep->peer_out.ensure(cnt * out_stride));
+            cudaError_t e = peer_copy(rep->peer_in.p, in_bytes, rep->dev, src + c0 * in_stride, in_stride, owner->dev, in_bytes, cnt, rep->stream);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(rep->stream);
+            if (e != cudaSuccess) return failf(H2V_ECUDA, "%s: peer copy %d -> %d: %s", what, owner->dev, rep->dev, cudaGetErrorString(e));
+        }
+        H2V_TRY(run(rep, rep->peer_in.p, in_bytes, rep->peer_out.p, out_stride, cnt));
+        // (cudaMemcpyPeer returns before the copy has landed and does not order against non-blocking streams: copy on the
+        // replica's stream and wait for it)
+        cudaError_t e = peer_copy(dst + c0 * out_stride, out_stride, owner->dev, rep->peer_out.p, out_stride, rep->dev, out_bytes, cnt, rep->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(rep->stream);
+        if (e != cudaSuccess) return failf(H2V_ECUDA, "%s: peer copy of the results: %s", what, cudaGetErrorString(e));
+        return H2V_OK;
+    });
+}
+
+// Host columns over several devices: column j goes to replica j mod G (each device has its own PCIe link and replica, no
+// collective).  run(rep, in, out, count) gets the replica's input and output columns in column order.
+template <class Rep, class In, class Out, class Run> int deal_columns(const std::vector<Rep *> &reps, const In *in, const Out *out, size_t n, Run run) {
+    const size_t G = reps.size();
+    std::vector<std::vector<In>> si(G);
+    std::vector<std::vector<Out>> so(G);
+    for (size_t j = 0; j < n; ++j) {
+        si[j % G].push_back(in[j]);
+        so[j % G].push_back(out[j]);
+    }
+    return fan_out(reps, [&](Rep *rep, size_t d) { return run(rep, si[d].data(), so[d].data(), si[d].size()); });
 }
 }  // namespace
 
@@ -2546,9 +2630,7 @@ int h2v_dev_alloc_on(int device, size_t bytes, void **d_out) {
     for (int d : g_devs) known = known || d == device;
     if (!known) return failf(H2V_EINVAL, "dev_alloc_on: device %d is not in the h2v_init list", device);
     if (!d_out || !bytes) return failf(H2V_EINVAL, "dev_alloc: bad argument");
-    t_dev = device;
-    int rc = use_device();
-    if (rc) return rc;
+    H2V_TRY(use_device(device));
     cudaError_t e = cudaMalloc(d_out, bytes);
     if (e != cudaSuccess) {
         cudaGetLastError();
@@ -2562,81 +2644,31 @@ int h2v_srs_load(uint32_t k, const uint64_t *g, const uint64_t *g_lagrange, h2v_
     if (!out) return failf(H2V_EINVAL, "h2v_srs_load: out is NULL");
     *out = nullptr;
     h2v_srs *h = new h2v_srs();
-    for (size_t i = 0; i < g_devs.size(); ++i) {
-        t_dev = g_devs[i];
-        SrsRep *r = nullptr;
-        int rc = i == 0 ? rep_srs_load(k, g, g_lagrange, &r) : rep_srs_clone(h->rep[0], &r);
-        if (rc) {
-            h2v_srs_free(h);
-            t_dev = -1;
-            return rc;
-        }
-        h->rep.push_back(r);
-    }
-    t_dev = -1;
-    *out = h;
-    return H2V_OK;
+    const int rc = make_replicas(h->rep, rep_srs_free, [&](int dev, SrsRep **r) {
+        return h->rep.empty() ? rep_srs_load(dev, k, g, g_lagrange, r) : rep_srs_clone(dev, h->rep[0], r);
+    });
+    if (rc) delete h;
+    else *out = h;
+    return rc;
 }
 void h2v_srs_free(h2v_srs_t h) {
     if (!h) return;
-    for (SrsRep *r : h->rep) {
-        t_dev = r->dev;
-        rep_srs_free(r);
-    }
-    t_dev = -1;
+    free_replicas(h->rep, rep_srs_free);
     delete h;
 }
 int h2v_commit_batch_dev(h2v_srs_t h, int basis, const void *d_polys, size_t col_stride, size_t n_polys, size_t len, void *d_out_affine) {
     if (!h) return failf(H2V_EINVAL, "commit: NULL srs");
     SrsRep *r = srs_on(h, device_of(d_polys));
     if (!r) return failf(H2V_EINVAL, "commit: the columns live on device %d, which is not in the h2v_init list", device_of(d_polys));
+    H2V_TRY(use_device(r->dev));
     const size_t G = h->rep.size();
-    static const bool no_split = getenv("H2V_NO_PEER_SPLIT") != nullptr;
-    if (G == 1 || no_split || n_polys < 8 * G || len == 0 || device_of(d_out_affine) != r->dev) {
-        t_dev = r->dev;
+    if (G == 1 || !peer_split_allowed() || n_polys < 8 * G || len == 0 || device_of(d_out_affine) != r->dev)
         return rep_commit_batch_dev(r, basis, d_polys, col_stride, n_polys, len, d_out_affine);
-    }
-    // Several devices, one resident batch (a phase of create_proof): the columns are independent, so the batch is cut
-    // into G contiguous blocks; the owner commits its block in place, every other device pulls its block over NVLink
-    // (peer copy, 32 B x len per column against ~10^3 x that in multiplier work), commits it against its own SRS replica
-    // and writes the 64-byte results back into the owner's output array.  No collective; results in column order.
-    const size_t per = (n_polys + G - 1) / G;
-    const fe *src = (const fe *)d_polys;
-    affine *dst = (affine *)d_out_affine;
-    int rc = fan_out(G, [&](size_t d) -> int {
-        SrsRep *rep = h->rep[d];
-        const size_t c0 = std::min(n_polys, d * per), cnt = std::min(n_polys, c0 + per) - c0;
-        if (!cnt) return H2V_OK;
-        t_dev = rep->dev;
-        if (rep == r) return rep_commit_batch_dev(rep, basis, src + c0 * col_stride, col_stride, cnt, len, dst + c0);
-        int rc2 = use_device();
-        if (rc2) return rc2;
-        std::lock_guard<std::mutex> plk(rep->peer_mu);
-        {
-            std::lock_guard<std::mutex> lk(rep->mu);
-            if ((rc2 = rep->peer_stage.ensure(cnt * len * sizeof(fe)))) return rc2;
-            if ((rc2 = rep->peer_out.ensure(cnt * sizeof(affine)))) return rc2;
-            cudaError_t e = cudaSuccess;
-            if (col_stride == len) {
-                e = cudaMemcpyPeerAsync(rep->peer_stage.p, rep->dev, src + c0 * col_stride, r->dev, cnt * len * sizeof(fe), rep->stream);
-            } else {
-                for (size_t c = 0; c < cnt && e == cudaSuccess; ++c)
-                    e = cudaMemcpyPeerAsync(rep->peer_stage.as<fe>() + c * len, rep->dev, src + (c0 + c) * col_stride, r->dev,
-                                            len * sizeof(fe), rep->stream);
-            }
-            if (e == cudaSuccess) e = cudaStreamSynchronize(rep->stream);
-            if (e != cudaSuccess) return failf(H2V_ECUDA, "commit: peer copy %d -> %d: %s", r->dev, rep->dev, cudaGetErrorString(e));
-        }
-        if ((rc2 = rep_commit_batch_dev(rep, basis, rep->peer_stage.p, len, cnt, len, rep->peer_out.p))) return rc2;
-        // (cudaMemcpyPeer returns before the copy has landed and does not order against non-blocking streams: copy on the
-        // replica's stream and wait for it)
-        cudaError_t e = cudaMemcpyPeerAsync(dst + c0, r->dev, rep->peer_out.p, rep->dev, cnt * sizeof(affine), rep->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(rep->stream);
-        if (e != cudaSuccess) return failf(H2V_ECUDA, "commit: peer copy of the results: %s", cudaGetErrorString(e));
-        return H2V_OK;
-    });
-    t_dev = r->dev;
-    return rc;
+    // 32 B x len per column cross NVLink against ~10^3 x that in multiplier work; 64 B of commitment come back
+    return split_blocks(h->rep, r, "commit", d_polys, len * sizeof(fe), col_stride * sizeof(fe), d_out_affine, sizeof(affine), sizeof(affine),
+                        n_polys, [&](SrsRep *rep, const void *in, size_t in_stride, void *out, size_t, size_t cnt) {
+                            return rep_commit_batch_dev(rep, basis, in, in_stride / sizeof(fe), cnt, len, out);
+                        });
 }
 // Host columns that are committed AND left resident (the advice phase of create_proof): every device uploads a contiguous
 // block of the columns over its own PCIe link in sub-batches (the next one crosses while the previous one is committed),
@@ -2652,22 +2684,21 @@ int h2v_commit_batch_resident(h2v_srs_t h, int basis, const uint64_t *const *pol
         if (!polys[c]) return failf(H2V_EINVAL, "commit_resident: polys[%zu] is NULL", c);
     SrsRep *r = srs_on(h, device_of(d_dst));
     if (!r) return failf(H2V_EINVAL, "commit_resident: the destination lives on device %d, which is not in the h2v_init list", device_of(d_dst));
-    const size_t G = (h->rep.size() > 1 && n_polys >= 8 * h->rep.size()) ? h->rep.size() : 1;
-    const size_t per = (n_polys + G - 1) / G;
+    H2V_TRY(use_device(r->dev));
+    const std::vector<SrsRep *> reps = h->rep.size() > 1 && n_polys >= 8 * h->rep.size() ? h->rep : std::vector<SrsRep *>{r};
+    const size_t per = (n_polys + reps.size() - 1) / reps.size();
     fe *dst = (fe *)d_dst;
-    int rc = fan_out(G, [&](size_t d) -> int {
-        SrsRep *rep = G == 1 ? r : h->rep[d];
+    return fan_out(reps, [&](SrsRep *rep, size_t d) -> int {
         const size_t c0 = std::min(n_polys, d * per), cnt = std::min(n_polys, c0 + per) - c0;
         if (!cnt) return H2V_OK;
-        t_dev = rep->dev;
-        int rc2 = use_device();
+        int rc2 = use_device(rep->dev);
         if (rc2) return rc2;
         const bool owner = rep == r;
         std::lock_guard<std::mutex> plk(rep->peer_mu);
-        if (!owner && (rc2 = rep->peer_stage.ensure(cnt * len * sizeof(fe)))) return rc2;
+        if (!owner && (rc2 = rep->peer_in.ensure(cnt * len * sizeof(fe)))) return rc2;
         if ((rc2 = rep->peer_out.ensure(cnt * sizeof(affine)))) return rc2;
         if (!rep->up_stream) H2V_CU(cudaStreamCreateWithFlags(&rep->up_stream, cudaStreamNonBlocking));
-        fe *stage = owner ? dst + c0 * dst_stride : rep->peer_stage.as<fe>();
+        fe *stage = owner ? dst + c0 * dst_stride : rep->peer_in.as<fe>();
         const size_t sstride = owner ? dst_stride : len;
         // few sub-batches: every commit call ends in a latency-bound reduction tail (~1 ms) that only size amortises
         const size_t sub = std::max<size_t>((cnt + 3) / 4, std::max<size_t>(1, ((size_t)64 << 20) / (len * sizeof(fe))));
@@ -2690,12 +2721,8 @@ int h2v_commit_batch_resident(h2v_srs_t h, int basis, const uint64_t *const *pol
             if (e != cudaSuccess) break;
             rc2 = rep_commit_batch_dev(rep, basis, stage + off * sstride, sstride, m, len, rep->peer_out.as<affine>() + off);
             if (rc2 || owner) continue;
-            if (dst_stride == len) {
-                e = cudaMemcpyPeerAsync(dst + (c0 + off) * dst_stride, r->dev, stage + off * len, rep->dev, m * len * sizeof(fe), rep->up_stream);
-            } else {
-                for (size_t c = 0; c < m && e == cudaSuccess; ++c)
-                    e = cudaMemcpyPeerAsync(dst + (c0 + off + c) * dst_stride, r->dev, stage + (off + c) * len, rep->dev, len * sizeof(fe), rep->up_stream);
-            }
+            e = peer_copy(dst + (c0 + off) * dst_stride, dst_stride * sizeof(fe), r->dev, stage + off * len, len * sizeof(fe), rep->dev,
+                          len * sizeof(fe), m, rep->up_stream);
         }
         if (e == cudaSuccess && !rc2)
             e = cudaMemcpyAsync(out_affine + 8 * c0, rep->peer_out.p, cnt * sizeof(affine), cudaMemcpyDeviceToHost, rep->up_stream);
@@ -2707,34 +2734,24 @@ int h2v_commit_batch_resident(h2v_srs_t h, int basis, const uint64_t *const *pol
             return failf(H2V_ECUDA, "commit_resident: %s", cudaGetErrorString(e != cudaSuccess ? e : e2));
         return H2V_OK;
     });
-    t_dev = r->dev;
-    return rc;
 }
-// Host columns: with several devices column j goes to device j mod G (each device has its own PCIe link and SRS
-// replica, no collective); the commitments come back in column order.
+// Host columns: with several devices column j goes to device j mod G; the commitments come back in column order.
 int h2v_commit_batch(h2v_srs_t h, int basis, const uint64_t *const *polys, size_t n_polys, size_t len, uint64_t *out_affine) {
     if (!h) return failf(H2V_EINVAL, "commit: NULL srs");
+    H2V_TRY(use_device(h->rep[0]->dev));
     const size_t G = h->rep.size();
-    if (G == 1 || n_polys < 2 * G || !polys || !out_affine) {
-        t_dev = h->rep[0]->dev;
-        return rep_commit_batch(h->rep[0], basis, polys, n_polys, len, out_affine);
-    }
-    std::vector<std::vector<const uint64_t *>> sub(G);
-    std::vector<std::vector<uint64_t>> outs(G);
-    for (size_t j = 0; j < n_polys; ++j) sub[j % G].push_back(polys[j]);
-    for (size_t d = 0; d < G; ++d) outs[d].resize(sub[d].size() * 8);
-    int rc = fan_out(G, [&](size_t d) {
-        t_dev = h->rep[d]->dev;
-        return rep_commit_batch(h->rep[d], basis, sub[d].data(), sub[d].size(), len, outs[d].data());
+    if (G == 1 || n_polys < 2 * G || !polys || !out_affine) return rep_commit_batch(h->rep[0], basis, polys, n_polys, len, out_affine);
+    std::vector<uint64_t *> outs(n_polys);
+    for (size_t j = 0; j < n_polys; ++j) outs[j] = out_affine + 8 * j;
+    return deal_columns(h->rep, polys, outs.data(), n_polys, [&](SrsRep *rep, const uint64_t *const *in, uint64_t *const *out, size_t cnt) {
+        std::vector<uint64_t> res(8 * cnt);
+        const int rc = rep_commit_batch(rep, basis, in, cnt, len, res.data());
+        for (size_t i = 0; i < cnt && !rc; ++i) memcpy(out[i], &res[8 * i], 64);
+        return rc;
     });
-    t_dev = -1;
-    if (rc) return rc;
-    for (size_t j = 0; j < n_polys; ++j) memcpy(out_affine + 8 * j, outs[j % G].data() + 8 * (j / G), 64);
-    return H2V_OK;
 }
 int h2v_commit(h2v_srs_t h, int basis, const uint64_t *poly, size_t len, uint64_t out_affine[8]) {
     if (!h) return failf(H2V_EINVAL, "commit: NULL srs");
-    t_dev = h->rep[0]->dev;
     return rep_commit_batch(h->rep[0], basis, &poly, 1, len, out_affine);
 }
 
@@ -2743,109 +2760,45 @@ int h2v_domain_new(uint32_t j, uint32_t k, h2v_domain_t *out) {
     if (!out) return failf(H2V_EINVAL, "domain_new: out is NULL");
     *out = nullptr;
     h2v_domain *h = new h2v_domain();
-    for (size_t i = 0; i < g_devs.size(); ++i) {
-        t_dev = g_devs[i];
-        DomRep *r = nullptr;
-        int rc = rep_domain_new(j, k, &r);
-        if (rc) {
-            h2v_domain_free(h);
-            t_dev = -1;
-            return rc;
-        }
-        h->rep.push_back(r);
-    }
-    t_dev = -1;
-    *out = h;
-    return H2V_OK;
+    const int rc = make_replicas(h->rep, rep_domain_free, [&](int dev, DomRep **r) { return rep_domain_new(dev, j, k, r); });
+    if (rc) delete h;
+    else *out = h;
+    return rc;
 }
 void h2v_domain_free(h2v_domain_t h) {
     if (!h) return;
-    for (DomRep *r : h->rep) {
-        t_dev = r->dev;
-        rep_domain_free(r);
-    }
-    t_dev = -1;
+    free_replicas(h->rep, rep_domain_free);
     delete h;
 }
 int h2v_domain_transform_dev(h2v_domain_t h, int op, const void *d_in, size_t in_stride, void *d_out, size_t out_stride, size_t n_cols) {
     DomRep *r = dom_rep(h, d_in);
     if (!r) return H2V_EINVAL;
+    H2V_TRY(use_device(r->dev));
     const size_t G = h->rep.size();
-    static const bool no_split = getenv("H2V_NO_PEER_SPLIT") != nullptr;
     // worth splitting when every device gets about 2^21 points of transform: 8 columns of a 2^18-point extended domain
     // (k = 16), a single column from 2^21 points up (k = 20: one coset transform is 0.8 ms, its NVLink round trip 0.2 ms)
-    const size_t pts = op >= 0 && op <= H2V_OP_DIVIDE_BY_VANISHING ? ((size_t)1 << (op >= H2V_OP_COEFF_TO_EXTENDED ? r->ek : r->k)) : 1;
-    const size_t min_per_dev = std::min<size_t>(8, std::max<size_t>(1, ((size_t)1 << 21) / pts));
-    if (G == 1 || no_split || n_cols < min_per_dev * G || op < 0 || op > H2V_OP_DIVIDE_BY_VANISHING || !d_out || device_of(d_out) != r->dev)
-        return rep_domain_transform_dev(r, op, d_in, in_stride, d_out, out_stride, n_cols);
-    // Several devices, one resident batch: contiguous blocks of columns, as h2v_commit_batch_dev splits them.  A device
-    // other than the owner pulls its input columns over NVLink, transforms them with its own twiddle tables and pushes
-    // the output columns back (32 B per input element in, 32 B per output element out: worth it for the extended
-    // transforms, whose 4n-point butterflies dominate).
-    const size_t nin = op_in_len(r, op), nout = op_out_len(r, op);
+    const bool known_op = op >= 0 && op <= H2V_OP_DIVIDE_BY_VANISHING;
     const size_t work_len = (size_t)1 << (op >= H2V_OP_COEFF_TO_EXTENDED ? r->ek : r->k);
-    if (in_stride < nin || out_stride < work_len) return rep_domain_transform_dev(r, op, d_in, in_stride, d_out, out_stride, n_cols);
-    const size_t per = (n_cols + G - 1) / G;
-    const fe *src = (const fe *)d_in;
-    fe *dst = (fe *)d_out;
-    int rc = fan_out(G, [&](size_t d) -> int {
-        DomRep *rep = h->rep[d];
-        const size_t c0 = std::min(n_cols, d * per), cnt = std::min(n_cols, c0 + per) - c0;
-        if (!cnt) return H2V_OK;
-        t_dev = rep->dev;
-        if (rep == r) return rep_domain_transform_dev(rep, op, src + c0 * in_stride, in_stride, dst + c0 * out_stride, out_stride, cnt);
-        int rc2 = use_device();
-        if (rc2) return rc2;
-        std::lock_guard<std::mutex> plk(rep->peer_mu);
-        cudaError_t e = cudaSuccess;
-        {
-            std::lock_guard<std::mutex> lk(rep->mu);
-            if ((rc2 = rep->peer_in.ensure(cnt * nin * sizeof(fe)))) return rc2;
-            if ((rc2 = rep->peer_out.ensure(cnt * work_len * sizeof(fe)))) return rc2;
-            if (in_stride == nin) {
-                e = cudaMemcpyPeerAsync(rep->peer_in.p, rep->dev, src + c0 * in_stride, r->dev, cnt * nin * sizeof(fe), rep->stream);
-            } else {
-                for (size_t c = 0; c < cnt && e == cudaSuccess; ++c)
-                    e = cudaMemcpyPeerAsync(rep->peer_in.as<fe>() + c * nin, rep->dev, src + (c0 + c) * in_stride, r->dev, nin * sizeof(fe),
-                                            rep->stream);
-            }
-            if (e == cudaSuccess) e = cudaStreamSynchronize(rep->stream);
-            if (e != cudaSuccess) return failf(H2V_ECUDA, "transform: peer copy %d -> %d: %s", r->dev, rep->dev, cudaGetErrorString(e));
-        }
-        if ((rc2 = rep_domain_transform_dev(rep, op, rep->peer_in.p, nin, rep->peer_out.p, work_len, cnt))) return rc2;
-        if (out_stride == work_len && nout == work_len) {
-            e = cudaMemcpyPeerAsync(dst + c0 * out_stride, r->dev, rep->peer_out.p, rep->dev, cnt * nout * sizeof(fe), rep->stream);
-        } else {
-            for (size_t c = 0; c < cnt && e == cudaSuccess; ++c)
-                e = cudaMemcpyPeerAsync(dst + (c0 + c) * out_stride, r->dev, rep->peer_out.as<fe>() + c * work_len, rep->dev,
-                                        nout * sizeof(fe), rep->stream);
-        }
-        if (e == cudaSuccess) e = cudaStreamSynchronize(rep->stream);
-        if (e != cudaSuccess) return failf(H2V_ECUDA, "transform: peer copy of the results: %s", cudaGetErrorString(e));
-        return H2V_OK;
-    });
-    t_dev = r->dev;
-    return rc;
+    const size_t min_per_dev = std::min<size_t>(8, std::max<size_t>(1, ((size_t)1 << 21) / (known_op ? work_len : 1)));
+    const size_t nin = op_in_len(r, op), nout = op_out_len(r, op);
+    if (G == 1 || !peer_split_allowed() || n_cols < min_per_dev * G || !known_op || !d_out || device_of(d_out) != r->dev || in_stride < nin ||
+        out_stride < work_len)
+        return rep_domain_transform_dev(r, op, d_in, in_stride, d_out, out_stride, n_cols);
+    // 32 B per input element in, 32 B per output element out: worth it for the extended transforms, whose 4n-point
+    // butterflies dominate
+    return split_blocks(h->rep, r, "transform", d_in, nin * sizeof(fe), in_stride * sizeof(fe), d_out, nout * sizeof(fe), out_stride * sizeof(fe),
+                        n_cols, [&](DomRep *rep, const void *in, size_t in_st, void *out, size_t out_st, size_t cnt) {
+                            return rep_domain_transform_dev(rep, op, in, in_st / sizeof(fe), out, out_st / sizeof(fe), cnt);
+                        });
 }
 int h2v_domain_transform_batch(h2v_domain_t h, int op, const uint64_t *const *in, uint64_t *const *out, size_t n_cols) {
     if (!h) return failf(H2V_EINVAL, "transform: NULL domain");
+    H2V_TRY(use_device(h->rep[0]->dev));
     const size_t G = h->rep.size();
-    if (G == 1 || n_cols < 2 * G || !in || !out) {
-        t_dev = h->rep[0]->dev;
-        return rep_domain_transform_batch(h->rep[0], op, in, out, n_cols);
-    }
-    std::vector<std::vector<const uint64_t *>> si(G);
-    std::vector<std::vector<uint64_t *>> so(G);
-    for (size_t j = 0; j < n_cols; ++j) {
-        si[j % G].push_back(in[j]);
-        so[j % G].push_back(out[j]);
-    }
-    int rc = fan_out(G, [&](size_t d) {
-        t_dev = h->rep[d]->dev;
-        return rep_domain_transform_batch(h->rep[d], op, si[d].data(), so[d].data(), si[d].size());
+    if (G == 1 || n_cols < 2 * G || !in || !out) return rep_domain_transform_batch(h->rep[0], op, in, out, n_cols);
+    return deal_columns(h->rep, in, out, n_cols, [&](DomRep *rep, const uint64_t *const *i, uint64_t *const *o, size_t cnt) {
+        return rep_domain_transform_batch(rep, op, i, o, cnt);
     });
-    t_dev = -1;
-    return rc;
 }
 
 }  // extern "C"

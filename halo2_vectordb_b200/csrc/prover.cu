@@ -325,7 +325,6 @@ int commit_dev(h2v_pk *pk, int basis, const fe *cols, size_t n_cols, std::vector
     if (!n_cols) return H2V_OK;
     H2V_TRY(pk->commits.ensure(n_cols * sizeof(affine)));
     H2V_TRY(h2v_commit_batch_dev(pk->srs, basis, cols, pk->n, n_cols, pk->n, pk->commits.p));
-    H2V_CU(cudaSetDevice(pk->dev));
     H2V_CU(cudaMemcpy(out.data(), pk->commits.p, n_cols * sizeof(affine), cudaMemcpyDeviceToHost));
     return H2V_OK;
 }
@@ -432,7 +431,6 @@ int h2v_pk_load(h2v_srs_t srs, const h2v_circuit_t *cs, const uint64_t *const *f
     h2v_domain_constant(pk->dom, 0, tmp); pk->omega = frh::load(tmp);
     h2v_domain_constant(pk->dom, 1, tmp); pk->omega_inv = frh::load(tmp);
     pk->delta = frh::pow_u64(frh::from_u64(7), (uint64_t)1 << 28);      // Fr::DELTA = MULTIPLICATIVE_GENERATOR^(2^S)
-    cudaSetDevice(pk->dev);      // h2v_domain_new built one replica per device and left this thread on the last one
     cudaError_t e = cudaStreamCreateWithFlags(&pk->st, cudaStreamNonBlocking);
     if (e != cudaSuccess) { h2v_pk_free(pk); return failf(H2V_ECUDA, "pk_load: %s", cudaGetErrorString(e)); }
 
@@ -725,7 +723,6 @@ int instances_and_advice(Group &g) {
         g.pts.resize(BA);
         H2V_TRY(h2v_commit_batch_resident(pk->srs, H2V_BASIS_LAGRANGE, adv.data(), BA, n, (const uint64_t *)tails.data(), g.u, bf + 1, pk->adv_L.p,
                                           n, (uint64_t *)g.pts.data()));
-        H2V_CU(cudaSetDevice(pk->dev));
     }
     return write_commitments(g, g.pts, A, true);      // hashed while the lookup permutations run
 }
@@ -760,7 +757,6 @@ int permuted_lookups(Group &g) {
             }
         }
         if (rc) return rc;
-        H2V_CU(cudaSetDevice(pk->dev));
         std::vector<Fr64> ta(BL * (bf + 1)), ts(BL * (bf + 1));
         for (size_t p = 0; p < B; ++p) {
             ChaCha20Rng &rng = g.P[p]->rng;

@@ -45,6 +45,11 @@ typedef struct h2v_domain *h2v_domain_t; /* EvaluationDomain: constants + device
  * entry points (h2v_commit_batch, h2v_domain_transform_batch) send column j to device j mod n_dev -- each device pulls
  * its columns over its own PCIe link, no collective -- and return results in column order; everything else runs on the
  * primary device.  Call once, before creating handles; NULL / 0 selects device 0 (the default without a call).
+ * An entry point that works on a device returns with the calling thread's current CUDA device set to the device the
+ * call was addressed to: the device that owns its buffers, or the primary device for host columns and for creating
+ * and freeing h2v_srs and h2v_domain handles.  This holds when the call split its work over several devices, and when
+ * it failed after its device work began; a call rejected for its arguments before that, or one that only computes on
+ * the host, leaves the current device as it was.
  * Mirrors nothing upstream: the reference is CPU-only and single-process (scaffold mod.rs:251-323). */
 int h2v_init(const int *devices, int n_dev);
 /* the device list in use; returns its length */

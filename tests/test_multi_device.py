@@ -69,6 +69,31 @@ def test_dev_entry_points_run_where_the_buffers_live(two_devices):
     dom.close()
 
 
+def test_calls_return_on_the_device_they_were_addressed_to(two_devices):
+    """an entry point leaves the calling thread's current device on the device its call was addressed to: the owner of
+    its buffers, also when a resident batch was split over both devices, and the primary device for host columns"""
+    import torch
+    h = two_devices
+    k, n, ncols = 9, 1 << 9, 21      # enough columns for both resident batches to be split
+    torch.cuda.init()
+    srs = h.ParamsKZG(k, None, O.gen_bases(n))
+    dom = h.EvaluationDomain(4, k)
+    cols = np.stack([O.fr_fill(n, 40 + i) for i in range(ncols)])
+    d_in = h.DeviceBuffer(cols.nbytes, device=1)
+    d_in.upload(cols)
+    d_pts = h.DeviceBuffer(ncols * 64, device=1)
+    d_c = h.DeviceBuffer(cols.nbytes, device=1)
+    srs.commit_batch_dev(d_in.ptr, n, ncols, n, d_pts.ptr)
+    assert torch.cuda.current_device() == 1
+    for host_call in (lambda: h.batch_invert(cols[0]), lambda: h.g1_sum(np.zeros((0, 8), dtype=np.uint64))):
+        dom.transform_dev(h.OP_LAGRANGE_TO_COEFF, d_in.ptr, n, d_c.ptr, n, ncols)
+        assert torch.cuda.current_device() == 1
+        host_call()
+        assert torch.cuda.current_device() == 0
+    srs.close()
+    dom.close()
+
+
 def test_init_rejects_bad_lists(h2v):
     with pytest.raises(ValueError):
         h2v.init([0, 0])
@@ -153,15 +178,16 @@ def test_proof_bytes_do_not_depend_on_the_device_count(h2v):
 
 
 @pytest.mark.parametrize("devices,k,cols_n", [pytest.param(1, 9, 19, id="1"), pytest.param(2, 9, 19, id="2"),
+                                              pytest.param(4, 9, 37, id="4"), pytest.param(8, 9, 70, id="8"),
                                               pytest.param(1, 16, 40, id="1-k16")])
 def test_commit_batch_resident(h2v, devices, k, cols_n):
     """h2v_commit_batch_resident: host columns are blinded, committed and left on the device (the advice phase of
-    create_proof); with two devices each uploads and commits a block and forwards it to the owner.  At k = 16 the 40
+    create_proof); with several devices each uploads and commits a block and forwards it to the owner.  At k = 16 the 40
     columns go up in two sub-batches of 32 and 8 (a full one holds 64 MiB of columns): the second crosses while the
     first is committed."""
     import torch
     if h2v.device_count() < devices:
-        pytest.skip("needs 2 GPUs")
+        pytest.skip(f"needs {devices} GPUs")
     h2v.init(list(range(devices)) if devices > 1 else 0)
     try:
         n, rows = 1 << k, 6
