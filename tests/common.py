@@ -29,3 +29,15 @@ def fr_arr(ints):
 
 def g1_arr(pts):
     return np.stack([O.g1_affine_from_ints(p) for p in pts]) if len(pts) else np.zeros((0, 8), dtype=np.uint64)
+
+
+def mem_available():
+    """MemAvailable of /proc/meminfo in bytes (0 when it cannot be read)"""
+    try:
+        with open("/proc/meminfo") as f:
+            for line in f:
+                if line.startswith("MemAvailable:"):
+                    return int(line.split()[1]) * 1024
+    except OSError:
+        pass
+    return 0

@@ -13,7 +13,7 @@ import sys
 import numpy as np
 import pytest
 
-from common import fr_arr
+from common import fr_arr, mem_available
 from oracle import oracle as O
 from oracle import pyref as P
 
@@ -25,17 +25,6 @@ GIB = 1 << 30
 
 def fe(x):
     return fr_arr([x])[0]
-
-
-def _mem_available():
-    try:
-        with open("/proc/meminfo") as f:
-            for line in f:
-                if line.startswith("MemAvailable:"):
-                    return int(line.split()[1]) * 1024
-    except OSError:
-        pass
-    return 0
 
 
 # ----------------------------------------------------------------------------- 1. best_fft at every large pass shape
@@ -58,7 +47,7 @@ def test_best_fft_largest_roundtrip(h2v, log_n):
     inverse (the omega^-1 twiddle table and the 1/n post-scale of lagrange_to_coeff) gives back the whole input, and
     sampled outputs equal the polynomial evaluated at omega^j."""
     n = 1 << log_n
-    if _mem_available() < 5 * n * 32:
+    if mem_available() < 5 * n * 32:
         pytest.skip(f"needs about {5 * n * 32 / GIB:.0f} GiB of free host memory")
     a = O.fr_fill(n, 6000 + log_n, mode=log_n % 2)
     wi = P.omega_for(log_n)
